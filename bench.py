@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """SAC learner hot-path benchmark (BASELINE.json metric: SAC updates/sec, Humanoid-v5 shape, B=256; PER samples/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (N=1) = BASELINE.json configs[1]: Humanoid-v5 SAC update (obs 348, act 17, 3x512 networks_model2 MLPs,
 batch 256) over a 1M-transition prioritized replay ring resident in HBM.  One STEP = what the trainer loop does
@@ -17,6 +17,8 @@ full update_parameters (target, twin-critic, actor, temperature, Adam, Polyak) -
           `sharded` object: C5 population (128 agents per GPU = 1024 on 8, batched fused updates, no inter-GPU traffic) and
           C4 large-batch data parallel (global batch 8192 and 65536 split over the N ranks, gradient all-reduce over NVLink).
   --impl reference : the CPU restatement of the reference (numpy/OpenBLAS update + C PER sampler) on the host cores.
+  --dump-outputs DIR : after the K timed steps of `value`, the arrays their last step computed (losses, alpha, network
+          parameters, priority table) as DIR/<name>.npy; the seeded inputs make two builds comparable output for output.
 """
 import argparse
 import ctypes
@@ -215,7 +217,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(3, min(args.steps, 1000))      # ~30 ms per step: 1000 steps stay within the driver's few minutes
+    steps = args.steps
     warmup = max(3, min(args.warmup, 50))
     best, runs = cpu_thread_sweep(steps, warmup)
     ups, ms = best["updates_per_s"], best["ms_per_step"]
@@ -247,6 +249,24 @@ def build_agent(hw, device, launch, math, seed):
         agent.replay_buffer.push_many(s, a, r, s2, d)
     agent.replay_buffer.set_priorities(synth_priorities(CAPACITY, seed))
     return agent
+
+
+def dump_outputs(N, agent, out_dir):
+    """What the timed steps computed, as float32 .npy files, so that two builds can be compared output for output: the three
+    losses of the last update, alpha and log_alpha, every parameter of the five networks (3.6 M floats) and the 1M-entry priority
+    table the last write-back updated; 18 MB in all.  Every input is seeded: the same arguments give the same inputs in every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    losses = np.zeros(3, np.float32)
+    N.check(N.lib().sacb_get_losses(agent._h, 0, N.ptr(losses)))
+    sc = agent._scalars()
+    out = {"losses": losses, "alpha": np.array([sc.alpha], np.float32), "log_alpha": np.array([sc.log_alpha], np.float32),
+           "priorities": agent.replay_buffer.priorities}
+    with agent._library_stream():
+        for net in ("policy", "q1", "q2", "q1_target", "q2_target"):
+            for k, v in getattr(agent, net).state_dict().items():
+                out[f"{net}.{k}"] = v.detach().cpu().numpy().astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def eager_cuda_baseline(device, steps=100):
@@ -456,6 +476,8 @@ def run_ours(args):
             time.sleep(0.15)
     barrier()
     launches = agent.stats()["kernel_launches"] - st0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(N, agent, args.dump_outputs)
     if world > 1:
         print(f"[rank {rank}] device {local}: {ms.value / args.steps:.4f} ms/step", file=sys.stderr)
     t = torch.tensor([ms.value], device=red_dev)
@@ -591,7 +613,12 @@ def main():
     ap.add_argument("--no-sharded", action="store_true", help="skip the population / data-parallel block")
     ap.add_argument("--agents-per-gpu", type=int, default=128)
     ap.add_argument("--no-pipeline", action="store_true", help="value: run sample / update / write-back sequentially on one stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -132,61 +132,50 @@ def test_range_sample_is_random_sample(hw):
         _range_sample(10, 11)
 
 
+def _layout(x):
+    """Structure of a checkpoint value as the reference's load code meets it: container types, keys, tensor shapes and dtypes."""
+    import collections
+    import numpy as np
+    import torch
+    if torch.is_tensor(x):
+        return ("tensor", tuple(x.shape), x.dtype)
+    if isinstance(x, np.ndarray):
+        return ("ndarray", x.shape)
+    if isinstance(x, dict):
+        return (type(x).__name__, {k: _layout(v) for k, v in x.items()})
+    if isinstance(x, (list, tuple, collections.deque)):
+        return (type(x).__name__, [_layout(v) for v in x])
+    return type(x).__name__
+
+
 def test_reference_loads_product_checkpoints():
     """Interop in the other direction: files written by the PRODUCT on a B200 (tests/test_gpu_networks_ckpt.py::
-    test_write_product_checkpoints_for_the_reference, committed under tests/golden/) go through the reference's own
-    SAC.load / SAC.load_checkpoint (sac_imp.py:164-173, :203-233); the reference then takes the same next step the product took.
-    Needs the live reference: skipped where /root/reference does not exist (the GPU box)."""
-    import functools
-    import sys
-    gold = os.path.join(ROOT, "tests", "golden")
-    files = [os.path.join(gold, f) for f in ("product_save.pt", "product_checkpoint.pt", "product_expected.npz")]
-    if not os.path.isdir("/root/reference") or not all(os.path.exists(f) for f in files):
-        pytest.skip("needs /root/reference and the product-written fixtures")
+    test_write_product_checkpoints_for_the_reference, committed under tests/golden/) can be resumed by the reference's
+    SAC.load / SAC.load_checkpoint (sac_imp.py:164-173, :203-233) and lead to the same next step the product took.
+    (1) Every key, container, tensor shape and dtype equals those of the save() / save_checkpoint() pair the reference itself
+    wrote after the same two updates (tests/golden/ckpt_ref_*.pt).  (2) The reference's resume and update, as restated by the
+    oracle (pinned to the reference resuming its own file: test_oracle_nets_ckpt_golden.py), take the product's third step.
+    The losses are the interop evidence; the oracle then steps the temperature like the product, whereas the reference's own
+    load_checkpoint (sac_imp.py:222-226) rebinds `log_alpha` away from its optimizer and keeps alpha = exp(loaded log_alpha)."""
     import numpy as np
     import torch
     from oracle import sac_oracle_np as O
     from tests.golden import cases
-    sys.dont_write_bytecode = True
-    saved = {k: sys.modules.get(k) for k in ("sac_imp", "networks_model1", "networks_model2", "replay_buffer")}
-    sys.path.insert(0, "/root/reference")
-    try:
-        for k in saved:
-            sys.modules.pop(k, None)
-        import sac_imp as ref_sac
-        case = cases.UPDATE_CASES["tiny_m1"]
-        real_load = torch.load
-        # the files hold CUDA tensors and a pickled list; the reference calls torch.load(path) bare (sac_imp.py:166, :205)
-        torch.load = functools.partial(real_load, map_location="cpu", weights_only=False)
-        try:
-            agent = ref_sac.SAC(case["obs"], case["act"], hidden_dim=case["hidden"], device="cpu")
-            agent.load(files[0])
-            ep, steps = agent.load_checkpoint(files[1])
-        finally:
-            torch.load = real_load
-        assert (ep, steps) == (3, 45) and len(agent.replay_buffer.buffer) == 20
-        assert agent.q1_optimizer.state_dict()["state"][0]["step"] == 2
-        b = O.make_batch(case["obs"], case["act"], case["batch"], seed=case["seed"] * 100 + 2)
-        agent.replay_buffer.sample = lambda n: (b["s"], b["a"], b["r"], b["s2"], b["d"])
-        queue = [b["eps_next"], b["eps_cur"]]
-        orig = torch.distributions.normal._standard_normal
-        torch.distributions.normal._standard_normal = lambda shape, dtype, device: torch.from_numpy(queue.pop(0)).to(dtype)
-        try:
-            info = agent.update_parameters(case["batch"])
-        finally:
-            torch.distributions.normal._standard_normal = orig
-        exp = np.load(files[2])
-        np.testing.assert_allclose([info["q1_loss"], info["q2_loss"], info["policy_loss"]], exp["next_losses"], rtol=3e-4)
-        # Reference quirk (sac_imp.py:222-226): load_checkpoint rebinds `self.log_alpha` to the loaded tensor while `alpha_optimizer`
-        # keeps stepping the tensor created in __init__, so after a resume the reference's temperature no longer trains: its alpha
-        # stays exp(loaded log_alpha).  The product resumes the temperature as well (exp["next_alpha"]); the losses above -- computed
-        # with the loaded alpha by both -- are the interop evidence.
-        ck = real_load(files[1], map_location="cpu", weights_only=False)
-        np.testing.assert_allclose(float(agent.alpha), float(np.exp(ck["log_alpha"].detach().numpy()[0])), rtol=1e-6)
-        assert abs(float(exp["next_alpha"]) - float(agent.alpha)) < 1e-3
-    finally:
-        sys.path.remove("/root/reference")
-        for k, v in saved.items():
-            sys.modules.pop(k, None)
-            if v is not None:
-                sys.modules[k] = v
+    from tests.util import state_from_checkpoint
+    gold = os.path.join(ROOT, "tests", "golden")
+    load = lambda f: torch.load(os.path.join(gold, f), map_location="cpu", weights_only=False)
+    for product, reference in (("product_save.pt", "ckpt_ref_save.pt"), ("product_checkpoint.pt", "ckpt_ref_checkpoint.pt")):
+        assert _layout(load(product)) == _layout(load(reference)), product
+    ck = load("product_checkpoint.pt")
+    for key, ref_value in load("ckpt_ref_checkpoint.pt")["q1_optimizer_state_dict"]["param_groups"][0].items():
+        assert ck["q1_optimizer_state_dict"]["param_groups"][0][key] == ref_value, key
+    assert (ck["episode"], ck["total_steps"]) == (3, 45) and len(ck["replay_buffer"]) == 20
+    assert float(ck["q1_optimizer_state_dict"]["state"][0]["step"]) == 2
+    case = cases.UPDATE_CASES["tiny_m1"]
+    st, _ = state_from_checkpoint(os.path.join(gold, "product_checkpoint.pt"), case)
+    np.testing.assert_allclose(st.alpha, float(np.exp(ck["log_alpha"].detach().numpy()[0])), rtol=1e-6)
+    b = O.make_batch(case["obs"], case["act"], case["batch"], seed=case["seed"] * 100 + 2)
+    info = O.update_parameters(st, b)
+    exp = np.load(os.path.join(gold, "product_expected.npz"))
+    np.testing.assert_allclose([info["q1_loss"], info["q2_loss"], info["policy_loss"]], exp["next_losses"], rtol=3e-4)
+    np.testing.assert_allclose(st.alpha, exp["next_alpha"], rtol=1e-5)

@@ -14,7 +14,6 @@ from tests.util import batch_of, make_agent, net_params, state_from_checkpoint
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SHIPPED = {"bipedal": dict(obs=24, act=4, hidden=256, n_hidden=2, batch=256, seed=31),
            "humanoid376": dict(obs=376, act=17, hidden=256, n_hidden=2, batch=256, seed=32)}
 
@@ -140,9 +139,10 @@ def test_resume_checkpoint_written_by_the_reference(hw):
     assert abs(float(other.alpha) - float(sv["alpha"])) < 1e-9
 
 
-def test_write_product_checkpoints_for_the_reference(hw):
-    """Writes save() / save_checkpoint() files from the product after two seeded updates; the CPU-side test
-    (tests/test_cabi.py::test_reference_loads_product_checkpoints) feeds the committed copies to the reference's own load code."""
+def test_write_product_checkpoints_for_the_reference(hw, tmp_path):
+    """Writes save() / save_checkpoint() files from the product after two seeded updates, then takes the next step.  The files
+    and that step are what tests/golden/product_*.pt and product_expected.npz hold (written by this test on a B200), which the
+    CPU-side test (tests/test_cabi.py::test_reference_loads_product_checkpoints) checks against the reference's load code."""
     case = cases.UPDATE_CASES["tiny_m1"]
     agent, st = make_agent(hw, case, math="fp32", capacity=128)
     for step in range(2):
@@ -150,8 +150,7 @@ def test_write_product_checkpoints_for_the_reference(hw):
         agent.update_from_batch(b, eps=(b["eps_next"], b["eps_cur"]))
     for t in cases.ckpt_transitions(case):
         agent.replay_buffer.push(*t)
-    out_dir = os.path.join(ROOT, "gpurun_out")
-    os.makedirs(out_dir, exist_ok=True)
+    out_dir = str(tmp_path)
     agent.save(os.path.join(out_dir, "product_save.pt"))
     agent.save_checkpoint(os.path.join(out_dir, "product_checkpoint.pt"), episode=3, total_steps=45)
     b = batch_of(case, 2)
@@ -160,6 +159,9 @@ def test_write_product_checkpoints_for_the_reference(hw):
              next_alpha=np.array(float(agent.alpha)))
     ck = torch.load(os.path.join(out_dir, "product_checkpoint.pt"), map_location="cpu", weights_only=False)
     assert len(ck["replay_buffer"]) == 20 and float(ck["policy_optimizer_state_dict"]["state"][0]["step"]) == 2.0
+    committed = np.load(os.path.join(GOLD, "product_expected.npz"))
+    np.testing.assert_allclose([l["q1_loss"], l["q2_loss"], l["policy_loss"]], committed["next_losses"], rtol=3e-4)
+    np.testing.assert_allclose(float(agent.alpha), committed["next_alpha"], rtol=1e-5)
 
 
 def test_resident_shadows_equal_rederived_shadows(hw):
