@@ -185,12 +185,23 @@ constexpr int kVariantEverything = 0, kVariantEverythingLn = 20;      // the bui
 constexpr uint32_t kLightTypes = tb(T_OUT_ADAM) | tb(T_BIAS_ADAM) | tb(T_SAMPLE_BWD);
 constexpr int variant_min_blocks(uint32_t types, uint32_t epis) { return (types != 0 && (types & ~kLightTypes) == 0 && epis == 0) ? 2 : 1; }
 
+// builds that carry the chained form of a launch (Stage::chain_map): tensor-core GEMMs with the plain epilogues, T_SHADOW riders.  The
+// others keep ONE call site of their task bodies (a second one makes the compiler outline them: stack frame, 4 us more per Adam stage)
+constexpr bool variant_chains(int math, uint32_t types, uint32_t epis) {
+    return math != SACB_MATH_FP32 && (types & tb(T_GEMM)) != 0 && (types & ~(tb(T_GEMM) | tb(T_SHADOW))) == 0 && (epis & ~kPlainEpis) == 0;
+}
 constexpr int kMaxStageTasks = 28;
+constexpr int kMaxChainClusters = 32;
 struct Stage {
     int32_t task_begin, task_end;
     int32_t n_tiles;          // per agent
-    int32_t ksplit;           // staged tensor-core launches: CTAs per output tile (thread-block cluster along K), 1 / 2 / 4
     int32_t tile_begin[kMaxStageTasks];   // first tile of each task of the stage (copy of Task::tile_begin: one load finds the task)
+    // Chained launch (program.cu: find_chains): consecutive row-local GEMM stages in ONE launch of thread-block clusters, cluster c
+    // owns one row block in every stage of the chain, CTA rank r its column tile r.  The chain's first stage holds the number of
+    // stages and of row clusters (further clusters of the launch walk the T_SHADOW riders of the chain's stages); every stage of the
+    // chain holds, per row cluster, (stage tile of the row block's first column tile) | (column tiles << 16), or -1: no tile.
+    int32_t chain_len, chain_clusters;
+    int32_t chain_map[kMaxChainClusters];
 };
 
 struct Program {

@@ -345,7 +345,6 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_selftest_kernel(const Task *
     const Task &t = *tp;
     tc::TcState st;
     st.g = 0; st.accum_uses = 0; st.tmem_base = 0; st.full_bar = s_bars; st.empty_bar = s_bars + kTStages; st.accum_bar = s_bars + 2 * kTStages; st.trace = nullptr;
-    st.krank = 0; st.ksplit = 1; st.reduce_uses = 0; st.reduce_bar = nullptr;
     constexpr bool kTc = kMath != SACB_MATH_FP32;
     st.tiles = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     if (kTc) {
@@ -428,7 +427,7 @@ extern "C" int sacb_selftest_gemm_stream(int device, int M, int N, int K, int a_
     Program P; memset(&P, 0, sizeof(P));
     P.tasks = d_tasks; P.n_agents = 1; P.bases = bases; P.scalars = null_ref(); P.error_flag = flag;
     Stage sg; memset(&sg, 0, sizeof(sg));
-    sg.task_begin = 1; sg.task_end = 2; sg.n_tiles = tk[1].n_tiles; sg.ksplit = 1;
+    sg.task_begin = 1; sg.task_end = 2; sg.n_tiles = tk[1].n_tiles;
     SACB_CUDA(cudaFuncSetAttribute(stream_selftest_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, stream::kSmemBytes));
     stream_selftest_kernel<<<std::min(tk[1].n_tiles, ctas), stream::kThreads, stream::kSmemBytes>>>(P, sg);
     SACB_CUDA(cudaDeviceSynchronize());

@@ -309,55 +309,15 @@ struct TcState {
     uint64_t *accum_bar;   //             tcgen05.commit -> everyone: the accumulator tile is complete
     unsigned long long *trace;   // optional per-CTA timestamps (profiling aid)
     const CUtensorMap *tmA, *tmB; // descriptors of the current task in GLOBAL memory (the task's other fields are read from a smem copy)
-    // split-K over a thread-block cluster: the ksplit CTAs of a cluster own consecutive K ranges of ONE output tile.  Every CTA
-    // PUSHES the rows of its partial accumulator to the CTA that finishes them (st.shared::cluster into that CTA's slot
-    // [source rank]), signals the owner's `reduce_bar` (mbarrier, release/acquire at cluster scope) and CTA r then sums the
-    // slots for rows [r, r+1) * 128 / ksplit and runs the epilogue on them.  The slots occupy operand stage 3, the main loop
-    // of a clustered launch uses stages 0-2 only (its K range is short), so a fast peer never overwrites live operands.
-    uint32_t krank, ksplit;
-    uint64_t *reduce_bar;
-    uint32_t reduce_uses;
-    // K blocks of the CTA's first tile whose B operand (a weight shadow no earlier stage of this step is still writing) was requested
-    // BEFORE the grid-dependency wait (tc_prefetch_b): their `full` barriers are armed with the whole stage's bytes already
+    // K blocks of the next tile whose B operand was requested ahead of its A operand (tc_prefetch_b): their `full` barriers are
+    // armed with the whole K block's bytes already
     uint32_t b_pre;
 };
-__device__ __forceinline__ int tc_stages(const TcState &st) { return st.ksplit > 1 ? kTStages - 1 : kTStages; }
 
 __device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
 __device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
 __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ uint32_t cluster_nctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r)); return r; }
-// address of the same shared-memory offset inside CTA `rank` of this cluster (distributed shared memory)
-__device__ __forceinline__ uint32_t dsmem_addr(const void *local_ptr, uint32_t rank) {
-    uint32_t remote;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_u32(local_ptr)), "r"(rank));
-    return remote;
-}
-__device__ __forceinline__ void st_dsmem_v4(uint32_t remote, float4 v) {
-    asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(remote), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_remote_release(uint32_t remote_bar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote_bar) : "memory");
-}
-// bounded wait with acquire semantics at cluster scope (the arrivals come from peer CTAs)
-__device__ __forceinline__ bool mbar_wait_cluster(uint64_t *bar, uint32_t parity, int *error_flag) {
-    const uint32_t addr = smem_u32(bar);
-    long long t0 = 0;
-#pragma unroll 1
-    for (uint32_t it = 0;; ++it) {
-        uint32_t done;
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done) : "r"(addr), "r"(parity) : "memory");
-        if (done) return true;
-        if (it == 0) t0 = clock64();
-        else if (clock64() - t0 > 2000000000ll) break;
-    }
-    if (error_flag) atomicExch(error_flag, 1);
-    return false;
-}
 
 // ---- main loop of one output tile: warp 0 = TMA producer, warp 1 = MMA issuer ----------------------------------
 // smem stage: A region 32 KB then B region 16 KB (a 64-row / 32-column task fills only the front of its region).
@@ -373,48 +333,49 @@ __device__ __forceinline__ void trace_stamp(unsigned long long *trace, int slot)
     trace[(size_t)blockIdx.x * kTraceSlots + slot] = ts;
 }
 
-// Staged launches: a stage's CTAs become resident and run their prologue while the previous stage still computes (programmatic
-// dependent launch).  The A operand of a GEMM (activations, gradients) is what the previous stage produces, but the B operand of a
-// forward / dX GEMM is a weight shadow that, for most stages, nothing has written since two stages ago or longer (Task::i[6], set by
-// the host builder): its first K blocks are requested here, before griddepcontrol.wait, so that after the release only the A
-// halves still have to cross the SM's L2 port -- the stage is bound by exactly that ingest.
-__device__ __forceinline__ void tc_prefetch_b(const Task &t, const Task *tg, int tile, int agent, TcState &st) {
+// The B operand of a forward / dX GEMM is a weight shadow that nothing the tile waits for writes, while its A operand (activations,
+// gradients) is what the tile waits for: the first K blocks of B are requested here, from the current ring position, so that after
+// the wait only the A halves still have to cross the SM's L2 port -- the tile is bound by exactly that ingest.  Callers: a staged
+// launch before griddepcontrol.wait (Task::i[6], set by the host builder), and a chained launch before the cluster barrier that
+// ends the previous layer (the previous tile's epilogue is done with the ring by then).
+__device__ __forceinline__ void tc_prefetch_b(const Task &t, const Task *tg, int tile, int agent, TcState &st, int *error_flag) {
     st.b_pre = 0;
-    if (st.ksplit != 1 || st.g != 0 || (threadIdx.x >> 5) != 0) return;
+    if ((threadIdx.x >> 5) != 0) return;
     const int nkb = cdiv(t.K, kTK), n_pre = min(nkb, kTStages);
     if (elect_one()) {
         const int n0 = (tile % t.tiles_n) * t.bn, nb = t.B.r0 + n0;
         const uint32_t tiles = smem_u32(st.tiles);
         for (int kb = 0; kb < n_pre; kb++) {
-            mbar_arrive_expect_tx(&st.full_bar[kb], (uint32_t)(t.bm + t.bn) * (kTK * 2 * 2));      // A + B bytes: the A loads follow in tc_mainloop
-            const uint32_t sb = tiles + kb * kTcStageBytes + kTcABytes;
-            if (!t.B.mn_major) tma_load_4d(&tg->tmB, &st.full_bar[kb], sb, kb * kTK, nb, 0, agent);
-            else tma_load_4d(&tg->tmB, &st.full_bar[kb], sb, nb, kb * kTK, 0, agent);
+            const uint32_t g = st.g + kb, s = g % kTStages;
+            mbar_wait(&st.empty_bar[s], ((g / kTStages) & 1) ^ 1, error_flag);
+            mbar_arrive_expect_tx(&st.full_bar[s], (uint32_t)(t.bm + t.bn) * (kTK * 2 * 2));      // A + B bytes: the A loads follow in tc_mainloop
+            const uint32_t sb = tiles + s * kTcStageBytes + kTcABytes;
+            if (!t.B.mn_major) tma_load_4d(&tg->tmB, &st.full_bar[s], sb, kb * kTK, nb, 0, agent);
+            else tma_load_4d(&tg->tmB, &st.full_bar[s], sb, nb, kb * kTK, 0, agent);
         }
     }
     __syncwarp();
     st.b_pre = (uint32_t)n_pre;      // uniform over warp 0 (the only warp that reads it)
 }
 
-// returns the number of K-blocks this CTA accumulated (0: its partial tile is zero)
+// returns the number of K-blocks accumulated (0: the tile is zero)
 __device__ __forceinline__ int tc_mainloop(const Task &t, int m0, int n0, int agent, TcState &st, int *error_flag, bool traced) {
     const int warp = threadIdx.x >> 5;
     if (traced && threadIdx.x == 0) trace_stamp(st.trace, 12);
-    const int nkb_all = cdiv(t.K, kTK), per = cdiv(nkb_all, (int)st.ksplit);
-    const int kb0 = (int)st.krank * per, nkb = max(0, min(nkb_all, kb0 + per) - kb0);      // this CTA's K range
+    const int nkb = cdiv(t.K, kTK);
     const uint32_t tiles = smem_u32(st.tiles);
     const int a_mn = t.A.mn_major, b_mn = t.B.mn_major;
-    const uint32_t g0 = st.g, nst = (uint32_t)tc_stages(st);
+    const uint32_t g0 = st.g, nst = (uint32_t)kTStages;
     if (warp == 0) {
         if (elect_one()) {
             for (int kb = 0; kb < nkb; kb++) {
                 const uint32_t g = g0 + kb, s = g % nst;
-                const bool pre = (uint32_t)kb < st.b_pre;      // B requested and the barrier armed before the dependency wait (first tile, g0 == 0)
+                const bool pre = (uint32_t)kb < st.b_pre;      // B requested and the barrier armed ahead (tc_prefetch_b)
                 if (!pre) mbar_wait(&st.empty_bar[s], ((g / nst) & 1) ^ 1, error_flag);
                 if (traced && kb < 16) trace_stamp(st.trace, 16 + kb);
                 if (!pre) mbar_arrive_expect_tx(&st.full_bar[s], (uint32_t)(t.bm + t.bn) * (kTK * 2 * 2));      // both planes of both operand tiles
                 const uint32_t sa = tiles + s * kTcStageBytes, sb = sa + kTcABytes;
-                const int k0 = (kb0 + kb) * kTK, ma = t.A.r0 + m0, nb = t.B.r0 + n0;
+                const int k0 = kb * kTK, ma = t.A.r0 + m0, nb = t.B.r0 + n0;
                 if (!a_mn) {
                     tma_load_4d(st.tmA, &st.full_bar[s], sa, k0, ma, 0, agent);        // box rows = bm (descriptor)
                 } else {
@@ -509,8 +470,8 @@ __device__ __forceinline__ AdamOut adam_math(const EpiR &e, float g, float w, fl
 //   pass B: the columns no aligned group covers (a0 leading ones, <= 3 trailing ones), one element per thread
 //   both passes leave the new weights in the staging tile; pass C writes the bf16 pair shadows from there with the
 //   tile-aligned mapping (the shadow rows are padded to 16 B)
-__device__ __forceinline__ void adam_epilogue_tile(const EpiR &e, float *Cs, int m0, int n0, int row_lo, int row_hi) {
-    const int tid = threadIdx.x;     // only rows [row_lo, row_hi) of the tile belong to this CTA (split-K cluster)
+__device__ __forceinline__ void adam_epilogue_tile(const EpiR &e, float *Cs, int m0, int n0, int bm) {
+    const int tid = threadIdx.x;     // rows [bm, 128) of the staging tile belong to no tile of this CTA (64-row tiles)
     const int ncols = min(kTN, e.N - n0);      // valid columns of this tile (> 0)
 #pragma unroll 1
     for (int half = 0; half < kAdamRowGroups; half++) {   // ---- pass A, kAdamRows rows of a thread at a time (register budget)
@@ -525,7 +486,7 @@ __device__ __forceinline__ void adam_epilogue_tile(const EpiR &e, float *Cs, int
             mrow[ii] = m0 + 32 * i + r0;
             const int a0 = (4 - (int)(((int64_t)mrow[ii] * e.N + n0) & 3)) & 3;
             c[ii] = a0 + 4 * j16;
-            vec[ii] = mrow[ii] < e.M && c[ii] + 3 < ncols && 32 * i + r0 >= row_lo && 32 * i + r0 < row_hi;
+            vec[ii] = mrow[ii] < e.M && c[ii] + 3 < ncols && 32 * i + r0 < bm;
             w[ii] = mm[ii] = vv[ii] = wt[ii] = make_float4(0.f, 0.f, 0.f, 0.f);
             if (vec[ii] && e.apply) {
                 const int64_t o = (int64_t)mrow[ii] * e.N + n0 + c[ii];
@@ -555,7 +516,7 @@ __device__ __forceinline__ void adam_epilogue_tile(const EpiR &e, float *Cs, int
     }
     if (e.N % 4 != 0 || ncols < kTN) {   // ---- pass B (warp-uniform condition): thread (row = tid / 4, q = tid % 4)
         const int row = tid >> 2, q = tid & 3, m = m0 + row;
-        if (m < e.M && row >= row_lo && row < row_hi) {
+        if (m < e.M && row < bm) {
             const int a0 = (4 - (int)(((int64_t)m * e.N + n0) & 3)) & 3;
             const int nv = ncols > a0 ? (ncols - a0) >> 2 : 0, tail0 = a0 + 4 * nv;
             int col[2];
@@ -595,7 +556,7 @@ __device__ __forceinline__ void adam_epilogue_tile(const EpiR &e, float *Cs, int
 #pragma unroll
         for (int i = 0; i < 4; i++) {
             const int m = m0 + 32 * i + r0;
-            if (m >= e.M || 32 * i + r0 < row_lo || 32 * i + r0 >= row_hi) continue;
+            if (m >= e.M || 32 * i + r0 >= bm) continue;
             const float4 v4 = *reinterpret_cast<const float4 *>(Cs + (32 * i + r0) * kCsLd + c4);
             const float w1[4] = {v4.x, v4.y, v4.z, v4.w};
             const int n = n0 + c4;
@@ -720,15 +681,11 @@ __device__ __forceinline__ void sample_epilogue_tile(const SampleEpi &e, const f
 template <int EPI>
 __device__ __forceinline__ void tc_epilogue(const EpiR &epi, int m0, int n0, int bm, int bn, TcState &st, int nkb_mine, int *error_flag, bool traced, const SampleEpi *se = nullptr) {
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int ks = (int)st.ksplit, rows_per = kTM / ks;
-    // staging: ks == 1 -> one tile [kTM][kCsLd] over operand stage 0 (all MMAs have retired);
-    //          ks  > 1 -> ks slots [rows_per][kCsLd] over operand stage 3 (never used by a clustered main loop), slot = source rank
-    float *Cs = reinterpret_cast<float *>(st.tiles + (ks > 1 ? (kTStages - 1) * kTcStageBytes : 0));
+    float *Cs = reinterpret_cast<float *>(st.tiles);      // staging tile [kTM][kCsLd] over operand stage 0 (all MMAs have retired)
     // phase-2 mapping: bn / 4 threads cover a row (4 columns each); the 512 threads cover 32 (bn = 64) or 64 (bn = 32) rows per
     // pass, four passes.  The rows' auxiliary operands (bias / activation signs) are fetched now, under the main loop.
     const int ct = bn >> 2, rs = kThreads / ct;
     const int c4 = (tid % ct) * 4, r0 = tid / ct;
-    const int row_lo = ks > 1 ? (int)st.krank * rows_per : 0, row_hi = ks > 1 ? row_lo + rows_per : bm;
     int m[4];
     float aux[4][4];
     float pre_eps[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, pre_b0 = 0.f, pre_b1 = 0.f;
@@ -747,7 +704,7 @@ __device__ __forceinline__ void tc_epilogue(const EpiR &epi, int m0, int n0, int
 #pragma unroll
         for (int i = 0; i < 4; i++) {
             const int row = rs * i + r0;
-            m[i] = (row >= row_lo && row < row_hi) ? m0 + row : 0x7fffffff;      // rows of another cluster rank / beyond the tile are skipped like rows beyond M
+            m[i] = row < bm ? m0 + row : 0x7fffffff;      // rows beyond the tile are skipped like rows beyond M
         }
         epilogue_aux4<EPI, 4>(epi, m, n0 + c4, aux);
     }
@@ -763,49 +720,21 @@ __device__ __forceinline__ void tc_epilogue(const EpiR &epi, int m0, int n0, int
             if (traced && tid == 64) trace_stamp(st.trace, 6);
             tc_fence_after();
             if (cols_live) tmem_ld16(st.tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)colh, v);
-        } else {      // a cluster rank beyond the last K-block contributes a zero partial tile
+        } else {      // K = 0: a zero tile
 #pragma unroll
             for (int j = 0; j < 16; j++) v[j] = 0.f;
         }
-        if (ks == 1) {
-            if (cols_live && (!half_m || lane < 16)) {
-                float4 *dst = reinterpret_cast<float4 *>(Cs + row * kCsLd + colh);
+        if (cols_live && (!half_m || lane < 16)) {
+            float4 *dst = reinterpret_cast<float4 *>(Cs + row * kCsLd + colh);
 #pragma unroll
-                for (int j = 0; j < 4; j++) dst[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-            }
-        } else {      // push the row to the CTA that finishes it (warp-uniform owner), slot = my rank (clustered tiles are 128 x 64)
-            const uint32_t owner = (uint32_t)(row / rows_per);
-            const uint32_t dst = dsmem_addr(Cs + ((int)st.krank * rows_per + row % rows_per) * kCsLd + colh, owner);
-#pragma unroll
-            for (int j = 0; j < 4; j++) st_dsmem_v4(dst + 16 * j, make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]));
+            for (int j = 0; j < 4; j++) dst[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
         }
     }
     tc_fence_before();
     __syncthreads();     // staging complete; all TMEM reads retired (the next tile's first MMA may overwrite the accumulator)
     if (traced && tid == 64) trace_stamp(st.trace, 7);
-    if (ks > 1) {
-        if (tid < ks && tid != (int)st.krank) {      // one release-arrive per peer: my rows have landed in its slots
-            asm volatile("fence.acq_rel.cluster;" ::: "memory");
-            mbar_arrive_remote_release(dsmem_addr(st.reduce_bar, (uint32_t)tid));
-        }
-        mbar_wait_cluster(st.reduce_bar, st.reduce_uses & 1, error_flag);      // ks - 1 peers have pushed their rows to me
-        st.reduce_uses++;
-        if (traced && tid == 64) trace_stamp(st.trace, 48);
-        const int cc = (tid & 15) * 4;
-        for (int l = tid >> 4; l < rows_per; l += 32) {      // sum the slots in rank order into slot 0 (deterministic)
-            float4 sum = *reinterpret_cast<const float4 *>(Cs + l * kCsLd + cc);
-            for (int r = 1; r < ks; r++) {
-                const float4 p = *reinterpret_cast<const float4 *>(Cs + (r * rows_per + l) * kCsLd + cc);
-                sum.x += p.x; sum.y += p.y; sum.z += p.z; sum.w += p.w;
-            }
-            *reinterpret_cast<float4 *>(Cs + l * kCsLd + cc) = sum;
-        }
-        __syncthreads();
-        if (traced && tid == 64) trace_stamp(st.trace, 49);
-        Cs -= row_lo * kCsLd;      // from here on Cs[row] addresses tile row `row` for row_lo <= row < row_hi
-    }
     if (EPI == EPI_ADAM) {
-        adam_epilogue_tile(epi, Cs, m0, n0, row_lo, row_hi);
+        adam_epilogue_tile(epi, Cs, m0, n0, bm);
     } else if (EPI == EPI_SAMPLE) {
         sample_epilogue_tile(*se, Cs, m0, bm, pre_eps, pre_b0, pre_b1);
     } else {   // phase 2: the staged accumulators of the thread's rows meet the prefetched auxiliary operands
@@ -834,7 +763,6 @@ __device__ __forceinline__ void gemm_tile_tc(const Task &t, const Task *tg, int 
     const int tm = tile / t.tiles_n, tn = tile % t.tiles_n;
     const int m0 = tm * t.bm, n0 = tn * t.bn;
     const bool traced = st.trace && first_tile;      // the CTA's first tile of the stage
-    if (st.ksplit > 1 && !first_tile) { cluster_arrive(); cluster_wait(); }      // peers are done with the previous tile's slots
     const int nkb_mine = tc_mainloop(t, m0, n0, agent, st, error_flag, traced);
     auto stamp = [&](int slot) { if (traced && threadIdx.x == 0) trace_stamp(st.trace, slot); };
     stamp(2);

@@ -90,9 +90,14 @@ struct ProgramKey {
     }
 };
 
+// One kernel launch of a staged program: one stage, or the stages [s0, s1) of a chain (Stage::chain_map) as `grid` CTAs in thread-block
+// clusters of `cluster` CTAs, run by kernel variant `kind`
+struct StageLaunch { int s0, s1, cluster, grid, kind; };
+
 struct ProgramInst {
     std::vector<Task> tasks;
     std::vector<Stage> stages;
+    std::vector<StageLaunch> launches;   // staged mode: the launches of one step, in order
     std::vector<int> stage_has_gemm;
     std::vector<int> stage_stream;       // 1: the stage holds only GEMM tasks and runs on the stream kernel (throughput programs, stream.cuh)
     std::vector<int> stage_kind;         // kernel variant (SACB_KERNEL_VARIANTS) that runs the stage in staged mode
@@ -103,7 +108,7 @@ struct ProgramInst {
     // the same step as two graphs split in front of the actor-loss stage (the TD errors exist since the critic-loss stage):
     // sacb_per_step runs the priority write-back and the next prioritized sample on a second stream under the tail of the update
     cudaGraphExec_t graph_part[2] = {nullptr, nullptr};
-    int split = -1;
+    int split = -1;                      // index into `launches`
     bool parts_built = false;
     // the whole pipelined learner step (sacb_per_step) as ONE graph: update stages on the main stream, priority write-back and the next
     // sample forked onto the second stream in front of stage `split`, joined at the end (valid for one buffer length / batch size)
@@ -145,6 +150,7 @@ struct sacb_handle_s {
     uint32_t dp_epoch = 0;
     int dp_device_eps = 1;               // data-parallel mode: eps of the current step drawn on device (phase 1 follows phase 0)
     int coop_blocks_per_sm = 0;
+    std::map<std::pair<int, int>, int> max_active_clusters;   // (kernel variant, cluster size) -> cudaOccupancyMaxActiveClusters
     // ---- replay (replay.cu) ----
     float *ring = nullptr;
     int64_t ring_row = 0;                // floats per transition: [s | s2 | a | r | d] padded to 4
@@ -194,6 +200,7 @@ int make_pm_tensor_map(CUtensorMap *out, const void *base, int64_t cols, int64_t
                        int64_t agent_stride_bytes, int n_agents, int box_rows);
 const void *update_kernel_for(int math_mode, int variant);      // variant: index into SACB_KERNEL_VARIANTS (0 = everything)
 bool variant_has_gemm(int variant);
+bool variant_can_chain(int variant);      // the build carries the chained launch form
 int variant_blocks_per_sm(int variant);      // resident CTAs per SM a build is compiled for (light column-sum builds: 2)
 int pick_variant(uint32_t task_types, uint32_t epilogues, bool allow_light_colsum = true);
 // program.cu

@@ -192,12 +192,23 @@ __device__ __noinline__ void task_out_adam_outlined(const Task &t, int tile, con
 __device__ __noinline__ void task_bias_adam_outlined(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) { task_bias_adam(t, tile, P, agent, scalars, smem); }
 __device__ __noinline__ void task_finish_outlined(const Task &t, const Program &P, int agent, float *scalars, float *smem) { task_finish(t, P, agent, scalars, smem); }
 
+// Between two layers of a chained launch: the epilogue's global stores (generic proxy) become visible to the TMA reads (async proxy)
+// of the other CTAs of the cluster, which own the rest of the row block.  A chain of one-CTA clusters only orders its own CTA.
+__device__ __forceinline__ void chain_barrier(uint32_t cluster_size) {
+    asm volatile("fence.proxy.async.global;" ::: "memory");
+    if (cluster_size > 1) { tc::cluster_arrive(); tc::cluster_wait(); }
+    else __syncthreads();
+    asm volatile("fence.proxy.async.global;" ::: "memory");
+}
+
 template <int kMath, uint32_t kTypes, uint32_t kEpis>
 __global__ void __launch_bounds__(kThreads, variant_min_blocks(kTypes, kEpis))
-sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Stage single, const int stage_begin, const int stage_end, const int tc_setup, const uint64_t seed) {
-    // `single` = the stage table entry when the launch covers exactly one stage (staged mode): no global load before the first task
+sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Stage single, const int stage_begin, const int stage_end, const int tc_setup,
+                  const int chained, const uint64_t seed) {
+    // `single` = the stage table entry when the launch covers exactly one stage (staged mode): no global load before the first task.
+    // chained != 0: the launch covers the stages of one chain (Stage::chain_map), as thread-block clusters.
     extern __shared__ __align__(16) uint8_t smem_raw[];
-    __shared__ uint64_t s_bars[2 * kTStages + 2];
+    __shared__ uint64_t s_bars[2 * kTStages + 1];
     __shared__ uint32_t s_tmem;
     __shared__ float s_red[kColsumSmem];      // >= kThreads floats
     __shared__ Stage s_stage;
@@ -211,8 +222,8 @@ sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Sta
         }
     };
     stamp(0);
-    auto timeline = [&](int slot, bool is_max) {
-        if (P.timeline && threadIdx.x == 0 && stage_end - stage_begin == 1) {
+    auto timeline = [&](int slot, bool is_max) {      // one entry per launch, under its first stage
+        if (P.timeline && threadIdx.x == 0 && (stage_end - stage_begin == 1 || chained)) {
             unsigned long long t;
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
             if (is_max) atomicMax(&P.timeline[stage_begin * 4 + slot], t); else atomicMin(&P.timeline[stage_begin * 4 + slot], t);
@@ -221,15 +232,12 @@ sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Sta
     timeline(0, false);
     tc::TcState st;
     st.g = 0; st.accum_uses = 0; st.tmem_base = 0; st.b_pre = 0;
-    st.krank = tc::cluster_ctarank(); st.ksplit = tc::cluster_nctarank(); st.reduce_uses = 0;
-    st.reduce_bar = s_bars + 2 * kTStages + 1;
     st.full_bar = s_bars; st.empty_bar = s_bars + kTStages; st.accum_bar = s_bars + 2 * kTStages; st.trace = P.trace;
     constexpr bool kTc = kMath != SACB_MATH_FP32;
     st.tiles = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     if (kTc && (kTypes & tb(T_GEMM)) != 0 && tc_setup) {
         if (threadIdx.x == 32) {      // warp 1 initialises the barriers while warp 0 allocates tensor memory
             for (int i = 0; i <= 2 * kTStages; i++) tc::mbar_init(&s_bars[i], 1);
-            tc::mbar_init(st.reduce_bar, st.ksplit > 1 ? st.ksplit - 1 : 1);
             tc::fence_barrier_init();
         }
         if (threadIdx.x < 32) tc::tmem_alloc(&s_tmem, kTN);
@@ -237,104 +245,161 @@ sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Sta
         __syncthreads();
         tc::tc_fence_after();
         st.tmem_base = s_tmem;
-        if (st.ksplit > 1) { tc::cluster_arrive(); tc::cluster_wait(); }      // every peer's reduce barrier is initialised
     }
 
     stamp(1);
-    unsigned int bar_target = 0;
     bool dep_synced = false;
     const Task *cached_task = nullptr;
-    for (int s = stage_begin; s < stage_end; s++) {
+    auto load_stage = [&](int s) {
+        __syncthreads();      // the previous stage's readers of s_stage are done
         if (threadIdx.x < sizeof(Stage) / 4) {
             const int32_t *src = (stage_end - stage_begin == 1) ? reinterpret_cast<const int32_t *>(&single) : reinterpret_cast<const int32_t *>(&P.stages[s]);
             reinterpret_cast<int32_t *>(&s_stage)[threadIdx.x] = src[threadIdx.x];
         }
         __syncthreads();
         stamp(9);
-        const int n_stage_tiles = s_stage.n_tiles, n_stage_tasks = s_stage.task_end - s_stage.task_begin;
-        const int total = n_stage_tiles * P.n_agents;
-        // a cluster of ksplit CTAs shares one work item (split-K GEMM tile); without a cluster launch ksplit == 1
-        const int cl = blockIdx.x / st.ksplit, n_cl = gridDim.x / st.ksplit;
-        for (int wi = cl; wi < total; wi += n_cl) {
-            const int agent = wi / n_stage_tiles, tile_in_stage = wi % n_stage_tiles;
-            int k = 0;
-            while (k + 1 < n_stage_tasks && tile_in_stage >= s_stage.tile_begin[k + 1]) k++;
-            const Task *tg = &P.tasks[s_stage.task_begin + k];
-            const int tile = tile_in_stage - s_stage.tile_begin[k];
-            if (tg != cached_task) {   // one parallel fetch of the task's fields instead of a chain of dependent global loads; a CTA that walks
-                                       // many tiles of the same task (population / large batch) keeps its copy
-                cached_task = tg;
-                constexpr int kSkip = 2 * sizeof(CUtensorMap) / 4, kWords = sizeof(Task) / 4 - kSkip;
-                static_assert(kWords <= kThreads, "task copy");
-                if (kTc && threadIdx.x == kThreads - 1) { tc::tma_prefetch_desc(&tg->tmA); tc::tma_prefetch_desc(&tg->tmB); }
-                __syncthreads();     // the previous tile's readers of s_task are done
-                if (wi == cl) stamp(10);
-                if ((int)threadIdx.x < kWords)
-                    reinterpret_cast<int32_t *>(&s_task)[kSkip + threadIdx.x] = __ldcg(reinterpret_cast<const int32_t *>(tg) + kSkip + threadIdx.x);
-                __syncthreads();
-                if (wi == cl) stamp(11);
-            }
-            const Task &t = s_task;
-            if (!dep_synced) {      // everything above only read launch parameters and the static task tables
-                if constexpr (kTc && (kTypes & tb(T_GEMM)) != 0) {
-                    if (t.type == T_GEMM && t.i[6] && tc_setup && stage_end - stage_begin == 1) tc::tc_prefetch_b(t, tg, tile, agent, st);
-                }
-                asm volatile("griddepcontrol.wait;" ::: "memory");
-                asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-                dep_synced = true;
-                timeline(1, false);
-            }
-            float *scalars = resolve(P.scalars, P.bases, agent);
-            if (t.type != T_GEMM && st.krank != 0) continue;      // element-wise tasks of a clustered stage run on rank 0 only
-            constexpr bool kOutlined = kTc && (kTypes & kBaseTypes) == kBaseTypes && kEpis == kAllEpis && !SACB_NO_OUTLINE;
-            if constexpr (kOutlined) {
-                switch (t.type) {
-                    case T_GEMM:
-                        switch (t.epi) {
-                            case EPI_F32: gemm_tile_tc_outlined<tb(EPI_F32)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, wi == cl, seed); break;
-                            case EPI_BIAS_RELU: gemm_tile_tc_outlined<tb(EPI_BIAS_RELU)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, wi == cl, seed); break;
-                            case EPI_MASK: gemm_tile_tc_outlined<tb(EPI_MASK)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, wi == cl, seed); break;
-                            case EPI_SAMPLE: gemm_tile_tc_outlined<tb(EPI_SAMPLE)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, wi == cl, seed); break;
-                            default: gemm_tile_tc_outlined<tb(EPI_ADAM)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, wi == cl, seed); break;
-                        }
-                        break;
-                    case T_SHADOW: task_shadow_outlined(t, tile, P, agent); break;
-                    case T_GATHER: task_gather_outlined(t, tile, P, agent, scalars, seed); break;
-                    case T_SAMPLE: task_sample_outlined(t, tile, P, agent, scalars, seed); break;
-                    case T_TARGET_LOSS: task_target_loss_outlined(t, tile, P, agent, scalars, s_red); break;
-                    case T_ACTOR_LOSS: task_actor_loss_outlined(t, tile, P, agent, scalars, s_red); break;
-                    case T_SAMPLE_BWD: task_sample_bwd_outlined(t, tile, P, agent, scalars); break;
-                    case T_OUT_ADAM: task_out_adam_outlined(t, tile, P, agent, scalars, s_red); break;
-                    case T_BIAS_ADAM: task_bias_adam_outlined(t, tile, P, agent, scalars, s_red); break;
-                    case T_FINISH: task_finish_outlined(t, P, agent, scalars, s_red); break;
-                    case T_LN_FWD: task_ln_fwd(t, tile, P, agent); break;
-                    case T_LN_BWD: task_ln_bwd(t, tile, P, agent); break;
-                }
-            } else
-            switch (t.type) {      // only the task types of this build's mask are compiled in
+    };
+    // task of stage tile `tile_in_stage` (s_stage) -> global record, tile index inside the task; its fields -> s_task
+    auto fetch_task = [&](int tile_in_stage, int &tile, bool first) -> const Task * {
+        int k = 0;
+        while (k + 1 < s_stage.task_end - s_stage.task_begin && tile_in_stage >= s_stage.tile_begin[k + 1]) k++;
+        const Task *tg = &P.tasks[s_stage.task_begin + k];
+        tile = tile_in_stage - s_stage.tile_begin[k];
+        if (tg != cached_task) {   // one parallel fetch of the task's fields instead of a chain of dependent global loads; a CTA that walks
+                                   // many tiles of the same task (population / large batch) keeps its copy
+            cached_task = tg;
+            constexpr int kSkip = 2 * sizeof(CUtensorMap) / 4, kWords = sizeof(Task) / 4 - kSkip;
+            static_assert(kWords <= kThreads, "task copy");
+            if (kTc && threadIdx.x == kThreads - 1) { tc::tma_prefetch_desc(&tg->tmA); tc::tma_prefetch_desc(&tg->tmB); }
+            __syncthreads();     // the previous tile's readers of s_task are done
+            if (first) stamp(10);
+            if ((int)threadIdx.x < kWords)
+                reinterpret_cast<int32_t *>(&s_task)[kSkip + threadIdx.x] = __ldcg(reinterpret_cast<const int32_t *>(tg) + kSkip + threadIdx.x);
+            __syncthreads();
+            if (first) stamp(11);
+        }
+        return tg;
+    };
+    auto dep_sync = [&]() {      // everything before only read launch parameters and the static task tables
+        if (dep_synced) return;
+        asm volatile("griddepcontrol.wait;" ::: "memory");
+        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+        dep_synced = true;
+        timeline(1, false);
+    };
+    auto run_task = [&](const Task *tg, int tile, int agent, bool first) {
+        const Task &t = s_task;
+        float *scalars = resolve(P.scalars, P.bases, agent);
+        constexpr bool kOutlined = kTc && (kTypes & kBaseTypes) == kBaseTypes && kEpis == kAllEpis && !SACB_NO_OUTLINE;
+        if constexpr (kOutlined) {
+            switch (t.type) {
                 case T_GEMM:
-                    if constexpr ((kTypes & tb(T_GEMM)) != 0) {
-                        if (kTc) gemm_tile_tc<kEpis>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, wi == cl, seed);
-                        else gemm_tile_ffma(t, tile, P.bases, agent, scalars, reinterpret_cast<float *>(smem_raw));
+                    switch (t.epi) {
+                        case EPI_F32: gemm_tile_tc_outlined<tb(EPI_F32)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
+                        case EPI_BIAS_RELU: gemm_tile_tc_outlined<tb(EPI_BIAS_RELU)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
+                        case EPI_MASK: gemm_tile_tc_outlined<tb(EPI_MASK)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
+                        case EPI_SAMPLE: gemm_tile_tc_outlined<tb(EPI_SAMPLE)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
+                        default: gemm_tile_tc_outlined<tb(EPI_ADAM)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
                     }
                     break;
-                case T_SHADOW: if constexpr ((kTypes & tb(T_SHADOW)) != 0) task_shadow(t, tile, P, agent); break;
-                case T_GATHER: if constexpr ((kTypes & tb(T_GATHER)) != 0) task_gather(t, tile, P, agent, scalars, seed); break;
-                case T_SAMPLE: if constexpr ((kTypes & tb(T_SAMPLE)) != 0) task_sample(t, tile, P, agent, scalars, seed); break;
-                case T_TARGET_LOSS: if constexpr ((kTypes & tb(T_TARGET_LOSS)) != 0) task_target_loss(t, tile, P, agent, scalars, s_red); break;
-                case T_ACTOR_LOSS: if constexpr ((kTypes & tb(T_ACTOR_LOSS)) != 0) task_actor_loss(t, tile, P, agent, scalars, s_red); break;
-                case T_SAMPLE_BWD: if constexpr ((kTypes & tb(T_SAMPLE_BWD)) != 0) task_sample_bwd(t, tile, P, agent, scalars); break;
-                case T_OUT_ADAM: if constexpr ((kTypes & tb(T_OUT_ADAM)) != 0) task_out_adam<variant_min_blocks(kTypes, kEpis) == 1>(t, tile, P, agent, scalars, s_red); break;
-                case T_BIAS_ADAM: if constexpr ((kTypes & tb(T_BIAS_ADAM)) != 0) task_bias_adam<variant_min_blocks(kTypes, kEpis) == 1>(t, tile, P, agent, scalars, s_red); break;
-                case T_FINISH: if constexpr ((kTypes & tb(T_FINISH)) != 0) task_finish(t, P, agent, scalars, s_red); break;
-                case T_LN_FWD: if constexpr ((kTypes & tb(T_LN_FWD)) != 0) task_ln_fwd(t, tile, P, agent); break;
-                case T_LN_BWD: if constexpr ((kTypes & tb(T_LN_BWD)) != 0) task_ln_bwd(t, tile, P, agent); break;
+                case T_SHADOW: task_shadow_outlined(t, tile, P, agent); break;
+                case T_GATHER: task_gather_outlined(t, tile, P, agent, scalars, seed); break;
+                case T_SAMPLE: task_sample_outlined(t, tile, P, agent, scalars, seed); break;
+                case T_TARGET_LOSS: task_target_loss_outlined(t, tile, P, agent, scalars, s_red); break;
+                case T_ACTOR_LOSS: task_actor_loss_outlined(t, tile, P, agent, scalars, s_red); break;
+                case T_SAMPLE_BWD: task_sample_bwd_outlined(t, tile, P, agent, scalars); break;
+                case T_OUT_ADAM: task_out_adam_outlined(t, tile, P, agent, scalars, s_red); break;
+                case T_BIAS_ADAM: task_bias_adam_outlined(t, tile, P, agent, scalars, s_red); break;
+                case T_FINISH: task_finish_outlined(t, P, agent, scalars, s_red); break;
+                case T_LN_FWD: task_ln_fwd(t, tile, P, agent); break;
+                case T_LN_BWD: task_ln_bwd(t, tile, P, agent); break;
             }
-            if (wi == cl) stamp(4);
+        } else
+        switch (t.type) {      // only the task types of this build's mask are compiled in
+            case T_GEMM:
+                if constexpr ((kTypes & tb(T_GEMM)) != 0) {
+                    if (kTc) gemm_tile_tc<kEpis>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed);
+                    else gemm_tile_ffma(t, tile, P.bases, agent, scalars, reinterpret_cast<float *>(smem_raw));
+                }
+                break;
+            case T_SHADOW: if constexpr ((kTypes & tb(T_SHADOW)) != 0) task_shadow(t, tile, P, agent); break;
+            case T_GATHER: if constexpr ((kTypes & tb(T_GATHER)) != 0) task_gather(t, tile, P, agent, scalars, seed); break;
+            case T_SAMPLE: if constexpr ((kTypes & tb(T_SAMPLE)) != 0) task_sample(t, tile, P, agent, scalars, seed); break;
+            case T_TARGET_LOSS: if constexpr ((kTypes & tb(T_TARGET_LOSS)) != 0) task_target_loss(t, tile, P, agent, scalars, s_red); break;
+            case T_ACTOR_LOSS: if constexpr ((kTypes & tb(T_ACTOR_LOSS)) != 0) task_actor_loss(t, tile, P, agent, scalars, s_red); break;
+            case T_SAMPLE_BWD: if constexpr ((kTypes & tb(T_SAMPLE_BWD)) != 0) task_sample_bwd(t, tile, P, agent, scalars); break;
+            case T_OUT_ADAM: if constexpr ((kTypes & tb(T_OUT_ADAM)) != 0) task_out_adam<variant_min_blocks(kTypes, kEpis) == 1>(t, tile, P, agent, scalars, s_red); break;
+            case T_BIAS_ADAM: if constexpr ((kTypes & tb(T_BIAS_ADAM)) != 0) task_bias_adam<variant_min_blocks(kTypes, kEpis) == 1>(t, tile, P, agent, scalars, s_red); break;
+            case T_FINISH: if constexpr ((kTypes & tb(T_FINISH)) != 0) task_finish(t, P, agent, scalars, s_red); break;
+            case T_LN_FWD: if constexpr ((kTypes & tb(T_LN_FWD)) != 0) task_ln_fwd(t, tile, P, agent); break;
+            case T_LN_BWD: if constexpr ((kTypes & tb(T_LN_BWD)) != 0) task_ln_bwd(t, tile, P, agent); break;
         }
-        if (s + 1 < stage_end) {
-            bar_target += gridDim.x;
-            grid_barrier(P.barrier, bar_target, P.error_flag);
+        if (first) stamp(4);
+    };
+
+    if (!chained) {
+        unsigned int bar_target = 0;
+        for (int s = stage_begin; s < stage_end; s++) {
+            load_stage(s);
+            const int n_stage_tiles = s_stage.n_tiles, total = n_stage_tiles * P.n_agents;
+            for (int wi = blockIdx.x; wi < total; wi += gridDim.x) {
+                const int agent = wi / n_stage_tiles;
+                int tile;
+                const Task *tg = fetch_task(wi % n_stage_tiles, tile, wi == (int)blockIdx.x);
+                if (!dep_synced) {
+                    if constexpr (kTc && (kTypes & tb(T_GEMM)) != 0) {
+                        if (s_task.type == T_GEMM && s_task.i[6] && tc_setup && stage_end - stage_begin == 1) tc::tc_prefetch_b(s_task, tg, tile, agent, st, P.error_flag);
+                    }
+                    dep_sync();
+                }
+                run_task(tg, tile, agent, wi == (int)blockIdx.x);
+            }
+            if (s + 1 < stage_end) {
+                bar_target += gridDim.x;
+                grid_barrier(P.barrier, bar_target, P.error_flag);
+            }
+        }
+    } else if constexpr (variant_chains(kMath, kTypes, kEpis)) {
+        // chained launch (one agent): cluster c < chain_clusters owns its row block in every stage of the chain, rank r its column tile r;
+        // a cluster stops behind the last stage that has a tile for it (a uniform decision: the map is per cluster).  The other clusters
+        // walk the riders (T_SHADOW tasks of the chain's stages, independent of the chain) without barriers.
+        const uint32_t cw = tc::cluster_nctarank(), r = tc::cluster_ctarank();
+        const int c = (int)(blockIdx.x / cw);
+        load_stage(stage_begin);
+        const int n_row = s_stage.chain_clusters;
+        if (c < n_row) {
+            int e = s_stage.chain_map[c], tile = 0;
+            bool have = e >= 0 && (int)r < (e >> 16);
+            const Task *tg = have ? fetch_task((e & 0xffff) + (int)r, tile, true) : nullptr;
+            dep_sync();
+            for (int s = stage_begin;; s++) {
+                if (have) run_task(tg, tile, 0, s == stage_begin);
+                if (s + 1 == stage_end) break;
+                load_stage(s + 1);
+                e = s_stage.chain_map[c];
+                if (e < 0) break;
+                have = (int)r < (e >> 16);
+                if (have) {      // the next layer's weights do not depend on this layer: request their first K blocks now
+                    tg = fetch_task((e & 0xffff) + (int)r, tile, false);
+                    tc::tc_prefetch_b(s_task, tg, tile, 0, st, P.error_flag);
+                }
+                chain_barrier(cw);
+            }
+        } else {
+            const int rider = (int)blockIdx.x - n_row * (int)cw, n_riders = (int)gridDim.x - n_row * (int)cw;
+            dep_sync();
+            int base = 0;      // riders of all stages of the chain as one list, dealt round-robin
+            for (int s = stage_begin; s < stage_end; s++) {
+                if (s != stage_begin) load_stage(s);
+                for (int k = 0; k < s_stage.task_end - s_stage.task_begin; k++) {
+                    const int tb0 = s_stage.tile_begin[k];
+                    int tile;
+                    const Task *tg = fetch_task(tb0, tile, false);
+                    if (s_task.type == T_GEMM) continue;
+                    for (int i = ((rider - base) % n_riders + n_riders) % n_riders; i < s_task.n_tiles; i += n_riders) run_task(tg, i, 0, false);
+                    base += s_task.n_tiles;
+                }
+            }
         }
     }
 
@@ -666,7 +731,7 @@ struct Builder {
         stage_stream.clear();
         auto emit = [&](const std::vector<Task> &ts, bool gemm) {
             Stage sg{};
-            sg.task_begin = (int)nt.size(); sg.n_tiles = 0; sg.ksplit = 1;
+            sg.task_begin = (int)nt.size(); sg.n_tiles = 0;
             for (size_t i = 0; i < ts.size(); i++) {
                 Task t = ts[i];
                 sg.tile_begin[i] = sg.n_tiles; t.tile_begin = sg.n_tiles; sg.n_tiles += t.n_tiles;
@@ -937,6 +1002,104 @@ struct Builder {
 
 };
 
+// ---- chains of row-local GEMM stages (one launch of thread-block clusters each) -----------------------------------------------
+// In consecutive MLP layers, row block r of layer l+1 reads only row block r of layer l, across all its columns: with 64 x 64 tiles
+// and at most 8 column tiles per layer, a cluster of CTAs holds the whole row block and a cluster barrier replaces the kernel
+// boundary (clusters never wait on each other).  Stage s+1 joins stage s when
+//   - both hold only GEMM tasks with a bias+ReLU, mask or fp32 epilogue, plus T_SHADOW riders, and s writes pair matrices (not fp32);
+//   - every GEMM of s+1 reads, as its K-major A operand, exactly the output of its own GEMM of s, with the same rows;
+//   - nothing else a GEMM of the chain reads (B, ReLU-mask source) is written by a stage of the chain;
+//   - every GEMM of the chain has at most kChainMaxCols 64-column tiles.
+// Results do not depend on the tile shape (the K order and the three products of every element stay the same).
+constexpr int kChainMaxCols = 8;
+struct Chain {
+    int s0, s1, cluster;
+    int n_row;                                 // row clusters (row blocks of the first stage's GEMMs)
+    int rider_tiles;                           // T_SHADOW tiles of the chain's stages
+    int rider_clusters = 0, kind = 0;          // clusters that walk the riders; kernel variant of the launch
+};
+
+static bool same_pm(const PmRef &a, const PmRef &b) { return a.base.v == b.base.v && a.ld == b.ld && a.plane == b.plane; }
+
+static std::vector<Chain> find_chains(const std::vector<Task> &tasks, const std::vector<Stage> &stages) {
+    auto gemms = [&](int s) { std::vector<int> g; for (int k = stages[s].task_begin; k < stages[s].task_end; k++) if (tasks[k].type == T_GEMM) g.push_back(k); return g; };
+    auto eligible = [&](int s) {
+        bool any = false;
+        for (int k = stages[s].task_begin; k < stages[s].task_end; k++) {
+            const Task &t = tasks[k];
+            if (t.type == T_SHADOW) continue;
+            if (t.type != T_GEMM || (t.epi != EPI_F32 && t.epi != EPI_BIAS_RELU && t.epi != EPI_MASK) || cdiv(t.N, 64) > kChainMaxCols) return false;
+            any = true;
+        }
+        return any;
+    };
+    auto joins = [&](int s) {      // s -> s+1
+        if (!eligible(s) || !eligible(s + 1)) return false;
+        const std::vector<int> prev = gemms(s), next = gemms(s + 1);
+        std::vector<int> used(prev.size(), 0);
+        for (int k : prev) if (tasks[k].epi == EPI_F32) return false;
+        for (int h : next) {
+            const Task &t = tasks[h];
+            if (t.A.mn_major || t.A.r0) return false;
+            int found = -1;
+            for (size_t i = 0; i < prev.size(); i++)
+                if (same_pm(tasks[prev[i]].Cpm, t.A.pm) && tasks[prev[i]].M == t.M && tasks[prev[i]].N == t.K) found = (int)i;
+            if (found < 0 || used[found]++) return false;
+        }
+        return true;
+    };
+    auto reads_written = [&](int s0, int s1) {      // a GEMM of [s0, s1) reads as B / mask what a task of [s0, s1) writes
+        std::vector<int64_t> out;
+        for (int s = s0; s < s1; s++)
+            for (int k = stages[s].task_begin; k < stages[s].task_end; k++)
+                out.push_back(tasks[k].type == T_GEMM ? tasks[k].Cpm.base.v : tasks[k].pm[0].base.v);
+        for (int s = s0; s < s1; s++)
+            for (int k : gemms(s))
+                for (int64_t o : out)
+                    if (o == tasks[k].B.pm.base.v || (tasks[k].epi == EPI_MASK && o == tasks[k].mask.base.v)) return true;
+        return false;
+    };
+    std::vector<Chain> out;
+    for (int s = 0; s + 1 < (int)stages.size();) {
+        int e = s + 1;
+        while (e < (int)stages.size() && joins(e - 1) && !reads_written(s, e + 1)) e++;
+        if (e - s < 2) { s++; continue; }
+        Chain c{s, e, 1, 0, 0};
+        for (int x = s; x < e; x++)
+            for (int k = stages[x].task_begin; k < stages[x].task_end; k++) {
+                if (tasks[k].type == T_GEMM) c.cluster = std::max(c.cluster, cdiv(tasks[k].N, 64));
+                else c.rider_tiles += tasks[k].n_tiles;
+            }
+        for (int k : gemms(s)) c.n_row += cdiv(tasks[k].M, 64);
+        if (c.n_row <= kMaxChainClusters) out.push_back(c);
+        s = e;
+    }
+    return out;
+}
+
+// Stage::chain_map of every stage of a chain (tasks built with 64 x 64 tiles)
+static void fill_chain_maps(const std::vector<Task> &tasks, std::vector<Stage> &stages, const Chain &c) {
+    std::map<int, int> first_cluster;      // GEMM task -> cluster of its row block 0 (row blocks r -> first + r)
+    int next = 0;
+    for (int s = c.s0; s < c.s1; s++) {
+        Stage &sg = stages[s];
+        for (int i = 0; i < kMaxChainClusters; i++) sg.chain_map[i] = -1;
+        sg.chain_len = s == c.s0 ? c.s1 - c.s0 : 0;
+        sg.chain_clusters = c.n_row;
+        for (int k = sg.task_begin; k < sg.task_end; k++) {
+            const Task &t = tasks[k];
+            if (t.type != T_GEMM) continue;
+            int c0 = -1;
+            if (s == c.s0) { c0 = next; next += t.tiles_m; }
+            else
+                for (int p = stages[s - 1].task_begin; p < stages[s - 1].task_end; p++)
+                    if (tasks[p].type == T_GEMM && same_pm(tasks[p].Cpm, t.A.pm)) c0 = first_cluster[p];
+            first_cluster[k] = c0;
+            for (int rb = 0; rb < t.tiles_m; rb++) sg.chain_map[c0 + rb] = (t.tile_begin + rb * t.tiles_n) | (t.tiles_n << 16);
+        }
+    }
+}
+
 }  // namespace
 
 void free_programs(sacb_handle h) {
@@ -961,7 +1124,7 @@ int check_error_flag(sacb_handle h) {
     return SACB_OK;
 }
 
-// one stage = one launch (staged mode): grid = tiles x ksplit, thread-block cluster of ksplit CTAs along x, optional PDL
+// one stage = one launch of the stream kernel, optional PDL
 static int launch_stream_stage(sacb_handle h, ProgramInst &p, int s, bool pdl) {
     uint64_t seed = h->cfg.seed;
     Stage single = p.stages[s];
@@ -977,29 +1140,31 @@ static int launch_stream_stage(sacb_handle h, ProgramInst &p, int s, bool pdl) {
     return SACB_OK;
 }
 
-static int launch_stage(sacb_handle h, ProgramInst &p, int s, bool pdl) {
+// launch `li` of a staged program: one stage, or a chain of stages as thread-block clusters; optional PDL
+static int launch_stage(sacb_handle h, ProgramInst &p, int li, bool pdl) {
+    const StageLaunch &L = p.launches[li];
+    const int s = L.s0;
     if (p.stage_stream[s]) return launch_stream_stage(h, p, s, pdl);
-    const bool tc = math_is_tc(h->cfg.math_mode);
-    const int kind = p.stage_kind[s];      // index of the kernel variant
+    const bool tc = math_is_tc(h->cfg.math_mode), chain = L.s1 - L.s0 > 1;
+    const int kind = L.kind;      // index of the kernel variant
     const size_t smem = variant_has_gemm(kind) ? math_smem(h->cfg.math_mode) : 0;      // element-wise stages only use static shared memory
     uint64_t seed = h->cfg.seed;
-    int s0 = s, s1 = s + 1, tc_setup = tc ? p.stage_has_gemm[s] : 0;
+    int s0 = L.s0, s1 = L.s1, tc_setup = tc ? p.stage_has_gemm[s] : 0, chained = chain ? 1 : 0;
     Stage single = p.stages[s];
-    const int ks = std::max(1, single.ksplit);
-    void *args[] = {(void *)&p.prog, (void *)&single, (void *)&s0, (void *)&s1, (void *)&tc_setup, (void *)&seed};
+    void *args[] = {(void *)&p.prog, (void *)&single, (void *)&s0, (void *)&s1, (void *)&tc_setup, (void *)&chained, (void *)&seed};
     cudaLaunchConfig_t cfg{};
+    int ctas = chain ? L.grid : std::max(1, single.n_tiles * h->cfg.n_agents);
     // population mode: a stage of many more tiles than SMs runs as one resident CTA per SM looping over tiles (barrier /
     // TMEM setup and teardown once per SM instead of once per tile); a single agent's stage (<= ~150 tiles) keeps one CTA per tile
-    int ctas = std::max(1, single.n_tiles * h->cfg.n_agents);
     static const int grid_cap = getenv("SACB_GRID_CAP") ? atoi(getenv("SACB_GRID_CAP")) : -1;     // 0 = never cap
     const int cap = grid_cap < 0 ? h->sm_count : grid_cap;
-    if (ks == 1 && cap > 0 && ctas > 2 * h->sm_count) {      // resident CTAs looping over tiles wi = blockIdx.x + i * gridDim.x
+    if (!chain && cap > 0 && ctas > 2 * h->sm_count) {      // resident CTAs looping over tiles wi = blockIdx.x + i * gridDim.x
         ctas = std::min(ctas, cap * (tc ? variant_blocks_per_sm(kind) : 1));
         // a grid that is a multiple of the stage's per-agent tile count keeps every CTA on ONE tile of ONE task across the agents it
         // walks: the task record is fetched once instead of once per tile (population mode: a column-sum stage holds 2-6 tasks)
         if (single.task_end - single.task_begin > 1 && single.n_tiles <= ctas / 2) ctas = (ctas / single.n_tiles) * single.n_tiles;
     }
-    cfg.gridDim = dim3(ctas * ks); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = h->stream;
+    cfg.gridDim = dim3(ctas); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = h->stream;
     cudaLaunchAttribute attr[2];
     int na = 0;
     if (pdl) {
@@ -1010,9 +1175,9 @@ static int launch_stage(sacb_handle h, ProgramInst &p, int s, bool pdl) {
         attr[na].val.programmaticStreamSerializationAllowed = 1;
         na++;
     }
-    if (ks > 1) {
+    if (chain && L.cluster > 1) {
         attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = ks; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
+        attr[na].val.clusterDim.x = L.cluster; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
         na++;
     }
     cfg.attrs = attr; cfg.numAttrs = na;
@@ -1020,35 +1185,52 @@ static int launch_stage(sacb_handle h, ProgramInst &p, int s, bool pdl) {
     return SACB_OK;
 }
 
-static int launch_range(sacb_handle h, ProgramInst &p, int s0, int s1, bool cooperative) {
+// the stages [s0, s1) as ONE cooperative launch of the build that carries every code path (persistent mode)
+static int launch_range(sacb_handle h, ProgramInst &p, int s0, int s1) {
     const bool tf32 = math_is_tc(h->cfg.math_mode);
     int needs_tc = 0, max_tiles = 1;
     for (int s = s0; s < s1; s++) { needs_tc |= p.stage_has_gemm[s]; max_tiles = std::max(max_tiles, p.stages[s].n_tiles * h->cfg.n_agents); }
     const size_t smem = math_smem(h->cfg.math_mode);
     uint64_t seed = h->cfg.seed;
-    int tc_setup = tf32 ? needs_tc : 0;
+    int tc_setup = tf32 ? needs_tc : 0, chained = 0;
     Stage single = p.stages[s0];
-    void *args[] = {(void *)&p.prog, (void *)&single, (void *)&s0, (void *)&s1, (void *)&tc_setup, (void *)&seed};
+    void *args[] = {(void *)&p.prog, (void *)&single, (void *)&s0, (void *)&s1, (void *)&tc_setup, (void *)&chained, (void *)&seed};
     const void *fn = update_kernel_for(h->cfg.math_mode, h->cfg.layer_norm ? kVariantEverythingLn : kVariantEverything);
-    if (cooperative) {
-        const int grid = std::min(max_tiles, h->sm_count * h->coop_blocks_per_sm);
-        SACB_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, h->stream));
-    } else {
-        return launch_stage(h, p, s0, h->use_pdl != 0);
-    }
+    const int grid = std::min(max_tiles, h->sm_count * h->coop_blocks_per_sm);
+    SACB_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, h->stream));
     return SACB_OK;
 }
 
 static int record_step(sacb_handle h, ProgramInst &p) {
     if (h->cfg.launch_mode == SACB_LAUNCH_PERSISTENT) {
         SACB_CUDA(cudaMemsetAsync(h->barrier, 0, sizeof(unsigned int), h->stream));
-        return launch_range(h, p, 0, (int)p.stages.size(), true);
+        return launch_range(h, p, 0, (int)p.stages.size());
     }
-    for (int s = 0; s < (int)p.stages.size(); s++) {
-        int rc = launch_range(h, p, s, s + 1, false);
+    for (int li = 0; li < (int)p.launches.size(); li++) {
+        int rc = launch_stage(h, p, li, h->use_pdl != 0);
         if (rc) return rc;
     }
     return SACB_OK;
+}
+
+// clusters of `cluster` CTAs of kernel variant `kind` the GPU holds at once (cached per handle); < 0: a CUDA error code
+static int max_active_clusters(sacb_handle h, int kind, int cluster) {
+    const auto key = std::make_pair(kind, cluster);
+    const auto it = h->max_active_clusters.find(key);
+    if (it != h->max_active_clusters.end()) return it->second;
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(cluster); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = math_smem(h->cfg.math_mode); cfg.stream = h->stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = cluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    int n = 0;
+    if (cudaOccupancyMaxActiveClusters(&n, update_kernel_for(h->cfg.math_mode, kind), &cfg) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(SACB_ERR_DEVICE, "cudaOccupancyMaxActiveClusters failed");
+    }
+    h->max_active_clusters[key] = n;
+    return n;
 }
 
 int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
@@ -1056,6 +1238,7 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
     if (it != h->programs.end()) { *out = &it->second; return SACB_OK; }
     if (key.B < 1 || key.B > h->cfg.max_batch) return fail(SACB_ERR_ARG, "batch size exceeds max_batch of the handle");
     std::vector<std::pair<int, int>> shapes;
+    std::vector<Chain> chains;
     bool stream_mode = false;
     {   // dry pass with the default 128 x 64 tiles: the per-stage tile counts drive the choice of tile shapes
         Builder d(h, key);
@@ -1066,8 +1249,29 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
         for (size_t s = 0; s < d.stages.size(); s++) if (d.has_gemm[s]) widest = std::max(widest, d.stages[s].n_tiles * h->cfg.n_agents);
         // throughput form: the widest GEMM stage has more than two waves of tiles (population of agents, large batches)
         stream_mode = math_is_tc(h->cfg.math_mode) && h->cfg.launch_mode == SACB_LAUNCH_STAGED && widest > 2 * h->sm_count &&
-                      !getenv("SACB_NO_STREAM") && !getenv("SACB_FUSE_SAMPLE") && !getenv("SACB_SPLITK");
+                      !getenv("SACB_NO_STREAM") && !getenv("SACB_FUSE_SAMPLE");
         shapes = stream_mode ? d.stream_tile_shapes() : d.choose_tile_shapes(h->sm_count);
+        // chained launches: latency programs of one agent (staged, tensor cores, no LayerNorm), where every cluster of the chain fits
+        // on the GPU at once (its CTAs hold one SM each)
+        if (math_is_tc(h->cfg.math_mode) && h->cfg.launch_mode == SACB_LAUNCH_STAGED && !stream_mode && h->cfg.n_agents == 1 && !h->cfg.layer_norm) {
+            for (Chain c : find_chains(d.tasks, d.stages)) {
+                uint32_t types = 0, epis = 0;
+                for (int k = d.stages[c.s0].task_begin; k < d.stages[c.s1 - 1].task_end; k++) {
+                    types |= tb(d.tasks[k].type);
+                    if (d.tasks[k].type == T_GEMM) epis |= tb(d.tasks[k].epi);
+                }
+                const int kind = pick_variant(types, epis, false);
+                const int fit = max_active_clusters(h, kind, c.cluster);
+                if (fit < 0) return fit;
+                if (!variant_can_chain(kind)) continue;
+                const int riders = c.rider_tiles ? std::min(cdiv(c.rider_tiles, c.cluster), fit - c.n_row) : 0;
+                if (c.n_row > fit || (c.rider_tiles && riders < 1)) continue;
+                c.rider_clusters = riders; c.kind = kind;
+                chains.push_back(c);
+                for (int k = d.stages[c.s0].task_begin; k < d.stages[c.s1 - 1].task_end; k++)
+                    if (d.tasks[k].type == T_GEMM) shapes[k] = {64, 64};
+            }
+        }
     }
     Builder b(h, key);
     b.shapes = shapes;
@@ -1076,21 +1280,7 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
     if (b.rc != SACB_OK) return b.rc;
     std::vector<int> stage_stream;
     if (stream_mode) b.split_mixed_stages(stage_stream);
-    // split-K (opt-in, SACB_SPLITK=1): a latency-bound stage with few tiles spreads every tile over a 2- or 4-CTA cluster so
-    // that more SMs pull operands (per-SM L2->SMEM ingest bounds the main loop); staged tensor-core launches only.
-    // Measured on B200 (profiles/r01_summary.md): the accumulator is ready 1.6 us (x2) / 2.8 us (x4) earlier, but pushing the
-    // partial tiles through DSMEM and the cluster-scope release/acquire cost 1.5-2.3 us, so it is a wash and stays off.
-    for (size_t s = 0; s < b.stages.size(); s++) {
-        Stage &sg = b.stages[s];
-        sg.ksplit = 1;
-        if (!math_is_tc(h->cfg.math_mode) || h->cfg.launch_mode != SACB_LAUNCH_STAGED || !b.has_gemm[s] || !getenv("SACB_SPLITK") || !getenv("SACB_FIXED_TILES")) continue;
-        int max_kb = 1;
-        for (int k = sg.task_begin; k < sg.task_end; k++)
-            if (b.tasks[k].type == T_GEMM) max_kb = std::max(max_kb, cdiv(b.tasks[k].K, kTK));
-        const int ctas = sg.n_tiles * h->cfg.n_agents;
-        for (int ks = 4; ks >= 2; ks /= 2)
-            if (ctas * ks <= h->sm_count && max_kb >= ks) { sg.ksplit = ks; break; }
-    }
+    for (const Chain &c : chains) fill_chain_maps(b.tasks, b.stages, c);
     ProgramInst &p = h->programs[key];
     p.tasks = b.tasks; p.stages = b.stages; p.stage_has_gemm = b.has_gemm;
     p.stage_stream = stage_stream.empty() ? std::vector<int>(b.stages.size(), 0) : stage_stream;
@@ -1104,6 +1294,16 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
         // population); a stage of a few long tiles (one agent, large batch) keeps the one-CTA build with 8 rows in flight
         const bool many = b.stages[s].n_tiles * h->cfg.n_agents > 2 * h->sm_count;
         p.stage_kind.push_back(getenv("SACB_ONE_KERNEL") ? (h->cfg.layer_norm ? kVariantEverythingLn : kVariantEverything) : pick_variant(types, epis, many));
+    }
+    for (int s = 0, ci = 0; s < (int)b.stages.size();) {
+        if (ci < (int)chains.size() && chains[ci].s0 == s) {
+            const Chain &c = chains[ci++];
+            p.launches.push_back({c.s0, c.s1, c.cluster, (c.n_row + c.rider_clusters) * c.cluster, c.kind});
+            s = c.s1;
+        } else {
+            p.launches.push_back({s, s + 1, 1, 0, p.stage_kind[s]});
+            s++;
+        }
     }
     for (auto &s : p.stages) { p.n_tiles_total += s.n_tiles; p.max_stage_tiles = std::max(p.max_stage_tiles, s.n_tiles); }
     SACB_CUDA(cudaMalloc(&p.d_tasks, p.tasks.size() * sizeof(Task)));
@@ -1126,7 +1326,7 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
     P.error_flag = h->error_flag;
     P.trace = nullptr; P.timeline = nullptr; P.adam_table = h->adam_table;
     P.host_losses = h->cfg.n_agents == 1 ? h->pin_small : nullptr;
-    p.kernels_per_step = h->cfg.launch_mode == SACB_LAUNCH_PERSISTENT ? 1 : (int)p.stages.size();
+    p.kernels_per_step = h->cfg.launch_mode == SACB_LAUNCH_PERSISTENT ? 1 : (int)p.launches.size();
 
     // capture one step into a CUDA graph (stage kernels, or memset + the single cooperative launch)
     cudaGraph_t graph = nullptr;
@@ -1173,8 +1373,12 @@ static int compute_split(ProgramInst &p) {
             if (p.tasks[k].type == T_ACTOR_LOSS && actor_stage < 0) actor_stage = s;
         }
     if (td_stage < 0) return fail(SACB_ERR_STATE, "program has no critic-loss stage");
-    p.split = actor_stage > td_stage ? actor_stage : td_stage + 1;
-    if (getenv("SACB_PER_SPLIT")) p.split = std::min(ns - 1, std::max(td_stage + 1, atoi(getenv("SACB_PER_SPLIT"))));      // experiment switch
+    int split = actor_stage > td_stage ? actor_stage : td_stage + 1;
+    if (getenv("SACB_PER_SPLIT")) split = std::min(ns - 1, std::max(td_stage + 1, atoi(getenv("SACB_PER_SPLIT"))));      // experiment switch
+    // the first launch from that stage on (neither the loss stages nor their neighbours are in a chain: a launch boundary)
+    const int nl = (int)p.launches.size();
+    p.split = nl;
+    for (int li = nl - 1; li >= 0 && p.launches[li].s0 >= split; li--) p.split = li;
     return SACB_OK;
 }
 
@@ -1182,7 +1386,7 @@ static int compute_split(ProgramInst &p) {
 int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
     static const bool off = getenv("SACB_NO_STEP_GRAPH") != nullptr;
     if (off || h->cfg.launch_mode != SACB_LAUNCH_STAGED || p.step_graph_failed) return 1;
-    const int ns = (int)p.stages.size();
+    const int nl = (int)p.launches.size();
     const int64_t n = h->r_len[0];
     if (!p.step_graph || p.step_graph_n != n || p.step_graph_k != k) {
         if (p.step_graph) { cudaGraphExecDestroy(p.step_graph); p.step_graph = nullptr; }
@@ -1193,15 +1397,15 @@ int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
         cudaGraph_t graph = nullptr;
         if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { cudaGetLastError(); p.step_graph_failed = true; return 1; }
         int rc = SACB_OK;
-        for (int s = 0; s < p.split && rc == SACB_OK; s++) rc = launch_stage(h, p, s, h->use_pdl != 0);
+        for (int li = 0; li < p.split && rc == SACB_OK; li++) rc = launch_stage(h, p, li, h->use_pdl != 0);
         if (rc == SACB_OK && (cudaEventRecord(h->ev_td, h->stream) != cudaSuccess || cudaStreamWaitEvent(h->stream2, h->ev_td, 0) != cudaSuccess)) rc = SACB_ERR_DEVICE;
         if (rc == SACB_OK) rc = per_writeback_launch(h, h->stream2, k, false);      // first kernel of the forked branch: a full dependency
         if (rc == SACB_OK) rc = per_sample_launch(h, h->stream2, nullptr, B, nullptr);
         if (rc == SACB_OK && cudaEventRecord(h->ev_sampled, h->stream2) != cudaSuccess) rc = SACB_ERR_DEVICE;
-        for (int s = p.split; s < ns && rc == SACB_OK; s++) rc = launch_stage(h, p, s, h->use_pdl != 0);
+        for (int li = p.split; li < nl && rc == SACB_OK; li++) rc = launch_stage(h, p, li, h->use_pdl != 0);
         if (rc == SACB_OK && cudaStreamWaitEvent(h->stream, h->ev_sampled, 0) != cudaSuccess) rc = SACB_ERR_DEVICE;
         const cudaError_t e2 = cudaStreamEndCapture(h->stream, &graph);
-        p.step_graph_launches = ns + (int)(h->kernel_launches - launches0);      // the stage kernels + what the replay helpers counted
+        p.step_graph_launches = nl + (int)(h->kernel_launches - launches0);      // the stage kernels + what the replay helpers counted
         p.step_graph_fused = h->per_fused;
         h->kernel_launches = launches0; h->per_frame[0] = frame0;
         if (rc != SACB_OK || e2 != cudaSuccess || !graph || cudaGraphInstantiate(&p.step_graph, graph, 0) != cudaSuccess) {
@@ -1223,12 +1427,12 @@ int launch_program_part(sacb_handle h, ProgramInst &p, int part) {
     if (h->cfg.launch_mode != SACB_LAUNCH_STAGED) {      // a single cooperative launch cannot be split: part 0 is the whole step
         return part == 0 ? launch_program(h, p) : SACB_OK;
     }
-    const int ns = (int)p.stages.size();
+    const int nl = (int)p.launches.size();
     if (!p.parts_built) {
         p.parts_built = true;
         if (p.split < 0) { if (int rc = compute_split(p)) return rc; }
         for (int part_i = 0; part_i < 2; part_i++) {
-            const int s0 = part_i ? p.split : 0, s1 = part_i ? ns : p.split;
+            const int s0 = part_i ? p.split : 0, s1 = part_i ? nl : p.split;
             cudaGraph_t graph = nullptr;
             if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) break;
             int rc = SACB_OK;
@@ -1239,7 +1443,7 @@ int launch_program_part(sacb_handle h, ProgramInst &p, int part) {
         }
         cudaGetLastError();
     }
-    const int s0 = part ? p.split : 0, s1 = part ? ns : p.split;
+    const int s0 = part ? p.split : 0, s1 = part ? nl : p.split;
     h->kernel_launches += s1 - s0;
     if (p.graph_part[part]) { SACB_CUDA(cudaGraphLaunch(p.graph_part[part], h->stream)); return SACB_OK; }
     for (int s = s0; s < s1; s++) { int rc = launch_stage(h, p, s, h->use_pdl != 0); if (rc) return rc; }
@@ -1273,21 +1477,31 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
     std::vector<unsigned long long> h_trace;
     if (trace) { SACB_CUDA(cudaMalloc(&d_trace, sizeof(unsigned long long) * kTraceSlots * 4096)); SACB_CUDA(cudaMemset(d_trace, 0, sizeof(unsigned long long) * kTraceSlots * 4096));
                  p->prog.trace = d_trace; h_trace.resize(kTraceSlots * 4096); }
-    const int n = std::min<int>(cap, (int)p->stages.size());
-    std::vector<cudaEvent_t> ev(p->stages.size() + 1);
+    const int nl = (int)p->launches.size();      // one entry per launch (a chain of stages is one)
+    const int n = std::min<int>(cap, nl);
+    std::vector<cudaEvent_t> ev(nl + 1);
     for (auto &e : ev) cudaEventCreate(&e);
-    std::vector<float> acc(p->stages.size(), 0.f);
+    std::vector<float> acc(nl, 0.f);
     const int reps = 20;
     for (int r = 0; r < reps + 3; r++) {
         cudaEventRecord(ev[0], h->stream);
-        for (int s = 0; s < (int)p->stages.size(); s++) {
-            // force the staged form regardless of launch_mode: this is a per-stage profile
-            { int rc2 = launch_stage(h, *p, s, false); if (rc2) return rc2; }
-            cudaEventRecord(ev[s + 1], h->stream);
-            if (trace && r == reps + 2) {
+        for (int li = 0; li < nl; li++) {
+            // force the staged form regardless of launch_mode: this is a per-launch profile
+            { int rc2 = launch_stage(h, *p, li, false); if (rc2) return rc2; }
+            cudaEventRecord(ev[li + 1], h->stream);
+            const StageLaunch &L = p->launches[li];
+            const int s = L.s0, ks = 1;
+            if (trace && r == reps + 2 && L.s1 - L.s0 > 1) {      // chain: span of the launch (per-CTA stamps cover its first tile only)
                 SACB_CUDA(cudaStreamSynchronize(h->stream));
-                const int ks = std::max(1, p->stages[s].ksplit);
-                const int grid = std::max(1, p->stages[s].n_tiles * h->cfg.n_agents) * ks;
+                const int g = std::min(L.grid, 4096);
+                SACB_CUDA(cudaMemcpy(h_trace.data(), d_trace, sizeof(unsigned long long) * kTraceSlots * g, cudaMemcpyDeviceToHost));
+                unsigned long long t0 = ~0ull, t5 = 0;
+                for (int b = 0; b < g; b++) { t0 = std::min(t0, h_trace[b * kTraceSlots]); t5 = std::max(t5, h_trace[b * kTraceSlots + 5]); }
+                fprintf(stderr, "[trace] stages %2d-%2d chain cluster %d grid %4d span %6.2f us\n", L.s0, L.s1 - 1, L.cluster, L.grid, (t5 - t0) * 1e-3);
+                SACB_CUDA(cudaMemset(d_trace, 0, sizeof(unsigned long long) * kTraceSlots * 4096));
+            } else if (trace && r == reps + 2) {
+                SACB_CUDA(cudaStreamSynchronize(h->stream));
+                const int grid = std::max(1, p->stages[s].n_tiles * h->cfg.n_agents);
                 SACB_CUDA(cudaMemcpy(h_trace.data(), d_trace, sizeof(unsigned long long) * kTraceSlots * std::min(grid, 4096), cudaMemcpyDeviceToHost));
                 double a[8] = {0}, mx_tile = 0, mx_main = 0; unsigned long long t0 = ~0ull, t0max = 0, t5 = 0;
                 const int g = std::min(grid, 4096);
@@ -1298,8 +1512,8 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
                     mx_tile = std::max(mx_tile, (double)(q[4] - q[1]));
                     if (p->stage_has_gemm[s]) { a[2] += (double)(q[2] - q[1]); a[3] += (double)(q[3] - q[2]); mx_main = std::max(mx_main, (double)(q[2] - q[1])); }
                 }
-                fprintf(stderr, "[trace] stage %2d ksplit %d grid %4d gemm %d span %6.2f us start-skew %5.2f | per-CTA avg: setup %.2f mainloop %.2f (max %.2f) epilogue %.2f tile %.2f (max %.2f) teardown %.2f\n",
-                        s, ks, grid, p->stage_has_gemm[s], (t5 - t0) * 1e-3, (t0max - t0) * 1e-3, a[1] / g * 1e-3, a[2] / g * 1e-3, mx_main * 1e-3, a[3] / g * 1e-3,
+                fprintf(stderr, "[trace] stage %2d grid %4d gemm %d span %6.2f us start-skew %5.2f | per-CTA avg: setup %.2f mainloop %.2f (max %.2f) epilogue %.2f tile %.2f (max %.2f) teardown %.2f\n",
+                        s, grid, p->stage_has_gemm[s], (t5 - t0) * 1e-3, (t0max - t0) * 1e-3, a[1] / g * 1e-3, a[2] / g * 1e-3, mx_main * 1e-3, a[3] / g * 1e-3,
                         a[4] / g * 1e-3, mx_tile * 1e-3, a[5] / g * 1e-3);
                 {   // slowest tile of every task of the stage (which task sets the span)
                     const Stage &sg = p->stages[s];
@@ -1314,14 +1528,14 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
                     fprintf(stderr, "\n");
                 }
                 if (p->stage_has_gemm[s]) {      // k-block timeline of CTA 0: TMA issue / arrival times relative to the end of setup
-                  for (int cta = 0; cta < std::min(ks, 2); cta++) {
+                  for (int cta = 0; cta < 1; cta++) {
                     const unsigned long long *q = &h_trace[cta * kTraceSlots];
                     fprintf(stderr, "[trace]   cta%d issue:", cta);
                     for (int kb = 0; kb < 16 && q[16 + kb] >= q[1]; kb++) fprintf(stderr, " %.2f", (q[16 + kb] - q[1]) * 1e-3);
                     fprintf(stderr, " | arrive:");
                     for (int kb = 0; kb < 16 && q[32 + kb] >= q[1]; kb++) fprintf(stderr, " %.2f", (q[32 + kb] - q[1]) * 1e-3);
-                    fprintf(stderr, " | accum %.2f staged %.2f cluster-sync %.2f reduced %.2f stored %.2f epi-end %.2f\n", (q[6] - q[1]) * 1e-3, (q[7] - q[1]) * 1e-3,
-                            q[48] > q[1] ? (q[48] - q[1]) * 1e-3 : 0.0, q[49] > q[1] ? (q[49] - q[1]) * 1e-3 : 0.0, (q[8] - q[1]) * 1e-3, (q[3] - q[1]) * 1e-3);
+                    fprintf(stderr, " | accum %.2f staged %.2f stored %.2f epi-end %.2f\n", (q[6] - q[1]) * 1e-3, (q[7] - q[1]) * 1e-3,
+                            (q[8] - q[1]) * 1e-3, (q[3] - q[1]) * 1e-3);
                   }
                     SACB_CUDA(cudaMemset(d_trace, 0, sizeof(unsigned long long) * kTraceSlots * 4096));
                 }
@@ -1329,12 +1543,12 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
         }
         SACB_CUDA(cudaStreamSynchronize(h->stream));
         if (r >= 3)
-            for (int s = 0; s < (int)p->stages.size(); s++) { float ms; cudaEventElapsedTime(&ms, ev[s], ev[s + 1]); acc[s] += ms * 1000.f / reps; }
+            for (int li = 0; li < nl; li++) { float ms; cudaEventElapsedTime(&ms, ev[li], ev[li + 1]); acc[li] += ms * 1000.f / reps; }
     }
     for (int s = 0; s < n; s++) us_out[s] = acc[s];
     if (getenv("SACB_TIMELINE")) {
-        // stage timeline of ONE graph replay as the update really runs (PDL, graph): per stage the earliest CTA start, the
-        // earliest release from griddepcontrol.wait and the latest CTA end, from %globaltimer
+        // launch timeline of ONE graph replay as the update really runs (PDL, graph): per launch the earliest CTA start, the
+        // earliest release from griddepcontrol.wait and the latest CTA end, from %globaltimer (stored under the launch's first stage)
         const int ns = (int)p->stages.size();
         unsigned long long *d_tl = nullptr;
         SACB_CUDA(cudaMalloc(&d_tl, sizeof(unsigned long long) * 4 * ns));
@@ -1344,7 +1558,7 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
         cudaGraph_t g = nullptr; cudaGraphExec_t ge = nullptr;
         SACB_CUDA(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
         int rc3 = SACB_OK;
-        for (int s = 0; s < ns && rc3 == SACB_OK; s++) rc3 = launch_stage(h, *p, s, h->use_pdl != 0);
+        for (int li = 0; li < nl && rc3 == SACB_OK; li++) rc3 = launch_stage(h, *p, li, h->use_pdl != 0);
         SACB_CUDA(cudaStreamEndCapture(h->stream, &g));
         p->prog.timeline = nullptr;
         if (rc3 == SACB_OK && cudaGraphInstantiate(&ge, g, 0) == cudaSuccess) {
@@ -1356,11 +1570,13 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
             }
             SACB_CUDA(cudaMemcpy(tl.data(), d_tl, sizeof(unsigned long long) * 4 * ns, cudaMemcpyDeviceToHost));
             const unsigned long long t0 = tl[0];
-            fprintf(stderr, "[timeline] stage: first-CTA-start  dependency-release  last-CTA-end | release-after-prev-end  release-to-end  (us, graph replay with PDL)\n");
-            for (int s = 0; s < ns; s++)
-                fprintf(stderr, "[timeline] %2d  %8.2f %8.2f %8.2f | %6.2f %6.2f\n", s, (tl[4 * s] - t0) * 1e-3, (tl[4 * s + 1] - t0) * 1e-3, (tl[4 * s + 2] - t0) * 1e-3,
-                        s ? ((double)tl[4 * s + 1] - (double)tl[4 * (s - 1) + 2]) * 1e-3 : 0.0, (tl[4 * s + 2] - tl[4 * s + 1]) * 1e-3);
-            fprintf(stderr, "[timeline] update = %.2f us\n", (tl[4 * (ns - 1) + 2] - t0) * 1e-3);
+            fprintf(stderr, "[timeline] stages: first-CTA-start  dependency-release  last-CTA-end | release-after-prev-end  release-to-end  (us, graph replay with PDL)\n");
+            for (int li = 0; li < nl; li++) {
+                const int s = p->launches[li].s0, sp = li ? p->launches[li - 1].s0 : 0;
+                fprintf(stderr, "[timeline] %2d-%2d  %8.2f %8.2f %8.2f | %6.2f %6.2f\n", s, p->launches[li].s1 - 1, (tl[4 * s] - t0) * 1e-3, (tl[4 * s + 1] - t0) * 1e-3, (tl[4 * s + 2] - t0) * 1e-3,
+                        li ? ((double)tl[4 * s + 1] - (double)tl[4 * sp + 2]) * 1e-3 : 0.0, (tl[4 * s + 2] - tl[4 * s + 1]) * 1e-3);
+            }
+            fprintf(stderr, "[timeline] update = %.2f us\n", (tl[4 * p->launches[nl - 1].s0 + 2] - t0) * 1e-3);
             cudaGraphExecDestroy(ge);
         }
         if (g) cudaGraphDestroy(g);
@@ -1371,8 +1587,8 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
         // printed relative to its own start (slot 9, right after the grid barrier)
         int a = 1, b = 4;
         sscanf(getenv("SACB_TRACE_RANGE"), "%d,%d", &a, &b);
-        int tc_setup = 1; uint64_t seed = h->cfg.seed; Stage single = p->stages[a];
-        void *args[] = {(void *)&p->prog, (void *)&single, (void *)&a, (void *)&b, (void *)&tc_setup, (void *)&seed};
+        int tc_setup = 1, chained = 0; uint64_t seed = h->cfg.seed; Stage single = p->stages[a];
+        void *args[] = {(void *)&p->prog, (void *)&single, (void *)&a, (void *)&b, (void *)&tc_setup, (void *)&chained, (void *)&seed};
         int grid = 1;
         for (int s = a; s < b; s++) grid = std::max(grid, p->stages[s].n_tiles);
         grid = std::min(grid, h->sm_count);
@@ -1394,8 +1610,8 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
     }
     if (trace) { p->prog.trace = nullptr; cudaFree(d_trace); }
     for (auto &e : ev) cudaEventDestroy(e);
-    h->kernel_launches += (int64_t)(reps + 3) * p->stages.size();
-    return (int)p->stages.size();
+    h->kernel_launches += (int64_t)(reps + 3) * nl;
+    return nl;
 }
 
 namespace sacb {
@@ -1406,6 +1622,7 @@ static const KernelVariant kVariants[kNumKernelVariants] = {
 #undef X
 };
 bool variant_has_gemm(int v) { return (kVariants[v].types & tb(T_GEMM)) != 0; }
+bool variant_can_chain(int v) { return variant_chains(SACB_MATH_BF16X3, kVariants[v].types, kVariants[v].epis); }
 int variant_blocks_per_sm(int v) { return variant_min_blocks(kVariants[v].types, kVariants[v].epis); }
 int pick_variant(uint32_t types, uint32_t epis, bool allow_light_colsum) {
     int best = 0, best_bits = 1 << 30;
