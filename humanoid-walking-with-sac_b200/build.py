@@ -22,7 +22,7 @@ def _newer(src_paths, target):
 
 def build(force=False, verbose=False):
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    extra = os.environ.get("SACB_EXTRA_NVCC", "").split()       # experiment switches, e.g. -DSACB_EXP_ONE_MMA
+    extra = os.environ.get("SACB_EXTRA_NVCC", "").split()       # extra nvcc flags, e.g. -DSOME_MACRO
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", "sacb200.h")]
     if not force and not _newer(deps, LIB):
         return LIB

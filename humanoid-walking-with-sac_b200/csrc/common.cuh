@@ -102,9 +102,7 @@ enum Epilogue : int32_t {
     EPI_F32 = 0,         // C[fp32] = acc (+ bias[n])
     EPI_BIAS_RELU,       // PM  = relu(acc + bias[n])
     EPI_MASK,            // PM  = acc * (mask_hi[m,n] > 0)
-    EPI_ADAM,            // acc = dW tile: Adam on W (+ Polyak into Wt, + shadow PM refresh, + optional grad export)
-    EPI_SAMPLE           // policy heads: C[fp32] = acc + bias (mean | log_std_raw), then the tanh-Gaussian sample + log-prob of
-                         // the tile's rows (the T_SAMPLE task fused into the heads GEMM; its arguments sit in the generic slots)
+    EPI_ADAM             // acc = dW tile: Adam on W (+ Polyak into Wt, + shadow PM refresh, + optional grad export)
 };
 
 struct AdamArgs {
@@ -149,7 +147,7 @@ struct alignas(64) Task {
 // spills in the forward / element-wise stages) and the instruction footprint of a 3-10 us kernel small.  X(index, task types, epilogues);
 // the host picks the smallest variant that covers a stage, variant 0 (everything) runs the persistent single-launch mode.
 constexpr uint32_t tb(int t) { return 1u << t; }
-constexpr uint32_t kAllTypes = (1u << (T_LN_BWD + 1)) - 1, kAllEpis = (1u << (EPI_SAMPLE + 1)) - 1;
+constexpr uint32_t kAllTypes = (1u << (T_LN_BWD + 1)) - 1, kAllEpis = (1u << (EPI_ADAM + 1)) - 1;
 // everything the reference architecture needs: the single persistent launch of a handle without LayerNorm does not carry the
 // LayerNorm tasks (their code alone cost the everything-build 0.265 -> 0.302 ms per update)
 constexpr uint32_t kBaseTypes = kAllTypes & ~((1u << T_LN_FWD) | (1u << T_LN_BWD));

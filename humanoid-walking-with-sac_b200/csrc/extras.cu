@@ -30,7 +30,7 @@ __device__ __forceinline__ float block_sum(float v, float *red) {
 }
 
 // one CTA per input row: y = W_out . relu(... relu(W_0 x + b_0) ...) + b_out ; warp-per-output-row dot products,
-// activations in shared memory (2 x hidden floats + in_dim).  B = 1 is the select_action latency path (sac_imp.py:54-72).
+// activations in shared memory (2 x hidden floats + in_dim).  Used by the QNetwork / GaussianPolicy callables.
 __global__ void __launch_bounds__(512) mlp_rows_kernel(MlpArgs a, const float *x, int ldx, const float *x2, int n2, float *out, int ldo) {
     extern __shared__ float sm[];
     float *cur = sm, *nxt = sm + max(a.in_dim, a.hidden);
@@ -70,18 +70,6 @@ __global__ void __launch_bounds__(512) mlp_rows_kernel(MlpArgs a, const float *x
         s = warp_sum(s);
         if (lane == 0) out[(int64_t)row * ldo + o] = s + __ldg(a.b_out + o);
     }
-}
-
-// head_raw [n, 2A] -> action [n, A]: evaluate => tanh(mean)*scale+bias (sac_imp.py:61-64), else policy.sample (:70)
-__global__ void action_kernel(const float *head, const float *eps, int n, int A, int evaluate, float scale, float bias, float *act,
-                              uint64_t seed, uint32_t counter) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n * A) return;
-    const int r = i / A, c = i % A;
-    const float mean = head[(int64_t)r * 2 * A + c], ls = head[(int64_t)r * 2 * A + A + c];
-    if (evaluate) { act[i] = tanhf(mean) * scale + bias; return; }
-    const float e = eps ? eps[i] : philox_normal(seed, 0x5e1ec7u, counter, (uint32_t)r, (uint32_t)c);
-    act[i] = sample_elem(mean, ls, e, scale, bias).action;
 }
 
 static MlpArgs mlp_args(sacb_handle h, int agent, int net) {
@@ -153,6 +141,7 @@ __global__ void __launch_bounds__(256) ln_relu_rows_kernel(float *y, int ldy, in
     for (int o = threadIdx.x; o < H; o += blockDim.x) yr[o] = fmaxf((__ldcg(yr + o) - mean) * rstd * __ldcg(g + ao + o) + __ldcg(be + ao + o), 0.f);
 }
 
+// head_raw [n, 2A] -> action [n, A]: evaluate => tanh(mean)*scale+bias (sac_imp.py:61-64), else policy.sample (:70)
 __global__ void action_pdl_kernel(const float *head, const float *eps, int n, int A, int evaluate, float scale, float bias, float *act, uint64_t seed, uint32_t counter) {
     asm volatile("griddepcontrol.wait;" ::: "memory");
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -224,27 +213,8 @@ static int select_action_rows(sacb_handle h, int agent0, int rows, int rows_per_
 }
 }  // namespace sacb
 
-// the first version (one CTA walks the whole policy, pageable copies), kept behind SACB_ACT_SINGLE_CTA=1 for A/B timing
-static int select_action_single_cta(sacb_handle h, int agent, const float *obs, int evaluate, const float *eps, float *action_out) {
-    const int O = h->cfg.obs_dim, A = h->cfg.act_dim;
-    float *d_obs = h->stage_rows, *d_head = d_obs + align_up(O, 4), *d_eps = d_head + align_up(2 * A, 4), *d_act = d_eps + align_up(A, 4);
-    SACB_CUDA(cudaMemcpyAsync(d_obs, obs, sizeof(float) * O, cudaMemcpyHostToDevice, h->stream));
-    if (eps && !evaluate) SACB_CUDA(cudaMemcpyAsync(d_eps, eps, sizeof(float) * A, cudaMemcpyHostToDevice, h->stream));
-    MlpArgs a = mlp_args(h, agent, SACB_NET_POLICY);
-    mlp_rows_kernel<<<1, 512, mlp_smem(a), h->stream>>>(a, d_obs, O, nullptr, 0, d_head, 2 * A);
-    action_kernel<<<1, std::max(32, (A + 31) / 32 * 32), 0, h->stream>>>(d_head, (eps && !evaluate) ? d_eps : nullptr, 1, A, evaluate, h->cfg.action_scale,
-                                                                        h->cfg.action_bias, d_act, h->cfg.seed, h->act_counter++);
-    h->kernel_launches += 2;
-    SACB_CUDA(cudaGetLastError());
-    SACB_CUDA(cudaMemcpyAsync(action_out, d_act, sizeof(float) * A, cudaMemcpyDeviceToHost, h->stream));
-    SACB_CUDA(cudaStreamSynchronize(h->stream));
-    return SACB_OK;
-}
-
 extern "C" int sacb_select_action(sacb_handle h, int agent, const float *obs, int evaluate, const float *eps, float *action_out) {
     if (!h || !obs || !action_out || agent < 0 || agent >= h->cfg.n_agents) return fail(SACB_ERR_ARG, "bad argument");
-    static const bool single = getenv("SACB_ACT_SINGLE_CTA") != nullptr;
-    if (single) return select_action_single_cta(h, agent, obs, evaluate, eps, action_out);
     return select_action_rows(h, agent, 1, 1, obs, evaluate, eps, action_out);
 }
 
@@ -354,7 +324,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_selftest_kernel(const Task *
         st.tmem_base = s_tmem;
     }
     for (int tile = blockIdx.x; tile < t.n_tiles; tile += gridDim.x) {
-        if (kTc) gemm_tile_tc(t, tp, tile, bases, 0, nullptr, st, error_flag, false, 0ull);
+        if (kTc) gemm_tile_tc(t, tp, tile, bases, 0, nullptr, st, error_flag, false);
         else gemm_tile_ffma(t, tile, bases, 0, nullptr, reinterpret_cast<float *>(smem_raw));
     }
     if (kTc) { tc::tc_fence_before(); __syncthreads(); if (threadIdx.x < 32) tc::tmem_dealloc(st.tmem_base, kTN); }
@@ -372,7 +342,7 @@ namespace sacb {
 __global__ void __launch_bounds__(stream::kThreads, 1) stream_selftest_kernel(const __grid_constant__ Program P, const __grid_constant__ Stage stage) {
     extern __shared__ __align__(1024) uint8_t smem_stream[];
     if ((tc::smem_u32(smem_stream) & 1023u) != 0) { if (threadIdx.x == 0) atomicExch(P.error_flag, 3); return; }
-    stream::gemm_stage(P, stage, smem_stream, 0ull);
+    stream::gemm_stage(P, stage, smem_stream);
 }
 }  // namespace sacb
 

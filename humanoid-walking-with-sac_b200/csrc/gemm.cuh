@@ -5,7 +5,6 @@
 // Both compute  C[M,N] = epilogue( A[M,K] * B[N,K]^T )  for one output tile of a Task.
 #pragma once
 #include "common.cuh"
-#include "sample.cuh"
 
 namespace sacb {
 
@@ -335,9 +334,8 @@ __device__ __forceinline__ void trace_stamp(unsigned long long *trace, int slot)
 
 // The B operand of a forward / dX GEMM is a weight shadow that nothing the tile waits for writes, while its A operand (activations,
 // gradients) is what the tile waits for: the first K blocks of B are requested here, from the current ring position, so that after
-// the wait only the A halves still have to cross the SM's L2 port -- the tile is bound by exactly that ingest.  Callers: a staged
-// launch before griddepcontrol.wait (Task::i[6], set by the host builder), and a chained launch before the cluster barrier that
-// ends the previous layer (the previous tile's epilogue is done with the ring by then).
+// the wait only the A halves still have to cross the SM's L2 port -- the tile is bound by exactly that ingest.  Caller: a chained
+// launch, before the cluster barrier that ends the previous layer (the previous tile's epilogue is done with the ring by then).
 __device__ __forceinline__ void tc_prefetch_b(const Task &t, const Task *tg, int tile, int agent, TcState &st, int *error_flag) {
     st.b_pre = 0;
     if ((threadIdx.x >> 5) != 0) return;
@@ -408,13 +406,9 @@ __device__ __forceinline__ int tc_mainloop(const Task &t, int m0, int n0, int ag
                     const uint64_t da_hi = make_desc(sa + kk * a_kstep, a_lbo), da_lo = make_desc(sa + a_lo + kk * a_kstep, a_lbo);
                     const uint64_t db_hi = make_desc(sb + kk * b_kstep, b_lbo), db_lo = make_desc(sb + b_lo + kk * b_kstep, b_lbo);
                     // small terms first: a_lo*b_hi + a_hi*b_lo, then a_hi*b_hi
-#ifdef SACB_EXP_ONE_MMA      // timing experiment only (wrong numerics): is the K loop bound by MMA issue or by operand ingest?
-                    umma_bf16(st.tmem_base, da_hi, db_hi, idesc, (kb | kk) ? 1u : 0u);
-#else
                     umma_bf16(st.tmem_base, da_lo, db_hi, idesc, (kb | kk) ? 1u : 0u);
                     umma_bf16(st.tmem_base, da_hi, db_lo, idesc, 1u);
                     umma_bf16(st.tmem_base, da_hi, db_hi, idesc, 1u);
-#endif
                 }
                 umma_commit(&st.empty_bar[s]);                 // implies tcgen05.fence::before_thread_sync
                 if (kb == nkb - 1) umma_commit(st.accum_bar);
@@ -645,41 +639,8 @@ __device__ __forceinline__ void epilogue_rows4(const EpiR &e, const int (&m)[R],
     }
 }
 
-// EPI_SAMPLE phase 2: the staging tile holds the raw head outputs (no bias) of rows [m0, m0 + bm) x 2A columns.  One warp per row
-// (lane = action component, A <= 32): head_raw = acc + bias, then exactly the arithmetic of task_sample.
-//   generic slots as T_SAMPLE: p1=eps [2B,A] (i4: 1 -> Philox draw, kept for the backward) ; pm0 = X PM ; p3=logp [2B] ;
-//   i0=B i1=A i2=obs ; f0=scale f1=bias
-struct SampleEpi {
-    float *head, *eps, *logp; const float *bias; Pm X;
-    int B, A, obs, device_eps; float scale, abias; uint32_t step, agent; uint64_t seed;
-};
-__device__ __forceinline__ void sample_epilogue_tile(const SampleEpi &e, const float *Cs, int m0, int bm, const float (&pre_eps)[8], float b_mean, float b_ls) {
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        const int row = warp + 16 * i, j = m0 + row;
-        if (row >= bm || j >= 2 * e.B) continue;      // warp-uniform
-        float lp = 0.f;
-        if (lane < e.A) {
-            const float mean = Cs[row * kCsLd + lane] + b_mean, ls = Cs[row * kCsLd + e.A + lane] + b_ls;
-            e.head[(int64_t)j * 2 * e.A + lane] = mean;
-            e.head[(int64_t)j * 2 * e.A + e.A + lane] = ls;
-            float ev = pre_eps[i];
-            if (e.device_eps) {
-                ev = philox_normal(e.seed, e.agent, e.step, (uint32_t)j, (uint32_t)lane);
-                e.eps[(int64_t)j * e.A + lane] = ev;
-            }
-            const SampleElem s = sample_elem(mean, ls, ev, e.scale, e.abias);
-            pm_store(e.X, j < e.B ? j : 2 * e.B + (j - e.B), e.obs + lane, s.action);
-            lp = s.logp;
-        }
-        lp = warp_sum(lp);
-        if (lane == 0) e.logp[j] = lp;
-    }
-}
-
 template <int EPI>
-__device__ __forceinline__ void tc_epilogue(const EpiR &epi, int m0, int n0, int bm, int bn, TcState &st, int nkb_mine, int *error_flag, bool traced, const SampleEpi *se = nullptr) {
+__device__ __forceinline__ void tc_epilogue(const EpiR &epi, int m0, int n0, int bm, int bn, TcState &st, int nkb_mine, int *error_flag, bool traced) {
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     float *Cs = reinterpret_cast<float *>(st.tiles);      // staging tile [kTM][kCsLd] over operand stage 0 (all MMAs have retired)
     // phase-2 mapping: bn / 4 threads cover a row (4 columns each); the 512 threads cover 32 (bn = 64) or 64 (bn = 32) rows per
@@ -688,19 +649,7 @@ __device__ __forceinline__ void tc_epilogue(const EpiR &epi, int m0, int n0, int
     const int c4 = (tid % ct) * 4, r0 = tid / ct;
     int m[4];
     float aux[4][4];
-    float pre_eps[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, pre_b0 = 0.f, pre_b1 = 0.f;
-    if (EPI == EPI_SAMPLE) {      // head biases and (injected-eps mode) the draws of this warp's rows
-        if (lane < se->A) {
-            pre_b0 = ldcg(se->bias + lane); pre_b1 = ldcg(se->bias + se->A + lane);
-            if (!se->device_eps) {
-#pragma unroll
-                for (int i = 0; i < 8; i++) {
-                    const int j = m0 + warp + 16 * i;
-                    if (warp + 16 * i < bm && j < 2 * se->B) pre_eps[i] = ldcg(se->eps + (int64_t)j * se->A + lane);
-                }
-            }
-        }
-    } else if (EPI != EPI_ADAM) {
+    if (EPI != EPI_ADAM) {
 #pragma unroll
         for (int i = 0; i < 4; i++) {
             const int row = rs * i + r0;
@@ -735,8 +684,6 @@ __device__ __forceinline__ void tc_epilogue(const EpiR &epi, int m0, int n0, int
     if (traced && tid == 64) trace_stamp(st.trace, 7);
     if (EPI == EPI_ADAM) {
         adam_epilogue_tile(epi, Cs, m0, n0, bm);
-    } else if (EPI == EPI_SAMPLE) {
-        sample_epilogue_tile(*se, Cs, m0, bm, pre_eps, pre_b0, pre_b1);
     } else {   // phase 2: the staged accumulators of the thread's rows meet the prefetched auxiliary operands
         float4 acc[4];
 #pragma unroll
@@ -757,7 +704,7 @@ __device__ __forceinline__ void tc_epilogue(const EpiR &epi, int m0, int n0, int
 // t = shared-memory copy of the task (fields), tg = the task in global memory (TMA descriptors)
 template <uint32_t kEpis = kAllEpis>
 __device__ __forceinline__ void gemm_tile_tc(const Task &t, const Task *tg, int tile, const AgentBases &bases, int agent,
-                                             const float *scalars, tc::TcState &st, int *error_flag, bool first_tile, uint64_t seed) {
+                                             const float *scalars, tc::TcState &st, int *error_flag, bool first_tile) {
     using namespace tc;
     st.tmA = &tg->tmA; st.tmB = &tg->tmB;
     const int tm = tile / t.tiles_n, tn = tile % t.tiles_n;
@@ -771,14 +718,6 @@ __device__ __forceinline__ void gemm_tile_tc(const Task &t, const Task *tg, int 
         case EPI_F32: if constexpr ((kEpis & tb(EPI_F32)) != 0) tc_epilogue<EPI_F32>(epi, m0, n0, t.bm, t.bn, st, nkb_mine, error_flag, traced); break;
         case EPI_BIAS_RELU: if constexpr ((kEpis & tb(EPI_BIAS_RELU)) != 0) tc_epilogue<EPI_BIAS_RELU>(epi, m0, n0, t.bm, t.bn, st, nkb_mine, error_flag, traced); break;
         case EPI_MASK: if constexpr ((kEpis & tb(EPI_MASK)) != 0) tc_epilogue<EPI_MASK>(epi, m0, n0, t.bm, t.bn, st, nkb_mine, error_flag, traced); break;
-        case EPI_SAMPLE: if constexpr ((kEpis & tb(EPI_SAMPLE)) != 0) {
-            SampleEpi se;
-            se.head = epi.C; se.bias = epi.bias; se.eps = resolve(t.p[1], bases, agent); se.logp = resolve(t.p[3], bases, agent);
-            se.X = resolve_pm(t.pm[0], bases, agent);
-            se.B = t.i[0]; se.A = t.i[1]; se.obs = t.i[2]; se.device_eps = t.i[4]; se.scale = t.f[0]; se.abias = t.f[1];
-            se.step = (uint32_t)__float_as_int(ldcg(scalars + SC_N_UPDATES)); se.agent = (uint32_t)agent; se.seed = seed;
-            tc_epilogue<EPI_SAMPLE>(epi, m0, n0, t.bm, t.bn, st, nkb_mine, error_flag, traced, &se);
-        } break;
         default: if constexpr ((kEpis & tb(EPI_ADAM)) != 0) tc_epilogue<EPI_ADAM>(epi, m0, n0, t.bm, t.bn, st, nkb_mine, error_flag, traced); break;
     }
     stamp(3);

@@ -116,7 +116,6 @@ struct ProgramInst {
     int64_t step_graph_n = -1, step_graph_k = -1;
     bool step_graph_failed = false;
     int step_graph_launches = 0;
-    bool step_graph_fused = false;       // which form of the sampler the capture recorded (sacb_handle_s::per_fused)
     int n_tiles_total = 0, max_stage_tiles = 0;
     int kernels_per_step = 0;
 };
@@ -127,7 +126,6 @@ struct sacb_handle_s {
     sacb_config cfg;
     int sm_count = 0;
     cudaStream_t stream = nullptr;
-    bool per_fused = false;              // the last prioritized sample ran chunk pass + search as one launch (where its flagged count is kept)
     cudaStream_t stream2 = nullptr;      // prioritized replay work that overlaps the update (sacb_per_step)
     cudaEvent_t ev_td = nullptr, ev_sampled = nullptr;
     int64_t sample_k = 0;                // rows of the minibatch the last prioritized sample left on the device (0: none)

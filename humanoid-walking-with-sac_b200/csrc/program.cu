@@ -15,10 +15,6 @@
 #include "tasks.cuh"
 #include "stream.cuh"
 
-#ifndef SACB_NO_OUTLINE
-#define SACB_NO_OUTLINE 1   // outlining measured SLOWER on B200 (persistent 0.265 -> 0.278 ms, one-kernel staged 0.242 -> 0.250): kept as an experiment switch
-#endif
-
 namespace sacb {
 
 // ================================================================================================================
@@ -174,24 +170,6 @@ __device__ __forceinline__ void grid_barrier(unsigned int *counter, unsigned int
     tc::fence_proxy_async();
 }
 
-// The build that carries every code path (variant 0: the single persistent launch) calls its task bodies through NON-inlined
-// functions, one per task type / GEMM epilogue: each body then gets its own register allocation and schedule (as in the per-stage
-// builds) instead of sharing the union of everybody's live ranges, which put spills into the MMA issue loop and the Adam epilogue.
-template <uint32_t kEpi>
-__device__ __noinline__ void gemm_tile_tc_outlined(const Task &t, const Task *tg, int tile, const AgentBases &bases, int agent, const float *scalars,
-                                                   tc::TcState &st, int *error_flag, bool first_tile, uint64_t seed) {
-    gemm_tile_tc<kEpi>(t, tg, tile, bases, agent, scalars, st, error_flag, first_tile, seed);
-}
-__device__ __noinline__ void task_shadow_outlined(const Task &t, int tile, const Program &P, int agent) { task_shadow(t, tile, P, agent); }
-__device__ __noinline__ void task_gather_outlined(const Task &t, int tile, const Program &P, int agent, const float *scalars, uint64_t seed) { task_gather(t, tile, P, agent, scalars, seed); }
-__device__ __noinline__ void task_sample_outlined(const Task &t, int tile, const Program &P, int agent, const float *scalars, uint64_t seed) { task_sample(t, tile, P, agent, scalars, seed); }
-__device__ __noinline__ void task_target_loss_outlined(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) { task_target_loss(t, tile, P, agent, scalars, smem); }
-__device__ __noinline__ void task_actor_loss_outlined(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) { task_actor_loss(t, tile, P, agent, scalars, smem); }
-__device__ __noinline__ void task_sample_bwd_outlined(const Task &t, int tile, const Program &P, int agent, const float *scalars) { task_sample_bwd(t, tile, P, agent, scalars); }
-__device__ __noinline__ void task_out_adam_outlined(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) { task_out_adam(t, tile, P, agent, scalars, smem); }
-__device__ __noinline__ void task_bias_adam_outlined(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) { task_bias_adam(t, tile, P, agent, scalars, smem); }
-__device__ __noinline__ void task_finish_outlined(const Task &t, const Program &P, int agent, float *scalars, float *smem) { task_finish(t, P, agent, scalars, smem); }
-
 // Between two layers of a chained launch: the epilogue's global stores (generic proxy) become visible to the TMA reads (async proxy)
 // of the other CTAs of the cluster, which own the rest of the row block.  A chain of one-CTA clusters only orders its own CTA.
 __device__ __forceinline__ void chain_barrier(uint32_t cluster_size) {
@@ -290,35 +268,10 @@ sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Sta
     auto run_task = [&](const Task *tg, int tile, int agent, bool first) {
         const Task &t = s_task;
         float *scalars = resolve(P.scalars, P.bases, agent);
-        constexpr bool kOutlined = kTc && (kTypes & kBaseTypes) == kBaseTypes && kEpis == kAllEpis && !SACB_NO_OUTLINE;
-        if constexpr (kOutlined) {
-            switch (t.type) {
-                case T_GEMM:
-                    switch (t.epi) {
-                        case EPI_F32: gemm_tile_tc_outlined<tb(EPI_F32)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
-                        case EPI_BIAS_RELU: gemm_tile_tc_outlined<tb(EPI_BIAS_RELU)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
-                        case EPI_MASK: gemm_tile_tc_outlined<tb(EPI_MASK)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
-                        case EPI_SAMPLE: gemm_tile_tc_outlined<tb(EPI_SAMPLE)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
-                        default: gemm_tile_tc_outlined<tb(EPI_ADAM)>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed); break;
-                    }
-                    break;
-                case T_SHADOW: task_shadow_outlined(t, tile, P, agent); break;
-                case T_GATHER: task_gather_outlined(t, tile, P, agent, scalars, seed); break;
-                case T_SAMPLE: task_sample_outlined(t, tile, P, agent, scalars, seed); break;
-                case T_TARGET_LOSS: task_target_loss_outlined(t, tile, P, agent, scalars, s_red); break;
-                case T_ACTOR_LOSS: task_actor_loss_outlined(t, tile, P, agent, scalars, s_red); break;
-                case T_SAMPLE_BWD: task_sample_bwd_outlined(t, tile, P, agent, scalars); break;
-                case T_OUT_ADAM: task_out_adam_outlined(t, tile, P, agent, scalars, s_red); break;
-                case T_BIAS_ADAM: task_bias_adam_outlined(t, tile, P, agent, scalars, s_red); break;
-                case T_FINISH: task_finish_outlined(t, P, agent, scalars, s_red); break;
-                case T_LN_FWD: task_ln_fwd(t, tile, P, agent); break;
-                case T_LN_BWD: task_ln_bwd(t, tile, P, agent); break;
-            }
-        } else
         switch (t.type) {      // only the task types of this build's mask are compiled in
             case T_GEMM:
                 if constexpr ((kTypes & tb(T_GEMM)) != 0) {
-                    if (kTc) gemm_tile_tc<kEpis>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first, seed);
+                    if (kTc) gemm_tile_tc<kEpis>(t, tg, tile, P.bases, agent, scalars, st, P.error_flag, first);
                     else gemm_tile_ffma(t, tile, P.bases, agent, scalars, reinterpret_cast<float *>(smem_raw));
                 }
                 break;
@@ -346,12 +299,7 @@ sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Sta
                 const int agent = wi / n_stage_tiles;
                 int tile;
                 const Task *tg = fetch_task(wi % n_stage_tiles, tile, wi == (int)blockIdx.x);
-                if (!dep_synced) {
-                    if constexpr (kTc && (kTypes & tb(T_GEMM)) != 0) {
-                        if (s_task.type == T_GEMM && s_task.i[6] && tc_setup && stage_end - stage_begin == 1) tc::tc_prefetch_b(s_task, tg, tile, agent, st, P.error_flag);
-                    }
-                    dep_sync();
-                }
+                dep_sync();
                 run_task(tg, tile, agent, wi == (int)blockIdx.x);
             }
             if (s + 1 < stage_end) {
@@ -418,13 +366,13 @@ sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Sta
 
 // throughput form of a stage that holds only GEMM tasks (stream.cuh): one resident CTA per SM, roles decoupled across tiles
 __global__ void __launch_bounds__(stream::kThreads, 1)
-sac_stream_kernel(const __grid_constant__ Program P, const __grid_constant__ Stage stage, const uint64_t seed) {
+sac_stream_kernel(const __grid_constant__ Program P, const __grid_constant__ Stage stage) {
     extern __shared__ __align__(1024) uint8_t smem_stream[];
     if ((tc::smem_u32(smem_stream) & 1023u) != 0) {      // SWIZZLE_128B operand tiles need 1024-byte alignment; the kernel owns all 227 KB
         if (threadIdx.x == 0) atomicExch(P.error_flag, 3);
         return;
     }
-    stream::gemm_stage(P, stage, smem_stream, seed);
+    stream::gemm_stage(P, stage, smem_stream);
 }
 
 // ================================================================================================================
@@ -449,7 +397,6 @@ struct Builder {
     int rc = SACB_OK;
     // tensor-core tile shape per task index (bm, bn), decided by choose_tile_shapes() from a dry first pass; empty = defaults
     std::vector<std::pair<int, int>> shapes;
-    std::map<int64_t, int> shadow_writer;      // arena offset of a weight shadow PM -> last stage of THIS program that writes it
     bool dry = false;      // first pass: count tiles only, no TMA descriptors
     bool stream = false;   // throughput program: GEMM stages run on the stream kernel (it alone understands split-K tasks)
 
@@ -518,16 +465,6 @@ struct Builder {
         t.type = T_GEMM; t.M = M; t.N = N; t.K = K;
         t.A.pm = a.ref; t.A.mn_major = a_mn; t.A.r0 = 0; t.B.pm = b.ref; t.B.mn_major = b_mn; t.B.r0 = b_r0;
         const size_t idx = tasks.size();
-        {   // B = a weight shadow (arena PM) that no stage later than two back has written: may be requested before the grid-dependency
-            // wait (gemm.cuh: tc_prefetch_b).  Writers: T_SHADOW tasks and Adam epilogues; the stage right before may still be running
-            const int cur = (int)stages.size() - 1;
-            const bool in_arena = ((b.ref.base.v >> 62) & 1) == 0;
-            const auto w = shadow_writer.find(b.ref.base.v);
-            // (opt-in, SACB_EARLY_B=1: measured no gain on B200 -- 0.1990 vs 0.1984 ms -- because with one 193 KB CTA per SM only the
-            //  ~20 CTAs of a stage that land on SMs the previous stage left idle are resident before the release at all)
-            t.i[6] = (in_arena && !stream && (w == shadow_writer.end() || w->second <= cur - 2) && getenv("SACB_EARLY_B")) ? 1 : 0;
-            for (const PmRef *r : {&t.adam.shadow, &t.adam.shadow2}) if (!is_null(r->base)) shadow_writer[r->base.v] = cur;
-        }
         t.bm = idx < shapes.size() && shapes[idx].first ? shapes[idx].first : tm;
         t.bn = idx < shapes.size() && shapes[idx].second ? shapes[idx].second : tn;
         t.tiles_m = cdiv(M, t.bm); t.tiles_n = cdiv(N, t.bn);
@@ -635,7 +572,6 @@ struct Builder {
     void shadow_task(int net, int64_t w_off, const PmView &dst, int src_ld, int col0 = 0) {
         Task t = blank(T_SHADOW);
         t.p[0] = A(L.param[net] + w_off); t.pm[0] = dst.ref; t.i[0] = dst.rows; t.i[1] = dst.cols; t.i[2] = col0; t.i[3] = src_ld;
-        shadow_writer[dst.ref.base.v] = (int)stages.size() - 1;
         add(t, cdiv(dst.rows, kShadowRows));
     }
 
@@ -651,7 +587,7 @@ struct Builder {
     }
     std::vector<std::pair<int, int>> choose_tile_shapes(int wave) const {
         std::vector<std::pair<int, int>> out(tasks.size(), {0, 0});
-        if (!math_is_tc(h->cfg.math_mode) || getenv("SACB_FIXED_TILES")) return out;
+        if (!math_is_tc(h->cfg.math_mode)) return out;
         for (size_t si = 0; si < stages.size(); si++) {
             const Stage &sg = stages[si];
             if (!has_gemm[si]) continue;
@@ -674,7 +610,7 @@ struct Builder {
                 const Task &t = tasks[b.task];
                 int nbm = b.bm, nbn = b.bn;
                 if (b.bm == kTM && t.M > 64) nbm = 64;
-                else if (b.bn == kTN && !t.B.mn_major && t.epi != EPI_ADAM && t.epi != EPI_SAMPLE && t.N > 32) nbn = 32;
+                else if (b.bn == kTN && !t.B.mn_major && t.epi != EPI_ADAM && t.N > 32) nbn = 32;
                 else { b.frozen = true; continue; }
                 const int ntiles = cdiv(t.M, nbm) * cdiv(t.N, nbn);
                 if (total + (ntiles - b.tiles) * h->cfg.n_agents > wave) { b.frozen = true; continue; }
@@ -690,8 +626,8 @@ struct Builder {
     // columns (64 where the output is narrower than 96 columns: policy heads, dL/da).
     // A stage that would hold fewer than kStreamWideMin x SMs tiles of 128 x 128 keeps 64-column tiles: twice the tiles for the
     // round-robin over the resident CTAs (mid-size batches: better wave quantisation and more tiles to overlap per CTA).
+    static constexpr int kStreamWideMin = 3;
     std::vector<std::pair<int, int>> stream_tile_shapes() const {
-        static const int wide_min = getenv("SACB_STREAM_WIDE_MIN") ? atoi(getenv("SACB_STREAM_WIDE_MIN")) : 3;
         // 128 x 256 tiles (two 96 KB ring slots, both 256-column accumulators) where the stage still holds kStreamN256Min x SMs of them:
         // 0.75x the L2 -> SM operand traffic per flop of the 128 x 128 tile, which is what bounds a large-batch GEMM stage
         // (SACB_STREAM_N256_MIN: waves of 256-wide tiles a stage needs, 0 = never).  Not where a task of the stage has only a handful
@@ -715,7 +651,7 @@ struct Builder {
                     tiles_256 += t256;
                     all_many = all_many && 2 * t256 >= h->sm_count;
                 }
-            const bool wide = wide_tiles >= wide_min * h->sm_count;
+            const bool wide = wide_tiles >= kStreamWideMin * h->sm_count;
             const bool very_wide = n256_min > 0 && all_many && tiles_256 >= n256_min * h->sm_count;
             for (int k = stages[si].task_begin; k < stages[si].task_end; k++)
                 if (tasks[k].type == T_GEMM) out[k] = {stream::kBM, (very_wide && takes_256(tasks[k])) ? 256 : ((wide && tasks[k].N >= 96) ? stream::kBN : 64)};
@@ -793,24 +729,11 @@ struct Builder {
                 }
             }
             // ---- policy heads -> head_raw [2B, 2A] (fp32) ------------------------------------------------------------
-            // opt-in experiment (SACB_FUSE_SAMPLE=1, tensor-core math, 2A <= 64): the tanh-Gaussian sample + log-prob of both batches
-            // in the epilogue of the heads GEMM (EPI_SAMPLE, one stage less).  Correct (parity tests pass) but slower on B200: the
-            // heads GEMM has only 2B / 64 = 8 tiles, so 8 SMs do the transcendental-heavy sampling of 512 rows (13.8 us) that the
-            // separate stage spreads over 32 CTAs (4 us + 1 us stage boundary); profiles/r01_summary.md
-            const bool fuse_sample = math_is_tc(h->cfg.math_mode) && A2 <= kTN && getenv("SACB_FUSE_SAMPLE");
             begin_stage();
-            if (fuse_sample) {
-                Task t = epi_f32(W(L.head_raw), A2, A(L.param[0] + P.b_out));
-                t.epi = EPI_SAMPLE;
-                t.p[1] = W(L.eps); t.pm[0] = xrows(0, 3 * B, L.ldx).ref; t.p[3] = W(L.logp);
-                t.i[0] = B; t.i[1] = act; t.i[2] = obs; t.i[4] = key.device_eps;
-                t.f[0] = h->cfg.action_scale; t.f[1] = h->cfg.action_bias;
-                gemm(hview(L.hp[nh - 1], 2 * B, 0, 2), 0, wsh_head(), 0, 2 * B, A2, H, t);
-            } else {
-                gemm(hview(L.hp[nh - 1], 2 * B, 0, 2), 0, wsh_head(), 0, 2 * B, A2, H, epi_f32(W(L.head_raw), A2, A(L.param[0] + P.b_out)));
-            }
+            gemm(hview(L.hp[nh - 1], 2 * B, 0, 2), 0, wsh_head(), 0, 2 * B, A2, H, epi_f32(W(L.head_raw), A2, A(L.param[0] + P.b_out)));
             // ---- reparameterised sample + log-prob for both batches -------------------------------------------------
-            if (!fuse_sample) {
+            // (its own stage: in the heads GEMM's epilogue the sampling ran on that GEMM's 8 tiles and was slower, profiles/r01_summary.md)
+            {
                 begin_stage();
                 Task t = blank(T_SAMPLE);
                 t.p[0] = W(L.head_raw); t.p[1] = W(L.eps); t.pm[0] = xrows(0, 3 * B, L.ldx).ref; t.p[3] = W(L.logp);
@@ -1126,9 +1049,8 @@ int check_error_flag(sacb_handle h) {
 
 // one stage = one launch of the stream kernel, optional PDL
 static int launch_stream_stage(sacb_handle h, ProgramInst &p, int s, bool pdl) {
-    uint64_t seed = h->cfg.seed;
     Stage single = p.stages[s];
-    void *args[] = {(void *)&p.prog, (void *)&single, (void *)&seed};
+    void *args[] = {(void *)&p.prog, (void *)&single};
     cudaLaunchConfig_t cfg{};
     const int tiles = std::max(1, single.n_tiles * h->cfg.n_agents);
     cfg.gridDim = dim3(std::min(tiles, h->sm_count)); cfg.blockDim = dim3(stream::kThreads); cfg.dynamicSmemBytes = stream::kSmemBytes; cfg.stream = h->stream;
@@ -1156,10 +1078,8 @@ static int launch_stage(sacb_handle h, ProgramInst &p, int li, bool pdl) {
     int ctas = chain ? L.grid : std::max(1, single.n_tiles * h->cfg.n_agents);
     // population mode: a stage of many more tiles than SMs runs as one resident CTA per SM looping over tiles (barrier /
     // TMEM setup and teardown once per SM instead of once per tile); a single agent's stage (<= ~150 tiles) keeps one CTA per tile
-    static const int grid_cap = getenv("SACB_GRID_CAP") ? atoi(getenv("SACB_GRID_CAP")) : -1;     // 0 = never cap
-    const int cap = grid_cap < 0 ? h->sm_count : grid_cap;
-    if (!chain && cap > 0 && ctas > 2 * h->sm_count) {      // resident CTAs looping over tiles wi = blockIdx.x + i * gridDim.x
-        ctas = std::min(ctas, cap * (tc ? variant_blocks_per_sm(kind) : 1));
+    if (!chain && ctas > 2 * h->sm_count) {      // resident CTAs looping over tiles wi = blockIdx.x + i * gridDim.x
+        ctas = std::min(ctas, h->sm_count * (tc ? variant_blocks_per_sm(kind) : 1));
         // a grid that is a multiple of the stage's per-agent tile count keeps every CTA on ONE tile of ONE task across the agents it
         // walks: the task record is fetched once instead of once per tile (population mode: a column-sum stage holds 2-6 tasks)
         if (single.task_end - single.task_begin > 1 && single.n_tiles <= ctas / 2) ctas = (ctas / single.n_tiles) * single.n_tiles;
@@ -1249,7 +1169,7 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
         for (size_t s = 0; s < d.stages.size(); s++) if (d.has_gemm[s]) widest = std::max(widest, d.stages[s].n_tiles * h->cfg.n_agents);
         // throughput form: the widest GEMM stage has more than two waves of tiles (population of agents, large batches)
         stream_mode = math_is_tc(h->cfg.math_mode) && h->cfg.launch_mode == SACB_LAUNCH_STAGED && widest > 2 * h->sm_count &&
-                      !getenv("SACB_NO_STREAM") && !getenv("SACB_FUSE_SAMPLE");
+                      !getenv("SACB_NO_STREAM");
         shapes = stream_mode ? d.stream_tile_shapes() : d.choose_tile_shapes(h->sm_count);
         // chained launches: latency programs of one agent (staged, tensor cores, no LayerNorm), where every cluster of the chain fits
         // on the GPU at once (its CTAs hold one SM each)
@@ -1293,7 +1213,7 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
         // the two-CTAs-per-SM column-sum build (4 rows in flight per thread) pays where resident CTAs walk thousands of small tiles (a
         // population); a stage of a few long tiles (one agent, large batch) keeps the one-CTA build with 8 rows in flight
         const bool many = b.stages[s].n_tiles * h->cfg.n_agents > 2 * h->sm_count;
-        p.stage_kind.push_back(getenv("SACB_ONE_KERNEL") ? (h->cfg.layer_norm ? kVariantEverythingLn : kVariantEverything) : pick_variant(types, epis, many));
+        p.stage_kind.push_back(pick_variant(types, epis, many));
     }
     for (int s = 0, ci = 0; s < (int)b.stages.size();) {
         if (ci < (int)chains.size() && chains[ci].s0 == s) {
@@ -1346,8 +1266,7 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
 
 ProgramKey update_key(sacb_handle h, int B, int with_gather, int export_grads, int device_eps, int use_isw) {
     ProgramKey k{B, with_gather, export_grads, device_eps, use_isw, -1};
-    static const bool always = getenv("SACB_ALWAYS_SHADOW") != nullptr;      // A/B switch: re-derive every shadow every step (round-1 behaviour)
-    k.resident = (h->shadows_valid && !always) ? 1 : 0;
+    k.resident = h->shadows_valid ? 1 : 0;
     return k;
 }
 void after_update_launch(sacb_handle h, const ProgramKey &key) {
@@ -1374,7 +1293,6 @@ static int compute_split(ProgramInst &p) {
         }
     if (td_stage < 0) return fail(SACB_ERR_STATE, "program has no critic-loss stage");
     int split = actor_stage > td_stage ? actor_stage : td_stage + 1;
-    if (getenv("SACB_PER_SPLIT")) split = std::min(ns - 1, std::max(td_stage + 1, atoi(getenv("SACB_PER_SPLIT"))));      // experiment switch
     // the first launch from that stage on (neither the loss stages nor their neighbours are in a chain: a launch boundary)
     const int nl = (int)p.launches.size();
     p.split = nl;
@@ -1384,8 +1302,7 @@ static int compute_split(ProgramInst &p) {
 
 // sacb_per_step as one graph launch (two graph launches + two events cost ~8 us per step: 206 against 198 us with no replay work at all)
 int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
-    static const bool off = getenv("SACB_NO_STEP_GRAPH") != nullptr;
-    if (off || h->cfg.launch_mode != SACB_LAUNCH_STAGED || p.step_graph_failed) return 1;
+    if (h->cfg.launch_mode != SACB_LAUNCH_STAGED || p.step_graph_failed) return 1;
     const int nl = (int)p.launches.size();
     const int64_t n = h->r_len[0];
     if (!p.step_graph || p.step_graph_n != n || p.step_graph_k != k) {
@@ -1406,7 +1323,6 @@ int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
         if (rc == SACB_OK && cudaStreamWaitEvent(h->stream, h->ev_sampled, 0) != cudaSuccess) rc = SACB_ERR_DEVICE;
         const cudaError_t e2 = cudaStreamEndCapture(h->stream, &graph);
         p.step_graph_launches = nl + (int)(h->kernel_launches - launches0);      // the stage kernels + what the replay helpers counted
-        p.step_graph_fused = h->per_fused;
         h->kernel_launches = launches0; h->per_frame[0] = frame0;
         if (rc != SACB_OK || e2 != cudaSuccess || !graph || cudaGraphInstantiate(&p.step_graph, graph, 0) != cudaSuccess) {
             if (graph) cudaGraphDestroy(graph);
@@ -1419,7 +1335,7 @@ int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
     }
     SACB_CUDA(cudaGraphLaunch(p.step_graph, h->stream));
     h->kernel_launches += p.step_graph_launches;
-    h->per_frame[0] += 1; h->sample_k = k; h->per_fused = p.step_graph_fused; h->prio_max_valid = true;
+    h->per_frame[0] += 1; h->sample_k = k; h->prio_max_valid = true;
     return SACB_OK;
 }
 

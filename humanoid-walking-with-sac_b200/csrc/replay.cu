@@ -4,17 +4,17 @@
 // Ring row = one transition [s (obs) | s2 (obs) | a (act) | r | d], fp32, padded to 16 B: a sampled row is one
 // contiguous ~2.9 KB read (Humanoid), gathered by one warp with coalesced loads.
 //
-// PER sampling reproduces np.random.choice(len, B, p=probs) bit-for-bit downstream of the p**alpha table:
-// Three launches per sample() call, chained with programmatic dependent launch and free of serial tails between them (capacity <= 2 M):
+// PER sampling reproduces np.random.choice(len, B, p=probs) bit-for-bit downstream of the p**alpha table, in three launches per
+// sample() call chained with programmatic dependent launch.  Up to 2 096 128 rows (the chunk prefixes fit into shared memory) there are
+// no serial tails between them:
 //   per_sum           CTA subtrees of numpy's pairwise-summation tree over p_alpha (float32, the exact same association)
 //   per_chunk_notail  every CTA adds the top of that tree itself (<= 512 values) -> total; probs = p_alpha / total (float32), float64 chunk
 //                     sums, count of "fine" elements
 //   per_search_scan   every CTA scans the chunk sums itself (shared memory), per-sample inverse-CDF search + provable ambiguity test
 //                     (see DESIGN.md "PER exactness"); the last group then runs the sequential float64 cumsum (numpy's own order) for
 //                     samples the test could not certify, IS weights (N p)^-beta / max, logical indices, ring slots for the update's gather
-// The forms that finish the sum / the scan in the last CTA to arrive (per_sum(tail), per_chunk, per_search: SACB_PER_TAILS=1, and any capacity
-// above 2 M), and the same work as one launch of ordered work items (per_sample_fused, SACB_PER_ONE_LAUNCH=1) or as two (per_chunk_search,
-// SACB_PER_TWO_LAUNCHES=1) are built too; all are bit-identical.
+// Above that the last CTA to arrive finishes the sum and the scan: per_sum(tail) -> per_chunk -> per_search, with the chunk prefixes
+// in global memory.  Both forms are bit-identical.
 #include <cmath>
 #include <cstring>
 #include <algorithm>
@@ -55,7 +55,7 @@ struct PerWs {            // device workspace of one agent's PER sampler
     double *chunk_sum;    // [n_chunks]
     double *chunk_carry;  // [n_chunks + 1] exclusive, last = cdf_last
     int *chunk_fine;      // [n_chunks]
-    int *counters;        // [0] total fine, [1] flagged count, [2] exact fallbacks run
+    int *counters;        // [0] total fine, [1] flagged count (running), [2] exact fallbacks run, [3] flagged count of the last call
     int *tickets;         // completion tickets of the three sample() kernels (kTicketInts each)
     float *block_max;     // [128] per-CTA maxima of the priority table (push reads max(priorities), replay_buffer.py:38)
     double *cdf_exact;    // [n_chunks + 1] exact sequential cdf at the chunk starts, only touched by the exact pass (sized for capacity)
@@ -556,15 +556,11 @@ __device__ __forceinline__ bool search_group(const SearchArgs &a, const double *
     return true;
 }
 
+// per_search behind per_chunk (capacity above 2 M: the chunk prefixes do not fit into shared memory and are read from global memory)
 __global__ void __launch_bounds__(256) per_search(const float *total, const double *carry, SearchArgs a) {
     SACB_PDL_ENTER();
-    const float tot = *total;
-    // the chunk prefixes in shared memory (one coalesced read instead of ten dependent L2 round trips per sample)
-    __shared__ double s_carry[kCarrySmem];
-    const bool staged = a.n_chunks + 1 <= kCarrySmem;
-    if (staged) for (int i = threadIdx.x; i <= a.n_chunks; i += blockDim.x) s_carry[i] = carry[i];
-    __syncthreads();
-    search_group(a, staged ? s_carry : carry, a.counters[0], tot, (int)blockIdx.x, (int)gridDim.x);
+    if (!search_group(a, carry, a.counters[0], *total, (int)blockIdx.x, (int)gridDim.x)) return;
+    if (threadIdx.x == 0) { a.counters[3] = a.counters[1]; a.counters[1] = 0; }      // flagged count of this call; reset for the next one
 }
 
 // per_search behind per_chunk_notail (capacity <= 2 M: the chunk prefixes fit into shared memory): every search group scans the chunk sums
@@ -584,108 +580,6 @@ __global__ void __launch_bounds__(256) per_search_scan(const float *total, doubl
     }
     if (!search_group(a, s_carry, s_cnt[0], tot, (int)blockIdx.x, (int)gridDim.x, uu_pre)) return;
     if (threadIdx.x == 0) { a.counters[3] = a.counters[1]; a.counters[1] = 0; }      // flagged count of this call; reset for the next one
-}
-
-// per_chunk and per_search as ONE launch (capacity <= 2 M: the chunk prefixes fit into shared memory).  CTAs claim work items in order
-// from a queue: first the chunk groups, then the search groups.  A search group waits until every chunk group has signalled -- those
-// were all claimed by CTAs that are running, so the wait cannot deadlock whatever the residency -- then scans the chunk sums ITSELF
-// into shared memory (1 K additions, redundantly per group: no second grid-wide rendezvous, no serial tail CTA) and searches its 8
-// samples.  queue[0] = next item, queue[32] = finished chunk groups; the tail of the last search group resets both.
-__global__ void __launch_bounds__(256) per_chunk_search(const float *total, double *chunk_sum, int *chunk_fine, double *carry, int *queue, SearchArgs a) {
-    SACB_PDL_ENTER();
-    __shared__ int s_item;
-    __shared__ double s_carry[kCarrySmem];
-    __shared__ int s_cnt[2];
-    if (threadIdx.x == 0) s_item = atomicAdd(queue, 1);
-    __syncthreads();
-    const int item = s_item, n_cg = (a.n_chunks + 7) / 8, n_sg = (a.B + 7) / 8;
-    const float tot = *total;
-    if (item < n_cg) {
-        chunk_group(a.p_alpha, a.n, tot, item, chunk_sum, chunk_fine);
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicAdd(queue + 32, 1);
-        return;
-    }
-    const int sg = item - n_cg;
-    if (sg >= n_sg) return;
-    if (threadIdx.x == 0) {
-        unsigned int it = 0;
-        int v;
-        do { asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(queue + 32) : "memory"); } while (v < n_cg && ++it < (1u << 26));
-    }
-    __syncthreads();
-    carry_scan(chunk_sum, chunk_fine, a.n_chunks, s_carry, s_cnt);      // chunk sums are read with ld.cg (L2): written by other CTAs of this launch
-    __syncthreads();
-    if (sg == 0) {      // the global copies (exact pass, statistics)
-        for (int i = threadIdx.x; i <= a.n_chunks; i += blockDim.x) carry[i] = s_carry[i];
-        if (threadIdx.x == 0) a.counters[0] = s_cnt[0];
-    }
-    if (!search_group(a, s_carry, s_cnt[0], tot, sg, n_sg)) return;
-    if (threadIdx.x == 0) { queue[0] = 0; queue[32] = 0; a.counters[3] = a.counters[1]; a.counters[1] = 0; }
-}
-
-// The whole sample() as ONE launch: the queue hands out the sum groups (CTA subtrees of the pairwise tree), then the chunk groups, then
-// the search groups.  A chunk group waits for every sum group, adds the top of the tree ITSELF (<= 4 K values in shared memory, the same
-// association in every CTA, so every CTA holds the same float32 total) and runs its chunk pass; a search group waits for every chunk
-// group as above.  Waits only ever point at lower-numbered items, which were claimed by running CTAs: no deadlock whatever the residency.
-// queue[0] = next item, queue[32] = finished chunk groups, queue[64] = finished sum groups.
-struct SumArgs { int top_depth; float *top_vals; float *total; double *u; int draw_B; uint64_t seed; const int64_t *frame; };
-__global__ void __launch_bounds__(256) per_sample_fused(SumArgs sm, double *chunk_sum, int *chunk_fine, double *carry, int *queue, SearchArgs a) {
-    SACB_PDL_ENTER();
-    __shared__ int s_item;
-    __shared__ double s_carry[kCarrySmem];
-    __shared__ int s_cnt[2];
-    if (threadIdx.x == 0) s_item = atomicAdd(queue, 1);
-    __syncthreads();
-    const int item = s_item, n_sum = (2 << sm.top_depth) - 1, n_cg = (a.n_chunks + 7) / 8, n_sg = (a.B + 7) / 8;
-    auto wait_for = [&](int *counter, int target) {
-        if (threadIdx.x == 0) {
-            unsigned int it = 0;
-            int v;
-            do { asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory"); } while (v < target && ++it < (1u << 26));
-        }
-        __syncthreads();
-    };
-    if (item < n_sum) {
-        __shared__ float s_heap[kSumHeap];
-        __shared__ unsigned char s_state[kSumHeap];
-        __shared__ int s_leaf[3 * 128];
-        const uint64_t counter = (uint64_t)__ldcg(sm.frame);
-        for (int j = item * blockDim.x + threadIdx.x; j < sm.draw_B; j += n_sum * blockDim.x) sm.u[j] = uniform_of(sm.seed, counter, j);
-        const unsigned id = (unsigned)item + 1;
-        int64_t s, m; bool leaf = false;
-        if (pw_node(0, a.n, kSumBlockMax, id, s, m, leaf) && leaf) {      // CTA-uniform
-            const float v = pw_block_sum(a.p_alpha, s, (int)m, s_heap, s_state, s_leaf);
-            if (threadIdx.x == 0) sm.top_vals[id] = v;
-        }
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicAdd(queue + 64, 1);
-        return;
-    }
-    if (item < n_sum + n_cg) {
-        wait_for(queue + 64, n_sum);
-        const float tot = top_tree_sum(a.n, sm.top_depth, sm.top_vals);
-        if (item == n_sum && threadIdx.x == 0) *sm.total = tot;      // the global copy (search groups, statistics, the exact pass)
-        chunk_group(a.p_alpha, a.n, tot, item - n_sum, chunk_sum, chunk_fine);
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicAdd(queue + 32, 1);
-        return;
-    }
-    const int sg = item - n_sum - n_cg;
-    if (sg >= n_sg) return;
-    wait_for(queue + 32, n_cg);
-    const float tot = __ldcg(sm.total);
-    carry_scan(chunk_sum, chunk_fine, a.n_chunks, s_carry, s_cnt);
-    __syncthreads();
-    if (sg == 0) {
-        for (int i = threadIdx.x; i <= a.n_chunks; i += blockDim.x) carry[i] = s_carry[i];
-        if (threadIdx.x == 0) a.counters[0] = s_cnt[0];
-    }
-    if (!search_group(a, s_carry, s_cnt[0], tot, sg, n_sg)) return;
-    if (threadIdx.x == 0) { queue[0] = 0; queue[32] = 0; queue[64] = 0; a.counters[3] = a.counters[1]; a.counters[1] = 0; }
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -999,8 +893,7 @@ extern "C" int sacb_push_rows(sacb_handle h, int agent, const float *rows, int64
         if (per) slot = h->r_pos[agent];
         else slot = h->r_len[agent] < cap ? (h->r_head[agent] + h->r_len[agent]) % cap : h->r_head[agent];
         const int64_t run = std::min(n - done_n, cap - slot);
-        static const bool copy_calls = getenv("SACB_PINNED_COPIES") != nullptr;      // A/B: cudaMemcpyAsync out of the pinned blocks instead
-        const bool by_kernel = per && staged && agent == 0 && !copy_calls;      // the push kernel moves the rows out of the pinned block itself
+        const bool by_kernel = per && staged && agent == 0;      // the push kernel moves the rows out of the pinned block itself
         if (!by_kernel) SACB_CUDA(cudaMemcpyAsync(ring + slot * row, rows + done_n * row, sizeof(float) * row * run, cudaMemcpyHostToDevice, h->stream));
         if (per) {
             int rc = per_push_priorities(h, slot, run, h->r_len[agent] == 0, by_kernel ? rows + done_n * row : nullptr);
@@ -1093,71 +986,35 @@ int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B
         if (h->u_in_flight) SACB_CUDA(cudaEventSynchronize(h->ev_u));      // the previous call's search kernel has read the block (long done)
         memcpy(h->pin_u, u, sizeof(double) * k);      // the search kernel reads them from here (host memory is addressable from the device): no copy call
     }
-    static const bool copy_calls = getenv("SACB_PINNED_COPIES") != nullptr;
-    if (u && copy_calls) SACB_CUDA(cudaMemcpyAsync(w.u, h->pin_u, sizeof(double) * k, cudaMemcpyHostToDevice, st));
-    const double *u_dev = u && !copy_calls ? h->pin_u : w.u;
-    auto sampled = [&]() -> int {      // behind the last kernel of the call
-        if (u) { SACB_CUDA(cudaEventRecord(h->ev_u, st)); h->u_in_flight = true; }
-        h->sample_k = k;
-        if (k_out) *k_out = k;
-        return SACB_OK;
-    };
+    const double *u_dev = u ? h->pin_u : w.u;
     const int depth = top_depth_of(n);
     if (depth > 11) return fail(SACB_ERR_ARG, "capacity too large for the summation heap");
     const float *pa = h->p_alpha;
     int *tickets = w.tickets;
-    // Three launches are the default.  The same work as ONE launch of ordered work items (per_sample_fused,
-    // SACB_PER_ONE_LAUNCH=1) or two (per_sum + per_chunk_search, SACB_PER_TWO_LAUNCHES=1) is bit-exact and faster back to back -- 30.7 / 30.2
-    // against 34.7 us per sample(256) at N = 1 M -- but not where it counts: the trainer's sequence push -> sample -> update runs 306-311 /
-    // 306 against 301.6 us per step (the spinning search / chunk groups hold SMs and load L2 while the others work), the pipelined
-    // learner step 211.3 / 213.2 against 211.5 us.
-    static const bool one_launch = getenv("SACB_PER_ONE_LAUNCH") != nullptr;
-    static const bool two_launches = getenv("SACB_PER_TWO_LAUNCHES") != nullptr;
-    const bool split_launch = !one_launch && !two_launches;
     const int n_chunks = (int)((n + kChunk - 1) / kChunk);
     SearchArgs sa;
     sa.p_alpha = pa; sa.n = n; sa.u = u_dev; sa.B = (int)k; sa.counters = w.counters; sa.idx_out = w.idx; sa.flagged = w.flagged;
     sa.ticket = tickets + 2 * kTicketInts; sa.carry_exact = w.cdf_exact; sa.chunk_sum = w.chunk_sum; sa.chunk_fine = w.chunk_fine; sa.n_chunks = n_chunks;
     sa.weights = w.weights; sa.slots = h->slots; sa.isw_ws = h->ws + h->L.isw; sa.idx_copy = h->last_idx_dev;
     sa.frame = frame_dev; sa.beta_start = (double)h->cfg.per_beta_start; sa.one_minus_start = 1.0 - (double)h->cfg.per_beta_start; sa.beta_frames = (double)h->cfg.per_beta_frames;
-    if (n_chunks + 1 <= kCarrySmem && !split_launch && !two_launches) {
-        // the whole call as ONE launch: CTAs claim sum groups, chunk groups, search groups, in that order, from a work queue
-        SumArgs sm;
-        sm.top_depth = depth; sm.top_vals = w.block_vals; sm.total = w.total; sm.u = w.u; sm.draw_B = u ? 0 : (int)k; sm.seed = h->cfg.seed; sm.frame = frame_dev;
-        SACB_CUDA(launch_pdl(per_sample_fused, dim3((2 << depth) - 1 + (n_chunks + 7) / 8 + (int)((k + 7) / 8)), dim3(256), 0, st, pdl, sm, w.chunk_sum, w.chunk_fine,
-                             w.chunk_carry, tickets + kTicketInts, sa));
-        h->kernel_launches += 1;
-        h->per_fused = true;
-        return sampled();
-    }
-    // three launches, no serial tails between them (SACB_PER_TAILS=1: the forms that finish the sum / the scan in the last CTA to arrive)
-    static const bool tails = getenv("SACB_PER_TAILS") != nullptr;
-    const bool no_tails = split_launch && !tails && n_chunks + 1 <= kCarrySmem;
+    // no serial tails while the chunk prefixes fit into shared memory (DESIGN.md section 4 records the one- and two-launch forms measured against this)
+    const bool no_tails = n_chunks + 1 <= kCarrySmem;
     SACB_CUDA(launch_pdl(per_sum, dim3((2 << depth) - 1), dim3(256), 0, st, pdl, pa, n, depth, w.block_vals, w.total, tickets + 0,
                          w.u, u ? 0 : (int)k, h->cfg.seed, (const int64_t *)frame_dev, no_tails ? 0 : 1));
-    h->kernel_launches += 1;
     if (no_tails) {
         SACB_CUDA(launch_pdl(per_chunk_notail, dim3((n_chunks + 7) / 8), dim3(256), 0, st, pdl, pa, n, depth, (const float *)w.block_vals, w.total,
                              w.chunk_sum, w.chunk_fine));
         SACB_CUDA(launch_pdl(per_search_scan, dim3((int)((k + 7) / 8)), dim3(256), 0, st, pdl, (const float *)w.total, w.chunk_carry, sa));
-        h->kernel_launches += 2;
-        h->per_fused = true;      // the flagged count of the call is kept in counters[3]
-        return sampled();
-    }
-    if (n_chunks + 1 <= kCarrySmem && !split_launch) {
-        // chunk pass and search as ONE launch: CTAs claim chunk groups, then search groups, in order from a work queue
-        SACB_CUDA(launch_pdl(per_chunk_search, dim3((n_chunks + 7) / 8 + (int)((k + 7) / 8)), dim3(256), 0, st, pdl, (const float *)w.total, w.chunk_sum, w.chunk_fine,
-                             w.chunk_carry, tickets + kTicketInts, sa));
-        h->kernel_launches += 1;
-        h->per_fused = true;
     } else {
         SACB_CUDA(launch_pdl(per_chunk, dim3((n_chunks + 7) / 8), dim3(256), 0, st, pdl, pa, n, (const float *)w.total, w.chunk_sum, w.chunk_fine,
                              n_chunks, w.chunk_carry, w.counters, tickets + kTicketInts));
         SACB_CUDA(launch_pdl(per_search, dim3((int)((k + 7) / 8)), dim3(256), 0, st, pdl, (const float *)w.total, (const double *)w.chunk_carry, sa));
-        h->kernel_launches += 2;
-        h->per_fused = false;
     }
-    return sampled();
+    h->kernel_launches += 3;
+    if (u) { SACB_CUDA(cudaEventRecord(h->ev_u, st)); h->u_in_flight = true; }      // behind the last kernel of the call
+    h->sample_k = k;
+    if (k_out) *k_out = k;
+    return SACB_OK;
 }
 
 int per_writeback_launch(sacb_handle h, cudaStream_t st, int64_t B, bool pdl_ok) {
@@ -1241,7 +1098,7 @@ extern "C" int sacb_per_get_stats(sacb_handle h, int agent, sacb_per_stats *out)
     SACB_CUDA(cudaMemcpyAsync(&last, w.chunk_carry + n_chunks, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     SACB_CUDA(cudaStreamSynchronize(h->stream));
     out->frame = h->per_frame[0]; out->pos = h->r_pos[0]; out->len = h->r_len[0];
-    out->n_fine = counters[0]; out->n_flagged = h->per_fused ? counters[3] : counters[1]; out->n_exact_fallbacks = counters[2];
+    out->n_fine = counters[0]; out->n_flagged = counters[3]; out->n_exact_fallbacks = counters[2];
     out->total_f32 = tot; out->cdf_last = last;
     return SACB_OK;
 }

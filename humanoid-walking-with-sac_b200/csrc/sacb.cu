@@ -329,10 +329,9 @@ static int finish_update(sacb_handle h, float *losses_out, uint32_t flags, int64
     }
     // the three losses (the `.item()` calls of sac_imp.py:141-143) and the device error flag: the last stage of the step (T_FINISH) has
     // stored them into the pinned block itself (Program::host_losses), ONE synchronisation and no copy behind the step.
-    // (population handles and SACB_PINNED_COPIES=1: one D2H copy of the five floats)
+    // (population handles: one D2H copy of the five floats)
     static_assert(SC_ERROR_FLAG == SC_LOSS_Q1 + 4, "losses and the flag copy are contiguous");
-    static const bool copy_calls = getenv("SACB_PINNED_COPIES") != nullptr;
-    if (h->cfg.n_agents != 1 || copy_calls)
+    if (h->cfg.n_agents != 1)
         SACB_CUDA(cudaMemcpyAsync(h->pin_small, h->arena + h->L.scalars + SC_LOSS_Q1, 5 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     if (write_back_B > 0) {
         if (!h->ev_loss) SACB_CUDA(cudaEventCreateWithFlags(&h->ev_loss, cudaEventDisableTiming));
@@ -470,26 +469,19 @@ static int per_step_enqueue(sacb_handle h, int64_t B) {
     ProgramInst *p;
     rc = get_program(h, key, &p);
     if (rc) return rc;
-    static const int exp_mode0 = getenv("SACB_EXP_PER_STEP") ? atoi(getenv("SACB_EXP_PER_STEP")) : 0;
-    if (exp_mode0 == 0) {      // the whole step -- update stages, forked write-back + next sample, join -- as ONE graph launch
-        rc = launch_per_step_graph(h, *p, B, k);
-        if (rc == SACB_OK) { after_update_launch(h, key); return SACB_OK; }
-        if (rc != 1) return rc;
-    }
+    // the whole step -- update stages, forked write-back + next sample, join -- as ONE graph launch
+    rc = launch_per_step_graph(h, *p, B, k);
+    if (rc == SACB_OK) { after_update_launch(h, key); return SACB_OK; }
+    if (rc != 1) return rc;
     if ((rc = launch_program_part(h, *p, 0))) return rc;
     after_update_launch(h, key);
-    static const int exp_mode = getenv("SACB_EXP_PER_STEP") ? atoi(getenv("SACB_EXP_PER_STEP")) : 0;      // timing experiments only (1: no replay work, 2: no events either)
-    if (exp_mode < 2) {
-        SACB_CUDA(cudaEventRecord(h->ev_td, h->stream));
-        SACB_CUDA(cudaStreamWaitEvent(h->stream2, h->ev_td, 0));
-    }
-    if (exp_mode == 0) {
-        if ((rc = per_writeback_launch(h, h->stream2, k))) return rc;
-        if ((rc = per_sample_launch(h, h->stream2, nullptr, B, nullptr))) return rc;
-    }
-    if (exp_mode < 2) SACB_CUDA(cudaEventRecord(h->ev_sampled, h->stream2));
+    SACB_CUDA(cudaEventRecord(h->ev_td, h->stream));
+    SACB_CUDA(cudaStreamWaitEvent(h->stream2, h->ev_td, 0));
+    if ((rc = per_writeback_launch(h, h->stream2, k))) return rc;
+    if ((rc = per_sample_launch(h, h->stream2, nullptr, B, nullptr))) return rc;
+    SACB_CUDA(cudaEventRecord(h->ev_sampled, h->stream2));
     if ((rc = launch_program_part(h, *p, 1))) return rc;
-    if (exp_mode < 2) SACB_CUDA(cudaStreamWaitEvent(h->stream, h->ev_sampled, 0));      // whatever follows on the main stream sees the new sample
+    SACB_CUDA(cudaStreamWaitEvent(h->stream, h->ev_sampled, 0));      // whatever follows on the main stream sees the new sample
     return SACB_OK;
 }
 

@@ -1,4 +1,4 @@
-// Tanh-Gaussian sampling arithmetic shared by the T_SAMPLE / T_SAMPLE_BWD tasks and the fused heads epilogue (EPI_SAMPLE).
+// Tanh-Gaussian sampling arithmetic shared by the T_SAMPLE / T_SAMPLE_BWD tasks and the forward / select_action kernels (extras.cu).
 #pragma once
 #include "common.cuh"
 

@@ -402,7 +402,7 @@ __device__ __forceinline__ void epilogue_tile(const EpiR &epi, float *Cs, float4
 }
 
 // the kernel body; P.tasks of the stage are all T_GEMM with bm = 128 and bn in {64, 128, 256}
-__device__ __forceinline__ void gemm_stage(const Program &P, const Stage &stage, uint8_t *smem, uint64_t seed) {
+__device__ __forceinline__ void gemm_stage(const Program &P, const Stage &stage, uint8_t *smem) {
     uint8_t *ring = smem;                                              // 1024-aligned (checked by the caller)
     float *Cs = reinterpret_cast<float *>(smem + kRingBytes);
     Misc &mi = *reinterpret_cast<Misc *>(smem + kRingBytes + kStagingBytes);

@@ -3,6 +3,7 @@
 // fills them.  Matrices that feed a GEMM are pair matrices (bf16 hi/lo planes, common.cuh).
 #pragma once
 #include "gemm.cuh"
+#include "sample.cuh"
 
 namespace sacb {
 

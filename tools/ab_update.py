@@ -15,4 +15,4 @@ for rep in range(5):
     ms = ctypes.c_float()
     N.check(N.lib().sacb_time_update(agent._h, 256, iters, ctypes.byref(ms)))
     best = min(best, ms.value)
-print(f"AB_UPDATE launch={launch} always_shadow={os.environ.get('SACB_ALWAYS_SHADOW', '0')} env={os.environ.get('SACB_AB_TAG', '')} best_ms={best:.4f} stages={agent.stats()['n_stages']}")
+print(f"AB_UPDATE launch={launch} env={os.environ.get('SACB_AB_TAG', '')} best_ms={best:.4f} stages={agent.stats()['n_stages']}")

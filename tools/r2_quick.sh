@@ -8,6 +8,4 @@ tail -${TAILN:-15} gpurun_out/pytest.log
 if [ "${TIMELINE:-0}" = "1" ]; then
 SACB_TIMELINE=1 timeout 300 python tools/trace_stages.py > gpurun_out/trace_resident.log 2>&1
 grep "timeline" gpurun_out/trace_resident.log | cut -c1-200
-SACB_ALWAYS_SHADOW=1 SACB_TIMELINE=1 timeout 300 python tools/trace_stages.py > gpurun_out/trace_always.log 2>&1
-grep "timeline" gpurun_out/trace_always.log | cut -c1-200
 fi
