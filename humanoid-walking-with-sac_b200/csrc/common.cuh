@@ -112,10 +112,109 @@ struct AdamArgs {
     PmRef shadow;       // bf16 pair shadow of w refreshed in place (null: not needed before the next step)
     PmRef shadow2;      // second shadow holding only columns >= shadow2_col0 of w (the action block of a critic's fc1)
     PmRef shadow_t;     // throughput programs only (stream.cuh): bf16 pair shadow of the Polyak target wt, refreshed in the epilogue too
-    int32_t shadow2_col0, pad0;
-    int32_t step_slot;  // ScalarSlot of the optimizer step counter (value BEFORE this step's increment)
+    int32_t shadow2_col0;
+    int32_t step_slot;  // ScalarSlot of the optimizer step counter (value BEFORE this step's increment); it also selects the cached
+                        // SC_FAC0 factors, which hold the step size (lr): a new learning rate does not touch the program
     int32_t apply;      // 0 = only export the gradient (data-parallel backward), 1 = apply Adam
-    float lr, tau;
+    float tau;          // Polyak rate
+};
+
+// ---- arguments of the non-GEMM task types (Task's union): the builder (program.cu) sets every field a type uses, the bodies
+// (tasks.cuh) read them.  Builder::blank() fills the union with 0xFF bytes first: an unset Ref / PmRef is null, an int -1, a
+// float NaN.  Extents: B = minibatch rows, H = hidden width, A = action dimension.
+
+struct ShadowArgs {           // T_SHADOW: columns [col0, col0 + cols) of an fp32 weight matrix -> their bf16 pair shadow
+    Ref src;                  // fp32 weight matrix, row stride src_ld
+    PmRef dst;                // shadow PM [rows, cols]
+    int32_t rows, cols, col0, src_ld;
+};
+struct GatherArgs {           // T_GATHER: replay ring rows -> minibatch PM
+    PmRef x;                  // X PM [3B, ldx]
+    Ref r, d;                 // out: reward, done [B]
+    int32_t B, obs, act;
+    int32_t device_draw;      // 1: positions drawn on the device (draw_position, uniform ring), 0: slots taken from Program::slots
+    int32_t capacity;         // ring slots per agent
+};
+struct SampleArgs {           // T_SAMPLE: policy head outputs -> tanh-Gaussian sample (into X) + log-prob
+    Ref head;                 // head_raw [2B, 2A] (mean | log_std_raw)
+    Ref eps;                  // standard normal draws [2B, A]
+    PmRef x;                  // X PM: row j < B -> X[j, obs:] (next state), j >= B -> X[2B + (j - B), obs:] (current state)
+    Ref logp;                 // out [2B]
+    int32_t B, A, obs;
+    int32_t device_eps;       // 1: eps drawn with Philox here and stored for the backward, 0: eps read
+    float scale, bias;        // action_scale, action_bias
+};
+struct TargetLossArgs {       // T_TARGET_LOSS
+    PmRef h[4];               // last hidden activations [B, H] of q1_target, q2_target on (s2, a2), of q1, q2 on (s, a)
+    PmRef dh[2];              // out: dL/dh of the last hidden layer of q1, q2 [B, H] (consumed by the critic backward GEMMs)
+    Ref w_out[4], b_out[4];   // output-layer weights [H] and biases [1] of the nets of h
+    Ref r, d, logp_next;      // [B]
+    Ref is_weights;           // [B], null: 1
+    Ref y, dq[2], td;         // out [B]: Bellman target, dL/dq1, dL/dq2, |q1 - y|
+    Ref partials;             // out: per-tile partial sums of w*(q-y)^2 [n_tiles, 2] (summed in tile order by T_FINISH: deterministic)
+    int32_t B, H;
+    int32_t R;                // batch rows per tile (kLossRows or kLossRowsMax, tasks.cuh)
+    float gamma;
+};
+struct ActorLossArgs {        // T_ACTOR_LOSS
+    PmRef h[2];               // last hidden activations [B, H] of q1, q2 on (s, a_new)
+    PmRef dh[2];              // out: dL/dh of the last hidden layer of q1, q2 (the Q weights are constants here, quirk Q2)
+    Ref w_out[2], b_out[2];   // output-layer weights [H] and biases [1] of q1, q2
+    Ref logp;                 // log-prob of the current-state sample [B]
+    Ref partials;             // out: per-tile partials [n_tiles, 2]: sum(alpha*logp - minq), sum(logp + target_entropy)
+    int32_t B, H;
+    int32_t R;                // batch rows per tile
+    float target_entropy;
+};
+struct SampleBwdArgs {        // T_SAMPLE_BWD: dL/da -> dL/dmean, dL/dlog_std
+    Ref da[2];                // dL/da through q1, q2 [B, A]
+    Ref head;                 // head_raw rows of the current-state sample [B, 2A]
+    Ref eps;                  // their draws [B, A]
+    PmRef g_head;             // out: PM [B, 2A]
+    int32_t B, A;
+    float scale, bias;
+};
+struct ColsumAdamArgs {       // T_BIAS_ADAM: db[n] = sum_b src[b, n], Adam, Polyak
+    AdamArgs adam;            // the bias (shadows unused)
+    // (B, N, chunk_rows ahead of src: there they are not read as one 16-byte load, which costs the 64-register build more spills)
+    int32_t B, N;
+    int32_t chunk_rows;       // batch rows per chunk (>= B: one chunk); several chunks add into adam.gexp with atomics
+    PmRef src;                // PM [B, N]
+};
+struct OutAdamArgs {          // T_OUT_ADAM: Q output layer Linear(H, 1): dW = dq^T h, db = sum dq, Adam, Polyak
+    AdamArgs w, b;            // weight [H] and bias [1] (shadows unused)
+    PmRef h;                  // last hidden activations [B, H]
+    Ref dq;                   // [B]
+    int32_t B, H;
+    int32_t chunk_rows;
+};
+struct FinishArgs {           // T_FINISH
+    Ref critic_part, actor_part;   // per-tile loss partials [n_part, 2] of T_TARGET_LOSS / T_ACTOR_LOSS (null: no such phase)
+    Ref alpha_grad;           // out: exported log_alpha gradient (null: not exported)
+    Ref loss_hist;            // per-agent ring of the last kLossHist updates' losses
+    int32_t bump[4];          // 1: +1 on SC_STEP_POLICY + k (policy, q1, q2, alpha)
+    int32_t bump_updates;     // 1: +1 on SC_N_UPDATES, losses recorded in loss_hist
+    int32_t n_part;           // rows of the partial arrays
+    int32_t auto_entropy;
+    int32_t apply;            // 1: Adam step on log_alpha and the next alpha written
+    float B;
+};
+struct LnFwdArgs {            // T_LN_FWD: h = relu(LN(z) * gamma + beta)
+    Ref z;                    // fp32 [rows, H]: Linear output incl. bias, written by the GEMM of the stage before
+    Ref gamma, beta;          // [H]
+    Ref stats;                // out: [rows][2] = (mean, rstd)
+    PmRef h;                  // out: PM [rows, H]
+    int32_t rows, H;
+    float eps;
+};
+struct LnBwdArgs {            // T_LN_BWD: dpre -> dz, gg
+    PmRef dpre;               // gradient at the LayerNorm output [rows, H] (ReLU mask applied)
+    Ref z;                    // fp32 Linear output, first of the rows
+    Ref gamma;                // [H]
+    Ref stats;                // (mean, rstd) of T_LN_FWD, first of the rows
+    PmRef dz;                 // out: gradient at the Linear output
+    PmRef gg;                 // out: dpre * xhat (null base: not wanted)
+    int32_t rows, H;
 };
 
 struct alignas(64) Task {
@@ -131,16 +230,27 @@ struct alignas(64) Task {
     int32_t M, N, K;
     int32_t epi;
     Ref C; int32_t ldc;       // EPI_F32
+    int32_t kb_per_chunk;     // split K (stream kernel, gradient export): K blocks per chunk, tile = [chunk][tm][tn]; 0 = no split
     PmRef Cpm;                // EPI_BIAS_RELU / EPI_MASK
     Ref bias;
     PmRef mask;
     AdamArgs adam;
-    // --- elementwise tasks: generic slots (meaning depends on type, see tasks.cuh)
-    Ref p[24];
-    PmRef pm[6];
-    int32_t i[8];
-    float f[6];
+    // --- the other task types: the arguments of `type`
+    union {
+        ShadowArgs shadow;
+        GatherArgs gather;
+        SampleArgs sample;
+        TargetLossArgs target_loss;
+        ActorLossArgs actor_loss;
+        SampleBwdArgs sample_bwd;
+        OutAdamArgs out_adam;
+        ColsumAdamArgs bias_adam;
+        FinishArgs finish;
+        LnFwdArgs ln_fwd;
+        LnBwdArgs ln_bwd;
+    };
 };
+static_assert(sizeof(Task) <= 1024, "every CTA copies the record of each task it runs into shared memory (fetch_task)");
 
 // Specialised builds of the stage kernel (staged mode): a launch only carries the code its stage can reach -- the task types and
 // GEMM epilogues in its masks -- which keeps the register allocation of the hot paths free of the other paths' pressure (no

@@ -275,17 +275,17 @@ sac_update_kernel(const __grid_constant__ Program P, const __grid_constant__ Sta
                     else gemm_tile_ffma(t, tile, P.bases, agent, scalars, reinterpret_cast<float *>(smem_raw));
                 }
                 break;
-            case T_SHADOW: if constexpr ((kTypes & tb(T_SHADOW)) != 0) task_shadow(t, tile, P, agent); break;
-            case T_GATHER: if constexpr ((kTypes & tb(T_GATHER)) != 0) task_gather(t, tile, P, agent, scalars, seed); break;
-            case T_SAMPLE: if constexpr ((kTypes & tb(T_SAMPLE)) != 0) task_sample(t, tile, P, agent, scalars, seed); break;
-            case T_TARGET_LOSS: if constexpr ((kTypes & tb(T_TARGET_LOSS)) != 0) task_target_loss(t, tile, P, agent, scalars, s_red); break;
-            case T_ACTOR_LOSS: if constexpr ((kTypes & tb(T_ACTOR_LOSS)) != 0) task_actor_loss(t, tile, P, agent, scalars, s_red); break;
-            case T_SAMPLE_BWD: if constexpr ((kTypes & tb(T_SAMPLE_BWD)) != 0) task_sample_bwd(t, tile, P, agent, scalars); break;
-            case T_OUT_ADAM: if constexpr ((kTypes & tb(T_OUT_ADAM)) != 0) task_out_adam<variant_min_blocks(kTypes, kEpis) == 1>(t, tile, P, agent, scalars, s_red); break;
-            case T_BIAS_ADAM: if constexpr ((kTypes & tb(T_BIAS_ADAM)) != 0) task_bias_adam<variant_min_blocks(kTypes, kEpis) == 1>(t, tile, P, agent, scalars, s_red); break;
-            case T_FINISH: if constexpr ((kTypes & tb(T_FINISH)) != 0) task_finish(t, P, agent, scalars, s_red); break;
-            case T_LN_FWD: if constexpr ((kTypes & tb(T_LN_FWD)) != 0) task_ln_fwd(t, tile, P, agent); break;
-            case T_LN_BWD: if constexpr ((kTypes & tb(T_LN_BWD)) != 0) task_ln_bwd(t, tile, P, agent); break;
+            case T_SHADOW: if constexpr ((kTypes & tb(T_SHADOW)) != 0) task_shadow(t.shadow, tile, P, agent); break;
+            case T_GATHER: if constexpr ((kTypes & tb(T_GATHER)) != 0) task_gather(t.gather, tile, P, agent, scalars, seed); break;
+            case T_SAMPLE: if constexpr ((kTypes & tb(T_SAMPLE)) != 0) task_sample(t.sample, tile, P, agent, scalars, seed); break;
+            case T_TARGET_LOSS: if constexpr ((kTypes & tb(T_TARGET_LOSS)) != 0) task_target_loss(t.target_loss, tile, P, agent, scalars, s_red); break;
+            case T_ACTOR_LOSS: if constexpr ((kTypes & tb(T_ACTOR_LOSS)) != 0) task_actor_loss(t.actor_loss, tile, P, agent, scalars, s_red); break;
+            case T_SAMPLE_BWD: if constexpr ((kTypes & tb(T_SAMPLE_BWD)) != 0) task_sample_bwd(t.sample_bwd, tile, P, agent, scalars); break;
+            case T_OUT_ADAM: if constexpr ((kTypes & tb(T_OUT_ADAM)) != 0) task_out_adam<variant_min_blocks(kTypes, kEpis) == 1>(t.out_adam, tile, P, agent, scalars, s_red); break;
+            case T_BIAS_ADAM: if constexpr ((kTypes & tb(T_BIAS_ADAM)) != 0) task_bias_adam<variant_min_blocks(kTypes, kEpis) == 1>(t.bias_adam, tile, P, agent, scalars, s_red); break;
+            case T_FINISH: if constexpr ((kTypes & tb(T_FINISH)) != 0) task_finish(t.finish, P, agent, scalars, s_red); break;
+            case T_LN_FWD: if constexpr ((kTypes & tb(T_LN_FWD)) != 0) task_ln_fwd(t.ln_fwd, tile, P, agent); break;
+            case T_LN_BWD: if constexpr ((kTypes & tb(T_LN_BWD)) != 0) task_ln_bwd(t.ln_bwd, tile, P, agent); break;
         }
         if (first) stamp(4);
     };
@@ -440,8 +440,9 @@ struct Builder {
         t.Cpm = t.mask = t.A.pm = t.B.pm = null_pm();
         t.adam.w = t.adam.m = t.adam.v = t.adam.wt = t.adam.gexp = null_ref();
         t.adam.shadow = t.adam.shadow2 = t.adam.shadow_t = null_pm();
-        for (auto &p : t.p) p = null_ref();
-        for (auto &p : t.pm) p = null_pm();
+        // the union of the non-GEMM arguments (the last member): a field its task type does not set stays null / -1 / NaN, never
+        // arena offset 0
+        memset(reinterpret_cast<char *>(&t) + offsetof(Task, shadow), 0xFF, sizeof(Task) - offsetof(Task, shadow));
         return t;
     }
     void add(Task t, int n_tiles) {
@@ -477,13 +478,14 @@ struct Builder {
                 rc = make_pm_tensor_map(&t.tmB, dev_ptr(b.ref.base), b_cols, b_rows, b.ref.ld, b.ref.plane, agent_stride_bytes(b.ref.base),
                                         h->cfg.n_agents, b_mn ? 64 : t.bn);
         }
-        int n_chunks = 1;
-        if (stream && t.epi == EPI_ADAM && !apply()) {      // gradient export over a long batch dimension: split K, accumulate with atomics
-            const int nkb = cdiv(K, stream::kBK);
-            n_chunks = std::max(1, std::min(16, nkb / 16));
-            if (n_chunks > 1) t.i[7] = cdiv(nkb, n_chunks);
-        }
+        const int n_chunks = stream ? k_chunks(t) : 1;
+        if (n_chunks > 1) t.kb_per_chunk = cdiv(cdiv(K, stream::kBK), n_chunks);
         add(t, t.tiles_m * t.tiles_n * n_chunks);
+    }
+    // split-K chunks of a GEMM task on the stream kernel: gradient export over a long batch dimension is cut into chunks of >= 16 K
+    // blocks (at most 16 chunks), accumulated into the zeroed gradient slab with atomics
+    int k_chunks(const Task &t) const {
+        return (t.epi == EPI_ADAM && !apply()) ? std::max(1, std::min(16, cdiv(t.K, stream::kBK) / 16)) : 1;
     }
     Task epi_bias_relu(const PmView &C, Ref bias) { Task t = blank(T_GEMM); t.epi = EPI_BIAS_RELU; t.Cpm = C.ref; t.bias = bias; return t; }
     Task epi_mask(const PmView &C, const PmView &mask) { Task t = blank(T_GEMM); t.epi = EPI_MASK; t.Cpm = C.ref; t.mask = mask.ref; return t; }
@@ -513,9 +515,9 @@ struct Builder {
         a.w = A(L.param[net] + off_in_net); a.m = A(L.adam_m[net] + off_in_net); a.v = A(L.adam_v[net] + off_in_net);
         a.wt = net == 0 ? null_ref() : A(L.param[net + 2] + off_in_net);     // q1 -> q1_target, q2 -> q2_target
         a.gexp = exporting() ? A(L.grad[net] + off_in_net) : null_ref();
-        a.shadow = a.shadow2 = a.shadow_t = null_pm(); a.shadow2_col0 = 0; a.pad0 = 0;
+        a.shadow = a.shadow2 = a.shadow_t = null_pm(); a.shadow2_col0 = 0;
         a.step_slot = step_slot(net); a.apply = apply() ? 1 : 0;
-        a.lr = h->cfg.lr; a.tau = h->cfg.tau;
+        a.tau = h->cfg.tau;
         return a;
     }
     // dW epilogue of hidden layer `layer`: the critics are read again (post-step) by the actor phase of the SAME update,
@@ -533,12 +535,10 @@ struct Builder {
 
     void bias_adam(int net, int64_t b_off, const PmView &dh, int Bn, int N) {
         Task t = blank(T_BIAS_ADAM);
-        t.pm[0] = dh.ref;
-        AdamArgs a = adam_args(net, b_off);
-        t.p[0] = a.w; t.p[1] = a.m; t.p[2] = a.v; t.p[3] = a.wt; t.p[4] = a.gexp;
-        t.i[0] = Bn; t.i[1] = N; t.i[2] = a.step_slot; t.i[3] = a.apply; t.f[0] = a.lr; t.f[1] = a.tau;
-        t.i[5] = colsum_rows(Bn);
-        add(t, cdiv(N, kColsumCols) * cdiv(Bn, t.i[5]));
+        ColsumAdamArgs &a = t.bias_adam;
+        a.adam = adam_args(net, b_off); a.src = dh.ref;
+        a.B = Bn; a.N = N; a.chunk_rows = colsum_rows(Bn);
+        add(t, cdiv(N, kColsumCols) * cdiv(Bn, a.chunk_rows));
     }
     // ---- opt-in LayerNorm variant (cfg.layer_norm): hidden layer = Linear -> LayerNorm (affine) -> ReLU.  The forward GEMM then writes the
     // Linear output z as fp32 (EPI_F32 with the bias) and a T_LN_FWD stage behind it normalises the rows into the activation PM; a
@@ -550,15 +550,17 @@ struct Builder {
     void ln_fwd(int net, int l, int64_t z_off, int64_t st_off, const PmView &hout, int rows) {
         const NetLayout &n = net == 0 ? L.pol : L.q;
         Task t = blank(T_LN_FWD);
-        t.p[0] = W(z_off); t.p[1] = A(L.param[net] + n.g[l]); t.p[2] = A(L.param[net] + n.be[l]); t.p[3] = W(st_off);
-        t.pm[0] = hout.ref; t.i[0] = rows; t.i[1] = L.hidden; t.f[0] = 1e-5f;      // torch.nn.LayerNorm default eps
+        LnFwdArgs &a = t.ln_fwd;
+        a.z = W(z_off); a.gamma = A(L.param[net] + n.g[l]); a.beta = A(L.param[net] + n.be[l]); a.stats = W(st_off);
+        a.h = hout.ref; a.rows = rows; a.H = L.hidden; a.eps = 1e-5f;      // torch.nn.LayerNorm default eps
         add(t, cdiv(rows, kLnRows));
     }
     void ln_bwd(int net, int l, const PmView &dpre, int64_t z_off, int64_t st_off, const PmView &dz, const PmView *gg, int rows) {
         const NetLayout &n = net == 0 ? L.pol : L.q;
         Task t = blank(T_LN_BWD);
-        t.pm[0] = dpre.ref; t.p[0] = W(z_off); t.p[1] = A(L.param[net] + n.g[l]); t.p[3] = W(st_off);
-        t.pm[1] = dz.ref; t.pm[2] = gg ? gg->ref : null_pm(); t.i[0] = rows; t.i[1] = L.hidden;
+        LnBwdArgs &a = t.ln_bwd;
+        a.dpre = dpre.ref; a.z = W(z_off); a.gamma = A(L.param[net] + n.g[l]); a.stats = W(st_off);
+        a.dz = dz.ref; a.gg = gg ? gg->ref : null_pm(); a.rows = rows; a.H = L.hidden;
         add(t, cdiv(rows, kLnRows));
     }
     // Adam on gamma / beta of hidden layer l of a trainable net: column sums of dpre * xhat (gg) and of dpre
@@ -571,7 +573,8 @@ struct Builder {
     // shadow of columns [col0, col0+dst.cols) of the fp32 matrix at w_off (row stride src_ld)
     void shadow_task(int net, int64_t w_off, const PmView &dst, int src_ld, int col0 = 0) {
         Task t = blank(T_SHADOW);
-        t.p[0] = A(L.param[net] + w_off); t.pm[0] = dst.ref; t.i[0] = dst.rows; t.i[1] = dst.cols; t.i[2] = col0; t.i[3] = src_ld;
+        ShadowArgs &a = t.shadow;
+        a.src = A(L.param[net] + w_off); a.dst = dst.ref; a.rows = dst.rows; a.cols = dst.cols; a.col0 = col0; a.src_ld = src_ld;
         add(t, cdiv(dst.rows, kShadowRows));
     }
 
@@ -644,8 +647,7 @@ struct Builder {
             bool all_many = true;
             for (int k = stages[si].task_begin; k < stages[si].task_end; k++)
                 if (tasks[k].type == T_GEMM) {
-                    // split-K chunks a gradient-export dW GEMM will be cut into (gemm(): the dry pass itself does not split)
-                    const int chunks = (tasks[k].epi == EPI_ADAM && !apply()) ? std::max(1, std::min(16, cdiv(tasks[k].K, stream::kBK) / 16)) : 1;
+                    const int chunks = k_chunks(tasks[k]);      // (the dry pass itself does not split)
                     wide_tiles += cdiv(tasks[k].M, stream::kBM) * cdiv(tasks[k].N, tasks[k].N >= 96 ? stream::kBN : 64) * h->cfg.n_agents;
                     const int t256 = cdiv(tasks[k].M, stream::kBM) * cdiv(tasks[k].N, takes_256(tasks[k]) ? 256 : (tasks[k].N >= 96 ? stream::kBN : 64)) * chunks * h->cfg.n_agents;
                     tiles_256 += t256;
@@ -706,10 +708,11 @@ struct Builder {
         }
         if (key.with_gather && critics) {
             Task t = blank(T_GATHER);
-            t.pm[0] = xrows(0, 3 * B, L.ldx).ref; t.p[0] = W(L.r); t.p[1] = W(L.d);
-            t.i[0] = B; t.i[1] = obs; t.i[2] = act;
-            t.i[3] = key.with_gather == 3 ? 1 : 0;      // 3: positions drawn on the device (uniform ring), see draw_position
-            t.i[4] = (int32_t)h->cfg.capacity;
+            GatherArgs &a = t.gather;
+            a.x = xrows(0, 3 * B, L.ldx).ref; a.r = W(L.r); a.d = W(L.d);
+            a.B = B; a.obs = obs; a.act = act;
+            a.device_draw = key.with_gather == 3 ? 1 : 0;      // 3: positions drawn on the device (uniform ring)
+            a.capacity = (int32_t)h->cfg.capacity;
             add(t, cdiv(B, 4));
         }
         if (critics) {
@@ -736,9 +739,10 @@ struct Builder {
             {
                 begin_stage();
                 Task t = blank(T_SAMPLE);
-                t.p[0] = W(L.head_raw); t.p[1] = W(L.eps); t.pm[0] = xrows(0, 3 * B, L.ldx).ref; t.p[3] = W(L.logp);
-                t.i[0] = B; t.i[1] = act; t.i[2] = obs; t.i[4] = key.device_eps;
-                t.f[0] = h->cfg.action_scale; t.f[1] = h->cfg.action_bias;
+                SampleArgs &a = t.sample;
+                a.head = W(L.head_raw); a.eps = W(L.eps); a.x = xrows(0, 3 * B, L.ldx).ref; a.logp = W(L.logp);
+                a.B = B; a.A = act; a.obs = obs; a.device_eps = key.device_eps;
+                a.scale = h->cfg.action_scale; a.bias = h->cfg.action_bias;
                 add(t, cdiv(2 * B, kThreads / 32));
             }
             // ---- target critics on (s2, a2) ---------------------------------------------------------------------------
@@ -757,15 +761,16 @@ struct Builder {
             begin_stage();
             {
                 Task t = blank(T_TARGET_LOSS);
-                t.pm[0] = hview(L.ht[0][nh - 1], B).ref; t.pm[1] = hview(L.ht[1][nh - 1], B).ref;
-                t.pm[2] = hview(L.hc[0][nh - 1], B).ref; t.pm[3] = hview(L.hc[1][nh - 1], B).ref;
-                t.pm[4] = hview(L.dhc[0][nh - 1], B).ref; t.pm[5] = hview(L.dhc[1][nh - 1], B).ref;
+                TargetLossArgs &a = t.target_loss;
+                a.h[0] = hview(L.ht[0][nh - 1], B).ref; a.h[1] = hview(L.ht[1][nh - 1], B).ref;
+                a.h[2] = hview(L.hc[0][nh - 1], B).ref; a.h[3] = hview(L.hc[1][nh - 1], B).ref;
+                a.dh[0] = hview(L.dhc[0][nh - 1], B).ref; a.dh[1] = hview(L.dhc[1][nh - 1], B).ref;
                 const int nets[4] = {3, 4, 1, 2};
-                for (int k = 0; k < 4; k++) { t.p[4 + k] = A(L.param[nets[k]] + Q.w_out); t.p[8 + k] = A(L.param[nets[k]] + Q.b_out); }
-                t.p[12] = W(L.r); t.p[13] = W(L.d); t.p[14] = W(L.logp); t.p[15] = key.use_isw ? W(L.isw) : null_ref();
-                t.p[16] = W(L.y); t.p[17] = W(L.dq[0]); t.p[18] = W(L.dq[1]); t.p[19] = W(L.td);
-                t.p[22] = W(L.loss_part);
-                t.i[0] = B; t.i[1] = H; t.i[2] = loss_rows(); t.f[0] = h->cfg.gamma;
+                for (int k = 0; k < 4; k++) { a.w_out[k] = A(L.param[nets[k]] + Q.w_out); a.b_out[k] = A(L.param[nets[k]] + Q.b_out); }
+                a.r = W(L.r); a.d = W(L.d); a.logp_next = W(L.logp); a.is_weights = key.use_isw ? W(L.isw) : null_ref();
+                a.y = W(L.y); a.dq[0] = W(L.dq[0]); a.dq[1] = W(L.dq[1]); a.td = W(L.td);
+                a.partials = W(L.loss_part);
+                a.B = B; a.H = H; a.R = loss_rows(); a.gamma = h->cfg.gamma;
                 add(t, cdiv(B, loss_rows()));
             }
             // gradient at the Linear output of critic k's hidden layer x: the dh PM itself, or (LayerNorm variant) the dz PM behind it
@@ -798,13 +803,11 @@ struct Builder {
                     if (s == nh) dW(0);
                     if (s == 1) {   // output layer
                         Task t = blank(T_OUT_ADAM);
-                        AdamArgs aw = adam_args(net, Q.w_out), ab = adam_args(net, Q.b_out);
-                        t.pm[0] = hview(L.hc[k][nh - 1], B).ref; t.p[1] = W(L.dq[k]);
-                        t.p[2] = aw.w; t.p[3] = aw.m; t.p[4] = aw.v; t.p[5] = aw.wt; t.p[6] = aw.gexp;
-                        t.p[7] = ab.w; t.p[8] = ab.m; t.p[9] = ab.v; t.p[10] = ab.wt; t.p[11] = ab.gexp;
-                        t.i[0] = B; t.i[1] = H; t.i[2] = aw.step_slot; t.i[3] = aw.apply; t.f[0] = aw.lr; t.f[1] = aw.tau;
-                        t.i[5] = colsum_rows(B);
-                        add(t, (cdiv(H, kColsumCols) + 1) * cdiv(B, t.i[5]));      // + the bias tile, per row chunk
+                        OutAdamArgs &a = t.out_adam;
+                        a.w = adam_args(net, Q.w_out); a.b = adam_args(net, Q.b_out);
+                        a.h = hview(L.hc[k][nh - 1], B).ref; a.dq = W(L.dq[k]);
+                        a.B = B; a.H = H; a.chunk_rows = colsum_rows(B);
+                        add(t, (cdiv(H, kColsumCols) + 1) * cdiv(B, a.chunk_rows));      // + the bias tile, per row chunk
                     }
                 }
                 if (l >= 1) ln_bwd_c(l - 1);
@@ -828,12 +831,13 @@ struct Builder {
             begin_stage();
             {
                 Task t = blank(T_ACTOR_LOSS);
-                t.pm[0] = hview(L.ha[0][nh - 1], B).ref; t.pm[1] = hview(L.ha[1][nh - 1], B).ref;
-                t.pm[2] = hview(L.dha[0][nh - 1], B).ref; t.pm[3] = hview(L.dha[1][nh - 1], B).ref;
-                t.p[2] = A(L.param[1] + Q.w_out); t.p[3] = A(L.param[2] + Q.w_out);
-                t.p[4] = A(L.param[1] + Q.b_out); t.p[5] = A(L.param[2] + Q.b_out);
-                t.p[6] = W(L.logp + B); t.p[9] = W(L.aloss_part);
-                t.i[0] = B; t.i[1] = H; t.i[2] = loss_rows(); t.f[0] = -(float)act;
+                ActorLossArgs &a = t.actor_loss;
+                a.h[0] = hview(L.ha[0][nh - 1], B).ref; a.h[1] = hview(L.ha[1][nh - 1], B).ref;
+                a.dh[0] = hview(L.dha[0][nh - 1], B).ref; a.dh[1] = hview(L.dha[1][nh - 1], B).ref;
+                a.w_out[0] = A(L.param[1] + Q.w_out); a.w_out[1] = A(L.param[2] + Q.w_out);
+                a.b_out[0] = A(L.param[1] + Q.b_out); a.b_out[1] = A(L.param[2] + Q.b_out);
+                a.logp = W(L.logp + B); a.partials = W(L.aloss_part);
+                a.B = B; a.H = H; a.R = loss_rows(); a.target_entropy = -(float)act;
                 add(t, cdiv(B, loss_rows()));
             }
             // ---- dL/da through both critics (input gradients only: the Q weights are constants here, quirk Q2) -------
@@ -859,9 +863,10 @@ struct Builder {
             begin_stage();
             {
                 Task t = blank(T_SAMPLE_BWD);
-                t.p[0] = W(L.da[0]); t.p[1] = W(L.da[1]); t.p[2] = W(L.head_raw + (int64_t)B * A2); t.p[3] = W(L.eps + (int64_t)B * act);
-                t.pm[0] = ghead(B).ref;
-                t.i[0] = B; t.i[1] = act; t.f[0] = h->cfg.action_scale; t.f[1] = h->cfg.action_bias;
+                SampleBwdArgs &a = t.sample_bwd;
+                a.da[0] = W(L.da[0]); a.da[1] = W(L.da[1]); a.head = W(L.head_raw + (int64_t)B * A2); a.eps = W(L.eps + (int64_t)B * act);
+                a.g_head = ghead(B).ref;
+                a.B = B; a.A = act; a.scale = h->cfg.action_scale; a.bias = h->cfg.action_bias;
                 add(t, cdiv(B * act, kThreads));
             }
             // ---- policy backward (current-state rows B..2B of the policy activations) --------------------------------
@@ -910,14 +915,15 @@ struct Builder {
         {   // own stage: the Adam epilogues of the previous stage still read the step counters
             begin_stage();
             Task t = blank(T_FINISH);
+            FinishArgs &a = t.finish;
             const int ap = apply() ? 1 : 0;
-            t.p[0] = critics ? W(L.loss_part) : null_ref();
-            t.p[1] = actor ? W(L.aloss_part) : null_ref();
-            t.p[2] = exporting() ? A(L.grad_scalars) : null_ref();
-            t.p[3] = A(L.loss_hist);
-            t.i[0] = ap; t.i[1] = ap; t.i[2] = ap; t.i[3] = ap && h->cfg.auto_entropy; t.i[4] = ap;
-            t.i[5] = cdiv(B, loss_rows()) * (loss_rows() / kLossRows); t.i[6] = h->cfg.auto_entropy; t.i[7] = ap;
-            t.f[0] = h->cfg.lr; t.f[1] = (float)B;
+            a.critic_part = critics ? W(L.loss_part) : null_ref();
+            a.actor_part = actor ? W(L.aloss_part) : null_ref();
+            a.alpha_grad = exporting() ? A(L.grad_scalars) : null_ref();
+            a.loss_hist = A(L.loss_hist);
+            a.bump[0] = ap; a.bump[1] = ap; a.bump[2] = ap; a.bump[3] = ap && h->cfg.auto_entropy; a.bump_updates = ap;
+            a.n_part = cdiv(B, loss_rows()) * (loss_rows() / kLossRows); a.auto_entropy = h->cfg.auto_entropy; a.apply = ap;
+            a.B = (float)B;
             add(t, 1);
 
         }
@@ -975,7 +981,7 @@ static std::vector<Chain> find_chains(const std::vector<Task> &tasks, const std:
         std::vector<int64_t> out;
         for (int s = s0; s < s1; s++)
             for (int k = stages[s].task_begin; k < stages[s].task_end; k++)
-                out.push_back(tasks[k].type == T_GEMM ? tasks[k].Cpm.base.v : tasks[k].pm[0].base.v);
+                out.push_back(tasks[k].type == T_GEMM ? tasks[k].Cpm.base.v : tasks[k].shadow.dst.base.v);      // eligible(): T_SHADOW
         for (int s = s0; s < s1; s++)
             for (int k : gemms(s))
                 for (int64_t o : out)

@@ -73,9 +73,9 @@ __device__ __forceinline__ TileRef locate(const Program &P, const Misc &mi, int 
     int tile = tis - mi.tile_begin[k];
     r.bm = r.tg->bm; r.bn = r.tg->bn;
     const int tn = r.tg->tiles_n, per = r.tg->tiles_m * tn;
-    // split K (gradient-export GEMMs of large batches, Task::i[7] = K blocks per chunk): tile = [chunk][tm][tn], the chunks of an
-    // output tile are accumulated into the zeroed gradient slab with atomics by their epilogues
-    const int chunk = r.tg->i[7], nkb_all = cdiv(r.tg->K, kBK);
+    // split K (gradient-export GEMMs of large batches): tile = [chunk][tm][tn], the chunks of an output tile are accumulated into the
+    // zeroed gradient slab with atomics by their epilogues
+    const int chunk = r.tg->kb_per_chunk, nkb_all = cdiv(r.tg->K, kBK);
     r.kb0 = 0; r.nkb = nkb_all;
     if (chunk > 0) { r.kb0 = (tile / per) * chunk; r.nkb = max(0, min(nkb_all - r.kb0, chunk)); tile %= per; }
     r.m0 = (tile / tn) * r.bm; r.n0 = (tile % tn) * r.bn;
@@ -393,7 +393,7 @@ __device__ __forceinline__ void epilogue_tile(const EpiR &epi, float *Cs, float4
         }
         epi_bar();
         if (EPI == EPI_ADAM) {
-            adam_epilogue(epi, Cs, state, r.m0, n0c, et, r.tg->i[7] > 0);
+            adam_epilogue(epi, Cs, state, r.m0, n0c, et, r.tg->kb_per_chunk > 0);
             // the next pass's first two groups: in flight across the barrier and the next TMEM -> staging copy
             if (state && !last) for (int g0 = 0; g0 < kStateDepth; g0++) adam_issue(epi, state, r.m0, n0c + 64, et, g0, g0);
         } else plain_epilogue<EPI>(epi, Cs, r.m0, n0c, et, aux);

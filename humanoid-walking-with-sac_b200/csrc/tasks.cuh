@@ -1,6 +1,6 @@
 // Non-GEMM tile tasks of the SAC update program (weight shadows, gather, sampling, losses, bias / output-layer
-// optimiser steps).  Slot meaning of Task::p / pm / i / f is documented per task; the host builder (program.cu)
-// fills them.  Matrices that feed a GEMM are pair matrices (bf16 hi/lo planes, common.cuh).
+// optimiser steps).  Each body reads its own argument struct of Task's union (common.cuh), which the host builder (program.cu)
+// fills.  Matrices that feed a GEMM are pair matrices (bf16 hi/lo planes, common.cuh).
 #pragma once
 #include "gemm.cuh"
 #include "sample.cuh"
@@ -9,15 +9,14 @@ namespace sacb {
 
 constexpr int kShadowRows = 64;      // weight rows per T_SHADOW tile (4 per warp)
 
-// T_SHADOW: p0 = fp32 weight matrix (row stride i3) ; pm0 = shadow PM of its columns [i2, i2+i1) ; i0=rows i1=cols.  One warp per row.
-// Runs at the start of every step, so weights written from outside the update (load_state_dict through the
-// aliased torch tensors, checkpoint loads, the data-parallel apply kernel) are always picked up.
-__device__ __forceinline__ void task_shadow(const Task &t, int tile, const Program &P, int agent) {
-    const int rows = t.i[0], cols = t.i[1];
+// T_SHADOW: one warp per row.  Runs at the start of every step, so weights written from outside the update (load_state_dict
+// through the aliased torch tensors, checkpoint loads, the data-parallel apply kernel) are always picked up.
+__device__ __forceinline__ void task_shadow(const ShadowArgs &t, int tile, const Program &P, int agent) {
+    const int rows = t.rows, cols = t.cols;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const Pm dst = resolve_pm(t.pm[0], P.bases, agent);
-    const float *src0 = resolve(t.p[0], P.bases, agent) + t.i[2];
-    const bool even = ((t.i[3] | t.i[2]) & 1) == 0;     // every row starts 8 B aligned in src and 4 B aligned in dst
+    const Pm dst = resolve_pm(t.dst, P.bases, agent);
+    const float *src0 = resolve(t.src, P.bases, agent) + t.col0;
+    const bool even = ((t.src_ld | t.col0) & 1) == 0;     // every row starts 8 B aligned in src and 4 B aligned in dst
     constexpr int kR = kShadowRows / (kThreads / 32);    // rows per warp, handled together: kR independent loads in flight per trip
     const int r0 = tile * kShadowRows + warp;
     constexpr int kU = 4;                                // column chunks handled together: kR * kU independent loads in flight per trip
@@ -31,7 +30,7 @@ __device__ __forceinline__ void task_shadow(const Task &t, int tile, const Progr
                 const int c = c0 + 64 * u;
                 x[i][u] = make_float2(0.f, 0.f);
                 if (r < rows && c < cols) {
-                    const float *src = src0 + (int64_t)r * t.i[3] + c;
+                    const float *src = src0 + (int64_t)r * t.src_ld + c;
                     if (even) x[i][u] = __ldcg(reinterpret_cast<const float2 *>(src));
                     else { x[i][u].x = ldcg(src); if (c + 1 < cols) x[i][u].y = ldcg(src + 1); }
                 }
@@ -56,7 +55,7 @@ __device__ __forceinline__ void task_shadow(const Task &t, int tile, const Progr
     }
 }
 
-// T_GATHER: pm0 = X PM [3B, ldx] ; p0=r ; p1=d ; i0=B i1=obs i2=act ; ring row = [s | s2 | a | r | d] (16 B aligned)
+// T_GATHER: ring row = [s | s2 | a | r | d] (16 B aligned)
 //   X rows [0,B) <- (s2, .)   rows [B,2B) <- (s, a)   rows [2B,3B) <- (s, .)
 // four rows per tile, four warps per sampled row: one warp per destination row (the fourth moves r and d).  A lane forms
 // pairs of neighbouring destination columns (one 4-byte store per bf16 plane); ring reads are coalesced streaming loads,
@@ -84,27 +83,27 @@ __device__ __forceinline__ uint32_t draw_position(uint32_t b, uint32_t n, uint64
     return x;
 }
 
-__device__ __forceinline__ void task_gather(const Task &t, int tile, const Program &P, int agent, const float *scalars, uint64_t seed) {
-    const int B = t.i[0], obs = t.i[1], act = t.i[2];
+__device__ __forceinline__ void task_gather(const GatherArgs &t, int tile, const Program &P, int agent, const float *scalars, uint64_t seed) {
+    const int B = t.B, obs = t.obs, act = t.act;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int b = tile * 4 + (warp >> 2), part = warp & 3;
     if (b >= B) return;
     int slot;
-    if (t.i[3]) {      // indices drawn here (the four warps of a row compute the same slot); recorded for the host / tests
+    if (t.device_draw) {      // indices drawn here (the four warps of a row compute the same slot); recorded for the host / tests
         const int64_t n = P.ring_meta[2 * agent], head = P.ring_meta[2 * agent + 1];
         const uint32_t step = (uint32_t)__float_as_int(ldcg(scalars + SC_N_UPDATES));
-        slot = (int)((head + draw_position((uint32_t)b, (uint32_t)n, seed, (uint32_t)agent, step)) % t.i[4]);
+        slot = (int)((head + draw_position((uint32_t)b, (uint32_t)n, seed, (uint32_t)agent, step)) % t.capacity);
         if (part == 3 && lane == 2) const_cast<int32_t *>(P.slots)[(int64_t)agent * P.slots_stride + b] = slot;
     } else {
         slot = P.slots[(int64_t)agent * P.slots_stride + b];
     }
     const float *row = P.ring + agent * P.ring_agent_stride + (int64_t)slot * P.ring_row;
     if (part == 3) {
-        if (lane == 0) resolve(t.p[0], P.bases, agent)[b] = __ldcs(row + 2 * obs + act);
-        if (lane == 1) resolve(t.p[1], P.bases, agent)[b] = __ldcs(row + 2 * obs + act + 1);
+        if (lane == 0) resolve(t.r, P.bases, agent)[b] = __ldcs(row + 2 * obs + act);
+        if (lane == 1) resolve(t.d, P.bases, agent)[b] = __ldcs(row + 2 * obs + act + 1);
         return;
     }
-    const Pm X = resolve_pm(t.pm[0], P.bases, agent);
+    const Pm X = resolve_pm(t.x, P.bases, agent);
     const int xrow = part == 0 ? b : (part == 1 ? B + b : 2 * B + b);
     const int ncols = part == 1 ? obs + act : obs;
     auto src = [&](int c) -> float {       // destination column -> ring element
@@ -133,34 +132,32 @@ __device__ __forceinline__ void task_gather(const Task &t, int tile, const Progr
     }
 }
 
-// T_SAMPLE: p0=head_raw [2B,2A] (mean | log_std_raw) ; p1=eps [2B,A] (i4: 1 -> Philox draw, kept for the backward) ;
-//   pm0 = X PM ; p3=logp [2B] ; i0=B i1=A i2=obs ; f0=scale f1=bias.
-//   row j<B: next-state sample -> X[j, obs:] ; j>=B: current-state sample -> X[2B + (j-B), obs:]
-__device__ __forceinline__ void task_sample(const Task &t, int tile, const Program &P, int agent, const float *scalars, uint64_t seed) {
-    const int B = t.i[0], A = t.i[1], obs = t.i[2];
+// T_SAMPLE: one warp per sampled row
+__device__ __forceinline__ void task_sample(const SampleArgs &t, int tile, const Program &P, int agent, const float *scalars, uint64_t seed) {
+    const int B = t.B, A = t.A, obs = t.obs;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int j = tile * (kThreads / 32) + warp;
     if (j >= 2 * B) return;
-    const float *head = resolve(t.p[0], P.bases, agent) + (int64_t)j * 2 * A;
-    float *eps = resolve(t.p[1], P.bases, agent);
-    const Pm X = resolve_pm(t.pm[0], P.bases, agent);
+    const float *head = resolve(t.head, P.bases, agent) + (int64_t)j * 2 * A;
+    float *eps = resolve(t.eps, P.bases, agent);
+    const Pm X = resolve_pm(t.x, P.bases, agent);
     const int xrow = j < B ? j : 2 * B + (j - B);
     const uint32_t step = (uint32_t)__float_as_int(ldcg(scalars + SC_N_UPDATES));
     float lp = 0.f;
     for (int a = lane; a < A; a += 32) {
         float e;
-        if (t.i[4]) {   // production mode: draw on device and keep the draw for the backward pass
+        if (t.device_eps) {   // production mode: draw on device and keep the draw for the backward pass
             e = philox_normal(seed, (uint32_t)agent, step, (uint32_t)j, (uint32_t)a);
             eps[(int64_t)j * A + a] = e;
         } else {
             e = ldcg(eps + (int64_t)j * A + a);
         }
-        const SampleElem s = sample_elem(ldcg(head + a), ldcg(head + A + a), e, t.f[0], t.f[1]);
+        const SampleElem s = sample_elem(ldcg(head + a), ldcg(head + A + a), e, t.scale, t.bias);
         pm_store(X, xrow, obs + a, s.action);
         lp += s.logp;
     }
     lp = warp_sum(lp);
-    if (lane == 0) resolve(t.p[3], P.bases, agent)[j] = lp;
+    if (lane == 0) resolve(t.logp, P.bases, agent)[j] = lp;
 }
 
 // dot product of one PM activation row with an fp32 weight vector (H % 8 == 0): 8 elements per lane per trip
@@ -251,7 +248,7 @@ __device__ __forceinline__ void write_dh_last4(const Pm &dh, const Pm &h, const 
     }
 }
 
-// The two loss tasks work on R = Task::i[2] batch rows per tile: R = 4 (latency programs: 4 warps per row, one per network, 64
+// The two loss tasks work on R batch rows per tile: R = 4 (latency programs: 4 warps per row, one per network, 64
 // tiles at B = 256) or R = 16 (throughput programs: a warp takes one network for 4 rows, all of their loads in flight together;
 // four times fewer dependent round trips per row).  Warp w handles the pairs (row, net) = (w / 4 + 4 j, w % 4), j < R / 4.
 constexpr int kLossRows = 4, kLossRowsMax = 16;
@@ -259,30 +256,24 @@ constexpr int kLossRows = 4, kLossRowsMax = 16;
 // T_TARGET_LOSS: Bellman target + critic MSE terms + dL/dq   (sac_imp.py:92-105).
 // Warp (row, k) forms the output-layer dot product of net k for its rows, one thread per row then does the scalar arithmetic,
 // the warps of nets 2, 3 (q1, q2) finally write dL/dh of the last hidden layer.
-//   pm0,pm1 = last hidden activations of q1_target,q2_target on (s2,a2) [B,H] ; pm2,pm3 = of q1,q2 on (s,a)
-//   p4..p7 = output-layer weights [H] of q1t,q2t,q1,q2 ; p8..p11 = their biases [1]
-//   p12=r p13=d p14=logp_next p15=is_weights(null -> 1) ; outputs p16=y p17=dq1 p18=dq2 p19=td (|q1-y|)
-//   pm4,pm5 = dL/dh of the last hidden layer of q1,q2 [B,H] (consumed by the critic backward GEMMs)
-//   p[22] = per-tile partial sums of w*(q-y)^2 [n_tiles, 2] (summed in tile order by T_FINISH: deterministic)
-//   i0=B i1=H i2=R ; f0=gamma
-__device__ __forceinline__ void task_target_loss(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
-    const int B = t.i[0], H = t.i[1], R = t.i[2], nj = R >> 2;
+__device__ __forceinline__ void task_target_loss(const TargetLossArgs &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
+    const int B = t.B, H = t.H, R = t.R, nj = R >> 2;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int k = warp & 3, r_w = warp >> 2;
     float *sq = smem, *sd = smem + 4 * kLossRowsMax, *sl = sd + 2 * kLossRowsMax;      // dots [R][4 nets], dq [R][2], loss terms [R][2]
-    const Pm h = resolve_pm(t.pm[k], P.bases, agent);
-    const float *w = resolve(t.p[4 + k], P.bases, agent);
+    const Pm h = resolve_pm(t.h[k], P.bases, agent);
+    const float *w = resolve(t.w_out[k], P.bases, agent);
     // the row's scalars are fetched by its scalar thread BEFORE the dot products, so their latency hides behind them
     float pre_bias[4] = {0.f, 0.f, 0.f, 0.f}, pre_alpha = 0.f, pre_logp = 0.f, pre_r = 0.f, pre_d = 0.f, pre_w = 1.f;
     if ((int)threadIdx.x < R && tile * R + (int)threadIdx.x < B) {
         const int br = tile * R + threadIdx.x;
-        for (int j = 0; j < 4; j++) pre_bias[j] = ldcg(resolve(t.p[8 + j], P.bases, agent));
+        for (int j = 0; j < 4; j++) pre_bias[j] = ldcg(resolve(t.b_out[j], P.bases, agent));
         const int n_upd = __float_as_int(ldcg(scalars + SC_N_UPDATES));
         pre_alpha = ldcg(scalars + SC_ALPHA0 + (n_upd & 1));
-        const float *isw = resolve(t.p[15], P.bases, agent);
-        pre_logp = ldcg(resolve(t.p[14], P.bases, agent) + br);
-        pre_r = ldcg(resolve(t.p[12], P.bases, agent) + br);
-        pre_d = ldcg(resolve(t.p[13], P.bases, agent) + br);
+        const float *isw = resolve(t.is_weights, P.bases, agent);
+        pre_logp = ldcg(resolve(t.logp_next, P.bases, agent) + br);
+        pre_r = ldcg(resolve(t.r, P.bases, agent) + br);
+        pre_d = ldcg(resolve(t.d, P.bases, agent) + br);
         if (isw) pre_w = ldcg(isw + br);
     }
     int64_t rows4[4];
@@ -308,22 +299,22 @@ __device__ __forceinline__ void task_target_loss(const Task &t, int tile, const 
             const float alpha = pre_alpha;
             const float qn = fminf(qq[0], qq[1]);
             const float vt = qn - alpha * pre_logp;                                   // sac_imp.py:97
-            const float yy = pre_r + (1.f - pre_d) * t.f[0] * vt;                     // :98
+            const float yy = pre_r + (1.f - pre_d) * t.gamma * vt;                     // :98
             const float wgt = pre_w;
             const float e1 = qq[2] - yy, e2 = qq[3] - yy;
             dq1 = 2.f * wgt * e1 / (float)B;                                                                          // d mean((q-y)^2) / dq
             dq2 = 2.f * wgt * e2 / (float)B;
-            resolve(t.p[16], P.bases, agent)[br] = yy;
-            resolve(t.p[17], P.bases, agent)[br] = dq1;
-            resolve(t.p[18], P.bases, agent)[br] = dq2;
-            resolve(t.p[19], P.bases, agent)[br] = fabsf(e1);
+            resolve(t.y, P.bases, agent)[br] = yy;
+            resolve(t.dq[0], P.bases, agent)[br] = dq1;
+            resolve(t.dq[1], P.bases, agent)[br] = dq2;
+            resolve(t.td, P.bases, agent)[br] = fabsf(e1);
             l1 = wgt * e1 * e1; l2 = wgt * e2 * e2;
         }
         sd[2 * r] = dq1; sd[2 * r + 1] = dq2; sl[2 * r] = l1; sl[2 * r + 1] = l2;
     }
     __syncthreads();
     if (k >= 2) {
-        const Pm dh = resolve_pm(t.pm[2 + k], P.bases, agent);
+        const Pm dh = resolve_pm(t.dh[k - 2], P.bases, agent);
         if (nj == 4) {
             float dq4[4];
             for (int j = 0; j < 4; j++) dq4[j] = sd[2 * (r_w + 4 * j) + (k - 2)];
@@ -336,7 +327,7 @@ __device__ __forceinline__ void task_target_loss(const Task &t, int tile, const 
         const int sub = threadIdx.x;
         float s1 = 0.f, s2 = 0.f;
         for (int i = kLossRows * sub; i < kLossRows * (sub + 1); i++) { s1 += sl[2 * i]; s2 += sl[2 * i + 1]; }
-        float *part = resolve(t.p[22], P.bases, agent);
+        float *part = resolve(t.partials, P.bases, agent);
         part[2 * (tile * nj + sub)] = s1; part[2 * (tile * nj + sub) + 1] = s2;
     }
     __syncthreads();
@@ -344,23 +335,19 @@ __device__ __forceinline__ void task_target_loss(const Task &t, int tile, const 
 
 // T_ACTOR_LOSS: policy-loss terms and min-Q routing (sac_imp.py:117-121).  Same tiling: the warps of "nets" 0, 1 form the two dot
 // products, those of 2, 3 write dL/dh of the last hidden layer of q1, q2.
-//   pm0,pm1 = last hidden activations of q1,q2 on (s, a_new) ; p2,p3 = output weights ; p4,p5 = output biases
-//   p6=logp_cur ; pm2,pm3 = dL/dh of the last hidden layer of q1,q2 (the Q weights are constants here, quirk Q2)
-//   p9 = per-tile partials [n_tiles,2]: sum(alpha*logp - minq), sum(logp + target_entropy)
-//   i0=B i1=H i2=R ; f0=target_entropy
-__device__ __forceinline__ void task_actor_loss(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
-    const int B = t.i[0], H = t.i[1], R = t.i[2], nj = R >> 2;
+__device__ __forceinline__ void task_actor_loss(const ActorLossArgs &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
+    const int B = t.B, H = t.H, R = t.R, nj = R >> 2;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int k = warp & 3, r_w = warp >> 2;
     float *sq = smem, *sd = smem + 4 * kLossRowsMax, *sl = sd + 2 * kLossRowsMax;
-    const Pm h = resolve_pm(t.pm[k & 1], P.bases, agent);
-    const float *w = resolve(t.p[2 + (k & 1)], P.bases, agent);
+    const Pm h = resolve_pm(t.h[k & 1], P.bases, agent);
+    const float *w = resolve(t.w_out[k & 1], P.bases, agent);
     float pre_b1 = 0.f, pre_b2 = 0.f, pre_alpha = 0.f, pre_logp = 0.f;      // fetched before the dot products (latency hidden)
     if ((int)threadIdx.x < R && tile * R + (int)threadIdx.x < B) {
-        pre_b1 = ldcg(resolve(t.p[4], P.bases, agent)); pre_b2 = ldcg(resolve(t.p[5], P.bases, agent));
+        pre_b1 = ldcg(resolve(t.b_out[0], P.bases, agent)); pre_b2 = ldcg(resolve(t.b_out[1], P.bases, agent));
         const int n_upd = __float_as_int(ldcg(scalars + SC_N_UPDATES));
         pre_alpha = ldcg(scalars + SC_ALPHA0 + (n_upd & 1));
-        pre_logp = ldcg(resolve(t.p[6], P.bases, agent) + tile * R + threadIdx.x);
+        pre_logp = ldcg(resolve(t.logp, P.bases, agent) + tile * R + threadIdx.x);
     }
     int64_t rows4[4];
     bool on4[4];
@@ -389,13 +376,13 @@ __device__ __forceinline__ void task_actor_loss(const Task &t, int tile, const P
             const float sel = q1 < q2 ? 1.f : (q1 == q2 ? 0.5f : 0.f);               // torch.minimum backward
             d1 = -sel / (float)B;
             d2 = -(1.f - sel) / (float)B;
-            ent = l + t.f[0];
+            ent = l + t.target_entropy;
         }
         sd[2 * r] = d1; sd[2 * r + 1] = d2; sl[2 * r] = pl; sl[2 * r + 1] = ent;
     }
     __syncthreads();
     if (k >= 2) {
-        const Pm dh = resolve_pm(t.pm[k], P.bases, agent);
+        const Pm dh = resolve_pm(t.dh[k - 2], P.bases, agent);
         if (nj == 4) {
             float dq4[4];
             for (int j = 0; j < 4; j++) dq4[j] = sd[2 * (r_w + 4 * j) + (k - 2)];
@@ -408,28 +395,27 @@ __device__ __forceinline__ void task_actor_loss(const Task &t, int tile, const P
         const int sub = threadIdx.x;
         float s1 = 0.f, s2 = 0.f;
         for (int i = kLossRows * sub; i < kLossRows * (sub + 1); i++) { s1 += sl[2 * i]; s2 += sl[2 * i + 1]; }
-        float *part = resolve(t.p[9], P.bases, agent);
+        float *part = resolve(t.partials, P.bases, agent);
         part[2 * (tile * nj + sub)] = s1; part[2 * (tile * nj + sub) + 1] = s2;
     }
     __syncthreads();
 }
 
-// T_SAMPLE_BWD: p0=da1 p1=da2 [B,A] ; p2=head_raw rows of the current-state sample ; p3=eps_cur ; pm0=g_head PM [B,2A]
-//   i0=B i1=A ; f0=scale f1=bias    (closed form of SURVEY 3.3)
-__device__ __forceinline__ void task_sample_bwd(const Task &t, int tile, const Program &P, int agent, const float *scalars) {
-    const int B = t.i[0], A = t.i[1];
+// T_SAMPLE_BWD: closed form of SURVEY 3.3, one thread per (row, action) element
+__device__ __forceinline__ void task_sample_bwd(const SampleBwdArgs &t, int tile, const Program &P, int agent, const float *scalars) {
+    const int B = t.B, A = t.A;
     const int idx = tile * kThreads + threadIdx.x;
     if (idx >= B * A) return;
     const int b = idx / A, a = idx % A;
     const int n_upd = __float_as_int(ldcg(scalars + SC_N_UPDATES));
     const float alpha = ldcg(scalars + SC_ALPHA0 + (n_upd & 1));
-    const float *head = resolve(t.p[2], P.bases, agent) + (int64_t)b * 2 * A;
-    const float eps = ldcg(resolve(t.p[3], P.bases, agent) + idx);
-    const SampleElem s = sample_elem(ldcg(head + a), ldcg(head + A + a), eps, t.f[0], t.f[1]);
-    const float da = ldcg(resolve(t.p[0], P.bases, agent) + idx) + ldcg(resolve(t.p[1], P.bases, agent) + idx);
-    const float sc = t.f[0], omy2 = 1.f - s.y * s.y, aB = alpha / (float)B;
+    const float *head = resolve(t.head, P.bases, agent) + (int64_t)b * 2 * A;
+    const float eps = ldcg(resolve(t.eps, P.bases, agent) + idx);
+    const SampleElem s = sample_elem(ldcg(head + a), ldcg(head + A + a), eps, t.scale, t.bias);
+    const float da = ldcg(resolve(t.da[0], P.bases, agent) + idx) + ldcg(resolve(t.da[1], P.bases, agent) + idx);
+    const float sc = t.scale, omy2 = 1.f - s.y * s.y, aB = alpha / (float)B;
     const float g_u = da * sc * omy2 + aB * (2.f * sc * s.y * omy2) / (sc * omy2 + kSquashEps);
-    const Pm g = resolve_pm(t.pm[0], P.bases, agent);
+    const Pm g = resolve_pm(t.g_head, P.bases, agent);
     pm_store(g, b, a, g_u);
     pm_store(g, b, A + a, (g_u * s.std * eps - aB) * s.in_range);
 }
@@ -511,15 +497,13 @@ __device__ __forceinline__ void colsum_finish(float g, bool chunked, float *ge, 
     if (apply) adam_prefetched(g, st, w, m, v, wt, ss, bs, tau);
 }
 
-// T_OUT_ADAM: Q output layer (Linear(H,1)).  pm0=h_L PM [B,H] p1=dq [B] ; p2..p6 = w,m,v,wt,gexp [H] ; p7..p11 = same for bias
-//   i0=B i1=H i2=step_slot i3=apply i5=rows per chunk (>= B: one chunk) ; f0=lr f1=tau.
-//   tiles: [row chunk][64-column tile] for the weight gradient, then one bias tile per row chunk
+// T_OUT_ADAM tiles: [row chunk][64-column tile] for the weight gradient, then one bias tile per row chunk
 template <bool kDeep = true>
-__device__ __forceinline__ void task_out_adam(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
-    const int B = t.i[0], H = t.i[1], R = t.i[5], n_ct = cdiv(H, kColsumCols), n_rc = cdiv(B, R);
-    const float *dq = resolve(t.p[1], P.bases, agent);
+__device__ __forceinline__ void task_out_adam(const OutAdamArgs &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
+    const int B = t.B, H = t.H, R = t.chunk_rows, n_ct = cdiv(H, kColsumCols), n_rc = cdiv(B, R);
+    const float *dq = resolve(t.dq, P.bases, agent);
     float ss, bs;
-    adam_factors_cached(scalars, t.i[2], ss, bs);
+    adam_factors_cached(scalars, t.w.step_slot, ss, bs);
     if (tile >= n_ct * n_rc) {      // bias tile of row chunk tile - n_ct * n_rc: db = sum_b dq[b] (32 lane partials, then the warp tree)
         const int rc = tile - n_ct * n_rc, r0 = rc * R, r1 = min(B, r0 + R);
         if (threadIdx.x < 32) {
@@ -527,20 +511,22 @@ __device__ __forceinline__ void task_out_adam(const Task &t, int tile, const Pro
             for (int b = r0 + threadIdx.x; b < r1; b += 32) gb += ldcg(dq + b);
             gb = warp_sum(gb);
             if (threadIdx.x == 0) {
-                float *w = resolve(t.p[7], P.bases, agent), *m = resolve(t.p[8], P.bases, agent), *v = resolve(t.p[9], P.bases, agent);
-                float *wt = resolve(t.p[10], P.bases, agent), *ge = resolve(t.p[11], P.bases, agent);
-                colsum_finish(gb, n_rc > 1, ge, t.i[3], prefetch_state(t.i[3] != 0, w, m, v, wt), w, m, v, wt, ss, bs, t.f[1]);
+                const AdamArgs &a = t.b;
+                float *w = resolve(a.w, P.bases, agent), *m = resolve(a.m, P.bases, agent), *v = resolve(a.v, P.bases, agent);
+                float *wt = resolve(a.wt, P.bases, agent), *ge = resolve(a.gexp, P.bases, agent);
+                colsum_finish(gb, n_rc > 1, ge, a.apply, prefetch_state(a.apply != 0, w, m, v, wt), w, m, v, wt, ss, bs, a.tau);
             }
         }
         return;
     }
     const int ct = tile % n_ct, rc = tile / n_ct, r0 = rc * R, r1 = min(B, r0 + R);
     const int n = ct * kColsumCols + threadIdx.x;
-    const Pm h = resolve_pm(t.pm[0], P.bases, agent);
+    const Pm h = resolve_pm(t.h, P.bases, agent);
     const bool owner = threadIdx.x < kColsumCols && n < H;
-    float *w = resolve(t.p[2], P.bases, agent) + n, *m = resolve(t.p[3], P.bases, agent) + n, *v = resolve(t.p[4], P.bases, agent) + n;
-    float *wt = resolve(t.p[5], P.bases, agent), *ge = resolve(t.p[6], P.bases, agent);
-    const PreState st = prefetch_state(owner && t.i[3], w, m, v, wt ? wt + n : nullptr);
+    const AdamArgs &a = t.w;
+    float *w = resolve(a.w, P.bases, agent) + n, *m = resolve(a.m, P.bases, agent) + n, *v = resolve(a.v, P.bases, agent) + n;
+    float *wt = resolve(a.wt, P.bases, agent), *ge = resolve(a.gexp, P.bases, agent);
+    const PreState st = prefetch_state(owner && a.apply, w, m, v, wt ? wt + n : nullptr);
     const int c0 = ct * kColsumCols;
     const float g = colsum64<kDeep>(r0, r1, smem, [&](int b, int c, float (&out)[8]) {
         if (c0 + c < h.ld) {
@@ -553,21 +539,21 @@ __device__ __forceinline__ void task_out_adam(const Task &t, int tile, const Pro
             for (int j = 0; j < 8; j++) out[j] = 0.f;
         }
     });
-    if (owner) colsum_finish(g, n_rc > 1, ge ? ge + n : nullptr, t.i[3], st, w, m, v, wt ? wt + n : nullptr, ss, bs, t.f[1]);
+    if (owner) colsum_finish(g, n_rc > 1, ge ? ge + n : nullptr, a.apply, st, w, m, v, wt ? wt + n : nullptr, ss, bs, a.tau);
 }
 
-// T_BIAS_ADAM: db[n] = sum_b dh[b,n].  pm0 = dh PM [B,N] ; p0..p4 = b,m,v,bt,gexp ; i0=B i1=N i2=step_slot i3=apply
-//   i5=rows per chunk ; f0=lr f1=tau.   tiles: [row chunk][64-column tile]
+// T_BIAS_ADAM tiles: [row chunk][64-column tile]
 template <bool kDeep = true>
-__device__ __forceinline__ void task_bias_adam(const Task &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
-    const int B = t.i[0], N = t.i[1], R = t.i[5], n_ct = cdiv(N, kColsumCols), n_rc = cdiv(B, R);
+__device__ __forceinline__ void task_bias_adam(const ColsumAdamArgs &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
+    const int B = t.B, N = t.N, R = t.chunk_rows, n_ct = cdiv(N, kColsumCols), n_rc = cdiv(B, R);
     const int ct = tile % n_ct, rc = tile / n_ct, r0 = rc * R, r1 = min(B, r0 + R);
     const int n = ct * kColsumCols + threadIdx.x;
-    const Pm dh = resolve_pm(t.pm[0], P.bases, agent);
+    const Pm dh = resolve_pm(t.src, P.bases, agent);
     const bool owner = threadIdx.x < kColsumCols && n < N;
-    float *w = resolve(t.p[0], P.bases, agent) + n, *m = resolve(t.p[1], P.bases, agent) + n, *v = resolve(t.p[2], P.bases, agent) + n;
-    float *bt = resolve(t.p[3], P.bases, agent), *ge = resolve(t.p[4], P.bases, agent);
-    const PreState st = prefetch_state(owner && t.i[3], w, m, v, bt ? bt + n : nullptr);
+    const AdamArgs &a = t.adam;
+    float *w = resolve(a.w, P.bases, agent) + n, *m = resolve(a.m, P.bases, agent) + n, *v = resolve(a.v, P.bases, agent) + n;
+    float *bt = resolve(a.wt, P.bases, agent), *ge = resolve(a.gexp, P.bases, agent);
+    const PreState st = prefetch_state(owner && a.apply, w, m, v, bt ? bt + n : nullptr);
     const int c0 = ct * kColsumCols;
     const float g = colsum64<kDeep>(r0, r1, smem, [&](int b, int c, float (&out)[8]) {
         if (c0 + c < dh.ld) pm_load8(dh, b, c0 + c, out);
@@ -578,8 +564,8 @@ __device__ __forceinline__ void task_bias_adam(const Task &t, int tile, const Pr
     });
     if (owner) {
         float ss, bs;
-        adam_factors_cached(scalars, t.i[2], ss, bs);
-        colsum_finish(g, n_rc > 1, ge ? ge + n : nullptr, t.i[3], st, w, m, v, bt ? bt + n : nullptr, ss, bs, t.f[1]);
+        adam_factors_cached(scalars, a.step_slot, ss, bs);
+        colsum_finish(g, n_rc > 1, ge ? ge + n : nullptr, a.apply, st, w, m, v, bt ? bt + n : nullptr, ss, bs, a.tau);
     }
 }
 
@@ -598,14 +584,12 @@ __device__ __forceinline__ void load8f(const float *p, float (&out)[8]) {
     const float4 a = __ldcg(reinterpret_cast<const float4 *>(p)), b = __ldcg(reinterpret_cast<const float4 *>(p + 4));
     out[0] = a.x; out[1] = a.y; out[2] = a.z; out[3] = a.w; out[4] = b.x; out[5] = b.y; out[6] = b.z; out[7] = b.w;
 }
-// T_LN_FWD: h = relu((z - mean) * rstd * gamma + beta), mean / biased variance over the H columns of the row (torch.nn.LayerNorm, eps f0).
-//   p0 = z fp32 [rows, H] (Linear output incl. bias, written by the GEMM of the stage before) ; p1 = gamma [H] ; p2 = beta [H] ;
-//   p3 = statistics out [rows][2] = (mean, rstd) ; pm0 = h PM [rows, H] ; i0 = rows ; i1 = H ; f0 = eps
-__device__ __forceinline__ void task_ln_fwd(const Task &t, int tile, const Program &P, int agent) {
-    const int rows = t.i[0], H = t.i[1], warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+// T_LN_FWD: h = relu((z - mean) * rstd * gamma + beta), mean / biased variance over the H columns of the row (torch.nn.LayerNorm)
+__device__ __forceinline__ void task_ln_fwd(const LnFwdArgs &t, int tile, const Program &P, int agent) {
+    const int rows = t.rows, H = t.H, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int row = tile * kLnRows + warp;
     if (row >= rows) return;      // warp-uniform
-    const float *z = resolve(t.p[0], P.bases, agent) + (int64_t)row * H, *gam = resolve(t.p[1], P.bases, agent), *bet = resolve(t.p[2], P.bases, agent);
+    const float *z = resolve(t.z, P.bases, agent) + (int64_t)row * H, *gam = resolve(t.gamma, P.bases, agent), *bet = resolve(t.beta, P.bases, agent);
     float v[kLnTrips][8];
     float s = 0.f;
 #pragma unroll
@@ -625,8 +609,8 @@ __device__ __forceinline__ void task_ln_fwd(const Task &t, int tile, const Progr
 #pragma unroll
             for (int i = 0; i < 8; i++) { const float d = v[u][i] - mean; q += d * d; }
         }
-    const float rstd = 1.0f / sqrtf(warp_sum(q) / (float)H + t.f[0]);
-    const Pm h = resolve_pm(t.pm[0], P.bases, agent);
+    const float rstd = 1.0f / sqrtf(warp_sum(q) / (float)H + t.eps);
+    const Pm h = resolve_pm(t.h, P.bases, agent);
 #pragma unroll
     for (int u = 0; u < kLnTrips; u++) {
         const int j = u * 256 + lane * 8;
@@ -638,22 +622,20 @@ __device__ __forceinline__ void task_ln_fwd(const Task &t, int tile, const Progr
             pm_store8(h, row, j, y);
         }
     }
-    if (lane == 0) { float *st = resolve(t.p[3], P.bases, agent) + 2 * (int64_t)row; st[0] = mean; st[1] = rstd; }
+    if (lane == 0) { float *st = resolve(t.stats, P.bases, agent) + 2 * (int64_t)row; st[0] = mean; st[1] = rstd; }
 }
 // T_LN_BWD: dpre = gradient at the LayerNorm output (ReLU mask already applied by the producer) -> dz = gradient at the Linear output:
 //   g = dpre * gamma ; xhat = (z - mean) * rstd ; dz = rstd * (g - mean_j(g) - xhat * mean_j(g * xhat)) ; gg = dpre * xhat (its column
 //   sums over the batch are dgamma, those of dpre are dbeta: T_BIAS_ADAM tasks)
-//   pm0 = dpre PM [B, H] ; p0 = z fp32 (first of the B rows) ; p1 = gamma ; p3 = statistics (first of the B rows) ;
-//   pm1 = dz PM out ; pm2 = gg PM out (null base: not wanted) ; i0 = B ; i1 = H
-__device__ __forceinline__ void task_ln_bwd(const Task &t, int tile, const Program &P, int agent) {
-    const int rows = t.i[0], H = t.i[1], warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+__device__ __forceinline__ void task_ln_bwd(const LnBwdArgs &t, int tile, const Program &P, int agent) {
+    const int rows = t.rows, H = t.H, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int row = tile * kLnRows + warp;
     if (row >= rows) return;
-    const float *z = resolve(t.p[0], P.bases, agent) + (int64_t)row * H, *gam = resolve(t.p[1], P.bases, agent);
-    const float *st = resolve(t.p[3], P.bases, agent) + 2 * (int64_t)row;
+    const float *z = resolve(t.z, P.bases, agent) + (int64_t)row * H, *gam = resolve(t.gamma, P.bases, agent);
+    const float *st = resolve(t.stats, P.bases, agent) + 2 * (int64_t)row;
     const float mean = ldcg(st), rstd = ldcg(st + 1);
-    const Pm dpre = resolve_pm(t.pm[0], P.bases, agent), dz = resolve_pm(t.pm[1], P.bases, agent);
-    const bool want_gg = !is_null(t.pm[2].base);
+    const Pm dpre = resolve_pm(t.dpre, P.bases, agent), dz = resolve_pm(t.dz, P.bases, agent);
+    const bool want_gg = !is_null(t.gg.base);
     float g[kLnTrips][8], xh[kLnTrips][8];
     float s1 = 0.f, s2 = 0.f;
 #pragma unroll
@@ -668,7 +650,7 @@ __device__ __forceinline__ void task_ln_bwd(const Task &t, int tile, const Progr
                 float gg[8];
 #pragma unroll
                 for (int i = 0; i < 8; i++) gg[i] = d[i] * xh[u][i];
-                pm_store8(resolve_pm(t.pm[2], P.bases, agent), row, j, gg);
+                pm_store8(resolve_pm(t.gg, P.bases, agent), row, j, gg);
             }
         }
     }
@@ -687,13 +669,10 @@ __device__ __forceinline__ void task_ln_bwd(const Task &t, int tile, const Progr
 
 // T_FINISH (one thread): finalise the loss scalars from the per-tile partials (fixed order), the temperature step
 // (sac_imp.py:128-135) and the optimizer step counters (+1 each, sac_imp.py:109,113,125,134).
-//   p0 = critic partials [nt,2] (null: skip) ; p1 = actor partials [nt,2] (null: skip) ; p2 = exported log_alpha gradient (or null)
-//   i0..i3 = bump step_policy,q1,q2,alpha ; i4 = bump n_updates ; i5 = n_tiles of the partial arrays ; i6 = auto_entropy ; i7 = apply
-//   f0 = lr ; f1 = B
-__device__ __forceinline__ void task_finish(const Task &t, const Program &P, int agent, float *scalars, float *smem) {
-    const int nt = t.i[5];
-    const float Bf = t.f[1];
-    const float *cp = resolve(t.p[0], P.bases, agent), *ap = resolve(t.p[1], P.bases, agent);
+__device__ __forceinline__ void task_finish(const FinishArgs &t, const Program &P, int agent, float *scalars, float *smem) {
+    const int nt = t.n_part;
+    const float Bf = t.B;
+    const float *cp = resolve(t.critic_part, P.bases, agent), *ap = resolve(t.actor_part, P.bases, agent);
     // the agent's scalar block is read ONCE into shared memory, edited there and written back at the end: the serial part below
     // would otherwise be a chain of ~8 dependent L2 round trips
     __shared__ float sc[32];
@@ -727,7 +706,7 @@ __device__ __forceinline__ void task_finish(const Task &t, const Program &P, int
     const int k = (int)threadIdx.x - 32;
     int new_step = 0;
     float2 fac = make_float2(0.f, 0.f);
-    const bool bump = k >= 0 && k < 4 && t.i[k];      // SC_STEP_POLICY, SC_STEP_Q1, SC_STEP_Q2, SC_STEP_ALPHA are consecutive
+    const bool bump = k >= 0 && k < 4 && t.bump[k];      // SC_STEP_POLICY, SC_STEP_Q1, SC_STEP_Q2, SC_STEP_ALPHA are consecutive
     if (bump) {
         new_step = __float_as_int(sc[SC_STEP_POLICY + k]) + 1;
         fac = __ldg(P.adam_table + min(new_step, kAdamTable - 1));
@@ -744,13 +723,13 @@ __device__ __forceinline__ void task_finish(const Task &t, const Program &P, int
             sc[SC_LOSS_PI] = s1 / Bf;
             const int n_upd = __float_as_int(sc[SC_N_UPDATES]);
             float alpha_next = sc[SC_ALPHA0 + (n_upd & 1)];
-            if (t.i[6]) {
+            if (t.auto_entropy) {
                 const float la = sc[SC_LOG_ALPHA];
                 const float g = -(s2 / Bf);                                      // d(-mean(log_alpha*(logp+H_t)))/dlog_alpha
                 sc[SC_LOSS_ALPHA] = la * g;
-                float *gexp = resolve(t.p[2], P.bases, agent);
+                float *gexp = resolve(t.alpha_grad, P.bases, agent);
                 if (gexp) *gexp = g;
-                if (t.i[7]) {      // adam_element on the shared-memory copy (same arithmetic)
+                if (t.apply) {      // adam_element on the shared-memory copy (same arithmetic)
                     const float ss = sc[SC_FAC0 + 2 * (SC_STEP_ALPHA - SC_STEP_POLICY)], bs = sc[SC_FAC0 + 2 * (SC_STEP_ALPHA - SC_STEP_POLICY) + 1];
                     float mm = sc[SC_LOG_ALPHA_M], vv = sc[SC_LOG_ALPHA_V];
                     mm = mm + (1.0f - kBeta1) * (g - mm);
@@ -761,12 +740,12 @@ __device__ __forceinline__ void task_finish(const Task &t, const Program &P, int
                 }
                 alpha_next = expf(sc[SC_LOG_ALPHA]);                            // self.alpha = self.log_alpha.exp()
             }
-            if (t.i[7]) sc[SC_ALPHA0 + ((n_upd + 1) & 1)] = alpha_next;
+            if (t.apply) sc[SC_ALPHA0 + ((n_upd + 1) & 1)] = alpha_next;
         }
-        if (t.i[4]) {
+        if (t.bump_updates) {
             sc[SC_N_UPDATES] = __int_as_float(__float_as_int(sc[SC_N_UPDATES]) + 1);
             const int pos = __float_as_int(sc[SC_HIST_POS]);
-            float *hist = resolve(t.p[3], P.bases, agent) + 4 * (pos % kLossHist);
+            float *hist = resolve(t.loss_hist, P.bases, agent) + 4 * (pos % kLossHist);
             hist[0] = sc[SC_LOSS_Q1]; hist[1] = sc[SC_LOSS_Q2]; hist[2] = sc[SC_LOSS_PI]; hist[3] = sc[SC_LOSS_ALPHA];
             sc[SC_HIST_POS] = __int_as_float(pos + 1);
         }
