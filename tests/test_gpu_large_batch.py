@@ -15,12 +15,9 @@ import torch
 
 from oracle import sac_oracle_np as O
 from tests.golden import cases
-from tests.test_gpu_update_parity import TOL as PARITY_TOL
-from tests.util import batch_of, grad_close, make_agent, net_params, relerr, relu_hint
+from tests.util import NETS, TOL, alpha_of, batch_of, check_losses, check_state, grad_close, make_agent, net_params, oracle_step, relerr, relu_hint, sac_state
 
 pytestmark = pytest.mark.gpu
-TOL = PARITY_TOL["bf16x3"]
-NETS = ("policy", "q1", "q2", "q1_target", "q2_target")
 # Data-parallel backward.  SPLIT_TOL: the same gradient summed in another order where every fp32 accumulation chain is short (the
 # bound of the GEMM self-tests).  A GEMM accumulates over K in fp32 in tensor memory, and that error grows with the chain: against the
 # oracle, the unsplit program's dW at B = K = 2048 / 8192 / 65536 is off by 1.2e-5 / 3e-5 / 3.3e-4, the split one (chains of
@@ -41,58 +38,12 @@ def case_of(name, B, steps, seed):
     return dict(cases.UPDATE_CASES[name], batch=B, steps=steps, seed=seed)
 
 
-def alpha_of(agent):
-    a = agent.alpha
-    return float(a) if not hasattr(a, "item") else float(a.item())
-
-
-def check_losses(got, ref, tag):
-    for k in ("q1_loss", "q2_loss", "policy_loss"):
-        assert abs(got[k] - ref[k]) <= TOL["loss"] * abs(ref[k]) + 1e-6, (tag, k, got[k], ref[k])
-
-
 def check_grads(grads, aux, nets, tag):
     """grads[net][name] against the oracle's aux[f"{net}_grads"][name]: every row within TOL["grad"], no ReLU flip allowed."""
     for net in nets:
         for nm, ref in aux[f"{net}_grads"].items():
             ok, overall, bad = grad_close(grads[net][nm], ref, TOL["grad"], max_flips=0)
             assert ok, (tag, net, nm, overall, bad)
-
-
-def oracle_step(agent, st, case, b, hint=None, per_weights=None):
-    """One oracle step on the masks the device used; every unit outside the rounding band must agree."""
-    hint = hint or relu_hint(agent, case)
-    ref, aux = O.update_parameters(st, b, per_weights=per_weights, return_aux=True, relu_hint=hint)
-    assert hint.mismatch == 0, (hint.mismatch, hint.adopted, hint.ambiguous)
-    return ref, aux
-
-
-def check_state(agent, st):
-    """All five nets, the Adam moments and step counts of the three optimizers, alpha -- after st.q1_opt.step steps.
-
-    Adam moves every weight by ~lr per step whatever |g| is: weights are compared in units of lr (0.02 lr per step, at most a fraction
-    5e-3 of the elements outside).  A Polyak target moves by only tau (w - w_t) per step, far inside that budget (a skipped or stale
-    Polyak step would pass it), so the targets also get the budget scaled by tau (an error of the online weights reaches the target
-    through tau), plus a few ulp of fp32 rounding per step."""
-    steps = st.q1_opt.step
-    budget = TOL["budget"] * st.lr * steps + 1e-7
-    for net in NETS:
-        mine = net_params(agent, net)
-        for nm, ref in getattr(st, net).items():
-            frac_bad = np.mean(np.abs(mine[nm] - ref) > budget)
-            assert frac_bad < TOL["frac"], (net, nm, frac_bad, np.abs(mine[nm] - ref).max())
-            if net.endswith("_target"):
-                tb = st.tau * steps * budget + 4 * steps * np.spacing(np.abs(ref))
-                frac_bad = np.mean(np.abs(mine[nm] - ref) > tb)
-                assert frac_bad < TOL["frac"], ("polyak", net, nm, frac_bad, np.abs(mine[nm] - ref).max())
-    for net, opt in (("policy", st.policy_opt), ("q1", st.q1_opt), ("q2", st.q2_opt)):
-        sd = getattr(agent, f"{net}_optimizer").state_dict()
-        for i, nm in enumerate(getattr(st, net)):
-            assert int(sd["state"][i]["step"]) == opt.step, (net, nm, sd["state"][i]["step"], opt.step)
-            assert grad_close(sd["state"][i]["exp_avg"].cpu().numpy(), opt.m[nm], TOL["adam"], max_flips=0)[0], (net, nm)
-            assert grad_close(sd["state"][i]["exp_avg_sq"].cpu().numpy(), opt.v[nm], 2 * TOL["adam"], max_flips=0)[0], (net, nm)
-    a = alpha_of(agent)
-    assert abs(a - st.alpha) <= 1e-5 * abs(st.alpha), (a, st.alpha)
 
 
 def n_stages_latency_form(hw, case, b, monkeypatch, **update_kw):
@@ -127,7 +78,7 @@ def test_throughput_update_matches_oracle(hw, monkeypatch, name, B, steps, seed)
         check_grads({net: agent.exported_grads(net) for net in ("q1", "q2", "policy")}, aux, ("q1", "q2", "policy"), step)
         a = alpha_of(agent)
         assert abs(a - st.alpha) <= 1e-5 * abs(st.alpha), (step, a, st.alpha)
-    check_state(agent, st)
+    check_state(sac_state(agent), st)
     # the program really took the throughput form: it has more stages than the latency form (mixed stages are cut in two)
     b = batch_of(case, 0)
     assert n_stages > n_stages_latency_form(hw, case, b, monkeypatch, export_grads=True), n_stages
@@ -184,7 +135,7 @@ def test_throughput_is_weighted_loss_and_td(hw, monkeypatch):
         assert td.shape == want.shape
         # |q1 - y| per row: within the loss tolerance of the scale of y (q1 and y each carry that relative error)
         np.testing.assert_allclose(td, want, rtol=TOL["loss"], atol=TOL["loss"] * float(np.sqrt(np.mean(aux["y"] ** 2))), err_msg=f"step {step}")
-    check_state(agent, st)
+    check_state(sac_state(agent), st)
 
 
 # ---- B. data-parallel backward, world = 1 -----------------------------------------------------------------------------------------
@@ -301,7 +252,7 @@ def test_dp_backward_matches_oracle_and_unsplit_program(hw, B):
     _close_oracle(grads[0], aux, ("q1", "q2"), "phase 0")
     _close_oracle(grads[1], aux, ("policy",), "phase 1")
     _check_log_alpha_grad(grads[1]["log_alpha"], aux)
-    check_state(dp.agent, st)
+    check_state(sac_state(dp.agent), st)
 
 
 def test_dp_two_shards_equal_fused_update(hw):
@@ -347,4 +298,4 @@ def test_dp_two_shards_equal_fused_update(hw):
         p0, p1 = net_params(shards[0].agent, net), net_params(shards[1].agent, net)
         for nm in p0:
             np.testing.assert_array_equal(p0[nm], p1[nm], err_msg=f"replicas diverged: {net}.{nm}")
-    check_state(shards[0].agent, st)
+    check_state(sac_state(shards[0].agent), st)

@@ -2,6 +2,7 @@
 handle must equal the same agents run one by one, and the data-parallel step over two logical shards must equal the
 single-agent step on the concatenated batch."""
 import ctypes
+import gc
 
 import numpy as np
 import pytest
@@ -252,32 +253,81 @@ def test_k_steps_per_call_equal_single_calls(hw, replay):
         np.testing.assert_array_equal(agents[0].replay_buffer.priorities, agents[1].replay_buffer.priorities)
 
 
-def test_population_stream_program_equals_single_agents(hw):
-    """12 agents of the C1 shape: the population's stages outnumber the SMs, so its program takes the throughput form (128 x 128
-    tiles on the stream kernel, mixed stages split) -- and must still equal twelve single agents on the latency form, bitwise."""
-    hw.use_networks("model1")
-    obs, act, hid, B, n = 24, 4, 256, 256, 12
+def _equal_states(got, want, tag):
+    for k, v in want.items():
+        if isinstance(v, dict):
+            for nm in v:
+                np.testing.assert_array_equal(got[k][nm], v[nm], err_msg=f"{tag} {k}.{nm}")
+        elif isinstance(v, tuple):      # (step, m, v) of an optimizer
+            assert got[k][0] == v[0], (tag, k, got[k][0], v[0])
+            _equal_states({"m": got[k][1], "v": got[k][2]}, {"m": v[1], "v": v[2]}, f"{tag} {k}")
+        else:
+            assert got[k] == v, (tag, k, got[k], v)
+
+
+def _n_tiles(hw, h):
+    st = hw._native.Stats()
+    hw._native.check(hw._native.lib().sacb_get_stats(h, ctypes.byref(st)))
+    return st.n_tiles
+
+
+# name, agents, wide: C1 x 12 (128 x 128 stream tiles, mixed stages split); C2 x 45 (odd count); C2 x 128, the benchmarked population:
+# 128 x 256 tiles, light column-sum builds, and arenas more than 2^31 / 2^32 bytes past agent 0's (64-bit agent offsets)
+STREAM_POPULATIONS = [("c1_bipedal_m1", 12, False), ("c2_humanoid_m2", 45, False), ("c2_humanoid_m2", 128, True)]
+
+
+@pytest.mark.parametrize("name,n,wide", STREAM_POPULATIONS)
+def test_population_stream_program_equals_single_agents(hw, monkeypatch, name, n, wide):
+    """A population whose stages outnumber the SMs takes the throughput form of the program (stream tiles, mixed stages split) -- and
+    must still equal the same agents run one by one on the latency form, bitwise: every agent's losses at both steps (step 1 derives
+    the weight shadows, step 2 reads the resident ones), and the whole state (nets, targets, Adam moments and steps, alpha) of agents
+    0, 1, the last, and the first ones past 2^31 / 2^32 bytes.  The single agents are built one at a time.
+    wide: the default program uses 128 x 256 tiles -- a build with SACB_STREAM_N256_MIN=0 (read at each program build) has more
+    tiles -- and that build equals the default one bit for bit."""
+    from tests.util import population_state, sac_state, selected_agents
+    monkeypatch.delenv("SACB_NO_STREAM", raising=False)
+    monkeypatch.delenv("SACB_STREAM_N256_MIN", raising=False)
+    case = cases.UPDATE_CASES[name]
+    hw.use_networks("model1" if case["n_hidden"] == 2 else "model2")
+    obs, act, hid, B = case["obs"], case["act"], case["hidden"], 256
     seeds = list(range(100, 100 + n))
-    pop = hw.PopulationSAC(n, obs, act, hidden_dim=hid, device="cuda", seeds=seeds, capacity=512, max_batch=B, seed=7)
     rng = np.random.RandomState(2)
-    singles = []
+    data = [O.make_batch(obs, act, 400, seed=900 + i) for i in range(n)]
+    idx = [np.stack([rng.permutation(400)[:B] for _ in seeds]).astype(np.int64) for _ in range(2)]
+    eps = [(rng.standard_normal((n, B, act)).astype(np.float32), rng.standard_normal((n, B, act)).astype(np.float32)) for _ in range(2)]
+
+    def run_population():
+        pop = hw.PopulationSAC(n, obs, act, hidden_dim=hid, device="cuda", seeds=seeds, capacity=512, max_batch=B, seed=7)
+        for i, b in enumerate(data):
+            pop.push_many(i, b["s"], b["a"], b["r"], b["s2"], b["d"])
+        losses = [pop.update_parameters(B, idx=idx[k], eps=eps[k]) for k in range(2)]
+        return pop, losses
+
+    pop, losses = run_population()
+    sel = selected_agents(pop, require_far=wide)
+    states = {i: population_state(pop, i) for i in sel}
+    n_tiles = _n_tiles(hw, pop._h)
+    del pop
+    gc.collect()
+    if wide:
+        with monkeypatch.context() as mp:
+            mp.setenv("SACB_STREAM_N256_MIN", "0")
+            narrow, narrow_losses = run_population()
+        assert _n_tiles(hw, narrow._h) > n_tiles, (_n_tiles(hw, narrow._h), n_tiles)
+        assert narrow_losses == losses
+        for i in sel:
+            _equal_states(population_state(narrow, i), states[i], f"128-wide tiles, agent {i}")
+        del narrow
+        gc.collect()
     for i, sd in enumerate(seeds):
         torch.manual_seed(sd)
         ag = hw.SAC(obs, act, hidden_dim=hid, device="cuda", capacity=512, max_batch=B, seed=7)
-        b = O.make_batch(obs, act, 400, seed=900 + i)
-        ag.replay_buffer.push_many(b["s"], b["a"], b["r"], b["s2"], b["d"])
-        pop.push_many(i, b["s"], b["a"], b["r"], b["s2"], b["d"])
-        singles.append(ag)
-    for step in range(2):
-        idx = np.stack([rng.permutation(400)[:B] for _ in seeds]).astype(np.int64)
-        e_next = rng.standard_normal((n, B, act)).astype(np.float32)
-        e_cur = rng.standard_normal((n, B, act)).astype(np.float32)
-        got = pop.update_parameters(B, idx=idx, eps=(e_next, e_cur))
-        for i, ag in enumerate(singles):
-            ref = ag.update_parameters(B, idx=idx[i], eps=(e_next[i], e_cur[i]))
-            assert got[i] == ref, (step, i, got[i], ref)
-    for i in (0, 5, n - 1):
-        st = pop.agent_state(i)
-        for net in ("policy", "q1", "q2", "q1_target", "q2_target"):
-            for k, v in net_params(singles[i], net).items():
-                np.testing.assert_array_equal(st[f"{net}_state_dict"][k].numpy(), v, err_msg=f"agent {i} {net}.{k}")
+        ag.replay_buffer.push_many(data[i]["s"], data[i]["a"], data[i]["r"], data[i]["s2"], data[i]["d"])
+        for k in range(2):
+            ref = ag.update_parameters(B, idx=idx[k][i], eps=(eps[k][0][i], eps[k][1][i]))
+            assert losses[k][i] == ref, (k, i, losses[k][i], ref)
+        if i in states:
+            _equal_states(states[i], sac_state(ag), f"agent {i}")
+        del ag
+        gc.collect()      # a SAC and its optimizer views reference each other: its handle (device arena) is freed by the collector
+    hw.use_networks("model1")

@@ -14,13 +14,12 @@ import pytest
 
 from oracle import sac_oracle_np as O
 from tests.golden import cases
+from tests.util import PARITY_TOL as TOL
 from tests.util import batch_of, grad_close, make_agent, net_params, relerr, relu_hint
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
-TOL = {"fp32": dict(loss=3e-4, grad=3e-4, adam=6e-4, frac=5e-3, budget=0.02),
-       "bf16x3": dict(loss=3e-4, grad=3e-4, adam=6e-4, frac=5e-3, budget=0.02)}
 CASES = [c for c in cases.UPDATE_CASES if not cases.UPDATE_CASES[c].get("loose")]
 
 
