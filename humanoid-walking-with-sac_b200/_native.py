@@ -49,7 +49,12 @@ class PerStats(ctypes.Structure):
 
 class Stats(ctypes.Structure):
     _fields_ = [("kernel_launches", ctypes.c_int64), ("n_stages", ctypes.c_int32), ("n_tasks", ctypes.c_int32), ("n_tiles", ctypes.c_int32),
-                ("grid", ctypes.c_int32), ("block", ctypes.c_int32), ("smem_bytes", ctypes.c_int32), ("sm_count", ctypes.c_int32)]
+                ("grid", ctypes.c_int32), ("block", ctypes.c_int32), ("smem_bytes", ctypes.c_int32), ("sm_count", ctypes.c_int32),
+                ("n_programs", ctypes.c_int32)]
+
+
+class Hparams(ctypes.Structure):
+    _fields_ = [("lr", ctypes.c_float), ("gamma", ctypes.c_float), ("tau", ctypes.c_float), ("target_entropy", ctypes.c_float)]
 
 
 H = ctypes.c_void_p
@@ -72,6 +77,9 @@ SIGNATURES = {
     "sacb_get_scalars": (I, [H, I, ctypes.POINTER(Scalars)]),
     "sacb_set_scalars": (I, [H, I, ctypes.POINTER(Scalars)]),
     "sacb_set_lr": (I, [H, ctypes.c_float]),
+    "sacb_get_hparams": (I, [H, I, ctypes.POINTER(Hparams)]),
+    "sacb_set_hparams": (I, [H, I, ctypes.POINTER(Hparams)]),
+    "sacb_copy_agents": (I, [H, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32), I]),
     "sacb_invalidate_shadows": (I, [H]),
     "sacb_push": (I, [H, I, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, I64]),
     "sacb_push_rows": (I, [H, I, c_f32p, I64]),

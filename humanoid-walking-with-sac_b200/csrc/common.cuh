@@ -68,9 +68,21 @@ enum ScalarSlot {
     SC_ERROR_FLAG,                   // copy of the device error flag made by T_FINISH: losses + flag come back in ONE D2H copy
     SC_COUNT = 16,
     SC_HIST_POS = 24,                // int32 bit pattern: completed updates since create, never reset: loss_hist[(pos % kLossHist)] = losses of that update
-    // Adam bias-correction factors of the NEXT step of each optimizer, refreshed whenever a step counter changes
-    // (T_FINISH, sacb_set_scalars, the data-parallel apply): [SC_FAC0 + 2*(step_slot - SC_STEP_POLICY)] = step_size, +1 = sqrt(bc2)
+    SC_DP_LOSS_Q1 = 25,              // 25..27: q1, q2, policy losses averaged over the data-parallel replicas (sacb_dp_exchange_apply)
+    // hyperparameters of the agent (sacb_set_hparams): every task reads them here, so a new value never rebuilds a program
+    SC_LR = 28, SC_GAMMA, SC_TAU, SC_TARGET_ENTROPY,
+    // Adam bias-correction factors of the NEXT step of each optimizer, refreshed whenever a step counter or SC_LR changes
+    // (T_FINISH, sacb_set_scalars, sacb_set_hparams, the data-parallel apply): [SC_FAC0 + 2*(step_slot - SC_STEP_POLICY)] = step_size, +1 = sqrt(bc2)
     SC_FAC0 = 16
+};
+static_assert(SC_TARGET_ENTROPY == 31, "the scalar block holds 32 floats");
+
+// Adam bias corrections of step t + 1 for t = index (host float64, independent of lr): step_size = (float)((double)lr / bc1) is formed
+// where the step counter moves, with the agent's SC_LR -- the same correctly rounded division as the host's adam_factors
+struct AdamBias {
+    double bc1;
+    float bc2_sqrt;
+    float pad;
 };
 
 // ---- GEMM operand: logical X[R, K] (R = M for A, N for B) held in a PM -----------------------------------
@@ -116,7 +128,7 @@ struct AdamArgs {
     int32_t step_slot;  // ScalarSlot of the optimizer step counter (value BEFORE this step's increment); it also selects the cached
                         // SC_FAC0 factors, which hold the step size (lr): a new learning rate does not touch the program
     int32_t apply;      // 0 = only export the gradient (data-parallel backward), 1 = apply Adam
-    float tau;          // Polyak rate
+                        // (the Polyak rate is the agent's SC_TAU)
 };
 
 // ---- arguments of the non-GEMM task types (Task's union): the builder (program.cu) sets every field a type uses, the bodies
@@ -153,18 +165,16 @@ struct TargetLossArgs {       // T_TARGET_LOSS
     Ref y, dq[2], td;         // out [B]: Bellman target, dL/dq1, dL/dq2, |q1 - y|
     Ref partials;             // out: per-tile partial sums of w*(q-y)^2 [n_tiles, 2] (summed in tile order by T_FINISH: deterministic)
     int32_t B, H;
-    int32_t R;                // batch rows per tile (kLossRows or kLossRowsMax, tasks.cuh)
-    float gamma;
+    int32_t R;                // batch rows per tile (kLossRows or kLossRowsMax, tasks.cuh); the discount is the agent's SC_GAMMA
 };
 struct ActorLossArgs {        // T_ACTOR_LOSS
     PmRef h[2];               // last hidden activations [B, H] of q1, q2 on (s, a_new)
     PmRef dh[2];              // out: dL/dh of the last hidden layer of q1, q2 (the Q weights are constants here, quirk Q2)
     Ref w_out[2], b_out[2];   // output-layer weights [H] and biases [1] of q1, q2
     Ref logp;                 // log-prob of the current-state sample [B]
-    Ref partials;             // out: per-tile partials [n_tiles, 2]: sum(alpha*logp - minq), sum(logp + target_entropy)
+    Ref partials;             // out: per-tile partials [n_tiles, 2]: sum(alpha*logp - minq), sum(logp + SC_TARGET_ENTROPY)
     int32_t B, H;
     int32_t R;                // batch rows per tile
-    float target_entropy;
 };
 struct SampleBwdArgs {        // T_SAMPLE_BWD: dL/da -> dL/dmean, dL/dlog_std
     Ref da[2];                // dL/da through q1, q2 [B, A]
@@ -326,7 +336,7 @@ struct Program {
     const int32_t *slots;     // physical ring slots of the minibatch rows [n_agents, B]
     int32_t slots_stride; int32_t pad1;
     int32_t *error_flag;      // set by watchdogs (mbarrier / grid barrier timeouts)
-    const float2 *adam_table;     // [kAdamTable] (step_size, sqrt(bc2)) of Adam step t+1 for t = index, computed on the host in float64
+    const AdamBias *adam_table;   // [kAdamTable] (bc1, sqrt(bc2)) of Adam step t+1 for t = index, computed on the host in float64
     unsigned long long *timeline; // optional [n_stages][4]: earliest CTA start, earliest dependency release, latest CTA end (profiling aid)
     unsigned long long *trace; // optional [grid][kTraceSlots] globaltimer stamps of each CTA's first tile (profiling aid), or null
     float *host_losses;       // pinned HOST memory (addressable from the device), or null: T_FINISH of agent 0 stores the three losses, the

@@ -10,14 +10,15 @@
 
 namespace sacb {
 
-__global__ void dp_apply_kernel(float *w, float *m, float *v, float *wt, const float *g, int64_t n, float scale, const float *scalars, int step_slot, float lr, float tau) {
+__global__ void dp_apply_kernel(float *w, float *m, float *v, float *wt, const float *g, int64_t n, float scale, const float *scalars, int step_slot) {
     float ss, bs;
     adam_factors_cached(scalars, step_slot, ss, bs);
+    const float tau = __ldcg(scalars + SC_TAU);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         adam_element(g[i] * scale, w + i, m + i, v + i, wt ? wt + i : nullptr, nullptr, 1, ss, bs, tau);
 }
 
-__global__ void dp_finish_kernel(float *scalars, const float *g_scalars, int phase, int auto_entropy, const float2 *adam_table) {
+__global__ void dp_finish_kernel(float *scalars, const float *g_scalars, int phase, int auto_entropy, const AdamBias *adam_table) {
     if (threadIdx.x || blockIdx.x) return;
     if (phase == 0) {
         for (int slot = SC_STEP_Q1; slot <= SC_STEP_Q2; slot++) {
@@ -98,12 +99,13 @@ __global__ void __launch_bounds__(256) dp_reduce_scatter_kernel(PeerSlabs ps, in
 
 // gathered != 0: second half of the two-shot exchange -- element i is already the replica mean, held by replica i / ceil(n4 / W)
 __global__ void __launch_bounds__(256) dp_reduce_apply_kernel(PeerSlabs ps, int rank, int world, uint32_t epoch, float *w, float *m, float *v, float *wt, int64_t n,
-                                                              int64_t n_first, const float *scalars, int slot_first, int slot_second, float tau, int *error_flag,
+                                                              int64_t n_first, const float *scalars, int slot_first, int slot_second, int *error_flag,
                                                               int gathered) {
     dp_wait_peers(ps, rank, world, epoch, error_flag);
     const int64_t per = (n / 4 + world - 1) / world;
     float ss[2], ibs[2];
     { float a, b; adam_factors_cached(scalars, slot_first, a, b); ss[0] = a; ibs[0] = 1.0f / b; adam_factors_cached(scalars, slot_second, a, b); ss[1] = a; ibs[1] = 1.0f / b; }
+    const float tau = __ldcg(scalars + SC_TAU);
     const float inv_w = 1.0f / (float)world;
     const int64_t n4 = n / 4;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
@@ -137,7 +139,7 @@ __global__ void __launch_bounds__(256) dp_reduce_apply_kernel(PeerSlabs ps, int 
 
 // phase 1 only: mean over the replicas of the log_alpha gradient and of the three loss scalars (each replica's mean over its own
 // rows), read from the peers' arenas behind the same barrier; then the temperature step and the step counters
-__global__ void dp_finish_peers_kernel(float *scalars, PeerSlabs gsc, PeerSlabs lss, int world, int phase, int auto_entropy, const float2 *adam_table) {
+__global__ void dp_finish_peers_kernel(float *scalars, PeerSlabs gsc, PeerSlabs lss, int world, int phase, int auto_entropy, const AdamBias *adam_table) {
     if (threadIdx.x || blockIdx.x) return;
     float g = 0.f, l[3] = {0.f, 0.f, 0.f};
     for (int p = 0; p < world; p++) {
@@ -146,14 +148,14 @@ __global__ void dp_finish_peers_kernel(float *scalars, PeerSlabs gsc, PeerSlabs 
     }
     const float inv_w = 1.0f / (float)world;
     if (phase == 0) {
-        scalars[SC_LOSS_Q1 + 16] = l[0] * inv_w; scalars[SC_LOSS_Q2 + 16] = l[1] * inv_w;      // replica means, kept apart from the local ones (slots 26, 27)
+        scalars[SC_DP_LOSS_Q1] = l[0] * inv_w; scalars[SC_DP_LOSS_Q1 + 1] = l[1] * inv_w;      // replica means, kept apart from the local ones
         for (int slot = SC_STEP_Q1; slot <= SC_STEP_Q2; slot++) {
             const int step = __float_as_int(scalars[slot]) + 1;
             scalars[slot] = __int_as_float(step);
             adam_factors_store(scalars, slot, step, adam_table);
         }
     } else {
-        scalars[SC_LOSS_PI + 16] = l[2] * inv_w;
+        scalars[SC_DP_LOSS_Q1 + 2] = l[2] * inv_w;
         g *= inv_w;
         const int n_upd = __float_as_int(scalars[SC_N_UPDATES]);
         float alpha_next = scalars[SC_ALPHA0 + (n_upd & 1)];
@@ -234,10 +236,10 @@ extern "C" int sacb_dp_exchange_apply(sacb_handle h, int phase) {
     }
     if (phase == 0)
         dp_reduce_apply_kernel<<<grid, 256, 0, h->stream>>>(ps, r, W, epoch, ar + L.param[1], ar + L.adam_m[1], ar + L.adam_v[1], ar + L.param[3], n, L.q.size, sc,
-                                                            SC_STEP_Q1, SC_STEP_Q2, h->cfg.tau, h->error_flag, gathered);
+                                                            SC_STEP_Q1, SC_STEP_Q2, h->error_flag, gathered);
     else
         dp_reduce_apply_kernel<<<grid, 256, 0, h->stream>>>(ps, r, W, epoch, ar + L.param[0], ar + L.adam_m[0], ar + L.adam_v[0], nullptr, n, L.pol.size, sc,
-                                                            SC_STEP_POLICY, SC_STEP_POLICY, h->cfg.tau, h->error_flag, gathered);
+                                                            SC_STEP_POLICY, SC_STEP_POLICY, h->error_flag, gathered);
     dp_finish_peers_kernel<<<1, 32, 0, h->stream>>>(sc, gsc, lss, W, phase, h->cfg.auto_entropy, h->adam_table);
     h->kernel_launches += 2;
     SACB_CUDA(cudaGetLastError());
@@ -247,7 +249,7 @@ extern "C" int sacb_dp_exchange_apply(sacb_handle h, int phase) {
 /* losses of the last data-parallel step averaged over the replicas (the local means stay in sacb_get_losses) */
 extern "C" int sacb_dp_get_losses(sacb_handle h, float *losses_out) {
     if (!h || !losses_out) return fail(SACB_ERR_ARG, "bad argument");
-    SACB_CUDA(cudaMemcpyAsync(losses_out, h->arena + h->L.scalars + SC_LOSS_Q1 + 16, 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    SACB_CUDA(cudaMemcpyAsync(losses_out, h->arena + h->L.scalars + SC_DP_LOSS_Q1, 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     SACB_CUDA(cudaStreamSynchronize(h->stream));
     return check_error_flag(h);
 }
@@ -301,7 +303,7 @@ extern "C" int sacb_dp_apply(sacb_handle h, int phase) {
     float *sc = ar + L.scalars;
     auto run = [&](int net, int64_t size) {
         dp_apply_kernel<<<296, 256, 0, h->stream>>>(ar + L.param[net], ar + L.adam_m[net], ar + L.adam_v[net], net ? ar + L.param[net + 2] : nullptr, ar + L.grad[net], size,
-                                                    1.0f, sc, net == 0 ? SC_STEP_POLICY : (net == 1 ? SC_STEP_Q1 : SC_STEP_Q2), h->cfg.lr, h->cfg.tau);
+                                                    1.0f, sc, net == 0 ? SC_STEP_POLICY : (net == 1 ? SC_STEP_Q1 : SC_STEP_Q2));
         h->kernel_launches++;
     };
     h->shadows_valid = false;      // the element-wise apply writes fp32 weights only: the next program re-derives the shadows

@@ -64,25 +64,31 @@ struct EpiR {
 
 // Adam bias corrections for step t (torch/optim/adam.py::_single_tensor_adam): python floats = double.  Double-precision
 // pow is slow on this part, so it runs once per optimizer per update (T_FINISH) and the tiles read the cached pair.
-__host__ __device__ inline void adam_factors(int step_before, float lr, float &step_size, float &bc2_sqrt) {
+__host__ inline AdamBias adam_bias(int step_before) {
     const double t = (double)(step_before + 1);
-    const double bc1 = 1.0 - pow((double)0.9, t);
-    const double bc2 = 1.0 - pow((double)0.999, t);
-    step_size = (float)((double)lr / bc1);
-    bc2_sqrt = (float)sqrt(bc2);
+    AdamBias b;
+    b.bc1 = 1.0 - pow((double)0.9, t);
+    b.bc2_sqrt = (float)sqrt(1.0 - pow((double)0.999, t));
+    b.pad = 0.f;
+    return b;
 }
+// step size from the table entry: one correctly rounded float64 division, on the host and on the device alike
+__host__ __device__ __forceinline__ float adam_step_size(float lr, double bc1) { return (float)((double)lr / bc1); }
 __device__ __forceinline__ void adam_factors_cached(const float *scalars, int step_slot, float &step_size, float &bc2_sqrt) {
     const float2 f = __ldcg(reinterpret_cast<const float2 *>(scalars + SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY)));
     step_size = f.x; bc2_sqrt = f.y;
 }
-__host__ inline void adam_factors_store(float *scalars, int step_slot, int step, float lr) {
-    adam_factors(step, lr, scalars[SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY)], scalars[SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY) + 1]);
+// host side: the factors for the agent's own learning rate (SC_LR of the same block)
+__host__ inline void adam_factors_store(float *scalars, int step_slot, int step) {
+    const AdamBias b = adam_bias(step);
+    scalars[SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY)] = adam_step_size(scalars[SC_LR], b.bc1);
+    scalars[SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY) + 1] = b.bc2_sqrt;
 }
-// device side: the factors come from the host-built table (float64 pow is very slow on this part)
-__device__ __forceinline__ void adam_factors_store(float *scalars, int step_slot, int step, const float2 *table) {
-    const float2 f = __ldg(table + min(step, kAdamTable - 1));
-    scalars[SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY)] = f.x;
-    scalars[SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY) + 1] = f.y;
+// device side: the bias corrections come from the host-built table (float64 pow is very slow on this part)
+__device__ __forceinline__ void adam_factors_store(float *scalars, int step_slot, int step, const AdamBias *table) {
+    const AdamBias b = table[min(step, kAdamTable - 1)];
+    scalars[SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY)] = adam_step_size(scalars[SC_LR], b.bc1);
+    scalars[SC_FAC0 + 2 * (step_slot - SC_STEP_POLICY) + 1] = b.bc2_sqrt;
 }
 
 // one Adam element update (+ Polyak, sac_imp.py:146-152); returns the new weight
@@ -132,7 +138,7 @@ __device__ __forceinline__ EpiR resolve_epilogue(const Task &t, const AgentBases
         e.shadow = resolve_pm(t.adam.shadow, b, agent);
         e.shadow2 = resolve_pm(t.adam.shadow2, b, agent); e.shadow2_col0 = t.adam.shadow2_col0;
         e.shadow_t = resolve_pm(t.adam.shadow_t, b, agent);
-        e.apply = t.adam.apply; e.tau = t.adam.tau;
+        e.apply = t.adam.apply; e.tau = __ldcg(scalars + SC_TAU);
         adam_factors_cached(scalars, t.adam.step_slot, e.step_size, e.bc2_sqrt);
         e.inv_bc2_sqrt = 1.0f / e.bc2_sqrt;
     }

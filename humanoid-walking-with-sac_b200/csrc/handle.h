@@ -134,7 +134,7 @@ struct sacb_handle_s {
     unsigned int *barrier = nullptr;
     int32_t *error_flag = nullptr;
     int32_t *slots = nullptr;            // [n_agents, maxB] physical ring slots of the current minibatch
-    float2 *adam_table = nullptr;        // [kAdamTable] Adam bias-correction factors per step count (host float64, lr of this handle)
+    sacb::AdamBias *adam_table = nullptr;     // [kAdamTable] Adam bias corrections per step count (host float64; the step size uses each agent's SC_LR)
     int32_t *slots_identity = nullptr;   // 0..maxB-1: "gather" straight from the upload staging rows (sacb_update_batch)
     int32_t *slots_staged = nullptr;     // pre-staged index sets (sacb_stage_indices)
     int64_t staged_steps = 0, staged_next = 0, staged_B = 0;

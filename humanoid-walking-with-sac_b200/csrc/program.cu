@@ -517,7 +517,6 @@ struct Builder {
         a.gexp = exporting() ? A(L.grad[net] + off_in_net) : null_ref();
         a.shadow = a.shadow2 = a.shadow_t = null_pm(); a.shadow2_col0 = 0;
         a.step_slot = step_slot(net); a.apply = apply() ? 1 : 0;
-        a.tau = h->cfg.tau;
         return a;
     }
     // dW epilogue of hidden layer `layer`: the critics are read again (post-step) by the actor phase of the SAME update,
@@ -770,7 +769,7 @@ struct Builder {
                 a.r = W(L.r); a.d = W(L.d); a.logp_next = W(L.logp); a.is_weights = key.use_isw ? W(L.isw) : null_ref();
                 a.y = W(L.y); a.dq[0] = W(L.dq[0]); a.dq[1] = W(L.dq[1]); a.td = W(L.td);
                 a.partials = W(L.loss_part);
-                a.B = B; a.H = H; a.R = loss_rows(); a.gamma = h->cfg.gamma;
+                a.B = B; a.H = H; a.R = loss_rows();
                 add(t, cdiv(B, loss_rows()));
             }
             // gradient at the Linear output of critic k's hidden layer x: the dh PM itself, or (LayerNorm variant) the dz PM behind it
@@ -837,7 +836,7 @@ struct Builder {
                 a.w_out[0] = A(L.param[1] + Q.w_out); a.w_out[1] = A(L.param[2] + Q.w_out);
                 a.b_out[0] = A(L.param[1] + Q.b_out); a.b_out[1] = A(L.param[2] + Q.b_out);
                 a.logp = W(L.logp + B); a.partials = W(L.aloss_part);
-                a.B = B; a.H = H; a.R = loss_rows(); a.target_entropy = -(float)act;
+                a.B = B; a.H = H; a.R = loss_rows();
                 add(t, cdiv(B, loss_rows()));
             }
             // ---- dL/da through both critics (input gradients only: the Q weights are constants here, quirk Q2) -------

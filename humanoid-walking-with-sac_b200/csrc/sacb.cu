@@ -2,6 +2,8 @@
 #include <cstdio>
 #include <cstring>
 #include <algorithm>
+#include <cmath>
+#include <functional>
 #include <vector>
 
 #include "handle.h"
@@ -43,7 +45,9 @@ extern "C" int sacb_device_count(void) {
 static int scalars_init(sacb_handle h) {
     std::vector<float> sc(32, 0.f);
     sc[SC_ALPHA0] = sc[SC_ALPHA1] = h->cfg.alpha0;     // python float 0.2 until the first update (quirk Q1)
-    for (int slot = SC_STEP_POLICY; slot <= SC_STEP_ALPHA; slot++) adam_factors_store(sc.data(), slot, 0, h->cfg.lr);
+    sc[SC_LR] = h->cfg.lr; sc[SC_GAMMA] = h->cfg.gamma; sc[SC_TAU] = h->cfg.tau;
+    sc[SC_TARGET_ENTROPY] = -(float)h->cfg.act_dim;    // sac_imp.py:46
+    for (int slot = SC_STEP_POLICY; slot <= SC_STEP_ALPHA; slot++) adam_factors_store(sc.data(), slot, 0);
     for (int a = 0; a < h->cfg.n_agents; a++)
         SACB_CUDA(cudaMemcpyAsync(h->arena + a * h->L.arena_size + h->L.scalars, sc.data(), 32 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     return cudaStreamSynchronize(h->stream) == cudaSuccess ? SACB_OK : SACB_ERR_DEVICE;
@@ -93,11 +97,11 @@ extern "C" int sacb_create(const sacb_config *cfg, sacb_handle *out) {
     cudaMemsetAsync(h->barrier, 0, 64, h->stream);
     cudaMemsetAsync(h->error_flag, 0, 64, h->stream);
     cudaMemsetAsync(h->slots, 0, sizeof(int32_t) * cfg->max_batch * n, h->stream);
-    {   // Adam bias corrections for every step count that still differs from (lr, 1) in float32
-        std::vector<float2> tab(kAdamTable);
-        for (int t = 0; t < kAdamTable; t++) adam_factors(t, cfg->lr, tab[t].x, tab[t].y);
-        if (cudaMalloc(&h->adam_table, sizeof(float2) * kAdamTable) != cudaSuccess) return bail(fail(SACB_ERR_NOMEM, "device allocation failed"));
-        cudaMemcpyAsync(h->adam_table, tab.data(), sizeof(float2) * kAdamTable, cudaMemcpyHostToDevice, h->stream);
+    {   // Adam bias corrections for every step count that still differs from (1, 1) in float32
+        std::vector<AdamBias> tab(kAdamTable);
+        for (int t = 0; t < kAdamTable; t++) tab[t] = adam_bias(t);
+        if (cudaMalloc(&h->adam_table, sizeof(AdamBias) * kAdamTable) != cudaSuccess) return bail(fail(SACB_ERR_NOMEM, "device allocation failed"));
+        cudaMemcpyAsync(h->adam_table, tab.data(), sizeof(AdamBias) * kAdamTable, cudaMemcpyHostToDevice, h->stream);
         cudaStreamSynchronize(h->stream);
     }
     if (cfg->layer_norm) {      // LayerNorm weights start at 1 (torch.nn.LayerNorm), biases at 0 (the memset above)
@@ -266,31 +270,75 @@ extern "C" int sacb_set_scalars(sacb_handle h, int agent, const sacb_scalars *in
     sc[SC_ALPHA0] = sc[SC_ALPHA1] = in->alpha;
     sc[SC_STEP_POLICY] = i2f(in->step_policy); sc[SC_STEP_Q1] = i2f(in->step_q1); sc[SC_STEP_Q2] = i2f(in->step_q2);
     sc[SC_STEP_ALPHA] = i2f(in->step_alpha); sc[SC_N_UPDATES] = i2f(in->n_updates);
-    adam_factors_store(sc, SC_STEP_POLICY, (int)in->step_policy, h->cfg.lr); adam_factors_store(sc, SC_STEP_Q1, (int)in->step_q1, h->cfg.lr);
-    adam_factors_store(sc, SC_STEP_Q2, (int)in->step_q2, h->cfg.lr); adam_factors_store(sc, SC_STEP_ALPHA, (int)in->step_alpha, h->cfg.lr);
+    for (int slot = SC_STEP_POLICY; slot <= SC_STEP_ALPHA; slot++) adam_factors_store(sc, slot, (int)f2i(sc[slot]));
     SACB_CUDA(cudaMemcpyAsync(dev, sc, sizeof(sc), cudaMemcpyHostToDevice, h->stream));
     SACB_CUDA(cudaStreamSynchronize(h->stream));
     h->act_counter = (uint32_t)in->act_counter;
     return SACB_OK;
 }
 
+// read-modify-write of an agent's scalar block, ordered on the handle's stream
+static int edit_scalars(sacb_handle h, int agent, const std::function<void(float *)> &edit) {
+    float sc[32];
+    float *dev = h->arena + agent * h->L.arena_size + h->L.scalars;
+    SACB_CUDA(cudaMemcpyAsync(sc, dev, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
+    SACB_CUDA(cudaStreamSynchronize(h->stream));
+    edit(sc);
+    SACB_CUDA(cudaMemcpyAsync(dev, sc, sizeof(sc), cudaMemcpyHostToDevice, h->stream));
+    SACB_CUDA(cudaStreamSynchronize(h->stream));
+    return SACB_OK;
+}
+// a new SC_LR: the cached factors of the NEXT step of every optimizer follow it
+static void refresh_factors(float *sc) {
+    for (int slot = SC_STEP_POLICY; slot <= SC_STEP_ALPHA; slot++) adam_factors_store(sc, slot, (int)f2i(sc[slot]));
+}
+
 extern "C" int sacb_set_lr(sacb_handle h, float lr) {
-    if (!h || !(lr > 0.f)) return fail(SACB_ERR_ARG, "bad learning rate");
-    if (lr == h->cfg.lr) return SACB_OK;
+    if (!h || !(lr > 0.f) || !std::isfinite(lr)) return fail(SACB_ERR_ARG, "bad learning rate");
     h->cfg.lr = lr;
-    std::vector<float2> tab(kAdamTable);
-    for (int t = 0; t < kAdamTable; t++) adam_factors(t, lr, tab[t].x, tab[t].y);
+    for (int a = 0; a < h->cfg.n_agents; a++)
+        if (int rc = edit_scalars(h, a, [&](float *sc) { sc[SC_LR] = lr; refresh_factors(sc); })) return rc;
+    return SACB_OK;
+}
+
+extern "C" int sacb_get_hparams(sacb_handle h, int agent, sacb_hparams *out) {
+    if (!h || !out || agent < 0 || agent >= h->cfg.n_agents) return fail(SACB_ERR_ARG, "bad argument");
+    float sc[32];
+    SACB_CUDA(cudaMemcpyAsync(sc, h->arena + agent * h->L.arena_size + h->L.scalars, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
     SACB_CUDA(cudaStreamSynchronize(h->stream));
-    SACB_CUDA(cudaMemcpyAsync(h->adam_table, tab.data(), sizeof(float2) * kAdamTable, cudaMemcpyHostToDevice, h->stream));
-    for (int a = 0; a < h->cfg.n_agents; a++) {      // cached factors of the NEXT step of every optimizer
-        float sc[32];
-        float *dev = h->arena + a * h->L.arena_size + h->L.scalars;
-        SACB_CUDA(cudaMemcpyAsync(sc, dev, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
-        SACB_CUDA(cudaStreamSynchronize(h->stream));
-        for (int slot = SC_STEP_POLICY; slot <= SC_STEP_ALPHA; slot++) adam_factors_store(sc, slot, (int)f2i(sc[slot]), lr);
-        SACB_CUDA(cudaMemcpyAsync(dev, sc, sizeof(sc), cudaMemcpyHostToDevice, h->stream));
+    out->lr = sc[SC_LR]; out->gamma = sc[SC_GAMMA]; out->tau = sc[SC_TAU]; out->target_entropy = sc[SC_TARGET_ENTROPY];
+    return SACB_OK;
+}
+
+extern "C" int sacb_set_hparams(sacb_handle h, int agent, const sacb_hparams *in) {
+    if (!h || !in || agent < 0 || agent >= h->cfg.n_agents) return fail(SACB_ERR_ARG, "bad argument");
+    if (!(in->lr > 0.f) || !std::isfinite(in->lr)) return fail(SACB_ERR_ARG, "lr must be finite and > 0");
+    if (!(in->gamma >= 0.f && in->gamma <= 1.f)) return fail(SACB_ERR_ARG, "gamma must lie in [0, 1]");
+    if (!(in->tau >= 0.f && in->tau <= 1.f)) return fail(SACB_ERR_ARG, "tau must lie in [0, 1]");
+    if (!std::isfinite(in->target_entropy)) return fail(SACB_ERR_ARG, "target_entropy must be finite");
+    return edit_scalars(h, agent, [&](float *sc) {
+        sc[SC_LR] = in->lr; sc[SC_GAMMA] = in->gamma; sc[SC_TAU] = in->tau; sc[SC_TARGET_ENTROPY] = in->target_entropy;
+        refresh_factors(sc);
+    });
+}
+
+/* exploit step of population-based training: agent dst[i] takes over the whole learner state of agent src[i] (one contiguous arena
+ * span: weights, targets, Adam moments, weight shadows, scalar block).  Replay rings and workspaces stay with their agent. */
+extern "C" int sacb_copy_agents(sacb_handle h, const int32_t *dst, const int32_t *src, int n) {
+    if (!h || n < 0 || (n > 0 && (!dst || !src))) return fail(SACB_ERR_ARG, "bad argument");
+    const int na = h->cfg.n_agents;
+    std::vector<char> is_dst(na, 0), is_src(na, 0);
+    for (int i = 0; i < n; i++) {
+        if (dst[i] < 0 || dst[i] >= na || src[i] < 0 || src[i] >= na) return fail(SACB_ERR_ARG, "agent index out of range");
+        if (is_dst[dst[i]]) return fail(SACB_ERR_ARG, "an agent appears twice as a destination");
+        is_dst[dst[i]] = 1; is_src[src[i]] = 1;
     }
-    SACB_CUDA(cudaStreamSynchronize(h->stream));
+    for (int a = 0; a < na; a++)
+        if (is_dst[a] && is_src[a]) return fail(SACB_ERR_ARG, "an agent appears as a source and as a destination");
+    const size_t bytes = sizeof(float) * h->L.arena_size;
+    for (int i = 0; i < n; i++)
+        SACB_CUDA(cudaMemcpyAsync(h->arena + (int64_t)dst[i] * h->L.arena_size, h->arena + (int64_t)src[i] * h->L.arena_size, bytes,
+                                  cudaMemcpyDeviceToDevice, h->stream));
     return SACB_OK;
 }
 
@@ -556,6 +604,7 @@ extern "C" int sacb_get_stats(sacb_handle h, sacb_stats *out) {
     memset(out, 0, sizeof(*out));
     out->kernel_launches = h->kernel_launches;
     out->sm_count = h->sm_count; out->block = kThreads;
+    out->n_programs = (int)h->programs.size();
     out->smem_bytes = (int)math_smem(h->cfg.math_mode);
     for (auto &kv : h->programs) {
         out->n_stages = (int)kv.second.stages.size(); out->n_tasks = (int)kv.second.tasks.size();

@@ -264,12 +264,13 @@ __device__ __forceinline__ void task_target_loss(const TargetLossArgs &t, int ti
     const Pm h = resolve_pm(t.h[k], P.bases, agent);
     const float *w = resolve(t.w_out[k], P.bases, agent);
     // the row's scalars are fetched by its scalar thread BEFORE the dot products, so their latency hides behind them
-    float pre_bias[4] = {0.f, 0.f, 0.f, 0.f}, pre_alpha = 0.f, pre_logp = 0.f, pre_r = 0.f, pre_d = 0.f, pre_w = 1.f;
+    float pre_bias[4] = {0.f, 0.f, 0.f, 0.f}, pre_alpha = 0.f, pre_gamma = 0.f, pre_logp = 0.f, pre_r = 0.f, pre_d = 0.f, pre_w = 1.f;
     if ((int)threadIdx.x < R && tile * R + (int)threadIdx.x < B) {
         const int br = tile * R + threadIdx.x;
         for (int j = 0; j < 4; j++) pre_bias[j] = ldcg(resolve(t.b_out[j], P.bases, agent));
         const int n_upd = __float_as_int(ldcg(scalars + SC_N_UPDATES));
         pre_alpha = ldcg(scalars + SC_ALPHA0 + (n_upd & 1));
+        pre_gamma = ldcg(scalars + SC_GAMMA);
         const float *isw = resolve(t.is_weights, P.bases, agent);
         pre_logp = ldcg(resolve(t.logp_next, P.bases, agent) + br);
         pre_r = ldcg(resolve(t.r, P.bases, agent) + br);
@@ -299,7 +300,7 @@ __device__ __forceinline__ void task_target_loss(const TargetLossArgs &t, int ti
             const float alpha = pre_alpha;
             const float qn = fminf(qq[0], qq[1]);
             const float vt = qn - alpha * pre_logp;                                   // sac_imp.py:97
-            const float yy = pre_r + (1.f - pre_d) * t.gamma * vt;                     // :98
+            const float yy = pre_r + (1.f - pre_d) * pre_gamma * vt;                   // :98
             const float wgt = pre_w;
             const float e1 = qq[2] - yy, e2 = qq[3] - yy;
             dq1 = 2.f * wgt * e1 / (float)B;                                                                          // d mean((q-y)^2) / dq
@@ -342,11 +343,12 @@ __device__ __forceinline__ void task_actor_loss(const ActorLossArgs &t, int tile
     float *sq = smem, *sd = smem + 4 * kLossRowsMax, *sl = sd + 2 * kLossRowsMax;
     const Pm h = resolve_pm(t.h[k & 1], P.bases, agent);
     const float *w = resolve(t.w_out[k & 1], P.bases, agent);
-    float pre_b1 = 0.f, pre_b2 = 0.f, pre_alpha = 0.f, pre_logp = 0.f;      // fetched before the dot products (latency hidden)
+    float pre_b1 = 0.f, pre_b2 = 0.f, pre_alpha = 0.f, pre_ent = 0.f, pre_logp = 0.f;      // fetched before the dot products (latency hidden)
     if ((int)threadIdx.x < R && tile * R + (int)threadIdx.x < B) {
         pre_b1 = ldcg(resolve(t.b_out[0], P.bases, agent)); pre_b2 = ldcg(resolve(t.b_out[1], P.bases, agent));
         const int n_upd = __float_as_int(ldcg(scalars + SC_N_UPDATES));
         pre_alpha = ldcg(scalars + SC_ALPHA0 + (n_upd & 1));
+        pre_ent = ldcg(scalars + SC_TARGET_ENTROPY);
         pre_logp = ldcg(resolve(t.logp, P.bases, agent) + tile * R + threadIdx.x);
     }
     int64_t rows4[4];
@@ -376,7 +378,7 @@ __device__ __forceinline__ void task_actor_loss(const ActorLossArgs &t, int tile
             const float sel = q1 < q2 ? 1.f : (q1 == q2 ? 0.5f : 0.f);               // torch.minimum backward
             d1 = -sel / (float)B;
             d2 = -(1.f - sel) / (float)B;
-            ent = l + t.target_entropy;
+            ent = l + pre_ent;
         }
         sd[2 * r] = d1; sd[2 * r + 1] = d2; sl[2 * r] = pl; sl[2 * r + 1] = ent;
     }
@@ -502,8 +504,10 @@ template <bool kDeep = true>
 __device__ __forceinline__ void task_out_adam(const OutAdamArgs &t, int tile, const Program &P, int agent, const float *scalars, float *smem) {
     const int B = t.B, H = t.H, R = t.chunk_rows, n_ct = cdiv(H, kColsumCols), n_rc = cdiv(B, R);
     const float *dq = resolve(t.dq, P.bases, agent);
-    float ss, bs;
-    adam_factors_cached(scalars, t.w.step_slot, ss, bs);
+    // the Adam factors and the Polyak rate (one L2 line): ahead of the column sum, where their latency hides; the light build
+    // (kDeep = false, 64 registers) loads them behind it instead, as task_bias_adam does -- holding them across it costs that build spills
+    float ss = 0.f, bs = 0.f, tau = 0.f;
+    if constexpr (kDeep) { adam_factors_cached(scalars, t.w.step_slot, ss, bs); tau = __ldcg(scalars + SC_TAU); }
     if (tile >= n_ct * n_rc) {      // bias tile of row chunk tile - n_ct * n_rc: db = sum_b dq[b] (32 lane partials, then the warp tree)
         const int rc = tile - n_ct * n_rc, r0 = rc * R, r1 = min(B, r0 + R);
         if (threadIdx.x < 32) {
@@ -512,9 +516,10 @@ __device__ __forceinline__ void task_out_adam(const OutAdamArgs &t, int tile, co
             gb = warp_sum(gb);
             if (threadIdx.x == 0) {
                 const AdamArgs &a = t.b;
+                if constexpr (!kDeep) { adam_factors_cached(scalars, a.step_slot, ss, bs); tau = __ldcg(scalars + SC_TAU); }
                 float *w = resolve(a.w, P.bases, agent), *m = resolve(a.m, P.bases, agent), *v = resolve(a.v, P.bases, agent);
                 float *wt = resolve(a.wt, P.bases, agent), *ge = resolve(a.gexp, P.bases, agent);
-                colsum_finish(gb, n_rc > 1, ge, a.apply, prefetch_state(a.apply != 0, w, m, v, wt), w, m, v, wt, ss, bs, a.tau);
+                colsum_finish(gb, n_rc > 1, ge, a.apply, prefetch_state(a.apply != 0, w, m, v, wt), w, m, v, wt, ss, bs, tau);
             }
         }
         return;
@@ -539,7 +544,10 @@ __device__ __forceinline__ void task_out_adam(const OutAdamArgs &t, int tile, co
             for (int j = 0; j < 8; j++) out[j] = 0.f;
         }
     });
-    if (owner) colsum_finish(g, n_rc > 1, ge ? ge + n : nullptr, a.apply, st, w, m, v, wt ? wt + n : nullptr, ss, bs, a.tau);
+    if (owner) {
+        if constexpr (!kDeep) { adam_factors_cached(scalars, a.step_slot, ss, bs); tau = __ldcg(scalars + SC_TAU); }
+        colsum_finish(g, n_rc > 1, ge ? ge + n : nullptr, a.apply, st, w, m, v, wt ? wt + n : nullptr, ss, bs, tau);
+    }
 }
 
 // T_BIAS_ADAM tiles: [row chunk][64-column tile]
@@ -565,7 +573,8 @@ __device__ __forceinline__ void task_bias_adam(const ColsumAdamArgs &t, int tile
     if (owner) {
         float ss, bs;
         adam_factors_cached(scalars, a.step_slot, ss, bs);
-        colsum_finish(g, n_rc > 1, ge ? ge + n : nullptr, a.apply, st, w, m, v, bt ? bt + n : nullptr, ss, bs, a.tau);
+        const float tau = __ldcg(scalars + SC_TAU);
+        colsum_finish(g, n_rc > 1, ge ? ge + n : nullptr, a.apply, st, w, m, v, bt ? bt + n : nullptr, ss, bs, tau);
     }
 }
 
@@ -702,14 +711,15 @@ __device__ __forceinline__ void task_finish(const FinishArgs &t, const Program &
     }
     __syncthreads();
     // threads 32..35: the step counter of one optimizer each (+1, sac_imp.py:109,113,125,134) and its next bias corrections
-    // from the host-built table, fetched while thread 0 works
+    // from the host-built table with the agent's learning rate, formed while thread 0 works
     const int k = (int)threadIdx.x - 32;
     int new_step = 0;
     float2 fac = make_float2(0.f, 0.f);
     const bool bump = k >= 0 && k < 4 && t.bump[k];      // SC_STEP_POLICY, SC_STEP_Q1, SC_STEP_Q2, SC_STEP_ALPHA are consecutive
     if (bump) {
         new_step = __float_as_int(sc[SC_STEP_POLICY + k]) + 1;
-        fac = __ldg(P.adam_table + min(new_step, kAdamTable - 1));
+        const AdamBias b = P.adam_table[min(new_step, kAdamTable - 1)];
+        fac = make_float2(adam_step_size(sc[SC_LR], b.bc1), b.bc2_sqrt);
     }
     if (threadIdx.x == 0) {
         if (cp) {

@@ -9,6 +9,8 @@ reference's `from networks_model1 import ...` (sac_imp.py:4): rebind them to net
 get the 3x512 variant.  Keyword-only arguments after `device` are extensions (replay kind, math mode...).
 """
 import ctypes
+import math
+import os
 import random
 
 import numpy as np
@@ -425,22 +427,34 @@ class PopulationSAC:
     SAC(state_dim, action_dim, ...)` builds: same initialiser calls in the same order, its own Adam state, temperature, Philox stream
     (stream id = agent index) and its own uniform replay ring of `capacity` transitions in HBM -- the agent index is a grid
     dimension of every stage kernel and the 4th coordinate of the TMA descriptors.  No inter-agent (or inter-GPU) traffic:
-    `distributed.partition_agents` assigns global agent ids to ranks.  Minibatch positions are drawn on the device."""
+    `distributed.partition_agents` assigns global agent ids to ranks.  Minibatch positions are drawn on the device.
+
+    Population-based training: `gamma`, `tau`, `lr`, `alpha` and `target_entropy` (default -action_dim, sac_imp.py:46) take one value
+    for all agents or one per agent.  They live in each agent's scalar block on the device, so `set_hyperparameters` (explore) never
+    rebuilds the update program, and `exploit(dst, src)` copies whole learner states on the device.  `automatic_entropy_tuning` is
+    shared by all agents."""
+
+    HPARAMS = ("lr", "gamma", "tau", "target_entropy", "alpha")
 
     def __init__(self, n_agents, state_dim, action_dim, hidden_dim=256, gamma=0.99, tau=0.005, lr=3e-4, alpha=0.2,
                  automatic_entropy_tuning=True, device="cuda", *, seeds=None, capacity=100000, max_batch=256, math="bf16x3",
-                 launch="staged", seed=None, action_bounds=None):
+                 launch="staged", seed=None, action_bounds=None, target_entropy=None):
         if not str(device).startswith("cuda"):
             raise RuntimeError("PopulationSAC runs on a B200 only (device='cuda[:i]'); there is no CPU path")
         self.n_agents, self.device = int(n_agents), device
         self.seeds = list(range(self.n_agents)) if seeds is None else [int(x) for x in seeds]
         if len(self.seeds) != self.n_agents:
             raise ValueError("one seed per agent")
+        hp = {k: self._per_agent(k, v) for k, v in (("lr", lr), ("gamma", gamma), ("tau", tau), ("alpha", alpha),
+                                                     ("target_entropy", -float(action_dim) if target_entropy is None else target_entropy))}
+        for i in range(self.n_agents):
+            self._check_hparams({k: v[i] for k, v in hp.items()})
         kw = {} if action_bounds is None else {"action_bounds": action_bounds}
         probe = GaussianPolicy(state_dim, action_dim, hidden_dim, **kw)
         cfg = N.default_config()
         cfg.obs_dim, cfg.act_dim, cfg.hidden_dim, cfg.n_hidden = state_dim, action_dim, hidden_dim, getattr(probe, "N_HIDDEN", 2)
-        cfg.gamma, cfg.tau, cfg.lr, cfg.alpha0, cfg.auto_entropy = gamma, tau, lr, alpha, int(bool(automatic_entropy_tuning))
+        cfg.gamma, cfg.tau, cfg.lr, cfg.alpha0 = hp["gamma"][0], hp["tau"][0], hp["lr"][0], hp["alpha"][0]
+        cfg.auto_entropy = int(bool(automatic_entropy_tuning))
         cfg.action_scale, cfg.action_bias = probe.action_scale, probe.action_bias
         cfg.replay_kind, cfg.capacity, cfg.max_batch, cfg.n_agents = N.REPLAY_UNIFORM, capacity, max_batch, self.n_agents
         cfg.device = torch.device(device).index or 0
@@ -461,6 +475,11 @@ class PopulationSAC:
                 for t, (_, p) in enumerate(mod.named_parameters()):
                     host = N.f32(p.detach().numpy())
                     N.check(lib.sacb_import_tensor(self._h, i, net_id, N.SLOT_PARAM, t, N.ptr(host), host.size))
+        default = (cfg.lr, cfg.gamma, cfg.tau, -float(action_dim), cfg.alpha0)
+        for i in range(self.n_agents):
+            mine = {k: float(np.float32(hp[k][i])) for k in self.HPARAMS}
+            if tuple(mine.values()) != tuple(float(np.float32(x)) for x in default):
+                self.set_hyperparameters(i, **mine)
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -544,3 +563,150 @@ class PopulationSAC:
         a = checkpoint["alpha"]
         sc.alpha = float(a.detach().reshape(-1)[0]) if torch.is_tensor(a) else float(a)
         N.check(lib.sacb_set_scalars(self._h, int(agent), ctypes.byref(sc)))
+
+    # ---- population-based training: per-agent hyperparameters, exploit, member checkpoints ---------------------------------------------
+    def _per_agent(self, name, value):
+        if np.ndim(value) == 0:
+            return [float(value)] * self.n_agents
+        vals = [float(x) for x in value]
+        if len(vals) != self.n_agents:
+            raise ValueError(f"{name}: one value or one per agent ({self.n_agents}), got {len(vals)}")
+        return vals
+
+    @staticmethod
+    def _check_hparams(hp):
+        """The library refuses the same values (sacb_set_hparams); alpha is checked here because it travels in sacb_set_scalars."""
+        if "alpha" in hp and not (math.isfinite(hp["alpha"]) and hp["alpha"] >= 0):
+            raise ValueError(f"alpha must be finite and >= 0, got {hp['alpha']}")
+        if "lr" in hp and not (math.isfinite(hp["lr"]) and hp["lr"] > 0):
+            raise ValueError(f"lr must be finite and > 0, got {hp['lr']}")
+        for k in ("gamma", "tau"):
+            if k in hp and not 0.0 <= hp[k] <= 1.0:
+                raise ValueError(f"{k} must lie in [0, 1], got {hp[k]}")
+        if "target_entropy" in hp and not math.isfinite(hp["target_entropy"]):
+            raise ValueError(f"target_entropy must be finite, got {hp['target_entropy']}")
+
+    def _agent_index(self, agent):
+        i = int(agent)
+        if not 0 <= i < self.n_agents:
+            raise ValueError(f"agent {agent} out of range [0, {self.n_agents})")
+        return i
+
+    def hyperparameters(self, agent):
+        """{lr, gamma, tau, target_entropy, alpha} of one agent as the device holds them (float32 values)."""
+        i, lib = self._agent_index(agent), N.lib()
+        hp, sc = N.Hparams(), N.Scalars()
+        N.check(lib.sacb_get_hparams(self._h, i, ctypes.byref(hp)))
+        N.check(lib.sacb_get_scalars(self._h, i, ctypes.byref(sc)))
+        return {"lr": hp.lr, "gamma": hp.gamma, "tau": hp.tau, "target_entropy": hp.target_entropy, "alpha": sc.alpha}
+
+    def set_hyperparameters(self, agent, **kw):
+        """Explore step: change only the given keys of one agent, effective from its next update (no program is rebuilt).  A new lr
+        applies to all four optimizers of the agent from their current step counts; a new alpha is the temperature of the next update
+        (with automatic entropy tuning, log_alpha keeps its value and the tuned alpha takes over after that update)."""
+        i, lib = self._agent_index(agent), N.lib()
+        unknown = set(kw) - set(self.HPARAMS)
+        if unknown:
+            raise ValueError(f"unknown hyperparameters {sorted(unknown)}; known: {self.HPARAMS}")
+        kw = {k: float(v) for k, v in kw.items()}
+        self._check_hparams(kw)
+        if set(kw) - {"alpha"}:
+            cur = N.Hparams()
+            N.check(lib.sacb_get_hparams(self._h, i, ctypes.byref(cur)))
+            for k in ("lr", "gamma", "tau", "target_entropy"):
+                if k in kw:
+                    setattr(cur, k, kw[k])
+            N.check(lib.sacb_set_hparams(self._h, i, ctypes.byref(cur)))
+        if "alpha" in kw:
+            sc = N.Scalars()
+            N.check(lib.sacb_get_scalars(self._h, i, ctypes.byref(sc)))
+            sc.alpha = kw["alpha"]
+            N.check(lib.sacb_set_scalars(self._h, i, ctypes.byref(sc)))
+
+    def exploit(self, dst, src):
+        """Exploit step: agent dst[k] takes over the whole learner state of agent src[k] (weights, targets, Adam state, temperature,
+        hyperparameters, step counts), copied on the device.  Replay rings stay with their agent, and dst[k] keeps drawing its own
+        minibatch positions and noise (the device streams are keyed by agent index).  A dst may appear once, and no agent may be both
+        a src and a dst of the same call (ValueError)."""
+        d = np.ascontiguousarray(np.asarray(dst, np.int64).ravel())
+        s = np.ascontiguousarray(np.asarray(src, np.int64).ravel())
+        if d.size != s.size:
+            raise ValueError("exploit: dst and src must have the same length")
+        if d.size and (min(d.min(), s.min()) < 0 or max(d.max(), s.max()) >= self.n_agents):
+            raise ValueError(f"exploit: agent index out of range [0, {self.n_agents})")
+        d32, s32 = d.astype(np.int32), s.astype(np.int32)
+        N.check(N.lib().sacb_copy_agents(self._h, N.ptr(d32, ctypes.c_int32), N.ptr(s32, ctypes.c_int32), int(d.size)))
+
+    def _optimizer_state(self, agent, net_id, sc, lr):
+        step = {N.NET_POLICY: sc.step_policy, N.NET_Q1: sc.step_q1, N.NET_Q2: sc.step_q2, None: sc.step_alpha}[net_id]
+        names = [None] if net_id is None else self._names[net_id]
+        state = {}
+        if step > 0:
+            lib = N.lib()
+            for t, entry in enumerate(names):
+                if net_id is None:
+                    m, v = torch.tensor([sc.log_alpha_m]), torch.tensor([sc.log_alpha_v])
+                else:
+                    m, v = (np.empty(entry[1], np.float32) for _ in range(2))
+                    for slot, host in ((N.SLOT_ADAM_M, m), (N.SLOT_ADAM_V, v)):
+                        N.check(lib.sacb_export_tensor(self._h, agent, net_id, slot, t, N.ptr(host), host.size))
+                    m, v = torch.from_numpy(m), torch.from_numpy(v)
+                state[t] = {"step": torch.tensor(float(step)), "exp_avg": m, "exp_avg_sq": v}
+        group = ArenaAdam(None, net_id, None, lr).param_groups[0]
+        group["params"] = list(range(len(names)))
+        return {"state": state, "param_groups": [group]}
+
+    def agent_checkpoint(self, agent):
+        """One member as a dictionary in the key layout of SAC.save_checkpoint without 'replay_buffer' (torch.save it): the five nets,
+        the three optimizer state_dicts, 'alpha', 'log_alpha' and 'alpha_optimizer_state_dict' (with automatic entropy tuning), and the
+        extension key 'sacb_hyperparameters' ({lr, gamma, tau, target_entropy}).  SAC.load_checkpoint accepts the file: that is how a
+        member leaves the population (SAC keeps its own gamma / tau / target_entropy; pass them to its constructor or sacb_set_hparams)."""
+        i = self._agent_index(agent)
+        self.synchronize()
+        hp = self.hyperparameters(i)
+        sc = N.Scalars()
+        N.check(N.lib().sacb_get_scalars(self._h, i, ctypes.byref(sc)))
+        ck = {k: v for k, v in self.agent_state(i).items() if k.endswith("_state_dict")}
+        for net_id, name in ((N.NET_POLICY, "policy"), (N.NET_Q1, "q1"), (N.NET_Q2, "q2")):
+            ck[f"{name}_optimizer_state_dict"] = self._optimizer_state(i, net_id, sc, hp["lr"])
+        auto = bool(self._cfg.auto_entropy)
+        ck["alpha"] = float(sc.alpha) if sc.n_updates == 0 or not auto else torch.tensor([sc.alpha])
+        if auto:
+            ck["log_alpha"] = torch.tensor([sc.log_alpha], requires_grad=True)
+            ck["alpha_optimizer_state_dict"] = self._optimizer_state(i, None, sc, hp["lr"])
+        ck["sacb_hyperparameters"] = {k: hp[k] for k in ("lr", "gamma", "tau", "target_entropy")}
+        return ck
+
+    def load_agent_checkpoint(self, agent, checkpoint):
+        """Inverse of `agent_checkpoint`; also takes a file (or dictionary) written by SAC.save_checkpoint.  Loads the nets, the Adam
+        state and step counts, alpha and log_alpha, and the hyperparameters: 'sacb_hyperparameters' when present, otherwise the
+        optimizers' learning rate (gamma, tau and target_entropy of the member then stay as they are)."""
+        i, lib = self._agent_index(agent), N.lib()
+        if isinstance(checkpoint, (str, bytes, os.PathLike)):
+            checkpoint = torch.load(checkpoint, map_location="cpu", weights_only=False)
+        hp = checkpoint.get("sacb_hyperparameters")
+        if hp is None:
+            groups = checkpoint.get("policy_optimizer_state_dict", {}).get("param_groups")
+            hp = {"lr": float(groups[0]["lr"])} if groups else {}
+        self.set_hyperparameters(i, **{k: float(v) for k, v in hp.items()})      # lr first: the step counts below take its factors
+        self.load_agent(i, checkpoint)
+        sc = N.Scalars()
+        N.check(lib.sacb_get_scalars(self._h, i, ctypes.byref(sc)))
+        for net_id, name, attr in ((N.NET_POLICY, "policy", "step_policy"), (N.NET_Q1, "q1", "step_q1"), (N.NET_Q2, "q2", "step_q2")):
+            state = checkpoint.get(f"{name}_optimizer_state_dict", {"state": {}})["state"]
+            setattr(sc, attr, int(float(state[min(state)]["step"])) if state else 0)
+            for t, st in state.items():
+                for slot, key in ((N.SLOT_ADAM_M, "exp_avg"), (N.SLOT_ADAM_V, "exp_avg_sq")):
+                    host = N.f32(torch.as_tensor(st[key]).detach().cpu().numpy())
+                    N.check(lib.sacb_import_tensor(self._h, i, net_id, slot, int(t), N.ptr(host), host.size))
+        if self._cfg.auto_entropy and "log_alpha" in checkpoint:
+            sc.log_alpha = float(torch.as_tensor(checkpoint["log_alpha"]).detach().reshape(-1)[0])
+            state = checkpoint.get("alpha_optimizer_state_dict", {"state": {}})["state"]
+            if state:
+                first = state[min(state)]
+                sc.step_alpha = int(float(first["step"]))
+                sc.log_alpha_m = float(torch.as_tensor(first["exp_avg"]).reshape(-1)[0])
+                sc.log_alpha_v = float(torch.as_tensor(first["exp_avg_sq"]).reshape(-1)[0])
+            else:
+                sc.step_alpha, sc.log_alpha_m, sc.log_alpha_v = 0, 0.0, 0.0
+        N.check(lib.sacb_set_scalars(self._h, i, ctypes.byref(sc)))

@@ -105,9 +105,24 @@ typedef struct {
 } sacb_scalars;
 int sacb_get_scalars(sacb_handle h, int agent, sacb_scalars *out);
 int sacb_set_scalars(sacb_handle h, int agent, const sacb_scalars *in);
-/* torch.optim.Adam.load_state_dict restores param_groups[0]['lr'] (sac_imp.py:215-218): rebuilds the Adam step-size table and the
- * cached bias-correction factors of every agent for the new learning rate (all four optimizers share it, sac_imp.py:39-49). */
+/* torch.optim.Adam.load_state_dict restores param_groups[0]['lr'] (sac_imp.py:215-218): sets the learning rate of every agent (all
+ * four optimizers of an agent share it, sac_imp.py:39-49) and refreshes their cached bias-correction factors.  No program is rebuilt. */
 int sacb_set_lr(sacb_handle h, float lr);
+/* Hyperparameters of one agent, kept in its scalar block on the device: every update reads them there, so changing one never rebuilds
+ * or re-captures an update program.  sacb_create gives every agent lr, gamma, tau of sacb_config and target_entropy = -act_dim
+ * (sac_imp.py:46).  lr drives all four optimizers of the agent; target_entropy matters with auto_entropy only.  Per-agent alpha:
+ * sacb_set_scalars.  sacb_set_hparams: lr finite and > 0, gamma and tau in [0, 1], target_entropy finite (SACB_ERR_ARG otherwise);
+ * the agent's cached Adam factors follow the new lr at its current step counts.  Both calls are ordered on the handle's stream. */
+typedef struct { float lr, gamma, tau, target_entropy; } sacb_hparams;
+int sacb_get_hparams(sacb_handle h, int agent, sacb_hparams *out);
+int sacb_set_hparams(sacb_handle h, int agent, const sacb_hparams *in);
+/* Exploit step of population-based training: for each i, agent dst[i] takes over the whole learner state of agent src[i] -- weights,
+ * Polyak targets, Adam moments, weight shadows and the scalar block (hyperparameters, step counts, log_alpha and its Adam state,
+ * alpha, cached factors, loss history).  Replay rings and workspaces are not copied.  Device-to-device copies enqueued on the handle's
+ * stream (no host synchronisation).  The destination keeps its own Philox streams: on-device draws are keyed by agent index, so after
+ * the copy dst[i] continues with src[i]'s step count but draws its own minibatch positions and noise.  SACB_ERR_ARG for an index out
+ * of range, a repeated dst, or an index that appears both as a src and as a dst in the same call. */
+int sacb_copy_agents(sacb_handle h, const int32_t *dst, const int32_t *src, int n);
 
 /* ---- replay: ReplayBuffer.push / PrioritizedReplayBuffer.push (replay_buffer.py:10-11, :36-46) ----------
  * n transitions, row-major float32 (the cast of sac_imp.py:81-85 happens in the shim); done as 0/1 floats. */
@@ -228,6 +243,7 @@ typedef struct {
     int64_t kernel_launches;   /* kernels of this library launched since create (graph nodes counted per replay) */
     int32_t n_stages, n_tasks, n_tiles;    /* of the current update program */
     int32_t grid, block, smem_bytes, sm_count;
+    int32_t n_programs;        /* update programs built since create (one per batch size / mode; never per hyperparameter value) */
 } sacb_stats;
 int sacb_get_stats(sacb_handle h, sacb_stats *out);
 /* CUDA-event stopwatch on the handle's stream (torch.cuda.Event only sees torch's stream). */
