@@ -284,16 +284,12 @@ extern "C" int sacb_dp_backward(sacb_handle h, int phase, int64_t B_local, const
             h->dp_device_eps = 1;
         }
     }
-    ProgramKey key{(int)B_local, phase == 0 ? 1 : 0, 1, h->dp_device_eps, 0, phase};
-    ProgramInst *p;
-    rc = get_program(h, key, &p);
-    if (rc) return rc;
     {   // large batches accumulate their gradients over K / row chunks with atomics: the phase's slab starts at zero
         const Layout &L = h->L;
         if (phase == 0) SACB_CUDA(cudaMemsetAsync(h->arena + L.grad[1], 0, sizeof(float) * 2 * L.q.size, h->stream));
         else SACB_CUDA(cudaMemsetAsync(h->arena + L.grad[0], 0, sizeof(float) * L.pol.size, h->stream));
     }
-    return launch_program(h, *p);
+    return run_update(h, ProgramKey{(int)B_local, phase == 0 ? 1 : 0, 1, h->dp_device_eps, 0, phase});
 }
 
 extern "C" int sacb_dp_apply(sacb_handle h, int phase) {

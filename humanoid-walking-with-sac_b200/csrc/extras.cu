@@ -153,17 +153,6 @@ __global__ void action_pdl_kernel(const float *head, const float *eps, int n, in
     act[i] = sample_elem(mean, ls, e, scale, bias).action;
 }
 
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_chain(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-
 // policy forward + action for `rows` observations (rows_per_agent consecutive rows belong to one agent, first agent = agent0);
 // obs / eps / action travel through pinned memory, one synchronisation
 static int select_action_rows(sacb_handle h, int agent0, int rows, int rows_per_agent, const float *obs, int evaluate, const float *eps, float *action_out) {
@@ -196,14 +185,14 @@ static int select_action_rows(sacb_handle h, int agent0, int rows, int rows_per_
         a.in = l == 0 ? O : H; a.out = l < nh ? H : 2 * A; a.relu = l < nh && !nl.layer_norm; a.agent_stride = h->L.arena_size;
         float *y = l < nh ? bufs[l & 1] : d_head;
         const int ldy = l < nh ? H : 2 * A;
-        SACB_CUDA(launch_chain(mlp_layer_kernel, dim3((a.out + 15) / 16, rows), dim3(512), sizeof(float) * a.in, h->stream, a, x, ldx, y, ldy, rows_per_agent));
+        SACB_CUDA(launch_pdl(mlp_layer_kernel, dim3((a.out + 15) / 16, rows), dim3(512), sizeof(float) * a.in, h->stream, true, a, x, ldx, y, ldy, rows_per_agent));
         if (l < nh && nl.layer_norm) {
-            SACB_CUDA(launch_chain(ln_relu_rows_kernel, dim3(rows), dim3(256), 0, h->stream, y, ldy, H, base + nl.g[l], base + nl.be[l], (int64_t)h->L.arena_size, rows_per_agent));
+            SACB_CUDA(launch_pdl(ln_relu_rows_kernel, dim3(rows), dim3(256), 0, h->stream, true, y, ldy, H, base + nl.g[l], base + nl.be[l], (int64_t)h->L.arena_size, rows_per_agent));
             h->kernel_launches++;
         }
         x = y; ldx = ldy;
     }
-    SACB_CUDA(launch_chain(action_pdl_kernel, dim3((rows * A + 127) / 128), dim3(128), 0, h->stream, (const float *)d_head, (const float *)(use_eps ? d_eps : nullptr),
+    SACB_CUDA(launch_pdl(action_pdl_kernel, dim3((rows * A + 127) / 128), dim3(128), 0, h->stream, true, (const float *)d_head, (const float *)(use_eps ? d_eps : nullptr),
                            rows, A, evaluate, h->cfg.action_scale, h->cfg.action_bias, d_act, h->cfg.seed, h->act_counter++));
     h->kernel_launches += nh + 2;
     SACB_CUDA(cudaMemcpyAsync(p_act, d_act, sizeof(float) * A * rows, cudaMemcpyDeviceToHost, h->stream));

@@ -104,21 +104,48 @@ struct ProgramInst {
     Task *d_tasks = nullptr;
     Stage *d_stages = nullptr;
     Program prog{};
+    // one update step (program.cu: enqueue_step) as a graph, and the kernel launches one replay of it stands for
     cudaGraphExec_t graph = nullptr;
-    // the same step as two graphs split in front of the actor-loss stage (the TD errors exist since the critic-loss stage):
-    // sacb_per_step runs the priority write-back and the next prioritized sample on a second stream under the tail of the update
-    cudaGraphExec_t graph_part[2] = {nullptr, nullptr};
+    int graph_launches = 0;
+    // the whole pipelined learner step (sacb_per_step, program.cu: enqueue_per_step) as ONE graph: update launches on the main stream,
+    // priority write-back and the next sample forked onto the second stream in front of launch `split` (the actor-loss stage: the TD
+    // errors exist since the critic-loss stage), joined at the end (valid for one buffer length / batch size)
     int split = -1;                      // index into `launches`
-    bool parts_built = false;
-    // the whole pipelined learner step (sacb_per_step) as ONE graph: update stages on the main stream, priority write-back and the next
-    // sample forked onto the second stream in front of stage `split`, joined at the end (valid for one buffer length / batch size)
     cudaGraphExec_t step_graph = nullptr;
     int64_t step_graph_n = -1, step_graph_k = -1;
     bool step_graph_failed = false;
     int step_graph_launches = 0;
     int n_tiles_total = 0, max_stage_tiles = 0;
-    int kernels_per_step = 0;
 };
+
+// Launch configuration of cudaLaunchKernelEx / cudaLaunchKernelExC: optional programmatic dependent launch (the kernel may become
+// resident while its predecessor on the stream still runs, and waits in griddepcontrol.wait) and optional thread-block clusters of
+// `cluster` CTAs along x (0: no cluster attribute).  Not copyable: `cfg.attrs` points into the object.
+struct LaunchConfig {
+    cudaLaunchConfig_t cfg{};
+    cudaLaunchAttribute attr[2];
+    LaunchConfig(dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool pdl, int cluster = 0) {
+        cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+        cfg.attrs = attr; cfg.numAttrs = 0;
+        if (pdl) {
+            attr[cfg.numAttrs].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+            attr[cfg.numAttrs++].val.programmaticStreamSerializationAllowed = 1;
+        }
+        if (cluster > 0) {
+            attr[cfg.numAttrs].id = cudaLaunchAttributeClusterDimension;
+            attr[cfg.numAttrs].val.clusterDim.x = cluster; attr[cfg.numAttrs].val.clusterDim.y = 1; attr[cfg.numAttrs].val.clusterDim.z = 1;
+            cfg.numAttrs++;
+        }
+    }
+    LaunchConfig(const LaunchConfig &) = delete;
+    LaunchConfig &operator=(const LaunchConfig &) = delete;
+};
+
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool pdl, Args... args) {
+    LaunchConfig lc(grid, block, smem, stream, pdl);
+    return cudaLaunchKernelEx(&lc.cfg, kernel, KArgs(args)...);
+}
 
 }  // namespace sacb
 
@@ -204,17 +231,22 @@ int pick_variant(uint32_t task_types, uint32_t epilogues, bool allow_light_colsu
 // program.cu
 int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out);
 int launch_program(sacb_handle h, ProgramInst &p);
-int launch_program_part(sacb_handle h, ProgramInst &p, int part);
-int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k);      // SACB_OK, an error, or 1: not available (caller falls back)   // 0: up to and including the critic-loss stage, 1: the rest
+// sacb_per_step's launches, enqueued directly (persistent mode: the whole update in front of the fork)
+int enqueue_per_step(sacb_handle h, ProgramInst &p, int64_t B, int64_t k);
+int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k);      // SACB_OK, an error, or 1: not available (caller falls back)
 void free_programs(sacb_handle h);
 int check_error_flag(sacb_handle h);
 // the key of the program that serves the next update of this handle (fills ProgramKey::resident), and the bookkeeping behind its launch
 ProgramKey update_key(sacb_handle h, int B, int with_gather, int export_grads, int device_eps, int use_isw);
 void after_update_launch(sacb_handle h, const ProgramKey &key);
+int run_update(sacb_handle h, const ProgramKey &key);      // get_program + launch_program + after_update_launch
+// the steady-state program of the timing entry points (shadows resident), behind one update that derives the shadows if they are not
+int steady_program(sacb_handle h, int64_t B, ProgramInst **out);
 // replay.cu
 int replay_create(sacb_handle h);
 void replay_destroy(sacb_handle h);
 int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B, int64_t *k_out);   // kernels of one sample() call
+int upload_per_frame(sacb_handle h, cudaStream_t st);                                                   // frame counter -> device, if sacb_per_set_frame changed it
 int upload_ring_meta(sacb_handle h);                                                                   // (len, head) of every agent's ring -> device, if a push changed them
 int per_writeback_launch(sacb_handle h, cudaStream_t st, int64_t B, bool pdl_ok = true);                                 // priorities <- |td| of the last update
 }  // namespace sacb

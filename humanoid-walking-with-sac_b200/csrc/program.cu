@@ -1033,7 +1033,6 @@ static void fill_chain_maps(const std::vector<Task> &tasks, std::vector<Stage> &
 void free_programs(sacb_handle h) {
     for (auto &kv : h->programs) {
         if (kv.second.graph) cudaGraphExecDestroy(kv.second.graph);
-        for (auto g : kv.second.graph_part) if (g) cudaGraphExecDestroy(g);
         if (kv.second.step_graph) cudaGraphExecDestroy(kv.second.step_graph);
         cudaFree(kv.second.d_tasks); cudaFree(kv.second.d_stages);
     }
@@ -1056,14 +1055,9 @@ int check_error_flag(sacb_handle h) {
 static int launch_stream_stage(sacb_handle h, ProgramInst &p, int s, bool pdl) {
     Stage single = p.stages[s];
     void *args[] = {(void *)&p.prog, (void *)&single};
-    cudaLaunchConfig_t cfg{};
     const int tiles = std::max(1, single.n_tiles * h->cfg.n_agents);
-    cfg.gridDim = dim3(std::min(tiles, h->sm_count)); cfg.blockDim = dim3(stream::kThreads); cfg.dynamicSmemBytes = stream::kSmemBytes; cfg.stream = h->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    SACB_CUDA(cudaLaunchKernelExC(&cfg, (const void *)sac_stream_kernel, args));
+    LaunchConfig lc(dim3(std::min(tiles, h->sm_count)), dim3(stream::kThreads), stream::kSmemBytes, h->stream, pdl);
+    SACB_CUDA(cudaLaunchKernelExC(&lc.cfg, (const void *)sac_stream_kernel, args));
     return SACB_OK;
 }
 
@@ -1079,7 +1073,6 @@ static int launch_stage(sacb_handle h, ProgramInst &p, int li, bool pdl) {
     int s0 = L.s0, s1 = L.s1, tc_setup = tc ? p.stage_has_gemm[s] : 0, chained = chain ? 1 : 0;
     Stage single = p.stages[s];
     void *args[] = {(void *)&p.prog, (void *)&single, (void *)&s0, (void *)&s1, (void *)&tc_setup, (void *)&chained, (void *)&seed};
-    cudaLaunchConfig_t cfg{};
     int ctas = chain ? L.grid : std::max(1, single.n_tiles * h->cfg.n_agents);
     // population mode: a stage of many more tiles than SMs runs as one resident CTA per SM looping over tiles (barrier /
     // TMEM setup and teardown once per SM instead of once per tile); a single agent's stage (<= ~150 tiles) keeps one CTA per tile
@@ -1089,24 +1082,11 @@ static int launch_stage(sacb_handle h, ProgramInst &p, int li, bool pdl) {
         // walks: the task record is fetched once instead of once per tile (population mode: a column-sum stage holds 2-6 tasks)
         if (single.task_end - single.task_begin > 1 && single.n_tiles <= ctas / 2) ctas = (ctas / single.n_tiles) * single.n_tiles;
     }
-    cfg.gridDim = dim3(ctas); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = h->stream;
-    cudaLaunchAttribute attr[2];
-    int na = 0;
-    if (pdl) {
-        // programmatic dependent launch: the next stage's CTAs may become resident (on SMs this stage leaves idle) and run
-        // their prologue -- barrier init, TMEM allocation, stage / task table fetch, TMA descriptor prefetch -- while this
-        // stage still computes; they block in griddepcontrol.wait before touching anything a previous stage wrote
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
-        na++;
-    }
-    if (chain && L.cluster > 1) {
-        attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = L.cluster; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
-        na++;
-    }
-    cfg.attrs = attr; cfg.numAttrs = na;
-    SACB_CUDA(cudaLaunchKernelExC(&cfg, update_kernel_for(h->cfg.math_mode, kind), args));
+    // programmatic dependent launch: the next stage's CTAs may become resident (on SMs this stage leaves idle) and run their prologue
+    // -- barrier init, TMEM allocation, stage / task table fetch, TMA descriptor prefetch -- while this stage still computes; they
+    // block in griddepcontrol.wait before touching anything a previous stage wrote
+    LaunchConfig lc(dim3(ctas), dim3(kThreads), smem, h->stream, pdl, chain && L.cluster > 1 ? L.cluster : 0);
+    SACB_CUDA(cudaLaunchKernelExC(&lc.cfg, update_kernel_for(h->cfg.math_mode, kind), args));
     return SACB_OK;
 }
 
@@ -1126,16 +1106,42 @@ static int launch_range(sacb_handle h, ProgramInst &p, int s0, int s1) {
     return SACB_OK;
 }
 
-static int record_step(sacb_handle h, ProgramInst &p) {
+// the launches [l0, l1) of a staged program
+static int enqueue_launches(sacb_handle h, ProgramInst &p, int l0, int l1) {
+    for (int li = l0; li < l1; li++)
+        if (int rc = launch_stage(h, p, li, h->use_pdl != 0)) return rc;
+    h->kernel_launches += l1 - l0;
+    return SACB_OK;
+}
+
+// one update step: the stage launches, or (persistent mode) the barrier reset + the single cooperative launch
+static int enqueue_step(sacb_handle h, ProgramInst &p) {
     if (h->cfg.launch_mode == SACB_LAUNCH_PERSISTENT) {
         SACB_CUDA(cudaMemsetAsync(h->barrier, 0, sizeof(unsigned int), h->stream));
+        h->kernel_launches++;
         return launch_range(h, p, 0, (int)p.stages.size());
     }
-    for (int li = 0; li < (int)p.launches.size(); li++) {
-        int rc = launch_stage(h, p, li, h->use_pdl != 0);
-        if (rc) return rc;
+    return enqueue_launches(h, p, 0, (int)p.launches.size());
+}
+
+// what `enqueue` puts on h->stream (and on the streams it forks from there) as one executable graph; nullptr if the capture fails.
+// The host counters the enqueue helpers advance are restored (a replay of the graph accounts for itself); `launches_counted` receives
+// the kernel launches they counted.
+template <typename Enqueue>
+static cudaGraphExec_t capture(sacb_handle h, Enqueue enqueue, int *launches_counted) {
+    const int64_t launches0 = h->kernel_launches, frame0 = h->per_frame[0];
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
+        const int rc = enqueue();
+        const cudaError_t e = cudaStreamEndCapture(h->stream, &graph);
+        if (rc == SACB_OK && e == cudaSuccess && graph && cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) exec = nullptr;
+        if (graph) cudaGraphDestroy(graph);
     }
-    return SACB_OK;
+    cudaGetLastError();
+    *launches_counted = (int)(h->kernel_launches - launches0);
+    h->kernel_launches = launches0; h->per_frame[0] = frame0;
+    return exec;
 }
 
 // clusters of `cluster` CTAs of kernel variant `kind` the GPU holds at once (cached per handle); < 0: a CUDA error code
@@ -1143,14 +1149,9 @@ static int max_active_clusters(sacb_handle h, int kind, int cluster) {
     const auto key = std::make_pair(kind, cluster);
     const auto it = h->max_active_clusters.find(key);
     if (it != h->max_active_clusters.end()) return it->second;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(cluster); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = math_smem(h->cfg.math_mode); cfg.stream = h->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = cluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
+    LaunchConfig lc(dim3(cluster), dim3(kThreads), math_smem(h->cfg.math_mode), h->stream, false, cluster);
     int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, update_kernel_for(h->cfg.math_mode, kind), &cfg) != cudaSuccess) {
+    if (cudaOccupancyMaxActiveClusters(&n, update_kernel_for(h->cfg.math_mode, kind), &lc.cfg) != cudaSuccess) {
         cudaGetLastError();
         return fail(SACB_ERR_DEVICE, "cudaOccupancyMaxActiveClusters failed");
     }
@@ -1251,20 +1252,7 @@ int get_program(sacb_handle h, const ProgramKey &key, ProgramInst **out) {
     P.error_flag = h->error_flag;
     P.trace = nullptr; P.timeline = nullptr; P.adam_table = h->adam_table;
     P.host_losses = h->cfg.n_agents == 1 ? h->pin_small : nullptr;
-    p.kernels_per_step = h->cfg.launch_mode == SACB_LAUNCH_PERSISTENT ? 1 : (int)p.launches.size();
-
-    // capture one step into a CUDA graph (stage kernels, or memset + the single cooperative launch)
-    cudaGraph_t graph = nullptr;
-    cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
-    if (e == cudaSuccess) {
-        int rc = record_step(h, p);
-        cudaError_t e2 = cudaStreamEndCapture(h->stream, &graph);
-        if (rc == SACB_OK && e2 == cudaSuccess && graph) {
-            if (cudaGraphInstantiate(&p.graph, graph, 0) != cudaSuccess) p.graph = nullptr;
-        }
-        if (graph) cudaGraphDestroy(graph);
-    }
-    cudaGetLastError();   // a failed capture falls back to direct launches
+    p.graph = capture(h, [&] { return enqueue_step(h, p); }, &p.graph_launches);      // none: launch_program enqueues the step directly
     *out = &p;
     return SACB_OK;
 }
@@ -1280,9 +1268,24 @@ void after_update_launch(sacb_handle h, const ProgramKey &key) {
 }
 
 int launch_program(sacb_handle h, ProgramInst &p) {
-    h->kernel_launches += p.kernels_per_step;
-    if (p.graph) { SACB_CUDA(cudaGraphLaunch(p.graph, h->stream)); return SACB_OK; }
-    return record_step(h, p);
+    if (!p.graph) return enqueue_step(h, p);
+    SACB_CUDA(cudaGraphLaunch(p.graph, h->stream));
+    h->kernel_launches += p.graph_launches;
+    return SACB_OK;
+}
+
+int run_update(sacb_handle h, const ProgramKey &key) {
+    ProgramInst *p;
+    int rc = get_program(h, key, &p);
+    if (rc == SACB_OK) rc = launch_program(h, *p);
+    if (rc == SACB_OK) after_update_launch(h, key);
+    return rc;
+}
+
+int steady_program(sacb_handle h, int64_t B, ProgramInst **out) {
+    if (!h->shadows_valid)
+        if (int rc = run_update(h, update_key(h, (int)B, 0, 0, 1, 0))) return rc;
+    return get_program(h, update_key(h, (int)B, 0, 0, 1, 0), out);
 }
 
 // The replay work may start anywhere behind the critic-loss stage (the TD errors exist from there on).  It is started in front
@@ -1305,69 +1308,39 @@ static int compute_split(ProgramInst &p) {
     return SACB_OK;
 }
 
-// sacb_per_step as one graph launch (two graph launches + two events cost ~8 us per step: 206 against 198 us with no replay work at all)
-int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
-    if (h->cfg.launch_mode != SACB_LAUNCH_STAGED || p.step_graph_failed) return 1;
+// One pipelined learner step (sacb_per_step): the update's launches in front of `split` on the main stream; the priority write-back
+// and the sample for the next step forked onto the second stream behind them; the rest of the update; the join.  Persistent mode cannot
+// split its single cooperative launch: the whole update runs in front of the fork.
+int enqueue_per_step(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
+    const bool staged = h->cfg.launch_mode == SACB_LAUNCH_STAGED;
     const int nl = (int)p.launches.size();
-    const int64_t n = h->r_len[0];
-    if (!p.step_graph || p.step_graph_n != n || p.step_graph_k != k) {
-        if (p.step_graph) { cudaGraphExecDestroy(p.step_graph); p.step_graph = nullptr; }
-        if (p.split < 0) { if (int rc = compute_split(p)) return rc; }
-        if (h->per_frame_dirty) return 1;      // the first (uncaptured) sample uploads the frame counter
-        // host-side bookkeeping of the launch helpers is replayed per graph launch below: undo what the capture pass does to it
-        const int64_t launches0 = h->kernel_launches, frame0 = h->per_frame[0];
-        cudaGraph_t graph = nullptr;
-        if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { cudaGetLastError(); p.step_graph_failed = true; return 1; }
-        int rc = SACB_OK;
-        for (int li = 0; li < p.split && rc == SACB_OK; li++) rc = launch_stage(h, p, li, h->use_pdl != 0);
-        if (rc == SACB_OK && (cudaEventRecord(h->ev_td, h->stream) != cudaSuccess || cudaStreamWaitEvent(h->stream2, h->ev_td, 0) != cudaSuccess)) rc = SACB_ERR_DEVICE;
-        if (rc == SACB_OK) rc = per_writeback_launch(h, h->stream2, k, false);      // first kernel of the forked branch: a full dependency
-        if (rc == SACB_OK) rc = per_sample_launch(h, h->stream2, nullptr, B, nullptr);
-        if (rc == SACB_OK && cudaEventRecord(h->ev_sampled, h->stream2) != cudaSuccess) rc = SACB_ERR_DEVICE;
-        for (int li = p.split; li < nl && rc == SACB_OK; li++) rc = launch_stage(h, p, li, h->use_pdl != 0);
-        if (rc == SACB_OK && cudaStreamWaitEvent(h->stream, h->ev_sampled, 0) != cudaSuccess) rc = SACB_ERR_DEVICE;
-        const cudaError_t e2 = cudaStreamEndCapture(h->stream, &graph);
-        p.step_graph_launches = nl + (int)(h->kernel_launches - launches0);      // the stage kernels + what the replay helpers counted
-        h->kernel_launches = launches0; h->per_frame[0] = frame0;
-        if (rc != SACB_OK || e2 != cudaSuccess || !graph || cudaGraphInstantiate(&p.step_graph, graph, 0) != cudaSuccess) {
-            if (graph) cudaGraphDestroy(graph);
-            cudaGetLastError();
-            p.step_graph = nullptr; p.step_graph_failed = true;
-            return 1;
-        }
-        cudaGraphDestroy(graph);
-        p.step_graph_n = n; p.step_graph_k = k;
-    }
-    SACB_CUDA(cudaGraphLaunch(p.step_graph, h->stream));
-    h->kernel_launches += p.step_graph_launches;
-    h->per_frame[0] += 1; h->sample_k = k; h->prio_max_valid = true;
+    int rc;
+    if (staged && p.split < 0 && (rc = compute_split(p))) return rc;
+    if ((rc = staged ? enqueue_launches(h, p, 0, p.split) : launch_program(h, p))) return rc;
+    SACB_CUDA(cudaEventRecord(h->ev_td, h->stream));
+    SACB_CUDA(cudaStreamWaitEvent(h->stream2, h->ev_td, 0));
+    if ((rc = per_writeback_launch(h, h->stream2, k, false))) return rc;      // first kernel of the forked branch: a full dependency
+    if ((rc = per_sample_launch(h, h->stream2, nullptr, B, nullptr))) return rc;
+    SACB_CUDA(cudaEventRecord(h->ev_sampled, h->stream2));
+    if (staged && (rc = enqueue_launches(h, p, p.split, nl))) return rc;
+    SACB_CUDA(cudaStreamWaitEvent(h->stream, h->ev_sampled, 0));      // whatever follows on the main stream sees the new sample
     return SACB_OK;
 }
 
-int launch_program_part(sacb_handle h, ProgramInst &p, int part) {
-    if (h->cfg.launch_mode != SACB_LAUNCH_STAGED) {      // a single cooperative launch cannot be split: part 0 is the whole step
-        return part == 0 ? launch_program(h, p) : SACB_OK;
+// sacb_per_step as one graph launch (two graph launches + two events cost ~8 us per step: 206 against 198 us with no replay work at all)
+int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
+    if (h->cfg.launch_mode != SACB_LAUNCH_STAGED || p.step_graph_failed) return 1;
+    const int64_t n = h->r_len[0];
+    if (!p.step_graph || p.step_graph_n != n || p.step_graph_k != k) {
+        if (p.step_graph) cudaGraphExecDestroy(p.step_graph);
+        p.step_graph = capture(h, [&] { return enqueue_per_step(h, p, B, k); }, &p.step_graph_launches);
+        if (!p.step_graph) { p.step_graph_failed = true; return 1; }
+        p.step_graph_n = n; p.step_graph_k = k;
     }
-    const int nl = (int)p.launches.size();
-    if (!p.parts_built) {
-        p.parts_built = true;
-        if (p.split < 0) { if (int rc = compute_split(p)) return rc; }
-        for (int part_i = 0; part_i < 2; part_i++) {
-            const int s0 = part_i ? p.split : 0, s1 = part_i ? nl : p.split;
-            cudaGraph_t graph = nullptr;
-            if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) break;
-            int rc = SACB_OK;
-            for (int s = s0; s < s1 && rc == SACB_OK; s++) rc = launch_stage(h, p, s, h->use_pdl != 0);
-            const cudaError_t e2 = cudaStreamEndCapture(h->stream, &graph);
-            if (rc == SACB_OK && e2 == cudaSuccess && graph && cudaGraphInstantiate(&p.graph_part[part_i], graph, 0) != cudaSuccess) p.graph_part[part_i] = nullptr;
-            if (graph) cudaGraphDestroy(graph);
-        }
-        cudaGetLastError();
-    }
-    const int s0 = part ? p.split : 0, s1 = part ? nl : p.split;
-    h->kernel_launches += s1 - s0;
-    if (p.graph_part[part]) { SACB_CUDA(cudaGraphLaunch(p.graph_part[part], h->stream)); return SACB_OK; }
-    for (int s = s0; s < s1; s++) { int rc = launch_stage(h, p, s, h->use_pdl != 0); if (rc) return rc; }
+    SACB_CUDA(cudaGraphLaunch(p.step_graph, h->stream));
+    // what the replay helpers do on the host when they enqueue the step directly
+    h->kernel_launches += p.step_graph_launches;
+    h->per_frame[0] += 1; h->sample_k = k; h->prio_max_valid = true;
     return SACB_OK;
 }
 
@@ -1381,18 +1354,12 @@ using namespace sacb;
 extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap) {
     if (!h) return fail(SACB_ERR_ARG, "null handle");
     ProgramInst *p;
-    int rc;
-    if (!h->shadows_valid) {      // one step that (re)derives the shadows, then the steady-state program is profiled
-        ProgramKey k0 = update_key(h, (int)B, 0, 0, 1, 0);
-        if ((rc = get_program(h, k0, &p)) || (rc = launch_program(h, *p))) return rc;
-        after_update_launch(h, k0);
-    }
-    ProgramKey key = update_key(h, (int)B, 0, 0, 1, 0);
-    if (getenv("SACB_TIME_DP_PHASE")) {      // profile the backward half of a data-parallel phase instead (gradients exported, nothing applied)
-        key = ProgramKey{(int)B, 0, 1, 1, 0, atoi(getenv("SACB_TIME_DP_PHASE"))};
-    }
-    rc = get_program(h, key, &p);
+    int rc = steady_program(h, B, &p);
     if (rc) return rc;
+    if (getenv("SACB_TIME_DP_PHASE")) {      // profile the backward half of a data-parallel phase instead (gradients exported, nothing applied)
+        rc = get_program(h, ProgramKey{(int)B, 0, 1, 1, 0, atoi(getenv("SACB_TIME_DP_PHASE"))}, &p);
+        if (rc) return rc;
+    }
     const bool trace = getenv("SACB_TRACE") != nullptr;
     unsigned long long *d_trace = nullptr;
     std::vector<unsigned long long> h_trace;
@@ -1476,13 +1443,10 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
         std::vector<unsigned long long> init(4 * ns, 0ull), tl(4 * ns);
         for (int s = 0; s < ns; s++) { init[4 * s] = ~0ull; init[4 * s + 1] = ~0ull; }
         p->prog.timeline = d_tl;
-        cudaGraph_t g = nullptr; cudaGraphExec_t ge = nullptr;
-        SACB_CUDA(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
-        int rc3 = SACB_OK;
-        for (int li = 0; li < nl && rc3 == SACB_OK; li++) rc3 = launch_stage(h, *p, li, h->use_pdl != 0);
-        SACB_CUDA(cudaStreamEndCapture(h->stream, &g));
+        int counted;
+        cudaGraphExec_t ge = capture(h, [&] { return enqueue_launches(h, *p, 0, nl); }, &counted);
         p->prog.timeline = nullptr;
-        if (rc3 == SACB_OK && cudaGraphInstantiate(&ge, g, 0) == cudaSuccess) {
+        if (ge) {
             for (int r = 0; r < 4; r++) {
                 SACB_CUDA(cudaMemcpyAsync(d_tl, init.data(), sizeof(unsigned long long) * 4 * ns, cudaMemcpyHostToDevice, h->stream));
                 SACB_CUDA(cudaStreamSynchronize(h->stream));
@@ -1500,34 +1464,7 @@ extern "C" int sacb_time_stages(sacb_handle h, int64_t B, float *us_out, int cap
             fprintf(stderr, "[timeline] update = %.2f us\n", (tl[4 * p->launches[nl - 1].s0 + 2] - t0) * 1e-3);
             cudaGraphExecDestroy(ge);
         }
-        if (g) cudaGraphDestroy(g);
         cudaFree(d_tl);
-    }
-    if (trace && getenv("SACB_TRACE_RANGE")) {
-        // warm-code experiment: stages [a, b) in ONE cooperative launch; the surviving stamps belong to stage b-1 and are
-        // printed relative to its own start (slot 9, right after the grid barrier)
-        int a = 1, b = 4;
-        sscanf(getenv("SACB_TRACE_RANGE"), "%d,%d", &a, &b);
-        int tc_setup = 1, chained = 0; uint64_t seed = h->cfg.seed; Stage single = p->stages[a];
-        void *args[] = {(void *)&p->prog, (void *)&single, (void *)&a, (void *)&b, (void *)&tc_setup, (void *)&chained, (void *)&seed};
-        int grid = 1;
-        for (int s = a; s < b; s++) grid = std::max(grid, p->stages[s].n_tiles);
-        grid = std::min(grid, h->sm_count);
-        for (int r = 0; r < 3; r++) {
-            SACB_CUDA(cudaMemsetAsync(h->barrier, 0, sizeof(unsigned int), h->stream));
-            SACB_CUDA(cudaLaunchCooperativeKernel(update_kernel_for(h->cfg.math_mode, h->cfg.layer_norm ? kVariantEverythingLn : kVariantEverything), dim3(grid), dim3(kThreads), args, math_smem(h->cfg.math_mode), h->stream));
-        }
-        SACB_CUDA(cudaStreamSynchronize(h->stream));
-        SACB_CUDA(cudaMemcpy(h_trace.data(), d_trace, sizeof(unsigned long long) * kTraceSlots * grid, cudaMemcpyDeviceToHost));
-        for (int c = 0; c < std::min(grid, 3); c++) {
-            const unsigned long long *q = &h_trace[c * kTraceSlots];
-            fprintf(stderr, "[warm] stages [%d,%d) cta%d: kernel %.2f us | last stage from its start: issue", a, b, c, (q[5] - q[0]) * 1e-3);
-            for (int kb = 0; kb < 16 && q[16 + kb] >= q[9]; kb++) fprintf(stderr, " %.2f", (q[16 + kb] - q[9]) * 1e-3);
-            fprintf(stderr, " | arrive");
-            for (int kb = 0; kb < 16 && q[32 + kb] >= q[9]; kb++) fprintf(stderr, " %.2f", (q[32 + kb] - q[9]) * 1e-3);
-            fprintf(stderr, " | accum %.2f staged %.2f stored %.2f epi-end %.2f || presync %.2f taskcopy %.2f mainloop-entry %.2f | acc-lds %.2f aux-ldg %.2f\n", (q[6] - q[9]) * 1e-3, (q[7] - q[9]) * 1e-3, (q[8] - q[9]) * 1e-3, (q[3] - q[9]) * 1e-3,
-                    (q[10] - q[9]) * 1e-3, (q[11] - q[9]) * 1e-3, (q[12] - q[9]) * 1e-3, (q[13] - q[9]) * 1e-3, (q[14] - q[9]) * 1e-3);
-        }
     }
     if (trace) { p->prog.trace = nullptr; cudaFree(d_trace); }
     for (auto &e : ev) cudaEventDestroy(e);

@@ -32,17 +32,6 @@ namespace sacb {
         asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   \
     } while (0)
 
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool pdl, Args... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-
 constexpr int kChunk = 1024;          // elements per scan chunk (one warp, 32 per lane)
 constexpr int kSumLeafMax = 128;      // numpy PW_BLOCKSIZE
 constexpr int kSumBlockMax = 4096;    // elements of one CTA subtree in per_sum
@@ -963,6 +952,17 @@ static int top_depth_of(int64_t n) {
 }
 
 namespace sacb {
+static int64_t *per_frame_dev(sacb_handle h) { return reinterpret_cast<int64_t *>(per_ws_of(h, 0).counters + 8); }
+
+// create / sacb_per_set_frame: the device copy of the frame counter follows the host's
+int upload_per_frame(sacb_handle h, cudaStream_t st) {
+    if (!h->per_frame_dirty) return SACB_OK;
+    SACB_CUDA(cudaMemcpyAsync(per_frame_dev(h), &h->per_frame[0], sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    SACB_CUDA(cudaStreamSynchronize(st));
+    h->per_frame_dirty = false;
+    return SACB_OK;
+}
+
 int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B, int64_t *k_out) {
     if (!h || h->cfg.replay_kind != SACB_REPLAY_PER) return fail(SACB_ERR_ARG, "handle has no prioritized buffer");
     const int64_t n = h->r_len[0];
@@ -971,12 +971,8 @@ int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B
     if (k > h->cfg.max_batch) return fail(SACB_ERR_ARG, "batch size exceeds max_batch");
     PerWs w = per_ws_of(h, 0);
     const bool pdl = h->use_pdl != 0;
-    int64_t *frame_dev = reinterpret_cast<int64_t *>(w.counters + 8);
-    if (h->per_frame_dirty) {      // create / sacb_per_set_frame: the device copy follows the host's
-        SACB_CUDA(cudaMemcpyAsync(frame_dev, &h->per_frame[0], sizeof(int64_t), cudaMemcpyHostToDevice, st));
-        SACB_CUDA(cudaStreamSynchronize(st));
-        h->per_frame_dirty = false;
-    }
+    int64_t *frame_dev = per_frame_dev(h);
+    if (int rc = upload_per_frame(h, st)) return rc;
     h->per_frame[0] += 1;      // host mirror (statistics, `frame` property); the kernels read and advance the device copy
     if (u) {      // host-drawn uniforms (np.random.random_sample inside np.random.choice): through pinned memory, no pageable staging
         if (!h->pin_u) {

@@ -427,13 +427,8 @@ extern "C" int sacb_update_batch(sacb_handle h, int64_t B, const float *s, const
     if (isw) SACB_CUDA(cudaMemcpyAsync(ws + L.isw, isw, sizeof(float) * B, cudaMemcpyHostToDevice, h->stream));
     int rc = upload_eps(h, 0, B, eps_next, eps_cur);
     if (rc) return rc;
-    ProgramKey key = update_key(h, (int)B, 2, (flags & SACB_EXPORT_GRADS) ? 1 : 0, eps_next ? 0 : 1, isw ? 1 : 0);
-    ProgramInst *p;
-    rc = get_program(h, key, &p);
+    rc = run_update(h, update_key(h, (int)B, 2, (flags & SACB_EXPORT_GRADS) ? 1 : 0, eps_next ? 0 : 1, isw ? 1 : 0));
     if (rc) return rc;
-    rc = launch_program(h, *p);
-    if (rc) return rc;
-    after_update_launch(h, key);
     if (td_abs_out) {
         SACB_CUDA(cudaMemcpyAsync(td_abs_out, ws + L.td, sizeof(float) * B, cudaMemcpyDeviceToHost, h->stream));
         SACB_CUDA(cudaStreamSynchronize(h->stream));
@@ -475,13 +470,8 @@ extern "C" int sacb_update(sacb_handle h, int64_t B, const int64_t *idx, const f
         if (rc) return rc;
     }
     const int use_isw = (h->cfg.per_weighted_loss && h->cfg.replay_kind == SACB_REPLAY_PER) ? 1 : 0;
-    ProgramKey key = update_key(h, (int)B, gather_mode, (flags & SACB_EXPORT_GRADS) ? 1 : 0, eps_next ? 0 : 1, use_isw);
-    ProgramInst *p;
-    rc = get_program(h, key, &p);
+    rc = run_update(h, update_key(h, (int)B, gather_mode, (flags & SACB_EXPORT_GRADS) ? 1 : 0, eps_next ? 0 : 1, use_isw));
     if (rc) return rc;
-    rc = launch_program(h, *p);
-    if (rc) return rc;
-    after_update_launch(h, key);
     int64_t write_back_B = 0;
     if (flags & SACB_WRITE_BACK_TD) {
         if (h->cfg.replay_kind != SACB_REPLAY_PER || h->cfg.n_agents != 1 || !(flags & SACB_USE_LAST_SAMPLE))
@@ -507,7 +497,10 @@ static int per_step_enqueue(sacb_handle h, int64_t B) {
         SACB_CUDA(cudaEventCreateWithFlags(&h->ev_td, cudaEventDisableTiming));
         SACB_CUDA(cudaEventCreateWithFlags(&h->ev_sampled, cudaEventDisableTiming));
     }
-    int rc;
+    // a frame counter set since the last sample reaches the device ahead of the step, whichever form enqueues it (the main stream has
+    // joined the previous step's sample)
+    int rc = upload_per_frame(h, h->stream);
+    if (rc) return rc;
     const int64_t k = std::min<int64_t>(B, h->r_len[0]);
     if (h->sample_k != k) {      // first call (or the batch size changed): draw this step's minibatch now
         rc = per_sample_launch(h, h->stream, nullptr, B, nullptr);
@@ -517,19 +510,11 @@ static int per_step_enqueue(sacb_handle h, int64_t B) {
     ProgramInst *p;
     rc = get_program(h, key, &p);
     if (rc) return rc;
-    // the whole step -- update stages, forked write-back + next sample, join -- as ONE graph launch
+    // the whole step -- update stages, forked write-back + next sample, join -- as ONE graph launch, else the same launches directly
     rc = launch_per_step_graph(h, *p, B, k);
-    if (rc == SACB_OK) { after_update_launch(h, key); return SACB_OK; }
-    if (rc != 1) return rc;
-    if ((rc = launch_program_part(h, *p, 0))) return rc;
+    if (rc == 1) rc = enqueue_per_step(h, *p, B, k);
+    if (rc) return rc;
     after_update_launch(h, key);
-    SACB_CUDA(cudaEventRecord(h->ev_td, h->stream));
-    SACB_CUDA(cudaStreamWaitEvent(h->stream2, h->ev_td, 0));
-    if ((rc = per_writeback_launch(h, h->stream2, k))) return rc;
-    if ((rc = per_sample_launch(h, h->stream2, nullptr, B, nullptr))) return rc;
-    SACB_CUDA(cudaEventRecord(h->ev_sampled, h->stream2));
-    if ((rc = launch_program_part(h, *p, 1))) return rc;
-    SACB_CUDA(cudaStreamWaitEvent(h->stream, h->ev_sampled, 0));      // whatever follows on the main stream sees the new sample
     return SACB_OK;
 }
 
@@ -616,14 +601,7 @@ extern "C" int sacb_get_stats(sacb_handle h, sacb_stats *out) {
 extern "C" int sacb_time_update(sacb_handle h, int64_t B, int iters, float *ms_per_step) {
     if (!h || !ms_per_step || iters < 1) return fail(SACB_ERR_ARG, "bad argument");
     ProgramInst *p;
-    int rc;
-    if (!h->shadows_valid) {      // one step that (re)derives the shadows, then the steady-state program is timed
-        ProgramKey k0 = update_key(h, (int)B, 0, 0, 1, 0);
-        if ((rc = get_program(h, k0, &p)) || (rc = launch_program(h, *p))) return rc;
-        after_update_launch(h, k0);
-    }
-    ProgramKey key = update_key(h, (int)B, 0, 0, 1, 0);
-    rc = get_program(h, key, &p);
+    int rc = steady_program(h, B, &p);
     if (rc) return rc;
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
