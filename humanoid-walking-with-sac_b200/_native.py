@@ -90,6 +90,7 @@ SIGNATURES = {
     "sacb_clear_replay": (I, [H, I]),
     "sacb_sample_uniform": (I, [H, I, c_i64p, I64, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p]),
     "sacb_per_sample": (I, [H, I, c_f64p, I64, c_i64p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p]),
+    "sacb_per_sample_all": (I, [H, c_f64p, I64, c_i64p, c_f32p]),
     "sacb_per_update": (I, [H, I, c_i64p, c_f32p, I64]),
     "sacb_per_update_final": (I, [H, I, c_i64p, c_f32p, I64]),
     "sacb_per_update_from_td": (I, [H, I, I64]),

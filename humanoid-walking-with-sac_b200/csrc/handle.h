@@ -155,7 +155,7 @@ struct sacb_handle_s {
     cudaStream_t stream = nullptr;
     cudaStream_t stream2 = nullptr;      // prioritized replay work that overlaps the update (sacb_per_step)
     cudaEvent_t ev_td = nullptr, ev_sampled = nullptr;
-    int64_t sample_k = 0;                // rows of the minibatch the last prioritized sample left on the device (0: none)
+    std::vector<int64_t> sample_k;       // per agent: rows of the minibatch the last prioritized sample left on the device (0: none)
     sacb::Layout L;
     float *arena = nullptr, *ws = nullptr;
     unsigned int *barrier = nullptr;
@@ -188,12 +188,12 @@ struct sacb_handle_s {
     // PER
     float *prio = nullptr, *p_alpha = nullptr;   // [n_agents, capacity]
     std::vector<int64_t> per_frame;
-    bool per_frame_dirty = true;         // the device copy of per_frame[0] (read and advanced by the sample kernels) has to be uploaded
-    void *per_ws = nullptr;                      // scan workspace (see replay.cu)
+    std::vector<char> per_frame_dirty;   // per agent: the device copy of per_frame[a] (read and advanced by the sample kernels) has to be uploaded
+    void *per_ws = nullptr;                      // [n_agents] sampler workspaces (see replay.cu: per_ws_of)
     int64_t *last_idx_dev = nullptr;             // [n_agents, maxB] logical indices of the last sample
     float *last_w_dev = nullptr;
     sacb_per_stats per_stats{};
-    bool prio_max_valid = false;                 // per-CTA maxima of the priority table are current (replay.cu: per_refresh_max)
+    std::vector<char> prio_max_valid;            // per agent: the CTA maxima of its priority table are current (replay.cu: per_refresh_max)
     // pinned host staging
     float *pin = nullptr;
     int64_t pin_floats = 0;
@@ -206,7 +206,7 @@ struct sacb_handle_s {
     bool push_in_flight = false;
     cudaEvent_t ev_slots = nullptr;      // the H2D copy of the minibatch slots out of `pin` has completed
     bool slots_in_flight = false;
-    double *pin_u = nullptr;             // pinned block for the host-drawn PER uniforms
+    double *pin_u = nullptr;             // pinned block for the host-drawn PER uniforms [n_agents, maxB]
     cudaEvent_t ev_u = nullptr;
     bool u_in_flight = false;
     float *act_ws = nullptr, *pin_act = nullptr;   // select_action scratch (device) and pinned obs / eps / action block
@@ -217,6 +217,8 @@ struct sacb_handle_s {
 
 namespace sacb {
 constexpr int kPinPushRows = 64;
+// largest capacity per agent of a prioritized population: the tail-free sampler form (chunk prefixes in shared memory)
+constexpr int64_t kPopulationPerCapacity = 2096128;
 inline bool math_is_tc(int m) { return m != SACB_MATH_FP32; }
 inline size_t math_smem(int m) { return math_is_tc(m) ? (size_t)kTcSmemBytes : (size_t)kSimtSmemBytes; }
 // TMA descriptor of a pair-matrix view (program.cu): dims {cols, rows, 2 planes, n_agents}, box {64, box_rows, 2, 1},
@@ -245,8 +247,9 @@ int steady_program(sacb_handle h, int64_t B, ProgramInst **out);
 // replay.cu
 int replay_create(sacb_handle h);
 void replay_destroy(sacb_handle h);
-int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B, int64_t *k_out);   // kernels of one sample() call
-int upload_per_frame(sacb_handle h, cudaStream_t st);                                                   // frame counter -> device, if sacb_per_set_frame changed it
+// kernels of one sample() call for agents [first, first + count) (u: [count][B] host uniforms or null); one chain for all of them
+int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B, int64_t *k_out, int first, int count);
+int upload_per_frame(sacb_handle h, cudaStream_t st);                                                   // frame counters -> device, where sacb_per_set_frame changed them
 int upload_ring_meta(sacb_handle h);                                                                   // (len, head) of every agent's ring -> device, if a push changed them
-int per_writeback_launch(sacb_handle h, cudaStream_t st, int64_t B, bool pdl_ok = true);                                 // priorities <- |td| of the last update
+int per_writeback_launch(sacb_handle h, cudaStream_t st, int64_t B, bool pdl_ok, int first, int count);   // priorities <- |td| of the last update
 }  // namespace sacb

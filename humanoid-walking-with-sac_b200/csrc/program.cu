@@ -1319,8 +1319,8 @@ int enqueue_per_step(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
     if ((rc = staged ? enqueue_launches(h, p, 0, p.split) : launch_program(h, p))) return rc;
     SACB_CUDA(cudaEventRecord(h->ev_td, h->stream));
     SACB_CUDA(cudaStreamWaitEvent(h->stream2, h->ev_td, 0));
-    if ((rc = per_writeback_launch(h, h->stream2, k, false))) return rc;      // first kernel of the forked branch: a full dependency
-    if ((rc = per_sample_launch(h, h->stream2, nullptr, B, nullptr))) return rc;
+    if ((rc = per_writeback_launch(h, h->stream2, k, false, 0, 1))) return rc;      // first kernel of the forked branch: a full dependency
+    if ((rc = per_sample_launch(h, h->stream2, nullptr, B, nullptr, 0, 1))) return rc;
     SACB_CUDA(cudaEventRecord(h->ev_sampled, h->stream2));
     if (staged && (rc = enqueue_launches(h, p, p.split, nl))) return rc;
     SACB_CUDA(cudaStreamWaitEvent(h->stream, h->ev_sampled, 0));      // whatever follows on the main stream sees the new sample
@@ -1340,7 +1340,7 @@ int launch_per_step_graph(sacb_handle h, ProgramInst &p, int64_t B, int64_t k) {
     SACB_CUDA(cudaGraphLaunch(p.step_graph, h->stream));
     // what the replay helpers do on the host when they enqueue the step directly
     h->kernel_launches += p.step_graph_launches;
-    h->per_frame[0] += 1; h->sample_k = k; h->prio_max_valid = true;
+    h->per_frame[0] += 1; h->sample_k[0] = k; h->prio_max_valid[0] = 1;
     return SACB_OK;
 }
 

@@ -15,6 +15,8 @@
 //                     samples the test could not certify, IS weights (N p)^-beta / max, logical indices, ring slots for the update's gather
 // Above that the last CTA to arrive finishes the sum and the scan: per_sum(tail) -> per_chunk -> per_search, with the chunk prefixes
 // in global memory.  Both forms are bit-identical.
+// Populations (n_agents > 1, capacity <= 2 096 128 per agent): the tail-free chain takes an agent grid dimension (blockIdx.y), so ONE
+// chain of three launches samples every agent's table (PerAgents below).
 #include <cmath>
 #include <cstring>
 #include <algorithm>
@@ -157,6 +159,40 @@ __device__ __forceinline__ bool last_block_done(int *ticket, int n_blocks = -1, 
     return s_last != 0;
 }
 
+// Agent dimension of one sampler chain: blockIdx.y = agent - first.  Every per-agent table and workspace sits at a fixed stride from
+// agent 0's, and the kernels receive agent 0's pointers.  meta = the (len, head) table of the rings (upload_ring_meta): each agent reads
+// its own length there, the grid being sized for the longest agent.  A chain over ONE agent passes meta = null and that agent's length
+// as `n`: a single-agent handle launches exactly the grids and argument values it launched before the agent dimension existed, and
+// the kernels' kAgents = false instantiation (single-agent handles) compiles the agent offsets out.
+struct PerAgents {
+    const int64_t *meta;
+    int first;
+    int64_t pa_stride;      // floats between two agents' prio / p_alpha tables (capacity)
+    int64_t ws_stride;      // bytes between two agents' sampler workspaces (PerWs)
+    int64_t u_stride;       // bytes between two agents' uniforms (host-drawn: a pinned row of max_batch; device-drawn: ws_stride)
+    int64_t batch_stride;   // entries between two agents' ring slots / last-sample indices (max_batch)
+    int64_t isw_stride;     // floats between two agents' update workspaces (Layout::ws_size)
+};
+__device__ __forceinline__ int per_agent(const PerAgents &g) { return g.first + (int)blockIdx.y; }
+template <typename T> __device__ __forceinline__ T *ws_at(T *p, const PerAgents &g, int a) { return (T *)((const char *)p + (int64_t)a * g.ws_stride); }
+__device__ __forceinline__ int64_t agent_len(const PerAgents &g, int a, int64_t n) { return g.meta ? __ldcg(g.meta + 2 * a) : n; }
+
+// depth of the top of numpy's summation tree above the CTA subtrees of <= kSumBlockMax elements
+__host__ __device__ inline int top_depth_of(int64_t n) {
+    int d = 0;
+    while (n > kSumBlockMax) { int64_t n2 = n / 2; n2 -= n2 % 8; n = n - n2; d++; }   // the right child is the larger one
+    return d;
+}
+
+// Key of agent a's device-drawn uniforms: seed ^ splitmix64(a) for a > 0 (splitmix64(x): x += 0x9E3779B97F4A7C15, then the
+// finaliser of uniform_of below), the handle's seed itself for agent 0 -- agent 0 of a population draws what a one-agent handle draws.
+__host__ __device__ inline uint64_t per_agent_seed(uint64_t seed, int a) {
+    if (a == 0) return seed;
+    uint64_t x = (uint64_t)a + 0x9E3779B97F4A7C15ull;
+    x ^= x >> 30; x *= 0xBF58476D1CE4E5B9ull; x ^= x >> 27; x *= 0x94D049BB133111EBull; x ^= x >> 31;
+    return seed ^ x;
+}
+
 __device__ __forceinline__ double uniform_of(uint64_t seed, uint64_t counter, int j) {      // splitmix64 -> [0, 1) with 53 bits
     uint64_t x = seed ^ (counter * 0x9E3779B97F4A7C15ull + (uint64_t)j * 0xBF58476D1CE4E5B9ull);
     x ^= x >> 30; x *= 0xBF58476D1CE4E5B9ull; x ^= x >> 27; x *= 0x94D049BB133111EBull; x ^= x >> 31;
@@ -188,12 +224,20 @@ __device__ float top_tree_sum(int64_t n, int top_depth, const float *top_vals) {
 // top of the tree (numpy's association) and publishes the float32 total.  draw_B > 0: the B uniforms of this call are drawn here.
 // tail = 0: no finishing step here -- the CTAs of the next kernel (per_chunk_notail) each add the top of the tree themselves (<= 512 values, the
 // same function, the same association), which takes the completion ticket (two dependent atomics) and the one-CTA tail off the chain.
+template <bool kAgents>
 __global__ void __launch_bounds__(256) per_sum(const float *p_alpha, int64_t n, int top_depth, float *top_vals, float *total, int *ticket,
-                                               double *u, int draw_B, uint64_t seed, const int64_t *frame, int tail) {
+                                               double *u, int draw_B, uint64_t seed, const int64_t *frame, int tail, PerAgents g) {
     SACB_PDL_ENTER();
     __shared__ float s_heap[kSumHeap];
     __shared__ unsigned char s_state[kSumHeap];
     __shared__ int s_leaf[3 * 128];          // a CTA subtree of <= kSumBlockMax elements has at most 128 leaves
+    if (kAgents) {      // CTAs beyond this agent's tree find no leaf below (pw_node)
+        const int ag = per_agent(g);
+        p_alpha += ag * g.pa_stride;
+        top_vals = ws_at(top_vals, g, ag); total = ws_at(total, g, ag); ticket = ws_at(ticket, g, ag); u = ws_at(u, g, ag); frame = ws_at(frame, g, ag);
+        if (g.meta) { n = agent_len(g, ag, n); top_depth = top_depth_of(n); }
+        seed = per_agent_seed(seed, ag);
+    }
     const uint64_t counter = (uint64_t)__ldcg(frame);
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < draw_B; j += gridDim.x * blockDim.x) u[j] = uniform_of(seed, counter, j);
     const unsigned id = blockIdx.x + 1;
@@ -331,9 +375,17 @@ __global__ void __launch_bounds__(256) per_chunk(const float *p_alpha, int64_t n
 
 // the same pass behind per_sum(tail = 0): every CTA first adds the top of the summation tree itself (CTA 0 publishes the total); no
 // completion ticket, no scan tail -- the search CTAs scan the chunk sums themselves (per_search_scan)
+template <bool kAgents>
 __global__ void __launch_bounds__(256) per_chunk_notail(const float *p_alpha, int64_t n, int top_depth, const float *top_vals, float *total,
-                                                        double *chunk_sum, int *chunk_fine) {
+                                                        double *chunk_sum, int *chunk_fine, PerAgents g) {
     SACB_PDL_ENTER();
+    if (kAgents) {
+        const int ag = per_agent(g);
+        if (g.meta) { n = agent_len(g, ag, n); top_depth = top_depth_of(n); }
+        if (blockIdx.x > 0 && (int64_t)blockIdx.x * 8 * kChunk >= n) return;      // beyond this agent's chunks (grid sized for the longest agent)
+        p_alpha += ag * g.pa_stride;
+        top_vals = ws_at(top_vals, g, ag); total = ws_at(total, g, ag); chunk_sum = ws_at(chunk_sum, g, ag); chunk_fine = ws_at(chunk_fine, g, ag);
+    }
     const float tot = top_tree_sum(n, top_depth, top_vals);
     if (blockIdx.x == 0 && threadIdx.x == 0) *total = tot;
     chunk_group(p_alpha, n, tot, (int)blockIdx.x, chunk_sum, chunk_fine);
@@ -554,8 +606,21 @@ __global__ void __launch_bounds__(256) per_search(const float *total, const doub
 
 // per_search behind per_chunk_notail (capacity <= 2 M: the chunk prefixes fit into shared memory): every search group scans the chunk sums
 // itself (1 K additions by carry_scan, the function the tail of per_chunk runs: same values) instead of reading prefixes a tail CTA wrote
-__global__ void __launch_bounds__(256) per_search_scan(const float *total, double *carry, SearchArgs a) {
+template <bool kAgents>
+__global__ void __launch_bounds__(256) per_search_scan(const float *total, double *carry, SearchArgs a, PerAgents g) {
     SACB_PDL_ENTER();
+    if (kAgents) {      // this CTA's agent (every agent draws the same B samples: no CTA is idle)
+        const int ag = per_agent(g);
+        if (g.meta) { a.n = agent_len(g, ag, a.n); a.n_chunks = (int)((a.n + kChunk - 1) / kChunk); }
+        a.p_alpha += ag * g.pa_stride;
+        a.u = reinterpret_cast<const double *>(reinterpret_cast<const char *>(a.u) + ag * g.u_stride);
+        total = ws_at(total, g, ag); carry = ws_at(carry, g, ag);
+        a.counters = ws_at(a.counters, g, ag); a.idx_out = ws_at(a.idx_out, g, ag); a.flagged = ws_at(a.flagged, g, ag);
+        a.ticket = ws_at(a.ticket, g, ag); a.carry_exact = ws_at(a.carry_exact, g, ag); a.chunk_sum = ws_at(a.chunk_sum, g, ag);
+        a.chunk_fine = ws_at(a.chunk_fine, g, ag); a.weights = ws_at(a.weights, g, ag); a.frame = ws_at(a.frame, g, ag);
+        a.slots += ag * g.batch_stride; a.idx_copy += ag * g.batch_stride;
+        if (a.isw_ws) a.isw_ws += ag * g.isw_stride;
+    }
     const float tot = *total;
     const int j = (int)blockIdx.x * 8 + (int)(threadIdx.x >> 5);
     const double uu_pre = j < a.B ? a.u[j] : -1.0;      // in flight during the scan
@@ -574,8 +639,11 @@ __global__ void __launch_bounds__(256) per_search_scan(const float *total, doubl
 // ---------------------------------------------------------------------------------------------------------------
 // priorities: update (last duplicate wins), push (max over the whole capacity array)
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(1024) per_update_kernel(float *prio, float *p_alpha, const int64_t *idx, const float *td, int B, float alpha, int is_final) {
+// one CTA per agent (blockIdx.x), tables / indices / |td| at the given strides from the first agent's
+__global__ void __launch_bounds__(1024) per_update_kernel(float *prio, float *p_alpha, const int64_t *idx, const float *td, int B, float alpha, int is_final,
+                                                          int64_t tab_stride, int64_t idx_stride, int64_t td_stride) {
     SACB_PDL_ENTER();
+    prio += blockIdx.x * tab_stride; p_alpha += blockIdx.x * tab_stride; idx += blockIdx.x * idx_stride; td += blockIdx.x * td_stride;
     extern __shared__ int64_t s_idx[];
     for (int j = threadIdx.x; j < B; j += blockDim.x) s_idx[j] = idx[j];
     __syncthreads();
@@ -592,8 +660,10 @@ __global__ void __launch_bounds__(1024) per_update_kernel(float *prio, float *p_
     }
 }
 
-__global__ void __launch_bounds__(1024) max_reduce_kernel(const float *x, int64_t n, float *block_out) {
+// blockIdx.y = agent: its table at x + y * x_stride, its CTA maxima at block_out + y * out_stride
+__global__ void __launch_bounds__(1024) max_reduce_kernel(const float *x, int64_t n, float *block_out, int64_t x_stride, int64_t out_stride) {
     __shared__ float s[32];
+    x += blockIdx.y * x_stride; block_out += blockIdx.y * out_stride;
     float m = -INFINITY;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) m = fmaxf(m, x[i]);
     for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
@@ -639,13 +709,15 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const float *ring, int
     for (int k = lane; k < ring_row / 4; k += 32) dst[k] = __ldcs(src + k);
 }
 
+static int64_t per_ws_bytes(sacb_handle h);
+// bytes between two agents' sampler workspaces
+static int64_t per_ws_stride(sacb_handle h) { return align_up(per_ws_bytes(h), 256); }
 static PerWs per_ws_of(sacb_handle h, int agent) {
     PerWs w;
-    char *base = (char *)h->per_ws;
+    char *base = (char *)h->per_ws + (int64_t)agent * per_ws_stride(h);
     const int64_t cap = h->cfg.capacity, nch = cap / kChunk + 2, B = h->cfg.max_batch;
     auto take = [&](size_t bytes) { char *p = base; base += align_up((int64_t)bytes, 256); return p; };
-    // same carve-up for every agent; agent stride computed by per_ws_bytes
-    (void)agent;
+    // the same carve-up for every agent, per_ws_stride apart
     w.block_vals = (float *)take(sizeof(float) * 4096);
     w.total = (float *)take(256);
     w.chunk_sum = (double *)take(sizeof(double) * nch);
@@ -671,19 +743,22 @@ int replay_create(sacb_handle h) {
     h->ring_row = align_up(2 * c.obs_dim + c.act_dim + 2, 4);
     const int n = c.n_agents;
     h->r_len.assign(n, 0); h->r_pos.assign(n, 0); h->r_head.assign(n, 0); h->per_frame.assign(n, 1);   // frame starts at 1 (replay_buffer.py:31)
+    h->per_frame_dirty.assign(n, 1); h->sample_k.assign(n, 0); h->prio_max_valid.assign(n, 0);
     const size_t ring_bytes = sizeof(float) * (size_t)h->ring_row * c.capacity * n;
     if (cudaMalloc(&h->ring, ring_bytes) != cudaSuccess) { cudaGetLastError(); return fail(SACB_ERR_NOMEM, "replay ring does not fit in device memory"); }
     h->stage_rows_cap = std::max<int64_t>(c.max_batch, 4096);
     if (cudaMalloc(&h->stage_rows, sizeof(float) * h->ring_row * h->stage_rows_cap) != cudaSuccess) return fail(SACB_ERR_NOMEM, "staging alloc failed");
     if (c.replay_kind == SACB_REPLAY_PER) {
-        if (n != 1) return fail(SACB_ERR_ARG, "prioritized replay is per-agent: use n_agents = 1 per handle");
+        if (n != 1 && c.capacity > kPopulationPerCapacity) return fail(SACB_ERR_ARG, "prioritized population: capacity <= 2096128 per agent");
         if (c.max_batch > 1024) return fail(SACB_ERR_ARG, "prioritized replay supports max_batch <= 1024");
-        if (cudaMalloc(&h->prio, sizeof(float) * c.capacity) != cudaSuccess || cudaMalloc(&h->p_alpha, sizeof(float) * c.capacity) != cudaSuccess ||
-            cudaMalloc(&h->per_ws, per_ws_bytes(h)) != cudaSuccess || cudaMalloc(&h->last_idx_dev, sizeof(int64_t) * c.max_batch) != cudaSuccess)
+        // per agent: prio / p_alpha [n, capacity], sampler workspace [n, per_ws_stride], last-sample indices [n, max_batch]
+        const size_t tab = sizeof(float) * c.capacity * n, ws = (size_t)per_ws_stride(h) * n;
+        if (cudaMalloc(&h->prio, tab) != cudaSuccess || cudaMalloc(&h->p_alpha, tab) != cudaSuccess ||
+            cudaMalloc(&h->per_ws, ws) != cudaSuccess || cudaMalloc(&h->last_idx_dev, sizeof(int64_t) * c.max_batch * n) != cudaSuccess)
             return fail(SACB_ERR_NOMEM, "PER tables do not fit in device memory");
-        cudaMemsetAsync(h->prio, 0, sizeof(float) * c.capacity, h->stream);
-        cudaMemsetAsync(h->p_alpha, 0, sizeof(float) * c.capacity, h->stream);
-        cudaMemsetAsync(h->per_ws, 0, per_ws_bytes(h), h->stream);
+        cudaMemsetAsync(h->prio, 0, tab, h->stream);
+        cudaMemsetAsync(h->p_alpha, 0, tab, h->stream);
+        cudaMemsetAsync(h->per_ws, 0, ws, h->stream);
     }
     return SACB_OK;
 }
@@ -770,33 +845,40 @@ extern "C" int sacb_clear_replay(sacb_handle h, int agent) {
     if (!h || agent < 0 || agent >= h->cfg.n_agents) return fail(SACB_ERR_ARG, "bad argument");
     h->r_len[agent] = h->r_pos[agent] = h->r_head[agent] = 0;
     h->ring_meta_dirty = true;
-    h->sample_k = 0;
-    h->prio_max_valid = false;
-    if (h->prio) { cudaMemsetAsync(h->prio, 0, sizeof(float) * h->cfg.capacity, h->stream); cudaMemsetAsync(h->p_alpha, 0, sizeof(float) * h->cfg.capacity, h->stream); }
+    h->sample_k[agent] = 0;
+    h->prio_max_valid[agent] = 0;
+    if (h->prio) {      // this agent's tables only
+        const int64_t cap = h->cfg.capacity;
+        cudaMemsetAsync(h->prio + agent * cap, 0, sizeof(float) * cap, h->stream); cudaMemsetAsync(h->p_alpha + agent * cap, 0, sizeof(float) * cap, h->stream);
+    }
     return SACB_OK;
 }
 
 // max(priorities) over the whole capacity array (replay_buffer.py:38) as 128 CTA maxima.  The table only changes through
 // update_priorities / set_priorities / clear (a push writes the maximum itself, which leaves it unchanged), so the reduction runs
 // right behind those -- off the push -> sample -> update critical path -- and push reuses it while `prio_max_valid`.
-static void per_refresh_max(sacb_handle h, cudaStream_t st) {
-    PerWs w = per_ws_of(h, 0);
-    max_reduce_kernel<<<128, 1024, 0, st>>>(h->prio, h->cfg.capacity, w.block_max);
+// agents [first, first + count), one launch (blockIdx.y = agent)
+static void per_refresh_max(sacb_handle h, cudaStream_t st, int first, int count) {
+    PerWs w = per_ws_of(h, first);
+    const int64_t cap = h->cfg.capacity;
+    max_reduce_kernel<<<dim3(128, count), 1024, 0, st>>>(h->prio + first * cap, cap, w.block_max, cap, per_ws_stride(h) / (int64_t)sizeof(float));
     h->kernel_launches++;
-    h->prio_max_valid = true;
+    for (int a = first; a < first + count; a++) h->prio_max_valid[a] = 1;
 }
 
-static int per_push_priorities(sacb_handle h, int64_t pos, int64_t count, bool empty, const float *pinned_rows = nullptr) {
-    PerWs w = per_ws_of(h, 0);
+// ring = the agent's ring (the push kernel moves pinned rows there itself)
+static int per_push_priorities(sacb_handle h, int agent, int64_t pos, int64_t count, bool empty, float *ring, const float *pinned_rows = nullptr) {
+    PerWs w = per_ws_of(h, agent);
     const int nb = 128;
-    if (!empty && !h->prio_max_valid) per_refresh_max(h, h->stream);
+    const int64_t cap = h->cfg.capacity;
+    if (!empty && !h->prio_max_valid[agent]) per_refresh_max(h, h->stream, agent, 1);
     const int row_vec4 = (int)(h->ring_row / 4);
     const int64_t work = pinned_rows ? std::max<int64_t>(count, count * row_vec4) : count;
-    per_push_kernel<<<(int)std::min<int64_t>(64, (work + 255) / 256), 256, 0, h->stream>>>(h->prio, h->p_alpha, w.block_max, nb, empty ? 1 : 0, pos, count,
-                                                                                         h->cfg.capacity, h->cfg.per_alpha, reinterpret_cast<const float4 *>(pinned_rows),
-                                                                                         reinterpret_cast<float4 *>(h->ring), row_vec4);
+    per_push_kernel<<<(int)std::min<int64_t>(64, (work + 255) / 256), 256, 0, h->stream>>>(h->prio + agent * cap, h->p_alpha + agent * cap, w.block_max, nb, empty ? 1 : 0,
+                                                                                         pos, count, cap, h->cfg.per_alpha, reinterpret_cast<const float4 *>(pinned_rows),
+                                                                                         reinterpret_cast<float4 *>(ring), row_vec4);
     h->kernel_launches++;
-    if (empty) h->prio_max_valid = false;      // the first push writes 1.0 into an all-zero table: reduce again next time
+    if (empty) h->prio_max_valid[agent] = 0;      // the first push writes 1.0 into an all-zero table: reduce again next time
     SACB_CUDA(cudaGetLastError());
     return SACB_OK;
 }
@@ -823,7 +905,7 @@ extern "C" int sacb_push(sacb_handle h, int agent, const float *s, const float *
         SACB_CUDA(cudaMemcpy2DAsync(dst + 2 * c.obs_dim + c.act_dim, pitch, r + done_n, sizeof(float), sizeof(float), run, cudaMemcpyHostToDevice, h->stream));
         SACB_CUDA(cudaMemcpy2DAsync(dst + 2 * c.obs_dim + c.act_dim + 1, pitch, done + done_n, sizeof(float), sizeof(float), run, cudaMemcpyHostToDevice, h->stream));
         if (per) {
-            int rc = per_push_priorities(h, slot, run, h->r_len[agent] == 0);
+            int rc = per_push_priorities(h, agent, slot, run, h->r_len[agent] == 0, ring);
             if (rc) return rc;
             h->r_pos[agent] = (slot + run) % cap;
             h->r_len[agent] = std::min(cap, h->r_len[agent] + run);
@@ -882,10 +964,10 @@ extern "C" int sacb_push_rows(sacb_handle h, int agent, const float *rows, int64
         if (per) slot = h->r_pos[agent];
         else slot = h->r_len[agent] < cap ? (h->r_head[agent] + h->r_len[agent]) % cap : h->r_head[agent];
         const int64_t run = std::min(n - done_n, cap - slot);
-        const bool by_kernel = per && staged && agent == 0;      // the push kernel moves the rows out of the pinned block itself
+        const bool by_kernel = per && staged;      // the push kernel moves the rows out of the pinned block itself
         if (!by_kernel) SACB_CUDA(cudaMemcpyAsync(ring + slot * row, rows + done_n * row, sizeof(float) * row * run, cudaMemcpyHostToDevice, h->stream));
         if (per) {
-            int rc = per_push_priorities(h, slot, run, h->r_len[agent] == 0, by_kernel ? rows + done_n * row : nullptr);
+            int rc = per_push_priorities(h, agent, slot, run, h->r_len[agent] == 0, ring, by_kernel ? rows + done_n * row : nullptr);
             if (rc) return rc;
             h->r_pos[agent] = (slot + run) % cap;
             h->r_len[agent] = std::min(cap, h->r_len[agent] + run);
@@ -945,42 +1027,53 @@ extern "C" int sacb_sample_uniform(sacb_handle h, int agent, const int64_t *idx,
 }
 
 // ---- PER --------------------------------------------------------------------------------------------------------
-static int top_depth_of(int64_t n) {
-    int d = 0;
-    while (n > kSumBlockMax) { int64_t n2 = n / 2; n2 -= n2 % 8; n = n - n2; d++; }   // the right child is the larger one
-    return d;
-}
-
 namespace sacb {
-static int64_t *per_frame_dev(sacb_handle h) { return reinterpret_cast<int64_t *>(per_ws_of(h, 0).counters + 8); }
+static int64_t *per_frame_dev(sacb_handle h, int agent) { return reinterpret_cast<int64_t *>(per_ws_of(h, agent).counters + 8); }
 
-// create / sacb_per_set_frame: the device copy of the frame counter follows the host's
+// create / sacb_per_set_frame: the device copy of every agent's frame counter follows the host's
 int upload_per_frame(sacb_handle h, cudaStream_t st) {
-    if (!h->per_frame_dirty) return SACB_OK;
-    SACB_CUDA(cudaMemcpyAsync(per_frame_dev(h), &h->per_frame[0], sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    bool any = false;
+    for (int a = 0; a < h->cfg.n_agents; a++) {
+        if (!h->per_frame_dirty[a]) continue;
+        SACB_CUDA(cudaMemcpyAsync(per_frame_dev(h, a), &h->per_frame[a], sizeof(int64_t), cudaMemcpyHostToDevice, st));
+        any = true;
+    }
+    if (!any) return SACB_OK;
     SACB_CUDA(cudaStreamSynchronize(st));
-    h->per_frame_dirty = false;
+    for (int a = 0; a < h->cfg.n_agents; a++) h->per_frame_dirty[a] = 0;
     return SACB_OK;
 }
 
-int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B, int64_t *k_out) {
+int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B, int64_t *k_out, int first, int count) {
     if (!h || h->cfg.replay_kind != SACB_REPLAY_PER) return fail(SACB_ERR_ARG, "handle has no prioritized buffer");
-    const int64_t n = h->r_len[0];
-    if (n < 1) return fail(SACB_ERR_STATE, "cannot sample from an empty buffer");
-    const int64_t k = std::min<int64_t>(B, n);                       // n_samples = min(batch_size, len)  (replay_buffer.py:50)
+    if (first < 0 || count < 1 || first + count > h->cfg.n_agents) return fail(SACB_ERR_ARG, "agent index out of range");
+    int64_t n = h->r_len[first], k;
+    if (count == 1) {
+        if (n < 1) return fail(SACB_ERR_STATE, "cannot sample from an empty buffer");
+        k = std::min<int64_t>(B, n);                                 // n_samples = min(batch_size, len)  (replay_buffer.py:50)
+    } else {      // every agent's minibatch has B rows (the batched update program): len >= B everywhere; grids sized for the longest agent
+        for (int a = first; a < first + count; a++) {
+            if (h->r_len[a] < B) return fail(SACB_ERR_STATE, "population sample: every agent's buffer must hold at least B transitions");
+            n = std::max(n, h->r_len[a]);
+        }
+        k = B;
+    }
     if (k > h->cfg.max_batch) return fail(SACB_ERR_ARG, "batch size exceeds max_batch");
-    PerWs w = per_ws_of(h, 0);
+    PerWs w = per_ws_of(h, 0);      // agent 0's pointers: the kernels add each agent's stride
     const bool pdl = h->use_pdl != 0;
-    int64_t *frame_dev = per_frame_dev(h);
+    int64_t *frame_dev = per_frame_dev(h, 0);
     if (int rc = upload_per_frame(h, st)) return rc;
-    h->per_frame[0] += 1;      // host mirror (statistics, `frame` property); the kernels read and advance the device copy
+    if (count > 1) { if (int rc = upload_ring_meta(h)) return rc; }      // each agent's length, read by the kernels
+    for (int a = first; a < first + count; a++) h->per_frame[a] += 1;    // host mirror (statistics, `frame`); the kernels read and advance the device copy
+    const int64_t mb = h->cfg.max_batch;
     if (u) {      // host-drawn uniforms (np.random.random_sample inside np.random.choice): through pinned memory, no pageable staging
         if (!h->pin_u) {
-            if (cudaMallocHost(&h->pin_u, sizeof(double) * h->cfg.max_batch) != cudaSuccess || cudaEventCreateWithFlags(&h->ev_u, cudaEventDisableTiming) != cudaSuccess)
+            if (cudaMallocHost(&h->pin_u, sizeof(double) * mb * h->cfg.n_agents) != cudaSuccess || cudaEventCreateWithFlags(&h->ev_u, cudaEventDisableTiming) != cudaSuccess)
                 return fail(SACB_ERR_NOMEM, "pinned allocation failed");
         }
         if (h->u_in_flight) SACB_CUDA(cudaEventSynchronize(h->ev_u));      // the previous call's search kernel has read the block (long done)
-        memcpy(h->pin_u, u, sizeof(double) * k);      // the search kernel reads them from here (host memory is addressable from the device): no copy call
+        // the search kernel reads them from here (host memory is addressable from the device): no copy call.  Row of agent a: pin_u + a * max_batch
+        for (int a = first; a < first + count; a++) memcpy(h->pin_u + a * mb, u + (a - first) * k, sizeof(double) * k);
     }
     const double *u_dev = u ? h->pin_u : w.u;
     const int depth = top_depth_of(n);
@@ -993,14 +1086,18 @@ int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B
     sa.ticket = tickets + 2 * kTicketInts; sa.carry_exact = w.cdf_exact; sa.chunk_sum = w.chunk_sum; sa.chunk_fine = w.chunk_fine; sa.n_chunks = n_chunks;
     sa.weights = w.weights; sa.slots = h->slots; sa.isw_ws = h->ws + h->L.isw; sa.idx_copy = h->last_idx_dev;
     sa.frame = frame_dev; sa.beta_start = (double)h->cfg.per_beta_start; sa.one_minus_start = 1.0 - (double)h->cfg.per_beta_start; sa.beta_frames = (double)h->cfg.per_beta_frames;
+    const int64_t ws_stride = per_ws_stride(h);
+    const PerAgents g{count > 1 ? h->ring_meta : nullptr, first, h->cfg.capacity, ws_stride, u ? (int64_t)sizeof(double) * mb : ws_stride, mb, h->L.ws_size};
     // no serial tails while the chunk prefixes fit into shared memory (DESIGN.md section 4 records the one- and two-launch forms measured against this)
     const bool no_tails = n_chunks + 1 <= kCarrySmem;
-    SACB_CUDA(launch_pdl(per_sum, dim3((2 << depth) - 1), dim3(256), 0, st, pdl, pa, n, depth, w.block_vals, w.total, tickets + 0,
-                         w.u, u ? 0 : (int)k, h->cfg.seed, (const int64_t *)frame_dev, no_tails ? 0 : 1));
+    if (!no_tails && h->cfg.n_agents != 1) return fail(SACB_ERR_ARG, "prioritized population: capacity <= 2096128 per agent");
+    const bool agents = h->cfg.n_agents > 1;      // population handles: the kernels with the agent offsets
+    SACB_CUDA(launch_pdl(agents ? per_sum<true> : per_sum<false>, dim3((2 << depth) - 1, count), dim3(256), 0, st, pdl, pa, n, depth, w.block_vals, w.total, tickets + 0,
+                         w.u, u ? 0 : (int)k, h->cfg.seed, (const int64_t *)frame_dev, no_tails ? 0 : 1, g));
     if (no_tails) {
-        SACB_CUDA(launch_pdl(per_chunk_notail, dim3((n_chunks + 7) / 8), dim3(256), 0, st, pdl, pa, n, depth, (const float *)w.block_vals, w.total,
-                             w.chunk_sum, w.chunk_fine));
-        SACB_CUDA(launch_pdl(per_search_scan, dim3((int)((k + 7) / 8)), dim3(256), 0, st, pdl, (const float *)w.total, w.chunk_carry, sa));
+        SACB_CUDA(launch_pdl(agents ? per_chunk_notail<true> : per_chunk_notail<false>, dim3((n_chunks + 7) / 8, count), dim3(256), 0, st, pdl, pa, n, depth, (const float *)w.block_vals, w.total,
+                             w.chunk_sum, w.chunk_fine, g));
+        SACB_CUDA(launch_pdl(agents ? per_search_scan<true> : per_search_scan<false>, dim3((int)((k + 7) / 8), count), dim3(256), 0, st, pdl, (const float *)w.total, w.chunk_carry, sa, g));
     } else {
         SACB_CUDA(launch_pdl(per_chunk, dim3((n_chunks + 7) / 8), dim3(256), 0, st, pdl, pa, n, (const float *)w.total, w.chunk_sum, w.chunk_fine,
                              n_chunks, w.chunk_carry, w.counters, tickets + kTicketInts));
@@ -1008,30 +1105,53 @@ int per_sample_launch(sacb_handle h, cudaStream_t st, const double *u, int64_t B
     }
     h->kernel_launches += 3;
     if (u) { SACB_CUDA(cudaEventRecord(h->ev_u, st)); h->u_in_flight = true; }      // behind the last kernel of the call
-    h->sample_k = k;
+    for (int a = first; a < first + count; a++) h->sample_k[a] = k;
     if (k_out) *k_out = k;
     return SACB_OK;
 }
 
-int per_writeback_launch(sacb_handle h, cudaStream_t st, int64_t B, bool pdl_ok) {
-    SACB_CUDA(launch_pdl(per_update_kernel, dim3(1), dim3(1024), sizeof(int64_t) * B, st, h->use_pdl != 0 && pdl_ok, h->prio, h->p_alpha,
-                         (const int64_t *)h->last_idx_dev, (const float *)(h->ws + h->L.td), (int)B, h->cfg.per_alpha, 0));
+// priorities <- |td| + 1e-6 of the last update for agents [first, first + count): one CTA per agent, then their CTA maxima
+int per_writeback_launch(sacb_handle h, cudaStream_t st, int64_t B, bool pdl_ok, int first, int count) {
+    const int64_t cap = h->cfg.capacity, mb = h->cfg.max_batch, wss = h->L.ws_size;
+    SACB_CUDA(launch_pdl(per_update_kernel, dim3(count), dim3(1024), sizeof(int64_t) * B, st, h->use_pdl != 0 && pdl_ok, h->prio + first * cap,
+                         h->p_alpha + first * cap, (const int64_t *)(h->last_idx_dev + first * mb), (const float *)(h->ws + first * wss + h->L.td), (int)B,
+                         h->cfg.per_alpha, 0, cap, mb, wss));
     h->kernel_launches++;
-    per_refresh_max(h, st);      // for the next push; same stream, behind the write-back
+    per_refresh_max(h, st, first, count);      // for the next push; same stream, behind the write-back
     return SACB_OK;
 }
 }  // namespace sacb
 
+static bool bad_per_agent(sacb_handle h, int agent) { return !h || agent < 0 || agent >= h->cfg.n_agents || h->cfg.replay_kind != SACB_REPLAY_PER; }
+
 extern "C" int sacb_per_sample(sacb_handle h, int agent, const double *u, int64_t B, int64_t *idx_out, float *weights_out,
                                float *s, float *a, float *r, float *s2, float *done) {
-    if (!h || agent != 0 || h->cfg.replay_kind != SACB_REPLAY_PER) return fail(SACB_ERR_ARG, "handle has no prioritized buffer");
+    if (!h || h->cfg.replay_kind != SACB_REPLAY_PER) return fail(SACB_ERR_ARG, "handle has no prioritized buffer");
+    if (agent < 0 || agent >= h->cfg.n_agents) return fail(SACB_ERR_ARG, "agent index out of range");
     int64_t k = 0;
-    int rc = per_sample_launch(h, h->stream, u, B, &k);
+    int rc = per_sample_launch(h, h->stream, u, B, &k, agent, 1);
     if (rc) return rc;
-    PerWs w = per_ws_of(h, 0);
+    PerWs w = per_ws_of(h, agent);
     if (idx_out) SACB_CUDA(cudaMemcpyAsync(idx_out, w.idx, sizeof(int64_t) * k, cudaMemcpyDeviceToHost, h->stream));
     if (weights_out) SACB_CUDA(cudaMemcpyAsync(weights_out, w.weights, sizeof(float) * k, cudaMemcpyDeviceToHost, h->stream));
-    if (s || a || r || s2 || done) return gather_to_host(h, 0, nullptr, k, s, a, r, s2, done);
+    if (s || a || r || s2 || done) return gather_to_host(h, agent, nullptr, k, s, a, r, s2, done);
+    if (idx_out || weights_out) SACB_CUDA(cudaStreamSynchronize(h->stream));
+    return SACB_OK;
+}
+
+extern "C" int sacb_per_sample_all(sacb_handle h, const double *u, int64_t B, int64_t *idx_out, float *weights_out) {
+    if (!h || h->cfg.replay_kind != SACB_REPLAY_PER) return fail(SACB_ERR_ARG, "handle has no prioritized buffer");
+    if (B < 1 || B > h->cfg.max_batch) return fail(SACB_ERR_ARG, "batch size out of range");
+    const int n = h->cfg.n_agents;
+    for (int a = 0; a < n; a++)
+        if (h->r_len[a] < B) return fail(SACB_ERR_STATE, "population sample: every agent's buffer must hold at least B transitions");
+    int rc = per_sample_launch(h, h->stream, u, B, nullptr, 0, n);
+    if (rc) return rc;
+    // the results sit at the same offset of every agent's workspace: one strided copy each
+    PerWs w = per_ws_of(h, 0);
+    const size_t pitch = (size_t)per_ws_stride(h);
+    if (idx_out) SACB_CUDA(cudaMemcpy2DAsync(idx_out, sizeof(int64_t) * B, w.idx, pitch, sizeof(int64_t) * B, n, cudaMemcpyDeviceToHost, h->stream));
+    if (weights_out) SACB_CUDA(cudaMemcpy2DAsync(weights_out, sizeof(float) * B, w.weights, pitch, sizeof(float) * B, n, cudaMemcpyDeviceToHost, h->stream));
     if (idx_out || weights_out) SACB_CUDA(cudaStreamSynchronize(h->stream));
     return SACB_OK;
 }
@@ -1040,68 +1160,71 @@ static int per_update_impl(sacb_handle h, int agent, const int64_t *idx, const f
 extern "C" int sacb_per_update(sacb_handle h, int agent, const int64_t *idx, const float *prio, int64_t B) { return per_update_impl(h, agent, idx, prio, B, 0); }
 extern "C" int sacb_per_update_final(sacb_handle h, int agent, const int64_t *idx, const float *prio, int64_t B) { return per_update_impl(h, agent, idx, prio, B, 1); }
 extern "C" int sacb_per_update_from_td(sacb_handle h, int agent, int64_t B) {
-    if (!h || agent != 0 || h->cfg.replay_kind != SACB_REPLAY_PER) return fail(SACB_ERR_ARG, "bad argument");
+    if (bad_per_agent(h, agent)) return fail(SACB_ERR_ARG, "bad argument");
     if (B < 1 || B > h->cfg.max_batch) return fail(SACB_ERR_ARG, "batch size out of range");
-    if (h->sample_k != B) return fail(SACB_ERR_STATE, "sacb_per_update_from_td: the last prioritized sample does not hold B rows");
-    return per_writeback_launch(h, h->stream, B);
+    if (h->sample_k[agent] != B) return fail(SACB_ERR_STATE, "sacb_per_update_from_td: the last prioritized sample does not hold B rows");
+    return per_writeback_launch(h, h->stream, B, true, agent, 1);
 }
 static int per_update_impl(sacb_handle h, int agent, const int64_t *idx, const float *prio, int64_t B, int is_final) {
-    if (!h || agent != 0 || h->cfg.replay_kind != SACB_REPLAY_PER || !prio) return fail(SACB_ERR_ARG, "bad argument");
+    if (bad_per_agent(h, agent) || !prio) return fail(SACB_ERR_ARG, "bad argument");
     if (B < 1 || B > h->cfg.max_batch) return fail(SACB_ERR_ARG, "batch size out of range");
-    PerWs w = per_ws_of(h, 0);
-    const int64_t *idx_dev = h->last_idx_dev;
+    PerWs w = per_ws_of(h, agent);
+    const int64_t cap = h->cfg.capacity;
+    const int64_t *idx_dev = h->last_idx_dev + agent * h->cfg.max_batch;
     if (idx) {
-        for (int64_t j = 0; j < B; j++) if (idx[j] < 0 || idx[j] >= h->cfg.capacity) return fail(SACB_ERR_STATE, "priority index out of range");
+        for (int64_t j = 0; j < B; j++) if (idx[j] < 0 || idx[j] >= cap) return fail(SACB_ERR_STATE, "priority index out of range");
         SACB_CUDA(cudaMemcpyAsync(w.idx, idx, sizeof(int64_t) * B, cudaMemcpyHostToDevice, h->stream));
         idx_dev = w.idx;
     }
     SACB_CUDA(cudaMemcpyAsync(w.weights, prio, sizeof(float) * B, cudaMemcpyHostToDevice, h->stream));
-    per_update_kernel<<<1, 1024, sizeof(int64_t) * B, h->stream>>>(h->prio, h->p_alpha, idx_dev, w.weights, (int)B, h->cfg.per_alpha, is_final);
+    per_update_kernel<<<1, 1024, sizeof(int64_t) * B, h->stream>>>(h->prio + agent * cap, h->p_alpha + agent * cap, idx_dev, w.weights, (int)B, h->cfg.per_alpha,
+                                                                   is_final, cap, h->cfg.max_batch, 0);
     h->kernel_launches++;
-    h->prio_max_valid = false;
+    h->prio_max_valid[agent] = 0;
     SACB_CUDA(cudaGetLastError());
     SACB_CUDA(cudaStreamSynchronize(h->stream));
     return SACB_OK;
 }
 
 extern "C" int sacb_per_get_priorities(sacb_handle h, int agent, float *prio, int64_t n) {
-    if (!h || agent != 0 || !h->prio || n > h->cfg.capacity) return fail(SACB_ERR_ARG, "bad argument");
-    SACB_CUDA(cudaMemcpyAsync(prio, h->prio, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
+    if (bad_per_agent(h, agent) || !h->prio || n > h->cfg.capacity) return fail(SACB_ERR_ARG, "bad argument");
+    SACB_CUDA(cudaMemcpyAsync(prio, h->prio + agent * h->cfg.capacity, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
     SACB_CUDA(cudaStreamSynchronize(h->stream));
     return SACB_OK;
 }
 
 extern "C" int sacb_per_set_priorities(sacb_handle h, int agent, const float *prio, const float *p_alpha, int64_t n) {
-    if (!h || agent != 0 || !h->prio || n > h->cfg.capacity || !prio) return fail(SACB_ERR_ARG, "bad argument");
-    h->sample_k = 0;      // a minibatch drawn from the old table is stale
-    h->prio_max_valid = false;
-    SACB_CUDA(cudaMemcpyAsync(h->prio, prio, sizeof(float) * n, cudaMemcpyHostToDevice, h->stream));
-    if (p_alpha) SACB_CUDA(cudaMemcpyAsync(h->p_alpha, p_alpha, sizeof(float) * n, cudaMemcpyHostToDevice, h->stream));
-    else { pow_alpha_kernel<<<256, 256, 0, h->stream>>>(h->prio, h->p_alpha, n, h->cfg.per_alpha); h->kernel_launches++; }
+    if (bad_per_agent(h, agent) || !h->prio || n > h->cfg.capacity || !prio) return fail(SACB_ERR_ARG, "bad argument");
+    h->sample_k[agent] = 0;      // a minibatch drawn from the old table is stale
+    h->prio_max_valid[agent] = 0;
+    float *pr = h->prio + agent * h->cfg.capacity, *pa = h->p_alpha + agent * h->cfg.capacity;
+    SACB_CUDA(cudaMemcpyAsync(pr, prio, sizeof(float) * n, cudaMemcpyHostToDevice, h->stream));
+    if (p_alpha) SACB_CUDA(cudaMemcpyAsync(pa, p_alpha, sizeof(float) * n, cudaMemcpyHostToDevice, h->stream));
+    else { pow_alpha_kernel<<<256, 256, 0, h->stream>>>(pr, pa, n, h->cfg.per_alpha); h->kernel_launches++; }
     SACB_CUDA(cudaStreamSynchronize(h->stream));
     return SACB_OK;
 }
 
 extern "C" int sacb_per_get_stats(sacb_handle h, int agent, sacb_per_stats *out) {
-    if (!h || agent != 0 || !h->prio || !out) return fail(SACB_ERR_ARG, "bad argument");
-    PerWs w = per_ws_of(h, 0);
+    if (bad_per_agent(h, agent) || !h->prio || !out) return fail(SACB_ERR_ARG, "bad argument");
+    PerWs w = per_ws_of(h, agent);
     int counters[4] = {0, 0, 0, 0};
     float tot = 0.f; double last = 0.0;
-    const int64_t n = std::max<int64_t>(1, h->r_len[0]);
+    const int64_t n = std::max<int64_t>(1, h->r_len[agent]);
     const int n_chunks = (int)((n + kChunk - 1) / kChunk);
     SACB_CUDA(cudaMemcpyAsync(counters, w.counters, sizeof(int) * 4, cudaMemcpyDeviceToHost, h->stream));
     SACB_CUDA(cudaMemcpyAsync(&tot, w.total, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     SACB_CUDA(cudaMemcpyAsync(&last, w.chunk_carry + n_chunks, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     SACB_CUDA(cudaStreamSynchronize(h->stream));
-    out->frame = h->per_frame[0]; out->pos = h->r_pos[0]; out->len = h->r_len[0];
+    out->frame = h->per_frame[agent]; out->pos = h->r_pos[agent]; out->len = h->r_len[agent];
     out->n_fine = counters[0]; out->n_flagged = counters[3]; out->n_exact_fallbacks = counters[2];
     out->total_f32 = tot; out->cdf_last = last;
     return SACB_OK;
 }
 
 extern "C" int sacb_per_set_frame(sacb_handle h, int agent, int64_t frame) {
-    if (!h || agent != 0) return fail(SACB_ERR_ARG, "bad argument");
-    h->per_frame[0] = frame;
-    h->per_frame_dirty = true;
+    if (!h || agent < 0 || agent >= h->cfg.n_agents) return fail(SACB_ERR_ARG, "bad argument");
+    h->per_frame[agent] = frame;
+    h->per_frame_dirty[agent] = 1;
     return SACB_OK;
 }

@@ -60,6 +60,8 @@ extern "C" int sacb_create(const sacb_config *cfg, sacb_handle *out) {
     if (cfg->max_batch < 1 || cfg->n_agents < 1 || cfg->capacity < 1) return fail(SACB_ERR_ARG, "bad max_batch / n_agents / capacity");
     if (2 * cfg->act_dim > 256) return fail(SACB_ERR_ARG, "act_dim > 128 unsupported");
     if (cfg->layer_norm && cfg->n_agents != 1) return fail(SACB_ERR_ARG, "layer_norm: single-agent handles only (the population programs are not validated with it)");
+    if (cfg->replay_kind == SACB_REPLAY_PER && cfg->n_agents > 1 && cfg->capacity > kPopulationPerCapacity)
+        return fail(SACB_ERR_ARG, "prioritized population: capacity <= 2096128 per agent (the tail-free sampler form)");
     if (cfg->layer_norm && cfg->hidden_dim > 1024) return fail(SACB_ERR_ARG, "layer_norm: hidden_dim > 1024 unsupported (a row is normalised in registers)");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || cfg->device >= ndev) { cudaGetLastError(); return fail(SACB_ERR_DEVICE, "no CUDA device: this library has no CPU fallback"); }
@@ -372,7 +374,7 @@ static int upload_eps(sacb_handle h, int agent, int64_t B, const float *eps_next
 // while the caller is back in Python
 static int finish_update(sacb_handle h, float *losses_out, uint32_t flags, int64_t write_back_B = 0) {
     if ((flags & SACB_NO_LOSS_READBACK) || !losses_out) {
-        if (write_back_B > 0) { if (int rc = per_writeback_launch(h, h->stream, write_back_B)) return rc; }
+        if (write_back_B > 0) { if (int rc = per_writeback_launch(h, h->stream, write_back_B, true, 0, h->cfg.n_agents)) return rc; }
         return (flags & SACB_NO_LOSS_READBACK) ? SACB_OK : sacb_synchronize(h);
     }
     // the three losses (the `.item()` calls of sac_imp.py:141-143) and the device error flag: the last stage of the step (T_FINISH) has
@@ -384,7 +386,7 @@ static int finish_update(sacb_handle h, float *losses_out, uint32_t flags, int64
     if (write_back_B > 0) {
         if (!h->ev_loss) SACB_CUDA(cudaEventCreateWithFlags(&h->ev_loss, cudaEventDisableTiming));
         SACB_CUDA(cudaEventRecord(h->ev_loss, h->stream));
-        if (int rc = per_writeback_launch(h, h->stream, write_back_B)) return rc;
+        if (int rc = per_writeback_launch(h, h->stream, write_back_B, true, 0, h->cfg.n_agents)) return rc;
         SACB_CUDA(cudaEventSynchronize(h->ev_loss));
     } else {
         SACB_CUDA(cudaStreamSynchronize(h->stream));
@@ -460,9 +462,10 @@ extern "C" int sacb_update(sacb_handle h, int64_t B, const int64_t *idx, const f
         gather_mode = 3;
     } else if (!(flags & SACB_USE_LAST_SAMPLE)) {
         return fail(SACB_ERR_ARG, "no indices: pass idx, stage them, set SACB_DEVICE_INDICES or SACB_USE_LAST_SAMPLE");
-    } else if (h->cfg.replay_kind == SACB_REPLAY_PER && h->sample_k != B) {
-        // set_priorities / clear / a sample of another size leave no (or a stale) minibatch behind
-        return fail(SACB_ERR_STATE, "SACB_USE_LAST_SAMPLE: the last prioritized sample does not hold B rows (sample again)");
+    } else if (h->cfg.replay_kind == SACB_REPLAY_PER) {
+        // set_priorities / clear / a sample of another size leave no (or a stale) minibatch behind; a population needs every agent's
+        for (int a = 0; a < h->cfg.n_agents; a++)
+            if (h->sample_k[a] != B) return fail(SACB_ERR_STATE, "SACB_USE_LAST_SAMPLE: the last prioritized sample does not hold B rows (sample again)");
     }
     if (eps_next) for (int a = 0; a < h->cfg.n_agents; a++) {
         const int64_t n = B * h->cfg.act_dim;
@@ -474,7 +477,7 @@ extern "C" int sacb_update(sacb_handle h, int64_t B, const int64_t *idx, const f
     if (rc) return rc;
     int64_t write_back_B = 0;
     if (flags & SACB_WRITE_BACK_TD) {
-        if (h->cfg.replay_kind != SACB_REPLAY_PER || h->cfg.n_agents != 1 || !(flags & SACB_USE_LAST_SAMPLE))
+        if (h->cfg.replay_kind != SACB_REPLAY_PER || !(flags & SACB_USE_LAST_SAMPLE))
             return fail(SACB_ERR_ARG, "SACB_WRITE_BACK_TD: needs the prioritized buffer and SACB_USE_LAST_SAMPLE");
         write_back_B = B;
     }
@@ -502,8 +505,8 @@ static int per_step_enqueue(sacb_handle h, int64_t B) {
     int rc = upload_per_frame(h, h->stream);
     if (rc) return rc;
     const int64_t k = std::min<int64_t>(B, h->r_len[0]);
-    if (h->sample_k != k) {      // first call (or the batch size changed): draw this step's minibatch now
-        rc = per_sample_launch(h, h->stream, nullptr, B, nullptr);
+    if (h->sample_k[0] != k) {      // first call (or the batch size changed): draw this step's minibatch now
+        rc = per_sample_launch(h, h->stream, nullptr, B, nullptr, 0, 1);
         if (rc) return rc;
     }
     ProgramKey key = update_key(h, (int)k, 1, 0, 1, h->cfg.per_weighted_loss ? 1 : 0);

@@ -429,6 +429,11 @@ class PopulationSAC:
     dimension of every stage kernel and the 4th coordinate of the TMA descriptors.  No inter-agent (or inter-GPU) traffic:
     `distributed.partition_agents` assigns global agent ids to ranks.  Minibatch positions are drawn on the device.
 
+    replay="per": every agent gets its own prioritized buffer instead (replay_buffer.py:25-90 each: priority table, max-priority
+    rule, frame counter and beta schedule per agent; `capacity` <= 2 096 128 per agent).  One chain of three sampler launches draws
+    every agent's minibatch, one launch writes every agent's |TD| priorities back (`per_weighted_loss`, as in `SAC`).  Per-agent
+    accessors mirror PrioritizedReplayBuffer: `priorities`, `set_priorities`, `sample`, `update_priorities`, `frame`, `set_frame`.
+
     Population-based training: `gamma`, `tau`, `lr`, `alpha` and `target_entropy` (default -action_dim, sac_imp.py:46) take one value
     for all agents or one per agent.  They live in each agent's scalar block on the device, so `set_hyperparameters` (explore) never
     rebuilds the update program, and `exploit(dst, src)` copies whole learner states on the device.  `automatic_entropy_tuning` is
@@ -438,9 +443,13 @@ class PopulationSAC:
 
     def __init__(self, n_agents, state_dim, action_dim, hidden_dim=256, gamma=0.99, tau=0.005, lr=3e-4, alpha=0.2,
                  automatic_entropy_tuning=True, device="cuda", *, seeds=None, capacity=100000, max_batch=256, math="bf16x3",
-                 launch="staged", seed=None, action_bounds=None, target_entropy=None):
+                 launch="staged", seed=None, action_bounds=None, target_entropy=None, replay="uniform", per_alpha=0.6, per_beta_start=0.4,
+                 per_beta_frames=100000, per_weighted_loss=False):
         if not str(device).startswith("cuda"):
             raise RuntimeError("PopulationSAC runs on a B200 only (device='cuda[:i]'); there is no CPU path")
+        if replay not in ("uniform", "per"):
+            raise ValueError(f"replay must be 'uniform' or 'per', got {replay!r}")
+        self._per = replay == "per"
         self.n_agents, self.device = int(n_agents), device
         self.seeds = list(range(self.n_agents)) if seeds is None else [int(x) for x in seeds]
         if len(self.seeds) != self.n_agents:
@@ -456,7 +465,9 @@ class PopulationSAC:
         cfg.gamma, cfg.tau, cfg.lr, cfg.alpha0 = hp["gamma"][0], hp["tau"][0], hp["lr"][0], hp["alpha"][0]
         cfg.auto_entropy = int(bool(automatic_entropy_tuning))
         cfg.action_scale, cfg.action_bias = probe.action_scale, probe.action_bias
-        cfg.replay_kind, cfg.capacity, cfg.max_batch, cfg.n_agents = N.REPLAY_UNIFORM, capacity, max_batch, self.n_agents
+        cfg.replay_kind, cfg.capacity, cfg.max_batch, cfg.n_agents = N.REPLAY_PER if self._per else N.REPLAY_UNIFORM, capacity, max_batch, self.n_agents
+        cfg.per_alpha, cfg.per_beta_start, cfg.per_beta_frames = per_alpha, per_beta_start, per_beta_frames
+        cfg.per_weighted_loss = int(bool(per_weighted_loss))
         cfg.device = torch.device(device).index or 0
         cfg.math_mode = {"fp32": N.MATH_FP32, "bf16x3": N.MATH_BF16X3}[math]
         cfg.launch_mode = {"staged": N.LAUNCH_STAGED, "persistent": N.LAUNCH_PERSISTENT}[launch]
@@ -505,6 +516,67 @@ class PopulationSAC:
     def buffer_len(self, agent):
         return int(N.lib().sacb_len(self._h, int(agent)))
 
+    # ---- per-agent prioritized buffer (replay="per"; PrioritizedReplayBuffer's interface with an agent index) -------------------------
+    def _per_agent_index(self, agent):
+        if not self._per:
+            raise ValueError("this population has uniform replay rings (construct it with replay='per')")
+        return self._agent_index(agent)
+
+    def priorities(self, agent):
+        """Host copy of agent `agent`'s float32[capacity] priority table (zeros for never-written slots)."""
+        i = self._per_agent_index(agent)
+        out = np.zeros(int(self._cfg.capacity), np.float32)
+        N.check(N.lib().sacb_per_get_priorities(self._h, i, N.ptr(out), out.size))
+        return out
+
+    def set_priorities(self, agent, priorities, p_alpha=None):
+        """Overwrite the first len(priorities) entries of one agent's table (p_alpha: its p**alpha table, else computed on the device)."""
+        i = self._per_agent_index(agent)
+        p = N.f32(priorities).ravel()
+        pa = None if p_alpha is None else N.f32(p_alpha).ravel()
+        if pa is not None and pa.size != p.size:
+            raise ValueError("p_alpha must have one entry per priority")
+        N.check(N.lib().sacb_per_set_priorities(self._h, i, N.ptr(p), N.ptr(pa), p.size))
+
+    def sample(self, agent, batch_size, u=None):
+        """PrioritizedReplayBuffer.sample of one agent: (s, a, r, s2, d, idx, weights); `u` = its min(batch_size, len) uniforms."""
+        i = self._per_agent_index(agent)
+        n = min(batch_size, self.buffer_len(i))
+        if u is None:
+            u = np.random.random_sample(n)
+        u = np.ascontiguousarray(u, np.float64)
+        o, k = self._cfg.obs_dim, self._cfg.act_dim
+        s, a, r = np.empty((n, o), np.float32), np.empty((n, k), np.float32), np.empty(n, np.float32)
+        s2, d = np.empty((n, o), np.float32), np.empty(n, np.float32)
+        idx, w = np.empty(n, np.int64), np.empty(n, np.float32)
+        N.check(N.lib().sacb_per_sample(self._h, i, N.ptr(u, ctypes.c_double), batch_size, N.ptr(idx, ctypes.c_int64), N.ptr(w),
+                                        N.ptr(s), N.ptr(a), N.ptr(r), N.ptr(s2), N.ptr(d)))
+        return s, a, r, s2, d, idx, w
+
+    def update_priorities(self, agent, indices, priorities):
+        """PrioritizedReplayBuffer.update_priorities of one agent (float32 priorities are stored + 1e-6 in float32, float64 ones in float64)."""
+        i = self._per_agent_index(agent)
+        idx = np.ascontiguousarray(np.asarray(indices), np.int64).ravel()
+        if hasattr(priorities, "detach"):
+            priorities = priorities.detach().cpu().numpy()
+        pr = np.asarray(priorities)
+        if pr.dtype == np.float32:
+            pr = np.ascontiguousarray(pr.ravel())
+            N.check(N.lib().sacb_per_update(self._h, i, N.ptr(idx, ctypes.c_int64), N.ptr(pr), idx.size))
+        else:      # priority.item() + 1e-6 in float64, then the float32 store (replay_buffer.py:87)
+            final = (pr.astype(np.float64).ravel() + 1e-6).astype(np.float32)
+            N.check(N.lib().sacb_per_update_final(self._h, i, N.ptr(idx, ctypes.c_int64), N.ptr(final), idx.size))
+
+    def frame(self, agent):
+        """The agent's frame counter (beta schedule, replay_buffer.py:53): starts at 1, +1 per sample of that agent."""
+        i = self._per_agent_index(agent)
+        st = N.PerStats()
+        N.check(N.lib().sacb_per_get_stats(self._h, i, ctypes.byref(st)))
+        return int(st.frame)
+
+    def set_frame(self, agent, v):
+        N.check(N.lib().sacb_per_set_frame(self._h, self._per_agent_index(agent), int(v)))
+
     # ---- acting / learning ------------------------------------------------------------------------------------------------
     def select_action(self, states, evaluate=False, *, eps=None):
         """states [n_agents, obs] -> actions [n_agents, act]: agent i acts on row i with its own policy (sac_imp.py:54-72 each)."""
@@ -514,14 +586,26 @@ class PopulationSAC:
         N.check(N.lib().sacb_select_action_batch(self._h, N.ptr(obs), int(bool(evaluate)), N.ptr(e), N.ptr(out)))
         return out
 
-    def update_parameters(self, batch_size=256, *, idx=None, eps=None, sync=True):
+    def update_parameters(self, batch_size=256, *, idx=None, u=None, eps=None, sync=True):
         """One update of EVERY agent (sac_imp.py:74-144 each) in one program.  idx [n_agents, B] positions / eps = (eps_next,
-        eps_cur) [n_agents, B, act] are test hooks; by default both are drawn on the device.  Returns a list of loss dicts."""
+        eps_cur) [n_agents, B, act] are test hooks; by default both are drawn on the device.  Returns a list of loss dicts.
+        replay="per": every agent's minibatch is one prioritized sample of B rows (each agent's buffer must hold at least B transitions),
+        drawn for all agents at once; `u` [n_agents, B] replaces the uniforms drawn on the device (idx does not apply).  With
+        per_weighted_loss the critic loss is IS-weighted and every agent's priorities of its minibatch become |q1 - y| + 1e-6."""
         lib = N.lib()
         e_next = e_cur = None
         if eps is not None:
             e_next, e_cur = N.f32(eps[0]), N.f32(eps[1])
-        if idx is not None:
+        if self._per:
+            if idx is not None:
+                raise ValueError("a prioritized population draws its minibatches with the sampler: pass u, not idx")
+            uu = None if u is None else np.ascontiguousarray(u, np.float64).reshape(self.n_agents, batch_size)
+            N.check(lib.sacb_per_sample_all(self._h, N.ptr(uu, ctypes.c_double), batch_size, None, None))
+            flags = N.NO_LOSS_READBACK | N.USE_LAST_SAMPLE | (N.WRITE_BACK_TD if self._cfg.per_weighted_loss else 0)
+            N.check(lib.sacb_update(self._h, batch_size, None, N.ptr(e_next), N.ptr(e_cur), None, flags))
+        elif u is not None:
+            raise ValueError("u: uniforms of the prioritized sampler (replay='per')")
+        elif idx is not None:
             ix = np.ascontiguousarray(idx, np.int64).reshape(self.n_agents, batch_size)
             N.check(lib.sacb_update(self._h, batch_size, N.ptr(ix, ctypes.c_int64), N.ptr(e_next), N.ptr(e_cur), None, N.NO_LOSS_READBACK))
         else:
@@ -625,8 +709,9 @@ class PopulationSAC:
 
     def exploit(self, dst, src):
         """Exploit step: agent dst[k] takes over the whole learner state of agent src[k] (weights, targets, Adam state, temperature,
-        hyperparameters, step counts), copied on the device.  Replay rings stay with their agent, and dst[k] keeps drawing its own
-        minibatch positions and noise (the device streams are keyed by agent index).  A dst may appear once, and no agent may be both
+        hyperparameters, step counts), copied on the device.  Replay rings -- and with replay="per" the priority tables and frame
+        counters -- stay with their agent, and dst[k] keeps drawing its own minibatch positions and noise (the device streams are keyed
+        by agent index).  A dst may appear once, and no agent may be both
         a src and a dst of the same call (ValueError)."""
         d = np.ascontiguousarray(np.asarray(dst, np.int64).ravel())
         s = np.ascontiguousarray(np.asarray(src, np.int64).ravel())

@@ -55,8 +55,10 @@ typedef struct {
     float gamma, tau, lr, alpha0;  /* sac_imp.py:13-17 */
     int32_t auto_entropy;          /* sac_imp.py:18 */
     float action_scale, action_bias; /* networks_model1.py:52-55 */
-    int32_t replay_kind;           /* SACB_REPLAY_* */
-    int64_t capacity;              /* replay_buffer.py:7 / :26 */
+    int32_t replay_kind;           /* SACB_REPLAY_*; a population (n_agents > 1) gives every agent its own ring, and with
+                                      SACB_REPLAY_PER its own priority table, frame counter and sampler workspace */
+    int64_t capacity;              /* replay_buffer.py:7 / :26, per agent.  SACB_REPLAY_PER with n_agents > 1: <= 2 096 128
+                                      (the sampler form without serial tails), SACB_ERR_ARG at sacb_create otherwise */
     float per_alpha, per_beta_start; /* replay_buffer.py:26 */
     int64_t per_beta_frames;
     int32_t max_batch;             /* largest batch_size update/sample will be called with */
@@ -147,18 +149,24 @@ int64_t sacb_host_first_distinct(const uint32_t *words, int64_t n_words, uint64_
 int sacb_sample_uniform(sacb_handle h, int agent, const int64_t *idx, int64_t B, float *s, float *a, float *r,
                         float *s2, float *done);
 
-/* PrioritizedReplayBuffer.sample (replay_buffer.py:48-82).  u = B float64 uniforms (what
- * np.random.random_sample(B) returns inside np.random.choice); NULL => drawn on device (Philox).
- * Outputs may be NULL to leave results on the device for sacb_update(..., SACB_USE_LAST_SAMPLE). */
+/* PrioritizedReplayBuffer.sample (replay_buffer.py:48-82) of one agent.  u = B float64 uniforms (what
+ * np.random.random_sample(B) returns inside np.random.choice); NULL => drawn on device (splitmix64 of the key, the frame counter and
+ * the row; agent a's key is cfg.seed for a = 0 and cfg.seed ^ splitmix64(a) otherwise, splitmix64(x) = the finaliser of x + 0x9E3779B97F4A7C15).
+ * Outputs may be NULL to leave results on the device for sacb_update(..., SACB_USE_LAST_SAMPLE).
+ * Every sacb_per_* entry point below takes agent in [0, n_agents) (SACB_ERR_ARG otherwise). */
 int sacb_per_sample(sacb_handle h, int agent, const double *u, int64_t B, int64_t *idx_out, float *weights_out,
                     float *s, float *a, float *r, float *s2, float *done);
+/* The same sample for EVERY agent of the handle in one chain of three launches: u_or_null [n_agents][B] (NULL: each agent draws from
+ * its own key on the device), idx_out / weights_out [n_agents][B] or NULL.  Every agent's buffer must hold at least B transitions
+ * (SACB_ERR_STATE otherwise), so each minibatch has B rows.  The minibatches stay on the device for sacb_update(SACB_USE_LAST_SAMPLE). */
+int sacb_per_sample_all(sacb_handle h, const double *u_or_null, int64_t B, int64_t *idx_out_or_null, float *weights_out_or_null);
 /* PrioritizedReplayBuffer.update_priorities (replay_buffer.py:84-87): sequential semantics, last duplicate wins. */
 int sacb_per_update(sacb_handle h, int agent, const int64_t *idx, const float *prio, int64_t B);
 /* same with prio already = float32(priority + 1e-6) computed by the caller in float64 (float64 inputs) */
 int sacb_per_update_final(sacb_handle h, int agent, const int64_t *idx, const float *prio_final, int64_t B);
 /* fused path: priorities <- |q1 - y| of the last update (extension, SURVEY H10), indices of the last sample */
 int sacb_per_update_from_td(sacb_handle h, int agent, int64_t B);
-/* throughput form of the trainer's learner step over the prioritized buffer (trainer.py:202-205 with PER), everything resident
+/* throughput form of the trainer's learner step over the prioritized buffer (single-agent handles; SACB_ERR_ARG on a population) (trainer.py:202-205 with PER), everything resident
  * in HBM: update on the minibatch the previous call sampled -> priorities <- |q1 - y| -> sample (device uniforms) for the next
  * call.  The write-back and the next sample run on a second stream under the tail of the update (from the actor-loss stage on), overlapping the rest of
  * the update; values are identical to sacb_per_sample / sacb_update(SACB_USE_LAST_SAMPLE) / sacb_per_update_from_td in sequence.
@@ -181,7 +189,8 @@ enum {
                                   Nothing of the step touches the host: population mode, K updates per call (sacb_update_steps) */
     SACB_WRITE_BACK_TD = 16    /* prioritized buffer, with SACB_USE_LAST_SAMPLE: priorities of the minibatch <- |q1 - y| + 1e-6
                                   (update_priorities, replay_buffer.py:84-87; = sacb_per_update_from_td) enqueued behind the loss copy:
-                                  the call returns when the losses have arrived, the write-back runs while the caller is back in Python */
+                                  the call returns when the losses have arrived, the write-back runs while the caller is back in Python.
+                                  A population writes back every agent's minibatch into its own table in one launch */
 };
 /* idx: B logical indices (NULL => SACB_USE_LAST_SAMPLE, or the next index set pre-staged with sacb_stage_indices; otherwise SACB_ERR_ARG);
  * eps_next / eps_cur: [B, act] N(0,1) draws of the two policy.sample calls (sac_imp.py:89, :116), NULL => Philox;
@@ -189,7 +198,7 @@ enum {
 int sacb_update(sacb_handle h, int64_t B, const int64_t *idx, const float *eps_next, const float *eps_cur,
                 float *losses_out, uint32_t flags);
 /* K learner steps per call with nothing of a step on the host (trainer.py:190-205 batched; SURVEY 8f rank 3): prioritized ring =
- * K x the sacb_per_step pipeline, uniform ring = K updates with SACB_DEVICE_INDICES; eps drawn on the device; then ONE read-back:
+ * K x the sacb_per_step pipeline (single-agent handles), uniform ring = K updates with SACB_DEVICE_INDICES; eps drawn on the device; then ONE read-back:
  * losses_out[K][3] (NULL or SACB_NO_LOSS_READBACK: none).  K <= 64.  Bitwise equal to K single calls. */
 int sacb_update_steps(sacb_handle h, int64_t B, int K, float *losses_out, uint32_t flags);
 /* update on a caller-supplied minibatch (no replay involved): test / bench entry. */
