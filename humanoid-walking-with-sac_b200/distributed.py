@@ -14,6 +14,7 @@ import torch
 import torch.distributed as dist
 
 from . import _native as N
+from .sac_imp import _loss_dict
 
 
 def partition_agents(n_agents, world_size, rank):
@@ -116,11 +117,10 @@ class DataParallelSAC:
         losses = np.zeros(3, np.float32)
         if self.mode == "peer" and self.exchange:      # the finish kernels averaged the replicas' loss scalars through peer memory
             N.check(lib.sacb_dp_get_losses(a._h, N.ptr(losses)))
-            return {"q1_loss": float(losses[0]), "q2_loss": float(losses[1]), "policy_loss": float(losses[2])}
+            return _loss_dict(losses)
         N.check(lib.sacb_get_losses(a._h, 0, N.ptr(losses)))
         t = torch.from_numpy(losses.copy()).to(self._bufs[0].device)
         with torch.cuda.stream(self._stream):
             allreduce_mean_([t], self.group)
         self._stream.synchronize()
-        q1, q2, pi = t.tolist()
-        return {"q1_loss": q1, "q2_loss": q2, "policy_loss": pi}
+        return _loss_dict(t.tolist())

@@ -51,6 +51,72 @@ def _as_row_parts(state, action, reward, next_state, done):
     return s, a, np.float32(reward), s2, np.float32(bool(done))
 
 
+def _transition_arrays(cfg, n):
+    """Host arrays (s, a, r, s2, d) for n transitions of a handle with config `cfg`."""
+    o, k = cfg.obs_dim, cfg.act_dim
+    return (np.empty((n, o), np.float32), np.empty((n, k), np.float32), np.empty(n, np.float32),
+            np.empty((n, o), np.float32), np.empty(n, np.float32))
+
+
+# ---- the prioritized buffer of one agent of a handle: PrioritizedReplayBuffer (agent 0) and PopulationSAC(replay="per") ----------
+# `owner` is anything that holds a library handle `_h` and its config `_cfg`.
+def _per_priorities(owner, agent):
+    """Host copy of the agent's float32[capacity] priority table (zeros for never-written slots)."""
+    out = np.zeros(int(owner._cfg.capacity), np.float32)
+    N.check(N.lib().sacb_per_get_priorities(owner._h, agent, N.ptr(out), out.size))
+    return out
+
+
+def _per_set_priorities(owner, agent, priorities, p_alpha=None):
+    """Overwrite the first len(priorities) entries of the agent's table (p_alpha: its p**alpha table, else computed on the device)."""
+    p = N.f32(priorities).ravel()
+    pa = None if p_alpha is None else N.f32(p_alpha).ravel()
+    if pa is not None and pa.size != p.size:      # the library copies p.size entries of each
+        raise ValueError("p_alpha must have one entry per priority")
+    N.check(N.lib().sacb_per_set_priorities(owner._h, agent, N.ptr(p), N.ptr(pa), p.size))
+
+
+def _per_sample(owner, agent, batch_size, u=None):
+    """The agent's (s, a, r, s2, d, idx, weights) of min(batch_size, len) rows; `u` = that many uniforms."""
+    n = min(batch_size, int(N.lib().sacb_len(owner._h, agent)))                # replay_buffer.py:50
+    if n > int(owner._cfg.max_batch):     # one call normalises the IS weights by the batch maximum on the device: no piecewise form
+        raise ValueError(f"prioritized sample of {n} rows exceeds the handle's max_batch={int(owner._cfg.max_batch)} "
+                         "(standalone buffers: 1024; a buffer of a SAC or PopulationSAC: its max_batch)")
+    if u is None:
+        u = np.random.random_sample(n)       # the draw np.random.choice(len, n, p=probs) makes (mtrand.pyx::choice)
+    u = np.ascontiguousarray(u, np.float64)
+    rows = _transition_arrays(owner._cfg, n)
+    idx, w = np.empty(n, np.int64), np.empty(n, np.float32)
+    N.check(N.lib().sacb_per_sample(owner._h, agent, N.ptr(u, ctypes.c_double), batch_size, N.ptr(idx, ctypes.c_int64), N.ptr(w),
+                                    *map(N.ptr, rows)))
+    return (*rows, idx, w)
+
+
+def _per_update_priorities(owner, agent, indices, priorities):
+    """The agent's update_priorities: float32 priorities are stored + 1e-6 in float32, float64 ones + 1e-6 in float64."""
+    idx = np.ascontiguousarray(np.asarray(indices), np.int64).ravel()
+    if hasattr(priorities, "detach"):
+        priorities = priorities.detach().cpu().numpy()
+    pr = np.asarray(priorities)
+    if pr.dtype == np.float32:
+        pr = np.ascontiguousarray(pr.ravel())
+        N.check(N.lib().sacb_per_update(owner._h, agent, N.ptr(idx, ctypes.c_int64), N.ptr(pr), idx.size))
+    else:   # priority.item() + 1e-6 in float64, then the float32 store (replay_buffer.py:87)
+        final = (pr.astype(np.float64).ravel() + 1e-6).astype(np.float32)
+        N.check(N.lib().sacb_per_update_final(owner._h, agent, N.ptr(idx, ctypes.c_int64), N.ptr(final), idx.size))
+
+
+def _per_stats(owner, agent):
+    st = N.PerStats()
+    N.check(N.lib().sacb_per_get_stats(owner._h, agent, ctypes.byref(st)))
+    return st
+
+
+def _per_set_frame(owner, agent, v):
+    """The agent's frame counter (beta schedule, replay_buffer.py:53): starts at 1, +1 per sample."""
+    N.check(N.lib().sacb_per_set_frame(owner._h, agent, int(v)))
+
+
 class _DeviceBuffer:
     _KIND = N.REPLAY_UNIFORM
 
@@ -122,11 +188,9 @@ class _DeviceBuffer:
     def _read(self, idx):
         self._flush()
         idx = np.ascontiguousarray(idx, np.int64)
-        n, o, k = idx.size, self._cfg.obs_dim, self._cfg.act_dim
-        s, a, r = np.empty((n, o), np.float32), np.empty((n, k), np.float32), np.empty(n, np.float32)
-        s2, d = np.empty((n, o), np.float32), np.empty(n, np.float32)
-        N.check(N.lib().sacb_read_transitions(self._h, 0, N.ptr(idx, ctypes.c_int64), n, N.ptr(s), N.ptr(a), N.ptr(r), N.ptr(s2), N.ptr(d)))
-        return s, a, r, s2, d
+        rows = _transition_arrays(self._cfg, idx.size)
+        N.check(N.lib().sacb_read_transitions(self._h, 0, N.ptr(idx, ctypes.c_int64), idx.size, *map(N.ptr, rows)))
+        return rows
 
     def _materialise(self):
         n = len(self)
@@ -166,12 +230,10 @@ class ReplayBuffer(_DeviceBuffer):
     def sample(self, batch_size):
         idx = self._draw(batch_size)        # ValueError("Sample larger than population...") like the reference
         self._flush()
-        n, o, k = idx.size, self._cfg.obs_dim, self._cfg.act_dim
-        s, a, r = np.empty((n, o), np.float32), np.empty((n, k), np.float32), np.empty(n, np.float32)
-        s2, d = np.empty((n, o), np.float32), np.empty(n, np.float32)
+        rows = _transition_arrays(self._cfg, idx.size)
         # any size up to len(buffer), like the reference: the library gathers through its staging area in pieces (replay.cu: gather_to_host)
-        N.check(N.lib().sacb_sample_uniform(self._h, 0, N.ptr(idx, ctypes.c_int64), n, N.ptr(s), N.ptr(a), N.ptr(r), N.ptr(s2), N.ptr(d)))
-        return s, a, r, s2, d
+        N.check(N.lib().sacb_sample_uniform(self._h, 0, N.ptr(idx, ctypes.c_int64), idx.size, *map(N.ptr, rows)))
+        return rows
 
 
 class PrioritizedReplayBuffer(_DeviceBuffer):
@@ -188,9 +250,7 @@ class PrioritizedReplayBuffer(_DeviceBuffer):
         cfg.per_alpha, cfg.per_beta_start, cfg.per_beta_frames = self.alpha, self.beta_start, self.beta_frames
 
     def _stats(self):
-        st = N.PerStats()
-        N.check(N.lib().sacb_per_get_stats(self._h, 0, ctypes.byref(st)))
-        return st
+        return _per_stats(self, 0)
 
     @property
     def frame(self):
@@ -198,7 +258,7 @@ class PrioritizedReplayBuffer(_DeviceBuffer):
 
     @frame.setter
     def frame(self, v):
-        N.check(N.lib().sacb_per_set_frame(self._h, 0, int(v)))
+        _per_set_frame(self, 0, v)
 
     @property
     def pos(self):
@@ -208,18 +268,15 @@ class PrioritizedReplayBuffer(_DeviceBuffer):
     @property
     def priorities(self):
         """Host copy of the float32[capacity] priority table (zeros for never-written slots)."""
-        out = np.zeros(self.capacity, np.float32)
-        if self._h is not None:
-            self._flush()
-            N.check(N.lib().sacb_per_get_priorities(self._h, 0, N.ptr(out), self.capacity))
-        return out
+        if self._h is None:
+            return np.zeros(self.capacity, np.float32)
+        self._flush()
+        return _per_priorities(self, 0)
 
     def set_priorities(self, priorities, p_alpha=None):
         """Overwrite the table (tests: inject numpy's own p**alpha, whose float32 pow is CPU-ISA dependent)."""
         self._flush()
-        p = N.f32(priorities)
-        pa = None if p_alpha is None else N.f32(p_alpha)
-        N.check(N.lib().sacb_per_set_priorities(self._h, 0, N.ptr(p), N.ptr(pa), p.size))
+        _per_set_priorities(self, 0, priorities, p_alpha)
 
     @property
     def buffer(self):
@@ -231,30 +288,8 @@ class PrioritizedReplayBuffer(_DeviceBuffer):
 
     def sample(self, batch_size, u=None):
         self._flush()
-        n = min(batch_size, len(self))                                           # replay_buffer.py:50
-        if n > int(self._cfg.max_batch):     # one call normalises the IS weights by the batch maximum on the device: no piecewise form
-            raise ValueError(f"prioritized sample of {n} rows exceeds this buffer's max_batch={int(self._cfg.max_batch)} "
-                             "(standalone buffers: 1024; a SAC-owned buffer: the agent's max_batch)")
-        if u is None:
-            u = np.random.random_sample(n)       # the draw np.random.choice(len, n, p=probs) makes (mtrand.pyx::choice)
-        u = np.ascontiguousarray(u, np.float64)
-        o, k = self._cfg.obs_dim, self._cfg.act_dim
-        s, a, r = np.empty((n, o), np.float32), np.empty((n, k), np.float32), np.empty(n, np.float32)
-        s2, d = np.empty((n, o), np.float32), np.empty(n, np.float32)
-        idx, w = np.empty(n, np.int64), np.empty(n, np.float32)
-        N.check(N.lib().sacb_per_sample(self._h, 0, N.ptr(u, ctypes.c_double), batch_size, N.ptr(idx, ctypes.c_int64), N.ptr(w),
-                                        N.ptr(s), N.ptr(a), N.ptr(r), N.ptr(s2), N.ptr(d)))
-        return s, a, r, s2, d, idx, w
+        return _per_sample(self, 0, batch_size, u)
 
     def update_priorities(self, indices, priorities):
         self._flush()
-        idx = np.ascontiguousarray(np.asarray(indices), np.int64)
-        if hasattr(priorities, "detach"):
-            priorities = priorities.detach().cpu().numpy()
-        pr = np.asarray(priorities)
-        if pr.dtype == np.float32:
-            pr = np.ascontiguousarray(pr.ravel())
-            N.check(N.lib().sacb_per_update(self._h, 0, N.ptr(idx, ctypes.c_int64), N.ptr(pr), idx.size))
-        else:   # priority.item() + 1e-6 in float64, then the float32 store (replay_buffer.py:87)
-            final = (pr.astype(np.float64).ravel() + 1e-6).astype(np.float32)
-            N.check(N.lib().sacb_per_update_final(self._h, 0, N.ptr(idx, ctypes.c_int64), N.ptr(final), idx.size))
+        _per_update_priorities(self, 0, indices, priorities)

@@ -18,9 +18,152 @@ import torch
 
 from . import _native as N
 from .networks_model1 import GaussianPolicy, QNetwork
-from .replay_buffer import PrioritizedReplayBuffer, ReplayBuffer
+from .replay_buffer import (PrioritizedReplayBuffer, ReplayBuffer, _per_priorities, _per_sample, _per_set_frame, _per_set_priorities,
+                            _per_stats, _per_update_priorities)
 
 _NETS = ("policy", "q1", "q2", "q1_target", "q2_target")
+_NET_OPTIMIZERS = ((N.NET_POLICY, "policy"), (N.NET_Q1, "q1"), (N.NET_Q2, "q2"))
+# torch.optim.Adam's state_dict layout: the param_group entries besides lr / params, and per moment: the arena slot of a network's
+# moment, its key in the state, and the scalar-block field of the temperature's (net id None) moment
+_ADAM_DEFAULTS = dict(betas=(0.9, 0.999), eps=1e-08, weight_decay=0, amsgrad=False, maximize=False, foreach=None, capturable=False,
+                      differentiable=False, fused=None, decoupled_weight_decay=False)
+_ADAM_MOMENTS = ((N.SLOT_ADAM_M, "exp_avg", "log_alpha_m"), (N.SLOT_ADAM_V, "exp_avg_sq", "log_alpha_v"))
+_STEP_FIELD = {N.NET_POLICY: "step_policy", N.NET_Q1: "step_q1", N.NET_Q2: "step_q2", None: "step_alpha"}
+
+
+def _adam_group(lr, n_params):
+    return dict(lr=lr, **_ADAM_DEFAULTS, params=list(range(n_params)))
+
+
+def _adam_lr(sd, default=None):
+    """Learning rate of a torch.optim.Adam state_dict (`default` if it holds none)."""
+    groups = sd.get("param_groups")
+    return float(groups[0]["lr"]) if groups and "lr" in groups[0] else default
+
+
+def _scalar(x):
+    """First element of a python number, array or tensor (the device's scalar block holds float32 values)."""
+    return float(torch.as_tensor(x).detach().reshape(-1)[0])
+
+
+def _loss_dict(losses):
+    """update_parameters' return value (sac_imp.py:74-144) from a [q1, q2, policy] loss triple."""
+    return {"q1_loss": float(losses[0]), "q2_loss": float(losses[1]), "policy_loss": float(losses[2])}
+
+
+def _config(n_agents, state_dim, action_dim, hidden_dim, n_hidden, policy, gamma, tau, lr, alpha, automatic_entropy_tuning, device, *,
+            replay, capacity, max_batch, math, launch, seed, per_alpha, per_beta_start, per_beta_frames, per_weighted_loss, layer_norm=False):
+    """The handle's sacb_config from constructor arguments (`policy`: a GaussianPolicy holding the action scale and bias)."""
+    cfg = N.default_config()
+    cfg.obs_dim, cfg.act_dim, cfg.hidden_dim, cfg.n_hidden = state_dim, action_dim, hidden_dim, n_hidden
+    cfg.gamma, cfg.tau, cfg.lr, cfg.alpha0, cfg.auto_entropy = gamma, tau, lr, alpha, int(bool(automatic_entropy_tuning))
+    cfg.action_scale, cfg.action_bias = policy.action_scale, policy.action_bias
+    cfg.replay_kind = N.REPLAY_PER if replay == "per" else N.REPLAY_UNIFORM
+    cfg.capacity, cfg.max_batch, cfg.n_agents, cfg.device = capacity, max_batch, n_agents, torch.device(device).index or 0
+    cfg.per_alpha, cfg.per_beta_start, cfg.per_beta_frames = per_alpha, per_beta_start, per_beta_frames
+    cfg.per_weighted_loss = int(bool(per_weighted_loss))
+    cfg.layer_norm = int(bool(layer_norm))
+    cfg.math_mode = {"fp32": N.MATH_FP32, "bf16x3": N.MATH_BF16X3}[math]
+    cfg.launch_mode = {"staged": N.LAUNCH_STAGED, "persistent": N.LAUNCH_PERSISTENT}[launch]
+    cfg.seed = random.getrandbits(63) if seed is None else int(seed)
+    return cfg
+
+
+def _param_names(module):
+    return [(name, tuple(p.shape)) for name, p in module.named_parameters()]
+
+
+class _Learner:
+    """What SAC and PopulationSAC share: a library handle `_h`, and per agent of it the scalar block, the torch.optim.Adam state of
+    the four optimizers and the reference's save() / save_checkpoint() layout.  A subclass sets `_cfg` and `_names` (net id -> [(parameter
+    name, shape)]) and says where tensors come from: `_tensor`, `_net_state_dicts`, `_load_nets`."""
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h is not None:
+            try:
+                N.lib().sacb_destroy(h)
+            except Exception:
+                pass
+            self._h = None
+
+    def synchronize(self):
+        N.check(N.lib().sacb_synchronize(self._h))
+
+    def _scalars(self, agent=0):
+        sc = N.Scalars()
+        N.check(N.lib().sacb_get_scalars(self._h, agent, ctypes.byref(sc)))
+        return sc
+
+    def _set_scalars(self, sc, agent=0):
+        N.check(N.lib().sacb_set_scalars(self._h, agent, ctypes.byref(sc)))
+
+    def _import(self, agent, net_id, slot, t, value):
+        host = N.f32(torch.as_tensor(value).detach().cpu().numpy())
+        N.check(N.lib().sacb_import_tensor(self._h, agent, net_id, slot, t, N.ptr(host), host.size))
+
+    def _alpha(self, sc, device, alpha_is_float=True):
+        """SAC.alpha of the agent whose scalar block is `sc` (a tensor lives on `device`)."""
+        if not self._cfg.auto_entropy or sc.n_updates == 0 and alpha_is_float:
+            return float(sc.alpha)
+        return torch.tensor([sc.alpha], device=device)
+
+    # ---- torch.optim.Adam state of one optimizer of one agent (net_id None: the temperature's) ----------------------------------------
+    def _adam_state_dict(self, agent, net_id, sc, lr):
+        """state_dict() of the optimizer (scalar block `sc`): like torch, no per-parameter state before the first step."""
+        step = getattr(sc, _STEP_FIELD[net_id])
+        n = 1 if net_id is None else len(self._names[net_id])
+        state = {}
+        for t in range(n if step > 0 else 0):
+            state[t] = {"step": torch.tensor(float(step))}
+            for slot, key, field in _ADAM_MOMENTS:
+                state[t][key] = (torch.tensor([getattr(sc, field)]) if net_id is None else
+                                 self._tensor(agent, net_id, slot, t, self._names[net_id][t][1]))
+        return {"state": state, "param_groups": [_adam_group(lr, n)]}
+
+    def _load_adam_state(self, agent, net_id, sd, sc):
+        """Inverse of `_adam_state_dict` into the device and `sc` (the caller stores `sc`).  A parameter without state gets the zero moments
+        a fresh torch.optim.Adam starts from; an empty state is step 0."""
+        state = sd["state"]
+        setattr(sc, _STEP_FIELD[net_id], int(float(state[min(state)]["step"])) if state else 0)
+        for slot, key, field in _ADAM_MOMENTS:
+            if net_id is None:
+                setattr(sc, field, _scalar(state[min(state)][key]) if state else 0.0)
+                continue
+            for t, (_, shape) in enumerate(self._names[net_id]):
+                self._import(agent, net_id, slot, t, state[t][key] if t in state else np.zeros(shape, np.float32))
+
+    # ---- the reference's save() / save_checkpoint() layout of one agent ---------------------------------------------------------------
+    def _learner_state(self, agent, device, alpha_is_float=True, lr=None):
+        """The learner keys of save() (sac_imp.py:154-162): the five nets and 'alpha'.  Given the learning rate, those of save_checkpoint()
+        (:177-201): the optimizers too, and 'log_alpha' with the temperature's optimizer under automatic entropy tuning."""
+        sc = self._scalars(agent)
+        out = self._net_state_dicts(agent)
+        if lr is not None:
+            for net_id, name in _NET_OPTIMIZERS:
+                out[f"{name}_optimizer_state_dict"] = self._adam_state_dict(agent, net_id, sc, lr)
+        out["alpha"] = self._alpha(sc, device, alpha_is_float)
+        if lr is not None and self._cfg.auto_entropy:
+            out["log_alpha"] = torch.tensor([sc.log_alpha], device=device, requires_grad=True)      # a leaf, like SAC.log_alpha
+            out["alpha_optimizer_state_dict"] = self._adam_state_dict(agent, None, sc, lr)
+        return out
+
+    def _load_learner(self, agent, checkpoint, optimizers=True):
+        """Inverse of `_learner_state`: the nets and alpha; with `optimizers`, each optimizer state and 'log_alpha' the checkpoint holds
+        (the temperature's under automatic entropy tuning only).  Returns the learning rate of the last optimizer state that has one."""
+        self._load_nets(agent, checkpoint)
+        sc, lr = self._scalars(agent), None
+        sc.alpha = _scalar(checkpoint["alpha"])
+        auto = bool(self._cfg.auto_entropy)
+        for net_id, name in (*_NET_OPTIMIZERS, (None, "alpha")) if optimizers else ():
+            sd = checkpoint.get(f"{name}_optimizer_state_dict")
+            if sd is not None and (net_id is not None or auto):
+                self._load_adam_state(agent, net_id, sd, sc)
+                lr = _adam_lr(sd, lr)
+        if optimizers and auto and "log_alpha" in checkpoint:
+            sc.log_alpha = _scalar(checkpoint["log_alpha"])
+        self._set_scalars(sc, agent)
+        return lr
 
 
 class ArenaAdam:
@@ -28,20 +171,8 @@ class ArenaAdam:
     this object only serves `state_dict()` / `load_state_dict()` in the reference checkpoint layout (SURVEY 5)."""
 
     def __init__(self, owner, net_id, module, lr):
-        self._owner, self._net_id, self._module = owner, net_id, module
-        n = len(list(module.parameters())) if module is not None else 1
-        self.param_groups = [dict(lr=lr, betas=(0.9, 0.999), eps=1e-08, weight_decay=0, amsgrad=False, maximize=False, foreach=None,
-                                  capturable=False, differentiable=False, fused=None, decoupled_weight_decay=False, params=list(range(n)))]
-
-    def _step_count(self):
-        sc = self._owner._scalars()
-        return {N.NET_POLICY: sc.step_policy, N.NET_Q1: sc.step_q1, N.NET_Q2: sc.step_q2, None: sc.step_alpha}[self._net_id]
-
-    def _set_step(self, v):
-        sc = self._owner._scalars()
-        name = {N.NET_POLICY: "step_policy", N.NET_Q1: "step_q1", N.NET_Q2: "step_q2", None: "step_alpha"}[self._net_id]
-        setattr(sc, name, int(v))
-        self._owner._set_scalars(sc)
+        self._owner, self._net_id = owner, net_id
+        self.param_groups = [_adam_group(lr, len(list(module.parameters())) if module is not None else 1)]
 
     def zero_grad(self, set_to_none=True):
         pass
@@ -50,49 +181,18 @@ class ArenaAdam:
         raise RuntimeError("the optimizer step is fused into SAC.update_parameters")
 
     def state_dict(self):
-        step = self._step_count()
-        state = {}
-        if step > 0:
-            if self._net_id is None:
-                sc = self._owner._scalars()
-                state[0] = {"step": torch.tensor(float(step)), "exp_avg": torch.tensor([sc.log_alpha_m]), "exp_avg_sq": torch.tensor([sc.log_alpha_v])}
-            else:
-                for i, p in enumerate(self._module.parameters()):
-                    state[i] = {"step": torch.tensor(float(step)),
-                                "exp_avg": self._owner._tensor(self._net_id, N.SLOT_ADAM_M, i, p.shape),
-                                "exp_avg_sq": self._owner._tensor(self._net_id, N.SLOT_ADAM_V, i, p.shape)}
-        return {"state": state, "param_groups": [dict(g) for g in self.param_groups]}
+        return self._owner._adam_state_dict(0, self._net_id, self._owner._scalars(), self.param_groups[0]["lr"])
 
     def load_state_dict(self, sd):
-        state = sd["state"]
-        if not state:
-            self._set_step(0)
-            self._restore_lr(sd)
-            return
-        first = state[min(state)]
-        self._set_step(int(float(first["step"])))
-        if self._net_id is None:
-            sc = self._owner._scalars()
-            sc.log_alpha_m = float(torch.as_tensor(first["exp_avg"]).reshape(-1)[0])
-            sc.log_alpha_v = float(torch.as_tensor(first["exp_avg_sq"]).reshape(-1)[0])
-            self._owner._set_scalars(sc)
-            self._restore_lr(sd)
-            return
-        for i, st in state.items():
-            for slot, key in ((N.SLOT_ADAM_M, "exp_avg"), (N.SLOT_ADAM_V, "exp_avg_sq")):
-                host = N.f32(torch.as_tensor(st[key]).detach().cpu().numpy())
-                N.check(N.lib().sacb_import_tensor(self._owner._h, 0, self._net_id, slot, int(i), N.ptr(host), host.size))
-        self._restore_lr(sd)
-
-    def _restore_lr(self, sd):
-        # torch.optim.Adam.load_state_dict restores the learning rate of the checkpoint (sac_imp.py:215-218); the device
-        # Adam of all four optimizers shares ONE rate (sac_imp.py:39-49), so a differing value re-derives its step-size table
-        if sd.get("param_groups") and "lr" in sd["param_groups"][0]:
-            lr = float(sd["param_groups"][0]["lr"])
+        sc = self._owner._scalars()
+        self._owner._load_adam_state(0, self._net_id, sd, sc)
+        self._owner._set_scalars(sc)
+        lr = _adam_lr(sd)
+        if lr is not None:      # torch.optim.Adam.load_state_dict restores the learning rate of the checkpoint (sac_imp.py:215-218)
             self._owner._set_lr(lr)
 
 
-class SAC:
+class SAC(_Learner):
     """Soft Actor-Critic for continuous actions; one fused device program per update_parameters call."""
 
     def __init__(self, state_dim, action_dim, hidden_dim=256, gamma=0.99, tau=0.005, lr=3e-4, alpha=0.2,
@@ -104,7 +204,6 @@ class SAC:
         self.gamma, self.tau, self.device = gamma, tau, device
         self.automatic_entropy_tuning = automatic_entropy_tuning
         self._lr = lr
-        dev_index = torch.device(device).index or 0
 
         # networks: built on the host with the reference's initialisers (same global-RNG consumption order as
         # sac_imp.py:28-36), then uploaded; afterwards every parameter aliases the device arena
@@ -122,21 +221,13 @@ class SAC:
         if getattr(self.policy, "N_HIDDEN", n_hidden) != n_hidden:
             raise ValueError("QNetwork and GaussianPolicy must come from the same networks_model* variant")
 
-        cfg = N.default_config()
-        cfg.obs_dim, cfg.act_dim, cfg.hidden_dim, cfg.n_hidden = state_dim, action_dim, hidden_dim, n_hidden
-        cfg.gamma, cfg.tau, cfg.lr, cfg.alpha0, cfg.auto_entropy = gamma, tau, lr, alpha, int(bool(automatic_entropy_tuning))
-        cfg.action_scale, cfg.action_bias = self.policy.action_scale, self.policy.action_bias
-        cfg.replay_kind = N.REPLAY_PER if replay == "per" else N.REPLAY_UNIFORM
-        cfg.capacity, cfg.max_batch, cfg.n_agents, cfg.device = capacity, max_batch, 1, dev_index
-        cfg.per_alpha, cfg.per_beta_start, cfg.per_beta_frames = per_alpha, per_beta_start, per_beta_frames
-        cfg.per_weighted_loss = int(bool(per_weighted_loss))
-        cfg.layer_norm = int(bool(layer_norm))
-        cfg.math_mode = {"fp32": N.MATH_FP32, "bf16x3": N.MATH_BF16X3}[math]
-        cfg.launch_mode = {"staged": N.LAUNCH_STAGED, "persistent": N.LAUNCH_PERSISTENT}[launch]
-        cfg.seed = random.getrandbits(63) if seed is None else int(seed)
-        self._cfg = cfg
-        self._h = N.create(cfg)
+        self._cfg = _config(1, state_dim, action_dim, hidden_dim, n_hidden, self.policy, gamma, tau, lr, alpha, automatic_entropy_tuning, device,
+                            replay=replay, capacity=capacity, max_batch=max_batch, math=math, launch=launch, seed=seed,
+                            per_alpha=per_alpha, per_beta_start=per_beta_start, per_beta_frames=per_beta_frames,
+                            per_weighted_loss=per_weighted_loss, layer_norm=layer_norm)
+        self._h = N.create(self._cfg)
         self._arena_base = None
+        self._names = {net_id: _param_names(getattr(self, name)) for net_id, name in enumerate(_NETS)}
         for net_id, name in enumerate(_NETS):
             getattr(self, name)._bind(self, net_id)
 
@@ -186,25 +277,9 @@ class SAC:
     def invalidate_shadows(self):
         N.check(N.lib().sacb_invalidate_shadows(self._h))
 
-    def __del__(self):
-        h = getattr(self, "_h", None)
-        if h is not None:
-            try:
-                N.lib().sacb_destroy(h)
-            except Exception:
-                pass
-            self._h = None
-
     # ---- scalars ---------------------------------------------------------------------------------------------
-    def _scalars(self):
-        sc = N.Scalars()
-        N.check(N.lib().sacb_get_scalars(self._h, 0, ctypes.byref(sc)))
-        return sc
-
-    def _set_scalars(self, sc):
-        N.check(N.lib().sacb_set_scalars(self._h, 0, ctypes.byref(sc)))
-
     def _set_lr(self, lr):
+        """The device Adam of all four optimizers shares ONE rate (sac_imp.py:39-49): a new one re-derives its step-size table."""
         N.check(N.lib().sacb_set_lr(self._h, lr))
         self._lr = lr
         for opt in ("policy_optimizer", "q1_optimizer", "q2_optimizer", "alpha_optimizer"):
@@ -220,24 +295,32 @@ class SAC:
             self._ext_stream = torch.cuda.ExternalStream(sp.value, device=f"cuda:{self._cfg.device}")
         return torch.cuda.stream(self._ext_stream)
 
-    def _tensor(self, net_id, slot, t, shape):
+    def _tensor(self, agent, net_id, slot, t, shape):
+        """A live view of one arena tensor (the state_dicts of this class alias the device memory)."""
         dev = ctypes.c_void_p()
-        N.check(N.lib().sacb_tensor_dev(self._h, 0, net_id, slot, t, ctypes.byref(dev)))
+        N.check(N.lib().sacb_tensor_dev(self._h, agent, net_id, slot, t, ctypes.byref(dev)))
         return torch.as_tensor(N.DevArray(dev.value, tuple(shape), self), device=f"cuda:{self._cfg.device}")
+
+    def _net_state_dicts(self, agent):
+        return {f"{n}_state_dict": getattr(self, n).state_dict() for n in _NETS}
+
+    def _load_nets(self, agent, checkpoint):
+        # the copies into the aliased arena run on the library's own stream (torch's current stream is not ordered against it)
+        with self._library_stream():
+            for n in _NETS:
+                getattr(self, n).load_state_dict(checkpoint[f"{n}_state_dict"])
+        self.synchronize()
 
     @property
     def alpha(self):
         """sac_imp.py:23 / :135: the constructor float until the first tuned update, then exp(log_alpha) (1-element tensor)."""
-        sc = self._scalars()
-        if not self.automatic_entropy_tuning or sc.n_updates == 0 and self._alpha_is_float:
-            return float(sc.alpha)
-        return torch.tensor([sc.alpha], device=self.device)
+        return self._alpha(self._scalars(), self.device, self._alpha_is_float)
 
     @alpha.setter
     def alpha(self, value):
         sc = self._scalars()
         self._alpha_is_float = not torch.is_tensor(value)
-        sc.alpha = float(value.detach().reshape(-1)[0]) if torch.is_tensor(value) else float(value)
+        sc.alpha = _scalar(value)
         self._set_scalars(sc)
 
     @property
@@ -249,7 +332,7 @@ class SAC:
     @log_alpha.setter
     def log_alpha(self, value):
         sc = self._scalars()
-        sc.log_alpha = float(torch.as_tensor(value).detach().reshape(-1)[0])
+        sc.log_alpha = _scalar(value)
         self._set_scalars(sc)
 
     # ---- acting ----------------------------------------------------------------------------------------------
@@ -292,7 +375,7 @@ class SAC:
         self._alpha_is_float = False
         if not sync:
             return None
-        return {"q1_loss": float(losses[0]), "q2_loss": float(losses[1]), "policy_loss": float(losses[2])}
+        return _loss_dict(losses)
 
     def learner_steps(self, batch_size=256, k=8, *, sync=True):
         """K learner steps per call, nothing of a step on the host (SURVEY 8f rank 3; trainer.py:190-205 with the updates of K
@@ -306,7 +389,7 @@ class SAC:
         self._alpha_is_float = False
         if not sync:
             return None
-        return [{"q1_loss": float(l[0]), "q2_loss": float(l[1]), "policy_loss": float(l[2])} for l in losses]
+        return [_loss_dict(l) for l in losses]
 
     def learner_step(self, batch_size=256, *, sync=False):
         """Throughput form of `update_parameters` over the prioritized buffer (per_weighted_loss mode), everything resident
@@ -324,7 +407,7 @@ class SAC:
         self._alpha_is_float = False
         if not sync:
             return None
-        return {"q1_loss": float(losses[0]), "q2_loss": float(losses[1]), "policy_loss": float(losses[2])}
+        return _loss_dict(losses)
 
     def update_from_batch(self, batch, eps=None, is_weights=None, export_grads=False, want_td=False):
         """Same step on a caller-supplied minibatch dict(s,a,r,s2,d) (parity tests / benchmarks; no replay involved)."""
@@ -340,14 +423,14 @@ class SAC:
         N.check(N.lib().sacb_update_batch(self._h, B, N.ptr(s), N.ptr(a), N.ptr(r), N.ptr(s2), N.ptr(d), N.ptr(w), N.ptr(e_next), N.ptr(e_cur),
                                           N.ptr(losses), N.ptr(td), N.EXPORT_GRADS if export_grads else 0))
         self._alpha_is_float = False
-        out = {"q1_loss": float(losses[0]), "q2_loss": float(losses[1]), "policy_loss": float(losses[2])}
+        out = _loss_dict(losses)
         return (out, td) if want_td else out
 
     def exported_grads(self, net):
         """Gradients of the last update run with export_grads=True, keyed like `named_parameters()`."""
         net_id = {"policy": N.NET_POLICY, "q1": N.NET_Q1, "q2": N.NET_Q2}[net]
         module = getattr(self, net)
-        return {name: self._tensor(net_id, N.SLOT_GRAD, i, p.shape).cpu().numpy() for i, (name, p) in enumerate(module.named_parameters())}
+        return {name: self._tensor(0, net_id, N.SLOT_GRAD, i, p.shape).cpu().numpy() for i, (name, p) in enumerate(module.named_parameters())}
 
     def _soft_update_target_networks(self):
         raise RuntimeError("the Polyak update is fused into update_parameters (sac_imp.py:146-152)")
@@ -356,33 +439,19 @@ class SAC:
     def save(self, path):
         self.synchronize()                  # an update enqueued with sync=False / learner_step may still be running
         with self._library_stream():
-            torch.save({f"{n}_state_dict": getattr(self, n).state_dict() for n in _NETS} | {"alpha": self.alpha}, path)
-
-    def _load_nets(self, checkpoint):
-        # the copies into the aliased arena run on the library's own stream (torch's current stream is not ordered against it)
-        with self._library_stream():
-            for n in _NETS:
-                getattr(self, n).load_state_dict(checkpoint[f"{n}_state_dict"])
-        self.synchronize()
+            torch.save(self._learner_state(0, self.device, self._alpha_is_float), path)
 
     def load(self, path):
         checkpoint = torch.load(path, map_location=self.device, weights_only=False)
-        self._load_nets(checkpoint)
-        self.alpha = checkpoint["alpha"]
+        self._load_learner(0, checkpoint, optimizers=False)
+        self._alpha_is_float = not torch.is_tensor(checkpoint["alpha"])
 
     def save_checkpoint(self, path, episode, total_steps, replay_buffer=True, *, rng_state=False):
         """sac_imp.py:177-201, same keys.  rng_state=True adds one extra key ('sacb_rng_state': the Philox counters of the
         on-device eps / exploration draws) so that a seeded run resumes its own random stream; the reference ignores it."""
         self.synchronize()
-        checkpoint = {"episode": episode, "total_steps": total_steps}
         with self._library_stream():
-            checkpoint.update({f"{n}_state_dict": getattr(self, n).state_dict() for n in _NETS})
-            for n in ("policy", "q1", "q2"):
-                checkpoint[f"{n}_optimizer_state_dict"] = getattr(self, f"{n}_optimizer").state_dict()
-            checkpoint["alpha"] = self.alpha
-            if self.automatic_entropy_tuning:
-                checkpoint["log_alpha"] = self.log_alpha
-                checkpoint["alpha_optimizer_state_dict"] = self.alpha_optimizer.state_dict()
+            checkpoint = {"episode": episode, "total_steps": total_steps, **self._learner_state(0, self.device, self._alpha_is_float, self._lr)}
             if replay_buffer:
                 checkpoint["replay_buffer"] = self.replay_buffer.buffer
             if rng_state:
@@ -393,15 +462,10 @@ class SAC:
 
     def load_checkpoint(self, path, load_replay_buffer=True):
         checkpoint = torch.load(path, map_location=self.device, weights_only=False)   # pickled deque / numpy inside
-        self._load_nets(checkpoint)
-        for n in ("policy", "q1", "q2"):
-            if f"{n}_optimizer_state_dict" in checkpoint:
-                getattr(self, f"{n}_optimizer").load_state_dict(checkpoint[f"{n}_optimizer_state_dict"])
-        self.alpha = checkpoint["alpha"]
-        if self.automatic_entropy_tuning and "log_alpha" in checkpoint:
-            self.log_alpha = checkpoint["log_alpha"]
-        if "alpha_optimizer_state_dict" in checkpoint and self.automatic_entropy_tuning:
-            self.alpha_optimizer.load_state_dict(checkpoint["alpha_optimizer_state_dict"])
+        lr = self._load_learner(0, checkpoint)
+        self._alpha_is_float = not torch.is_tensor(checkpoint["alpha"])
+        if lr is not None:
+            self._set_lr(lr)
         if load_replay_buffer and "replay_buffer" in checkpoint:
             self.replay_buffer.buffer = checkpoint["replay_buffer"]
         rs = checkpoint.get("sacb_rng_state")
@@ -417,11 +481,8 @@ class SAC:
         N.check(N.lib().sacb_get_stats(self._h, ctypes.byref(st)))
         return {k: getattr(st, k) for k, _ in st._fields_}
 
-    def synchronize(self):
-        N.check(N.lib().sacb_synchronize(self._h))
 
-
-class PopulationSAC:
+class PopulationSAC(_Learner):
     """`n_agents` independent SAC agents (distinct seeds) trained by ONE batched update program per step on one GPU
     (BASELINE.json configs[4]; the per-agent step is sac_imp.py:74-144).  Agent i = exactly what `torch.manual_seed(seeds[i]);
     SAC(state_dim, action_dim, ...)` builds: same initialiser calls in the same order, its own Adam state, temperature, Philox stream
@@ -460,46 +521,27 @@ class PopulationSAC:
             self._check_hparams({k: v[i] for k, v in hp.items()})
         kw = {} if action_bounds is None else {"action_bounds": action_bounds}
         probe = GaussianPolicy(state_dim, action_dim, hidden_dim, **kw)
-        cfg = N.default_config()
-        cfg.obs_dim, cfg.act_dim, cfg.hidden_dim, cfg.n_hidden = state_dim, action_dim, hidden_dim, getattr(probe, "N_HIDDEN", 2)
-        cfg.gamma, cfg.tau, cfg.lr, cfg.alpha0 = hp["gamma"][0], hp["tau"][0], hp["lr"][0], hp["alpha"][0]
-        cfg.auto_entropy = int(bool(automatic_entropy_tuning))
-        cfg.action_scale, cfg.action_bias = probe.action_scale, probe.action_bias
-        cfg.replay_kind, cfg.capacity, cfg.max_batch, cfg.n_agents = N.REPLAY_PER if self._per else N.REPLAY_UNIFORM, capacity, max_batch, self.n_agents
-        cfg.per_alpha, cfg.per_beta_start, cfg.per_beta_frames = per_alpha, per_beta_start, per_beta_frames
-        cfg.per_weighted_loss = int(bool(per_weighted_loss))
-        cfg.device = torch.device(device).index or 0
-        cfg.math_mode = {"fp32": N.MATH_FP32, "bf16x3": N.MATH_BF16X3}[math]
-        cfg.launch_mode = {"staged": N.LAUNCH_STAGED, "persistent": N.LAUNCH_PERSISTENT}[launch]
-        cfg.seed = random.getrandbits(63) if seed is None else int(seed)
-        self._cfg = cfg
+        self._cfg = cfg = _config(self.n_agents, state_dim, action_dim, hidden_dim, getattr(probe, "N_HIDDEN", 2), probe,
+                                  hp["gamma"][0], hp["tau"][0], hp["lr"][0], hp["alpha"][0], automatic_entropy_tuning, device,
+                                  replay=replay, capacity=capacity, max_batch=max_batch, math=math, launch=launch, seed=seed,
+                                  per_alpha=per_alpha, per_beta_start=per_beta_start, per_beta_frames=per_beta_frames,
+                                  per_weighted_loss=per_weighted_loss)
         self._h = N.create(cfg)
         self._names = {}
-        lib = N.lib()
         for i, sd in enumerate(self.seeds):
             torch.manual_seed(sd)                      # the construction order of sac_imp.py:28-36 under this agent's seed
             pol = GaussianPolicy(state_dim, action_dim, hidden_dim, **kw)
             q1, q2 = QNetwork(state_dim, action_dim, hidden_dim), QNetwork(state_dim, action_dim, hidden_dim)
             QNetwork(state_dim, action_dim, hidden_dim); QNetwork(state_dim, action_dim, hidden_dim)     # the targets' own (discarded) init draws
             for net_id, mod in ((N.NET_POLICY, pol), (N.NET_Q1, q1), (N.NET_Q2, q2), (N.NET_Q1_TARGET, q1), (N.NET_Q2_TARGET, q2)):
-                self._names[net_id] = [(n, tuple(p.shape)) for n, p in mod.named_parameters()]
-                for t, (_, p) in enumerate(mod.named_parameters()):
-                    host = N.f32(p.detach().numpy())
-                    N.check(lib.sacb_import_tensor(self._h, i, net_id, N.SLOT_PARAM, t, N.ptr(host), host.size))
+                self._names[net_id] = _param_names(mod)
+                for t, p in enumerate(mod.parameters()):
+                    self._import(i, net_id, N.SLOT_PARAM, t, p)
         default = (cfg.lr, cfg.gamma, cfg.tau, -float(action_dim), cfg.alpha0)
         for i in range(self.n_agents):
             mine = {k: float(np.float32(hp[k][i])) for k in self.HPARAMS}
             if tuple(mine.values()) != tuple(float(np.float32(x)) for x in default):
                 self.set_hyperparameters(i, **mine)
-
-    def __del__(self):
-        h = getattr(self, "_h", None)
-        if h is not None:
-            try:
-                N.lib().sacb_destroy(h)
-            except Exception:
-                pass
-            self._h = None
 
     def __len__(self):
         return self.n_agents
@@ -524,58 +566,26 @@ class PopulationSAC:
 
     def priorities(self, agent):
         """Host copy of agent `agent`'s float32[capacity] priority table (zeros for never-written slots)."""
-        i = self._per_agent_index(agent)
-        out = np.zeros(int(self._cfg.capacity), np.float32)
-        N.check(N.lib().sacb_per_get_priorities(self._h, i, N.ptr(out), out.size))
-        return out
+        return _per_priorities(self, self._per_agent_index(agent))
 
     def set_priorities(self, agent, priorities, p_alpha=None):
         """Overwrite the first len(priorities) entries of one agent's table (p_alpha: its p**alpha table, else computed on the device)."""
-        i = self._per_agent_index(agent)
-        p = N.f32(priorities).ravel()
-        pa = None if p_alpha is None else N.f32(p_alpha).ravel()
-        if pa is not None and pa.size != p.size:
-            raise ValueError("p_alpha must have one entry per priority")
-        N.check(N.lib().sacb_per_set_priorities(self._h, i, N.ptr(p), N.ptr(pa), p.size))
+        _per_set_priorities(self, self._per_agent_index(agent), priorities, p_alpha)
 
     def sample(self, agent, batch_size, u=None):
         """PrioritizedReplayBuffer.sample of one agent: (s, a, r, s2, d, idx, weights); `u` = its min(batch_size, len) uniforms."""
-        i = self._per_agent_index(agent)
-        n = min(batch_size, self.buffer_len(i))
-        if u is None:
-            u = np.random.random_sample(n)
-        u = np.ascontiguousarray(u, np.float64)
-        o, k = self._cfg.obs_dim, self._cfg.act_dim
-        s, a, r = np.empty((n, o), np.float32), np.empty((n, k), np.float32), np.empty(n, np.float32)
-        s2, d = np.empty((n, o), np.float32), np.empty(n, np.float32)
-        idx, w = np.empty(n, np.int64), np.empty(n, np.float32)
-        N.check(N.lib().sacb_per_sample(self._h, i, N.ptr(u, ctypes.c_double), batch_size, N.ptr(idx, ctypes.c_int64), N.ptr(w),
-                                        N.ptr(s), N.ptr(a), N.ptr(r), N.ptr(s2), N.ptr(d)))
-        return s, a, r, s2, d, idx, w
+        return _per_sample(self, self._per_agent_index(agent), batch_size, u)
 
     def update_priorities(self, agent, indices, priorities):
         """PrioritizedReplayBuffer.update_priorities of one agent (float32 priorities are stored + 1e-6 in float32, float64 ones in float64)."""
-        i = self._per_agent_index(agent)
-        idx = np.ascontiguousarray(np.asarray(indices), np.int64).ravel()
-        if hasattr(priorities, "detach"):
-            priorities = priorities.detach().cpu().numpy()
-        pr = np.asarray(priorities)
-        if pr.dtype == np.float32:
-            pr = np.ascontiguousarray(pr.ravel())
-            N.check(N.lib().sacb_per_update(self._h, i, N.ptr(idx, ctypes.c_int64), N.ptr(pr), idx.size))
-        else:      # priority.item() + 1e-6 in float64, then the float32 store (replay_buffer.py:87)
-            final = (pr.astype(np.float64).ravel() + 1e-6).astype(np.float32)
-            N.check(N.lib().sacb_per_update_final(self._h, i, N.ptr(idx, ctypes.c_int64), N.ptr(final), idx.size))
+        _per_update_priorities(self, self._per_agent_index(agent), indices, priorities)
 
     def frame(self, agent):
         """The agent's frame counter (beta schedule, replay_buffer.py:53): starts at 1, +1 per sample of that agent."""
-        i = self._per_agent_index(agent)
-        st = N.PerStats()
-        N.check(N.lib().sacb_per_get_stats(self._h, i, ctypes.byref(st)))
-        return int(st.frame)
+        return int(_per_stats(self, self._per_agent_index(agent)).frame)
 
     def set_frame(self, agent, v):
-        N.check(N.lib().sacb_per_set_frame(self._h, self._per_agent_index(agent), int(v)))
+        _per_set_frame(self, self._per_agent_index(agent), v)
 
     # ---- acting / learning ------------------------------------------------------------------------------------------------
     def select_action(self, states, evaluate=False, *, eps=None):
@@ -614,39 +624,34 @@ class PopulationSAC:
             return None
         losses = np.zeros((self.n_agents, 3), np.float32)
         N.check(lib.sacb_get_losses_all(self._h, N.ptr(losses)))
-        return [{"q1_loss": float(l[0]), "q2_loss": float(l[1]), "policy_loss": float(l[2])} for l in losses]
-
-    def synchronize(self):
-        N.check(N.lib().sacb_synchronize(self._h))
+        return [_loss_dict(l) for l in losses]
 
     # ---- per-agent state in the reference's save() layout (sac_imp.py:154-162) ---------------------------------------
-    def agent_state(self, agent):
-        lib, out = N.lib(), {}
+    def _tensor(self, agent, net_id, slot, t, shape):
+        """A host copy of one arena tensor of `agent`."""
+        host = np.empty(shape, np.float32)
+        N.check(N.lib().sacb_export_tensor(self._h, agent, net_id, slot, t, N.ptr(host), host.size))
+        return torch.from_numpy(host)
+
+    def _net_state_dicts(self, agent):
+        out = {}
         for net_id, name in enumerate(_NETS):
-            sd = {}
-            for t, (pname, shape) in enumerate(self._names[net_id]):
-                host = np.empty(shape, np.float32)
-                N.check(lib.sacb_export_tensor(self._h, int(agent), net_id, N.SLOT_PARAM, t, N.ptr(host), host.size))
-                sd[pname] = torch.from_numpy(host)
-            out[f"{name}_state_dict"] = sd
-        sc = N.Scalars()
-        N.check(lib.sacb_get_scalars(self._h, int(agent), ctypes.byref(sc)))
-        out["alpha"] = float(sc.alpha) if sc.n_updates == 0 or not self._cfg.auto_entropy else torch.tensor([sc.alpha])
+            out[f"{name}_state_dict"] = {pname: self._tensor(agent, net_id, N.SLOT_PARAM, t, shape)
+                                         for t, (pname, shape) in enumerate(self._names[net_id])}
         return out
 
-    def load_agent(self, agent, checkpoint):
-        """Inverse of `agent_state` (accepts a file written by the reference's or the product's `SAC.save`)."""
-        lib = N.lib()
+    def _load_nets(self, agent, checkpoint):
         for net_id, name in enumerate(_NETS):
             sd = checkpoint[f"{name}_state_dict"]
             for t, (pname, _) in enumerate(self._names[net_id]):
-                host = N.f32(torch.as_tensor(sd[pname]).detach().cpu().numpy())
-                N.check(lib.sacb_import_tensor(self._h, int(agent), net_id, N.SLOT_PARAM, t, N.ptr(host), host.size))
-        sc = N.Scalars()
-        N.check(lib.sacb_get_scalars(self._h, int(agent), ctypes.byref(sc)))
-        a = checkpoint["alpha"]
-        sc.alpha = float(a.detach().reshape(-1)[0]) if torch.is_tensor(a) else float(a)
-        N.check(lib.sacb_set_scalars(self._h, int(agent), ctypes.byref(sc)))
+                self._import(agent, net_id, N.SLOT_PARAM, t, sd[pname])
+
+    def agent_state(self, agent):
+        return self._learner_state(int(agent), None)
+
+    def load_agent(self, agent, checkpoint):
+        """Inverse of `agent_state` (accepts a file written by the reference's or the product's `SAC.save`)."""
+        self._load_learner(int(agent), checkpoint, optimizers=False)
 
     # ---- population-based training: per-agent hyperparameters, exploit, member checkpoints ---------------------------------------------
     def _per_agent(self, name, value):
@@ -678,11 +683,9 @@ class PopulationSAC:
 
     def hyperparameters(self, agent):
         """{lr, gamma, tau, target_entropy, alpha} of one agent as the device holds them (float32 values)."""
-        i, lib = self._agent_index(agent), N.lib()
-        hp, sc = N.Hparams(), N.Scalars()
-        N.check(lib.sacb_get_hparams(self._h, i, ctypes.byref(hp)))
-        N.check(lib.sacb_get_scalars(self._h, i, ctypes.byref(sc)))
-        return {"lr": hp.lr, "gamma": hp.gamma, "tau": hp.tau, "target_entropy": hp.target_entropy, "alpha": sc.alpha}
+        i, hp = self._agent_index(agent), N.Hparams()
+        N.check(N.lib().sacb_get_hparams(self._h, i, ctypes.byref(hp)))
+        return {"lr": hp.lr, "gamma": hp.gamma, "tau": hp.tau, "target_entropy": hp.target_entropy, "alpha": self._scalars(i).alpha}
 
     def set_hyperparameters(self, agent, **kw):
         """Explore step: change only the given keys of one agent, effective from its next update (no program is rebuilt).  A new lr
@@ -702,10 +705,9 @@ class PopulationSAC:
                     setattr(cur, k, kw[k])
             N.check(lib.sacb_set_hparams(self._h, i, ctypes.byref(cur)))
         if "alpha" in kw:
-            sc = N.Scalars()
-            N.check(lib.sacb_get_scalars(self._h, i, ctypes.byref(sc)))
+            sc = self._scalars(i)
             sc.alpha = kw["alpha"]
-            N.check(lib.sacb_set_scalars(self._h, i, ctypes.byref(sc)))
+            self._set_scalars(sc, i)
 
     def exploit(self, dst, src):
         """Exploit step: agent dst[k] takes over the whole learner state of agent src[k] (weights, targets, Adam state, temperature,
@@ -722,25 +724,6 @@ class PopulationSAC:
         d32, s32 = d.astype(np.int32), s.astype(np.int32)
         N.check(N.lib().sacb_copy_agents(self._h, N.ptr(d32, ctypes.c_int32), N.ptr(s32, ctypes.c_int32), int(d.size)))
 
-    def _optimizer_state(self, agent, net_id, sc, lr):
-        step = {N.NET_POLICY: sc.step_policy, N.NET_Q1: sc.step_q1, N.NET_Q2: sc.step_q2, None: sc.step_alpha}[net_id]
-        names = [None] if net_id is None else self._names[net_id]
-        state = {}
-        if step > 0:
-            lib = N.lib()
-            for t, entry in enumerate(names):
-                if net_id is None:
-                    m, v = torch.tensor([sc.log_alpha_m]), torch.tensor([sc.log_alpha_v])
-                else:
-                    m, v = (np.empty(entry[1], np.float32) for _ in range(2))
-                    for slot, host in ((N.SLOT_ADAM_M, m), (N.SLOT_ADAM_V, v)):
-                        N.check(lib.sacb_export_tensor(self._h, agent, net_id, slot, t, N.ptr(host), host.size))
-                    m, v = torch.from_numpy(m), torch.from_numpy(v)
-                state[t] = {"step": torch.tensor(float(step)), "exp_avg": m, "exp_avg_sq": v}
-        group = ArenaAdam(None, net_id, None, lr).param_groups[0]
-        group["params"] = list(range(len(names)))
-        return {"state": state, "param_groups": [group]}
-
     def agent_checkpoint(self, agent):
         """One member as a dictionary in the key layout of SAC.save_checkpoint without 'replay_buffer' (torch.save it): the five nets,
         the three optimizer state_dicts, 'alpha', 'log_alpha' and 'alpha_optimizer_state_dict' (with automatic entropy tuning), and the
@@ -749,16 +732,7 @@ class PopulationSAC:
         i = self._agent_index(agent)
         self.synchronize()
         hp = self.hyperparameters(i)
-        sc = N.Scalars()
-        N.check(N.lib().sacb_get_scalars(self._h, i, ctypes.byref(sc)))
-        ck = {k: v for k, v in self.agent_state(i).items() if k.endswith("_state_dict")}
-        for net_id, name in ((N.NET_POLICY, "policy"), (N.NET_Q1, "q1"), (N.NET_Q2, "q2")):
-            ck[f"{name}_optimizer_state_dict"] = self._optimizer_state(i, net_id, sc, hp["lr"])
-        auto = bool(self._cfg.auto_entropy)
-        ck["alpha"] = float(sc.alpha) if sc.n_updates == 0 or not auto else torch.tensor([sc.alpha])
-        if auto:
-            ck["log_alpha"] = torch.tensor([sc.log_alpha], requires_grad=True)
-            ck["alpha_optimizer_state_dict"] = self._optimizer_state(i, None, sc, hp["lr"])
+        ck = self._learner_state(i, None, lr=hp["lr"])
         ck["sacb_hyperparameters"] = {k: hp[k] for k in ("lr", "gamma", "tau", "target_entropy")}
         return ck
 
@@ -766,32 +740,11 @@ class PopulationSAC:
         """Inverse of `agent_checkpoint`; also takes a file (or dictionary) written by SAC.save_checkpoint.  Loads the nets, the Adam
         state and step counts, alpha and log_alpha, and the hyperparameters: 'sacb_hyperparameters' when present, otherwise the
         optimizers' learning rate (gamma, tau and target_entropy of the member then stay as they are)."""
-        i, lib = self._agent_index(agent), N.lib()
+        i = self._agent_index(agent)
         if isinstance(checkpoint, (str, bytes, os.PathLike)):
             checkpoint = torch.load(checkpoint, map_location="cpu", weights_only=False)
+        lr = self._load_learner(i, checkpoint)
         hp = checkpoint.get("sacb_hyperparameters")
         if hp is None:
-            groups = checkpoint.get("policy_optimizer_state_dict", {}).get("param_groups")
-            hp = {"lr": float(groups[0]["lr"])} if groups else {}
-        self.set_hyperparameters(i, **{k: float(v) for k, v in hp.items()})      # lr first: the step counts below take its factors
-        self.load_agent(i, checkpoint)
-        sc = N.Scalars()
-        N.check(lib.sacb_get_scalars(self._h, i, ctypes.byref(sc)))
-        for net_id, name, attr in ((N.NET_POLICY, "policy", "step_policy"), (N.NET_Q1, "q1", "step_q1"), (N.NET_Q2, "q2", "step_q2")):
-            state = checkpoint.get(f"{name}_optimizer_state_dict", {"state": {}})["state"]
-            setattr(sc, attr, int(float(state[min(state)]["step"])) if state else 0)
-            for t, st in state.items():
-                for slot, key in ((N.SLOT_ADAM_M, "exp_avg"), (N.SLOT_ADAM_V, "exp_avg_sq")):
-                    host = N.f32(torch.as_tensor(st[key]).detach().cpu().numpy())
-                    N.check(lib.sacb_import_tensor(self._h, i, net_id, slot, int(t), N.ptr(host), host.size))
-        if self._cfg.auto_entropy and "log_alpha" in checkpoint:
-            sc.log_alpha = float(torch.as_tensor(checkpoint["log_alpha"]).detach().reshape(-1)[0])
-            state = checkpoint.get("alpha_optimizer_state_dict", {"state": {}})["state"]
-            if state:
-                first = state[min(state)]
-                sc.step_alpha = int(float(first["step"]))
-                sc.log_alpha_m = float(torch.as_tensor(first["exp_avg"]).reshape(-1)[0])
-                sc.log_alpha_v = float(torch.as_tensor(first["exp_avg_sq"]).reshape(-1)[0])
-            else:
-                sc.step_alpha, sc.log_alpha_m, sc.log_alpha_v = 0, 0.0, 0.0
-        N.check(lib.sacb_set_scalars(self._h, i, ctypes.byref(sc)))
+            hp = {} if lr is None else {"lr": lr}
+        self.set_hyperparameters(i, **hp)
